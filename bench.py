@@ -29,6 +29,7 @@ import numpy as np  # noqa: E402
 
 SR, CLIP_LEN, FL, HOP, N_MELS, N_MFCC = 44_100, 220_500, 1024, 512, 40, 13
 CLIP_SECONDS = CLIP_LEN / SR
+DUMP_CLIPS = 512                            # --dump-outputs: 512 x 429 x (13 + 40) float32 = 46.6 MB
 
 
 def parse_args():
@@ -45,7 +46,25 @@ def parse_args():
     ap.add_argument("--retrieval-steps", type=int, default=3, help="secondary cosine top-20 measurement (0 = skip)")
     ap.add_argument("--cpu-seconds", type=float, default=12.0, help="budget of the cpu_baseline leg")
     ap.add_argument("--no-cpu-baseline", action="store_true")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", type=Path, default=None,
+                    help=f"after the timed steps, write the last step's features of a fixed, seeded sample of "
+                         f"{DUMP_CLIPS} of rank 0's clips as float32 DIR/<name>.npy")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs is not None and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
+    return args
+
+
+def dump_outputs(out_dir: Path, outputs: dict, n_clips: int) -> None:
+    """Write rows of each [clips, frames, coeffs] output for a sample of clips that depends only on n_clips."""
+    import torch
+
+    sel = np.sort(np.random.default_rng(0).choice(n_clips, min(n_clips, DUMP_CLIPS), replace=False))
+    out_dir.mkdir(parents=True, exist_ok=True)
+    for name, t in outputs.items():
+        np.save(out_dir / f"{name}.npy", t[torch.as_tensor(sel, device=t.device)].cpu().numpy())
 
 
 def algorithmic_bytes_per_clip(outputs: str, n_frames: int) -> int:
@@ -218,14 +237,8 @@ def run_reference(args) -> None:
     n_frames = 1 + (CLIP_LEN - FL) // HOP
     O, cfg, cores, want, clips = cpu_arm(args, n_frames)
     per_step = clips.shape[0]
-    t0 = time.perf_counter()
-    O.features_batch(clips, cfg, want=want, n_threads=cores)                       # calibration step (counts as warm-up)
-    one = time.perf_counter() - t0
-    # keep the whole run within a few minutes whatever K is
-    budget = 150.0
+    O.features_batch(clips, cfg, want=want, n_threads=cores)                       # first step (counts as warm-up)
     steps, warm = args.steps, max(0, args.warmup - 1)
-    if one * (steps + warm) > budget:                       # never below 4 clips per core: cut steps instead
-        steps = max(1, int(budget / one) - warm)
     for _ in range(warm):
         O.features_batch(clips, cfg, want=want, n_threads=cores)
     t0 = time.perf_counter()
@@ -308,6 +321,8 @@ def run_ours(args) -> None:
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
     total_ms = float(t.item())
     value = world * b * CLIP_SECONDS * args.steps / (total_ms * 1e-3)
+    if args.dump_outputs is not None and rank == 0:
+        dump_outputs(args.dump_outputs, {name: out for name, out in (("mfcc", mf), ("log_mel", lm)) if out is not None}, b)
 
     # roofline of the dominant (only) kernel of the step
     bytes_per_launch = b * algorithmic_bytes_per_clip(args.outputs, n_frames)

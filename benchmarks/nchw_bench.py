@@ -1,4 +1,4 @@
-import sys; sys.path.insert(0,'/root/repo')
+import sys; sys.path.insert(0, str(__import__('pathlib').Path(__file__).resolve().parents[1]))
 import torch, json
 from dsp_final_b200 import synth
 from dsp_final_b200.batch import features_batch, log_mel_nchw

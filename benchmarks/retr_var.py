@@ -1,5 +1,5 @@
 import sys, time
-sys.path.insert(0,'/root/repo')
+sys.path.insert(0, str(__import__('pathlib').Path(__file__).resolve().parents[1]))
 import torch
 from dsp_final_b200 import retrieval as R
 dev=torch.device('cuda'); g=torch.Generator(device=dev); g.manual_seed(5)

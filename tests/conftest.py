@@ -2,6 +2,7 @@
 from __future__ import annotations
 
 import json
+import os
 import sys
 from pathlib import Path
 
@@ -12,17 +13,18 @@ REPO = Path(__file__).resolve().parents[1]
 if str(REPO) not in sys.path:
     sys.path.insert(0, str(REPO))
 GOLDEN = REPO / "tests" / "golden"
-REFERENCE = Path("/root/reference")
+# A checkout of the original Python project, for the few tests that import its modules (optional)
+REFERENCE = Path(os.environ["DSP_REF_PATH"]) if os.environ.get("DSP_REF_PATH") else None
 
 
 def pytest_configure(config):
     config.addinivalue_line("markers", "gpu: needs a CUDA device (run on the B200 box with -m gpu)")
-    config.addinivalue_line("markers", "needs_reference: imports /root/reference (dev container only)")
+    config.addinivalue_line("markers", "needs_reference: imports the original project from DSP_REF_PATH")
 
 
 def pytest_collection_modifyitems(config, items):
-    have_ref = (REFERENCE / "src" / "dsp" / "fft.py").exists()
-    skip_ref = pytest.mark.skip(reason="/root/reference not present (GPU box)")
+    have_ref = REFERENCE is not None and (REFERENCE / "src" / "dsp" / "fft.py").exists()
+    skip_ref = pytest.mark.skip(reason="DSP_REF_PATH does not name a checkout of the original project")
     for item in items:
         if "needs_reference" in item.keywords and not have_ref:
             item.add_marker(skip_ref)

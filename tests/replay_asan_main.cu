@@ -2,7 +2,7 @@
 #include <cstdlib>
 #include <vector>
 #include <cmath>
-#include "/root/repo/include/dspx.h"
+#include "../include/dspx.h"
 extern "C" int emu_features_generic(const dspx_config *cfg, const float *clips, int64_t n_clips, int64_t clip_len, int64_t clip_stride, int stft_mode, int stft_pre, float *logmel, float *mfcc, float *stft_out, int fpc);
 extern "C" int emu_features_warp8(const dspx_config *cfg, const float *clips, int64_t n_clips, int64_t clip_len, int64_t clip_stride, float *logmel, float *mfcc, float *stft_out, int stft_pre);
 int main() {

@@ -2,15 +2,13 @@
 from __future__ import annotations
 
 import hashlib
-import importlib.util
 import json
-import sys
 from types import SimpleNamespace
 
 import numpy as np
 import pytest
 
-from conftest import REFERENCE
+from conftest import GOLDEN
 
 
 def _items(n):
@@ -65,44 +63,32 @@ def test_save_load_manifest_roundtrip(tmp_path):
     assert not list(tmp_path.rglob("*.tmp"))
 
 
-@pytest.mark.needs_reference
-def test_reference_cache_reads_our_files_and_bytes_match(tmp_path):
-    """The reference's FeatureCache (imported from its checkout) and ours are interchangeable on disk."""
+def test_reference_cache_reads_our_files_and_bytes_match(tmp_path, known_answers):
+    """Our cache files are the reference's, byte for byte, so its FeatureCache reads them as its own.
+
+    tests/golden/pipeline.npz holds what the reference's FeatureCache wrote for the 40-item pipeline set
+    (tests/golden/make_pipeline_golden.py): the header of its first .npy file, that file's path under the cache root
+    and np.load of every file.  Header + payload is therefore the reference's file exactly; all 40 share one shape and
+    so one header.  Its params dict and digest for this config are in known_answers.json."""
     from dsp_final_b200.cache import BatchFeatureCache
     from dsp_final_b200.dsp.mfcc import MfccConfig
 
-    sys.dont_write_bytecode = True
-    sys.path.insert(0, str(REFERENCE))
-    try:
-        saved = {k: sys.modules.pop(k) for k in list(sys.modules) if k == "src" or k.startswith("src.")}
-        ref_cache = importlib.import_module("src.features.cache")
-        ref_cfg_cls = importlib.import_module("src.dsp.mfcc").MfccConfig
-    finally:
-        sys.path.remove(str(REFERENCE))
-    try:
-        items = _items(3)
-        feats = np.random.default_rng(1).standard_normal((3, 215, 40)).astype(np.float32)
-        ours, theirs = BatchFeatureCache(tmp_path / "ours"), ref_cache.FeatureCache(tmp_path / "theirs")
-        cfg, rcfg = MfccConfig(44100, 1024, 1024), ref_cfg_cls(44100, 1024, 1024)
-        recs = ours.save_features(items, feats, "log_mel", cfg)
-        reader = ref_cache.FeatureCache(tmp_path / "ours")                    # reference code reads OUR files
-        for i, it in enumerate(items):
-            assert np.array_equal(reader.load_feature(it, "log_mel", rcfg), feats[i])
-            theirs.save_feature(theirs.feature_path(it, "log_mel", rcfg), feats[i])
-            a = ours.feature_path(it, "log_mel", cfg).read_bytes()
-            b = theirs.feature_path(it, "log_mel", rcfg).read_bytes()
-            assert hashlib.sha1(a).hexdigest() == hashlib.sha1(b).hexdigest()  # identical .npy bytes
-            assert ours.feature_path(it, "log_mel", cfg).relative_to(tmp_path / "ours") == \
-                theirs.feature_path(it, "log_mel", rcfg).relative_to(tmp_path / "theirs")
-        m_ours = json.loads(ours.write_manifest("log_mel", cfg, recs).read_text())
-        m_ref = json.loads(theirs.write_manifest("log_mel", rcfg, recs).read_text())
-        assert list(m_ours) == list(m_ref)
-        for k in ("feature_type", "hash", "params", "num_files"):
-            assert m_ours[k] == m_ref[k]
-    finally:
-        for k in [k for k in sys.modules if k == "src" or k.startswith("src.")]:
-            del sys.modules[k]
-        sys.modules.update(saved)
+    g = np.load(GOLDEN / "pipeline.npz")
+    feats, header = g["mfcc_f32"], bytes(g["npy_header"])
+    items = [SimpleNamespace(filename=f"{1 + n // 8}-{100000 + n}-A-{n % 5}.wav", fold=1 + n // 8)   # item_table()
+             for n in range(feats.shape[0])]
+    cfg = MfccConfig(44100, 1024, 512)
+    ours = BatchFeatureCache(tmp_path)
+    recs = ours.save_features(items, feats, "mfcc", cfg)
+    assert str(ours.feature_path(items[0], "mfcc", cfg).relative_to(tmp_path)) == bytes(g["first_path"]).decode()
+    for i, it in enumerate(items):
+        blob = ours.feature_path(it, "mfcc", cfg).read_bytes()
+        assert hashlib.sha1(blob).hexdigest() == hashlib.sha1(header + feats[i].tobytes()).hexdigest(), it.filename
+    m = json.loads(ours.write_manifest("mfcc", cfg, recs).read_text())
+    assert list(m) == ["feature_type", "hash", "params", "created_at", "num_files", "files"]
+    assert m["feature_type"] == "mfcc" and m["num_files"] == len(items)
+    assert m["hash"] == known_answers["cache_digests"]["mfcc/1024/512"]
+    assert m["params"] == known_answers["cache_params_mfcc_1024_512"]
 
 
 @pytest.mark.gpu

@@ -1,8 +1,8 @@
 """The reference's own src/features and src/retrieval run unchanged on top of our src/dsp shims.
 
-Dev-container test (needs /root/reference): a path overlay puts integration/src/dsp in place of the
+Runs when DSP_REF_PATH names a reference checkout: a path overlay puts integration/src/dsp in place of the
 reference's src/dsp while every other reference module is imported from the reference checkout.
-The GPU box has no reference checkout; there the same pipeline (Esc50Meta -> FeatureCache-format files ->
+Without a checkout the same pipeline (Esc50Meta -> FeatureCache-format files ->
 compute_embeddings -> evaluate_retrieval / run_mfcc_retrieval) is exercised by tests/test_pipeline.py
 against golden outputs that the reference produced here (tests/golden/make_pipeline_golden.py).
 """

@@ -12,7 +12,7 @@ import hashlib
 import numpy as np
 import pytest
 
-from conftest import rel_err
+from conftest import REFERENCE, rel_err
 from oracle import oracle as O
 
 TIGHT = 1e-12
@@ -176,15 +176,15 @@ def test_batch_front_end_matches_single(golden_small):
 
 @pytest.mark.needs_reference
 def test_oracle_against_live_reference():
-    """Dev-container only: a fresh random case straight against the imported reference."""
+    """A fresh random case straight against the original project (its checkout named by DSP_REF_PATH)."""
     import sys
 
     sys.dont_write_bytecode = True
-    sys.path.insert(0, "/root/reference")
+    sys.path.insert(0, str(REFERENCE))
     try:
         from src.dsp.mfcc import MfccConfig, mfcc
     finally:
-        sys.path.remove("/root/reference")
+        sys.path.remove(str(REFERENCE))
     x = np.random.default_rng(99).standard_normal(6000).astype(np.float32)
     cfg = MfccConfig(sample_rate=16000, frame_length=400, hop_length=160, n_mels=23, n_mfcc=13)
     ours = O.mfcc(x, O.OracleConfig(16000, 400, 160, n_mels=23, n_mfcc=13))

@@ -19,7 +19,7 @@ OK, EINVAL, ENOMEM, ECUDA, ENODEVICE, EUNSUPPORTED = 0, -1, -2, -3, -4, -5
 WINDOWS = {"hann": 0, "hamming": 1, "rect": 2}
 KERNELS = {"auto": 0, "generic": 1, "warp8": 2}
 KERNEL_NAMES = {v: k for k, v in KERNELS.items()}
-DTYPE_F32, DTYPE_F64 = 0, 1
+DTYPE_F32, DTYPE_F64, DTYPE_PCM16 = 0, 1, 2
 MAX_K = 128
 
 
@@ -54,6 +54,18 @@ class DspxPlanInfo(C.Structure):
     ]
 
 
+class DspxRaggedClip(C.Structure):
+    """struct dspx_ragged_clip: one row of a ragged batch's table (dspx_ragged_layout)."""
+
+    _fields_ = [
+        ("start", C.c_int64),
+        ("length", C.c_int64),
+        ("n_frames", C.c_int64),
+        ("first_frame", C.c_int64),
+        ("first_pair", C.c_int64),
+    ]
+
+
 class DspxError(RuntimeError):
     pass
 
@@ -83,6 +95,10 @@ _SIGNATURES = {
     "dspx_features_pcm16": (_I32, [_VP, _VP, _I64, _I64, _I64, _I32, _VP, _VP, _VP, _VP, _SZ, _VP]),
     "dspx_features_host_pcm16": (_I32, [_VP, _VP, _I64, _I64, _I64, _I32, _VP, _VP, _VP]),
     "dspx_stft_host": (_I32, [_VP, _VP, _I64, _I64, _I64, _I32, _VP]),
+    "dspx_ragged_layout": (_I64, [C.POINTER(DspxConfig), _VP, _VP, _I64, _I32, _VP]),
+    "dspx_features_ragged_workspace": (_SZ, [_VP, _VP, _I64, _I32, _I32, _I32, _I32, _I32]),
+    "dspx_features_ragged": (_I32, [_VP, _VP, _I32, _I32, _VP, _VP, _I64, _I64, _VP, _VP, _VP, _VP, _SZ, _VP]),
+    "dspx_embed_stats_ragged": (_I32, [_VP, _VP, _I64, _I32, _VP, _VP]),
     "dspx_next_pow_two": (_I64, [_I64]),
     "dspx_fft_c2c": (_I32, [_VP, _I64, _I64, _I64, _I32, _VP, _VP, _VP]),
     "dspx_cosine_topk_workspace": (_SZ, [_I64, _I64, _I32, _I32]),

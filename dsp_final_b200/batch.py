@@ -11,15 +11,19 @@ over them and keep the reference signatures.
   * NumPy array (or CPU tensor) in -> NumPy arrays out through the host-buffer
     C ABI (dspx_features_host / dspx_stft_host: pinned staging + copy/compute
     overlap inside the library).
+
+features_ragged takes clips of different lengths in one call (dspx_features_ragged):
+outputs are stacked along the frame axis and split per clip with "frame_offsets".
 """
 from __future__ import annotations
 
+import ctypes as C
 from typing import Any, Iterable
 
 import numpy as np
 
 from . import _lib
-from .plan import Plan, get_plan
+from .plan import Plan, config_key, config_struct, get_plan
 
 FEATURES = ("log_mel", "mfcc", "embed")
 
@@ -185,6 +189,157 @@ def features_batch(clips, cfg: Any, want: Iterable[str] = ("mfcc",), device: int
     return out
 
 
+RAGGED_ALIGN = 4       # samples: clip starts in the packed buffer (float32 needs even ones; 4 keeps 16-byte alignment)
+
+
+def ragged_layout(lengths, cfg, dtype=np.float32, starts=None) -> tuple[np.ndarray, np.ndarray, int]:
+    """(starts, table, total_frames) of a ragged batch: dspx_ragged_layout on the host, no device needed.
+
+    `starts` defaults to the clips packed back to back at multiples of RAGGED_ALIGN samples.  table is int64
+    [n_clips, 5], the rows of struct dspx_ragged_clip: start, length, n_frames, first_frame, first_pair.
+    """
+    lengths = np.ascontiguousarray(lengths, dtype=np.int64).reshape(-1)
+    if starts is None:
+        padded = (lengths + RAGGED_ALIGN - 1) // RAGGED_ALIGN * RAGGED_ALIGN
+        starts = np.concatenate(([0], np.cumsum(padded)[:-1])).astype(np.int64) if len(lengths) else lengths.copy()
+    starts = np.ascontiguousarray(starts, dtype=np.int64).reshape(-1)
+    if starts.shape != lengths.shape:
+        raise ValueError("one start per clip expected")
+    code = _lib.DTYPE_PCM16 if np.dtype(dtype) == np.int16 else _lib.DTYPE_F32
+    table = np.zeros((len(lengths), 5), np.int64)
+    c = config_struct(config_key(cfg))
+    total = _lib.check(_lib.load().dspx_ragged_layout(C.byref(c), starts.ctypes.data, lengths.ctypes.data, len(lengths),
+                                                      code, table.ctypes.data), "dspx_ragged_layout")
+    return starts, table, int(total)
+
+
+def _ragged_inputs(clips) -> tuple[list, bool, bool]:
+    """-> (1-D clips, on the GPU, PCM16); all NumPy float32 / int16, or all torch CUDA tensors of one dtype."""
+    clips = list(clips)
+    cuda = [_is_cuda_tensor(c) for c in clips]
+    if any(cuda) and not all(cuda):
+        raise ValueError("clips must be all NumPy arrays or all torch CUDA tensors")
+    pcm = [_is_pcm16(c) for c in clips]
+    if any(pcm) and not all(pcm):
+        raise ValueError("clips must all be float or all be int16 PCM")
+    on_gpu, is_pcm = bool(clips) and all(cuda), bool(clips) and all(pcm)
+    if on_gpu:
+        import torch
+
+        dt = torch.int16 if is_pcm else torch.float32
+        out = [c.reshape(-1).to(dt) for c in clips]
+        if len({c.device for c in out}) > 1:
+            raise ValueError("clips must be on one device")
+    else:
+        if clips and type(clips[0]).__module__.startswith("torch"):
+            clips = [c.detach().cpu().numpy() for c in clips]
+        out = [np.asarray(c, dtype=np.int16 if is_pcm else np.float32).reshape(-1) for c in clips]
+    return out, on_gpu, is_pcm
+
+
+def ragged_launch(plan: Plan, samples, pcm: bool, table: np.ndarray, table_dev, total: int, want, normalize: bool = True,
+                  out=None) -> tuple[dict, Any]:
+    """One dspx_features_ragged call on torch's current stream: `samples` a packed torch CUDA tensor (float32 or
+    int16), table / table_dev the layout on the host and on the device.  Returns ({name: torch CUDA view}, the flat
+    float32 tensor that holds all of them in FEATURES order); `out`, when given, is that flat tensor."""
+    import torch
+
+    lib = _lib.load()
+    n = len(table)
+    sizes = {"log_mel": (total, plan.n_mels), "mfcc": (total, plan.n_mfcc), "embed": (n, 2 * plan.n_mfcc)}
+    counts = [sizes[k][0] * sizes[k][1] for k in FEATURES if k in want]
+    dev = samples.device
+    if out is None:
+        out = torch.empty(sum(counts), dtype=torch.float32, device=dev)
+    res, off = {}, 0
+    for k in FEATURES:
+        if k in want:
+            m = sizes[k][0] * sizes[k][1]
+            res[k] = out[off:off + m].view(sizes[k])
+            off += m
+    code = _lib.DTYPE_PCM16 if pcm else _lib.DTYPE_F32
+    flags = [1 if k in want else 0 for k in FEATURES]
+    ws_bytes = int(lib.dspx_features_ragged_workspace(plan.handle, table.ctypes.data, n, code, 1 if normalize else 0, *flags))
+    with torch.cuda.device(dev.index):
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+        ptr = [res[k].data_ptr() if k in res else None for k in FEATURES]
+        _lib.check(lib.dspx_features_ragged(plan.handle, samples.data_ptr(), code, 1 if normalize else 0, table_dev.data_ptr(),
+                                           table.ctypes.data, n, total, *ptr, ws.data_ptr(), ws_bytes,
+                                           torch.cuda.current_stream(dev.index).cuda_stream), "dspx_features_ragged")
+    return res, out
+
+
+def features_ragged(clips, cfg: Any, want: Iterable[str] = ("mfcc",), device: int | None = None,
+                    normalize: bool = True) -> dict:
+    """log-mel / MFCC / clip embeddings of clips of different lengths, in one launch.
+
+    `clips` is a sequence of 1-D arrays: all NumPy (float32, or int16 PCM converted like features_batch does), or all
+    torch CUDA tensors of one dtype.  Returns {"log_mel": [total_frames, n_mels], "mfcc": [total_frames, n_mfcc],
+    "embed": [B, 2*n_mfcc]} restricted to `want`, plus "frame_offsets" (int64 [B+1]): clip i owns rows
+    frame_offsets[i]:frame_offsets[i+1].  Every clip gets the values features_batch gives it alone.  NumPy in ->
+    NumPy out (one pinned staging buffer, one copy each way); torch CUDA in -> torch CUDA out on torch's current
+    stream.  A clip shorter than frame_length raises ValueError naming its index.
+    """
+    import torch
+
+    want = _want(want)
+    xs, on_gpu, pcm = _ragged_inputs(clips)
+    starts, table, total = ragged_layout([len(x) for x in xs], cfg, np.int16 if pcm else np.float32)
+    offsets = np.concatenate((table[:, 3], [total])).astype(np.int64) if len(xs) else np.zeros(1, np.int64)
+    if not xs:
+        key = config_key(cfg)
+        shapes = {"log_mel": (0, key[4]), "mfcc": (0, key[5]), "embed": (0, 2 * key[5])}
+        res = {k: np.zeros(shapes[k], np.float32) for k in want}
+        res["frame_offsets"] = offsets
+        return res
+    n_samples = int(starts[-1] + len(xs[-1]))
+    if on_gpu:
+        dev = xs[0].device
+        parts = []
+        pad = torch.zeros(RAGGED_ALIGN, dtype=xs[0].dtype, device=dev)
+        for i, x in enumerate(xs):
+            parts.append(x)
+            gap = int(starts[i + 1] - starts[i] - len(x)) if i + 1 < len(xs) else 0
+            if gap:
+                parts.append(pad[:gap])
+        plan = get_plan(cfg, dev.index if device is None else device)
+        with torch.cuda.device(dev.index):
+            samples = torch.cat(parts)
+            table_dev = torch.from_numpy(table).to(dev)
+            res, _ = ragged_launch(plan, samples, pcm, table, table_dev, total, want, normalize)
+        res["frame_offsets"] = torch.from_numpy(offsets).to(dev)
+        return res
+    plan = get_plan(cfg, device)
+    dev = torch.device("cuda", plan.device)
+    staging = torch.empty(n_samples, dtype=torch.int16 if pcm else torch.float32, pin_memory=True)
+    host = staging.numpy()
+    for s, x in zip(starts, xs):
+        host[s:s + len(x)] = x
+    with torch.cuda.device(plan.device):
+        stream = torch.cuda.current_stream(plan.device)
+        samples = staging.to(dev, non_blocking=True)
+        table_dev = torch.from_numpy(table).to(dev)
+        res, flat = ragged_launch(plan, samples, pcm, table, table_dev, total, want, normalize)
+        out_host = torch.empty(flat.shape, dtype=torch.float32, pin_memory=True)
+        out_host.copy_(flat, non_blocking=True)
+        stream.synchronize()
+    out, off = {}, 0
+    host_out = out_host.numpy()
+    for k in FEATURES:
+        if k in res:
+            m = res[k].numel()
+            out[k] = host_out[off:off + m].reshape(tuple(res[k].shape))
+            off += m
+    out["frame_offsets"] = offsets
+    return out
+
+
+def split_ragged(stacked, frame_offsets) -> list:
+    """[total_frames, C] stacked features -> one [T_i, C] view per clip."""
+    o = [int(v) for v in (frame_offsets.tolist() if hasattr(frame_offsets, "tolist") else frame_offsets)]
+    return [stacked[o[i]:o[i + 1]] for i in range(len(o) - 1)]
+
+
 def mfcc_batch(clips, cfg, **kw):
     return features_batch(clips, cfg, ("mfcc",), **kw)["mfcc"]
 
@@ -260,11 +415,42 @@ def stft_batch(clips, frame_length: int, hop_length: int, window: str = "hann", 
     return out
 
 
+def _embed_stats_ragged(feats: list):
+    """embed_stats of a list of [T_i, C] arrays (all NumPy or all torch CUDA) through dspx_embed_stats_ragged."""
+    import torch
+
+    host = not all(_is_cuda_tensor(f) for f in feats)
+    fs = [torch.as_tensor(np.asarray(f, dtype=np.float32)) if host else f.to(torch.float32) for f in feats]
+    if any(f.dim() != 2 or f.shape[1] != fs[0].shape[1] or f.shape[0] < 1 for f in fs):
+        raise ValueError("embed_stats takes [T_i, C] arrays with T_i >= 1 and one C")
+    c = int(fs[0].shape[1])
+    rows = np.array([f.shape[0] for f in fs], np.int64)
+    table = np.zeros((len(fs), 5), np.int64)
+    table[:, 2] = rows
+    table[:, 3] = np.cumsum(rows) - rows
+    dev = torch.device("cuda", torch.cuda.current_device()) if host else fs[0].device
+    with torch.cuda.device(dev.index):
+        stacked = torch.cat(fs).to(dev).contiguous()
+        table_dev = torch.from_numpy(table).to(dev)
+        out = torch.empty((len(fs), 2 * c), dtype=torch.float32, device=dev)
+        _lib.check(_lib.load().dspx_embed_stats_ragged(stacked.data_ptr(), table_dev.data_ptr(), len(fs), c, out.data_ptr(),
+                                                       torch.cuda.current_stream(dev.index).cuda_stream),
+                   "dspx_embed_stats_ragged")
+    return out.cpu().numpy() if host else out
+
+
 def embed_stats(feats):
-    """concat(mean_t, std_t) of [B, T, C] float32 features (retrieval.py:38-41). torch CUDA in/out."""
+    """concat(mean_t, std_t) of [B, T, C] float32 features (retrieval.py:38-41). torch CUDA in/out.
+
+    A list or tuple of [T_i, C] arrays (clips of different lengths) is reduced in one launch, with the same
+    per-clip summation order."""
     import torch
 
     _lib.require_device()
+    if isinstance(feats, (list, tuple)):
+        if not feats:
+            raise ValueError("embed_stats of an empty list")
+        return _embed_stats_ragged(list(feats))
     if not _is_cuda_tensor(feats):
         feats = torch.as_tensor(np.asarray(feats, dtype=np.float32)).cuda()
         to_host = True

@@ -77,6 +77,18 @@ def read_npy_shape(path: Path) -> tuple:
         return tuple(reader(handle)[0])
 
 
+def _features_per_clip(clips: list, cfg: Any, feature_types: tuple, normalize: bool = True) -> dict:
+    """{feature_type: one [n_frames, n_coef] array per clip}: one batch when the clips have one length, else one
+    ragged launch."""
+    from .batch import features_batch, features_ragged, split_ragged
+
+    if len({c.shape for c in clips}) == 1:
+        out = features_batch(np.stack(clips, axis=0), cfg, feature_types, normalize=normalize)
+        return {ft: list(out[ft]) for ft in feature_types}
+    out = features_ragged(clips, cfg, feature_types, normalize=normalize)
+    return {ft: split_ragged(out[ft], out["frame_offsets"]) for ft in feature_types}
+
+
 def _record(item, path: Path, shape) -> dict:
     return {"filename": item.filename, "fold": item.fold, "path": str(path), "shape": [int(s) for s in shape]}
 
@@ -127,20 +139,13 @@ class BatchFeatureCache:
         return self.get_features([item], feature_type, cfg)[0]
 
     def _compute(self, items: Sequence[Any], feature_type: str, cfg: Any, loader) -> list:
-        from .batch import features_batch
-        from .retrieval import _by_length, _load_clips
+        from .retrieval import _load_clips
 
         if feature_type not in FEATURE_TYPES:
             raise ValueError(f"Unsupported feature_type: {feature_type}")
         if isinstance(cfg, Mapping):
             raise ValueError("get_feature requires MfccConfig for mfcc/log_mel")      # cache.py:83
-        clips = _load_clips(list(items), cfg, loader)
-        feats: list = [None] * len(clips)
-        for _shape, rows in _by_length(clips).items():
-            out = features_batch(np.stack([clips[i] for i in rows], axis=0), cfg, (feature_type,))[feature_type]
-            for j, i in enumerate(rows):
-                feats[i] = out[j]
-        return feats
+        return _features_per_clip(_load_clips(list(items), cfg, loader), cfg, (feature_type,))[feature_type]
 
     def get_features(self, items: Sequence[Any], feature_type: str, cfg: Any, loader=None, batch: int = 256,
                      workers: int = 8) -> list:
@@ -164,11 +169,13 @@ class BatchFeatureCache:
 
     def save_features(self, items: Sequence[Any], feats: np.ndarray, feature_type: str, cfg: Any,
                       workers: int = 8) -> list[dict]:
-        """Write feats[i] ([n_frames, n_coef]) for items[i]; returns the manifest records."""
+        """Write feats[i] ([n_frames, n_coef]) for items[i]; returns the manifest records.  feats is one array
+        [N, n_frames, n_coef] or a list of N arrays (clips of different lengths)."""
         if feature_type not in FEATURE_TYPES:
             raise ValueError(f"Unsupported feature_type: {feature_type}")
-        feats = np.asarray(feats)
-        if feats.shape[0] != len(items):
+        if not isinstance(feats, (list, tuple)):
+            feats = np.asarray(feats)
+        if len(feats) != len(items):
             raise ValueError("one feature array per item expected")
         base = self.feature_dir(feature_type, cfg)                      # hash once per batch, not per file
         jobs = [(base.joinpath(f"fold{it.fold}", it.filename + ".npy"), np.ascontiguousarray(feats[i], dtype=np.float32))
@@ -199,11 +206,10 @@ class BatchFeatureCache:
         """Fill the cache for `items`: the batched twin of precompute_features.py:62-113.
 
         Audio comes from `clips` ([N, L] float32 already loaded/normalised, or int16 PCM which is
-        converted and peak-normalised on the GPU) or from `loader(item)` (decoding files is out of
-        scope here).  Returns {feature_type: manifest path}.
+        converted and peak-normalised on the GPU; or a list of N clips of different lengths) or from
+        `loader(item)` (decoding files is out of scope here).  A batch of clips of different lengths is
+        one ragged launch.  Returns {feature_type: manifest path}.
         """
-        from .batch import features_batch
-
         feature_types = tuple(feature_types)
         for ft in feature_types:
             if ft not in FEATURE_TYPES:
@@ -220,10 +226,10 @@ class BatchFeatureCache:
                     if not (skip_existing and all(paths[ft][i].is_file() for ft in feature_types))]
             if todo:
                 if clips is not None:
-                    x = np.asarray(clips[s:s + batch])[todo]
+                    x = [np.asarray(clips[s + i]) for i in todo]
                 else:
-                    x = np.stack([np.asarray(loader(chunk[i])) for i in todo])
-                out = features_batch(x, cfg, feature_types, normalize=normalize)
+                    x = [np.asarray(loader(chunk[i])) for i in todo]
+                out = _features_per_clip(x, cfg, feature_types, normalize=normalize)
                 for ft in feature_types:
                     self.save_features([chunk[i] for i in todo], out[ft], ft, cfg, workers=workers)
             for ft in feature_types:

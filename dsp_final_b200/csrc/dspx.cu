@@ -47,6 +47,8 @@ static int upload(const std::vector<T> &h, T **d)
     return DSPX_OK;
 }
 
+static size_t align256(size_t x) { return (x + 255) & ~(size_t)255; }
+
 struct DeviceGuard {
     int prev = -1;
     bool ok = false;
@@ -176,13 +178,15 @@ int launch_generic_fallback(const dspx_plan *pl, const float *clips, int64_t n_c
                           pl->cfg.pre_emphasis > 0.0 ? 1 : 0, logmel, mfcc, nullptr, st, nchw);
 }
 
-static int launch_embed(const float *feats, int64_t n_clips, int64_t T, int C, float *out, cudaStream_t st)
+static int launch_embed(const float *feats, int64_t n_clips, int64_t T, int C, float *out, cudaStream_t st,
+                        const dspx_ragged_clip *rtab = nullptr)
 {
     const int cw = C < 128 ? C : 128;
     const int groups = 128 / cw;
     const size_t smem = ((size_t)groups * C + C) * sizeof(double);
     DSPX_REQUIRE(smem <= 48 * 1024, "n_coef %d too large for embed_stats", C);
-    embed_stats_kernel<<<(unsigned)n_clips, 128, smem, st>>>(feats, T, C, out);
+    DSPX_REQUIRE(n_clips < (int64_t)2147483647, "too many clips for one launch");
+    embed_stats_kernel<<<(unsigned)n_clips, 128, smem, st>>>(feats, T, C, out, rtab);
     DSPX_CUDA_CHECK(cudaGetLastError());
     return DSPX_OK;
 }
@@ -256,6 +260,106 @@ static int stft_device(const dspx_plan *pl, const float *clips, int64_t n_clips,
         warp8_can_launch(clips, n_clips, clip_stride, T) && warp8_aligned(pl, clips, clip_stride))
         return launch_warp8(pl, clips, n_clips, clip_len, clip_stride, T, nullptr, nullptr, st, 0, out, pre);
     return launch_generic(pl, clips, n_clips, clip_len, clip_stride, T, pl->take_stft, pre, nullptr, nullptr, out, st);
+}
+
+// ---- ragged batches (dspx_features_ragged) ------------------------------------------------------------
+// Workspace of one call, carved the same way by the size query and the launch (offsets from a 256-byte aligned base):
+// the compact first-pair array the ragged kernel searches, PCM16 peaks, fixed-point embedding sums, MFCC scratch for
+// embeddings without an MFCC output (when the fused path does not apply), and on plans without a ragged kernel a
+// float32 copy of one PCM16 clip at a time.
+struct RaggedWs {
+    uint32_t *rpairs = nullptr;
+    int *peaks = nullptr;
+    long long *eacc = nullptr;
+    float *mfcc = nullptr;
+    float *f32 = nullptr;
+};
+
+static bool ragged_kernel(const dspx_plan *pl) { return pl->kernel == DSPX_KERNEL_WARP8 && !warp8_x2(pl); }
+
+static size_t ragged_ws_carve(const dspx_plan *pl, const dspx_ragged_clip *tab, int64_t n_clips, int dtype, int normalize,
+                              bool want_mfcc, bool want_embed, char *base, RaggedWs *ws)
+{
+    const bool pcm = dtype == DSPX_DTYPE_PCM16, rk = ragged_kernel(pl);
+    const bool fused = want_embed && !want_mfcc && rk && warp8_ragged_aligned(pl, pcm);
+    int64_t total_frames = 0, max_len = 0;
+    if (n_clips > 0) total_frames = tab[n_clips - 1].first_frame + tab[n_clips - 1].n_frames;
+    for (int64_t i = 0; i < n_clips; i++) max_len = std::max(max_len, tab[i].length);
+    const size_t b_pairs = rk ? (size_t)(n_clips + 1) * sizeof(uint32_t) : 0;
+    const size_t b_peaks = rk && pcm && normalize ? (size_t)n_clips * sizeof(int) : 0;
+    const size_t b_eacc = fused ? (size_t)n_clips * 2 * pl->cfg.n_mfcc * sizeof(long long) : 0;
+    const size_t b_mfcc = want_embed && !want_mfcc && !fused ? (size_t)total_frames * pl->cfg.n_mfcc * sizeof(float) : 0;
+    const size_t b_f32 = !rk && pcm ? (size_t)max_len * sizeof(float) : 0;
+    size_t off = 0;
+    auto take = [&](size_t bytes) -> char * {
+        char *p = bytes && base ? base + off : nullptr;
+        off += align256(bytes);
+        return p;
+    };
+    RaggedWs w;
+    w.rpairs = reinterpret_cast<uint32_t *>(take(b_pairs));
+    w.peaks = reinterpret_cast<int *>(take(b_peaks));
+    w.eacc = reinterpret_cast<long long *>(take(b_eacc));
+    w.mfcc = reinterpret_cast<float *>(take(b_mfcc));
+    w.f32 = reinterpret_cast<float *>(take(b_f32));
+    if (ws) *ws = w;
+    return off + 256;
+}
+
+// Plans without a ragged kernel: one stream-ordered feature call per clip into its rows of the stacked outputs, the
+// embeddings from the stacked MFCCs at the end.  Each clip is computed exactly as a [1, length] call computes it.
+static int features_ragged_per_clip(const dspx_plan *pl, const void *samples, int pcm, int normalize,
+                                    const dspx_ragged_clip *tab_dev, const dspx_ragged_clip *tab, int64_t n_clips,
+                                    float *logmel, float *mfcc, float *embed, const RaggedWs &ws, cudaStream_t st)
+{
+    float *mf = mfcc ? mfcc : (embed ? ws.mfcc : nullptr);
+    for (int64_t i = 0; i < n_clips; i++) {
+        const int64_t len = tab[i].length, ff = tab[i].first_frame;
+        const float *x = static_cast<const float *>(samples) + tab[i].start;
+        if (pcm) {
+            pcm16_to_float_kernel<<<1, 256, 0, st>>>(static_cast<const int16_t *>(samples) + tab[i].start, len, len,
+                                                     normalize ? 1 : 0, ws.f32, len);
+            DSPX_CUDA_CHECK(cudaGetLastError());
+            x = ws.f32;
+        }
+        const int rc = features_device(pl, x, 1, len, len, logmel ? logmel + ff * pl->cfg.n_mels : nullptr,
+                                       mf ? mf + ff * pl->cfg.n_mfcc : nullptr, nullptr, st);
+        if (rc != DSPX_OK) return rc;
+    }
+    return embed ? launch_embed(mf, n_clips, 1, pl->cfg.n_mfcc, embed, st, tab_dev) : DSPX_OK;
+}
+
+static int features_ragged(const dspx_plan *pl, const void *samples, int dtype, int normalize, const dspx_ragged_clip *tab_dev,
+                           const dspx_ragged_clip *tab, int64_t n_clips, float *logmel, float *mfcc, float *embed,
+                           char *ws_base, cudaStream_t st)
+{
+    const int pcm = dtype == DSPX_DTYPE_PCM16 ? 1 : 0;
+    RaggedWs ws;
+    ragged_ws_carve(pl, tab, n_clips, dtype, normalize, mfcc != nullptr, embed != nullptr, ws_base, &ws);
+    if (!ragged_kernel(pl))
+        return features_ragged_per_clip(pl, samples, pcm, normalize, tab_dev, tab, n_clips, logmel, mfcc, embed, ws, st);
+    const int C = pl->cfg.n_mfcc;
+    const uint32_t n_items = (uint32_t)(tab[n_clips - 1].first_pair + (tab[n_clips - 1].n_frames + 1) / 2);
+    ragged_pairs_kernel<<<(unsigned)((n_clips + 256) / 256), 256, 0, st>>>(tab_dev, n_clips, ws.rpairs);
+    DSPX_CUDA_CHECK(cudaGetLastError());
+    if (ws.peaks) {
+        pcm16_peak_kernel<<<(unsigned)n_clips, 256, 0, st>>>(static_cast<const int16_t *>(samples), 0, 0, ws.peaks, tab_dev);
+        DSPX_CUDA_CHECK(cudaGetLastError());
+    }
+    if (ws.eacc) {                                   // embeddings alone, accumulated inside the feature kernel
+        DSPX_CUDA_CHECK(cudaMemsetAsync(ws.eacc, 0, (size_t)n_clips * 2 * C * sizeof(long long), st));
+        int rc = launch_warp8_ragged(pl, samples, pcm, tab_dev, ws.rpairs, n_clips, n_items, logmel, nullptr, ws.eacc,
+                                     nullptr, st);
+        if (rc != DSPX_OK) return rc;
+        const int64_t total = n_clips * C;
+        embed_finalize_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(ws.eacc, n_clips, 1, C, embed, tab_dev);
+        DSPX_CUDA_CHECK(cudaGetLastError());
+        return DSPX_OK;
+    }
+    float *mf = mfcc ? mfcc : (embed ? ws.mfcc : nullptr);
+    int rc = launch_warp8_ragged(pl, samples, pcm, tab_dev, ws.rpairs, n_clips, n_items, logmel, mf, nullptr, ws.peaks, st);
+    if (rc != DSPX_OK) return rc;
+    return embed ? launch_embed(mf, n_clips, 1, C, embed, st, tab_dev) : DSPX_OK;
 }
 
 static int ensure_pipe(dspx_plan *pl, size_t in_bytes, size_t out_bytes, bool stage_in, bool stage_out, HostPipe **out,
@@ -344,8 +448,6 @@ static bool is_pinned(const void *p)
     if (cudaPointerGetAttributes(&a, p) != cudaSuccess) { cudaGetLastError(); return false; }
     return a.type == cudaMemoryTypeHost || a.type == cudaMemoryTypeManaged;
 }
-
-static size_t align256(size_t x) { return (x + 255) & ~(size_t)255; }
 
 // Chunked host pipeline shared by dspx_features_host and dspx_stft_host.
 // mode 0: features (logmel/mfcc/embed), mode 1: stft (complex out in `o_stft`).
@@ -711,6 +813,81 @@ int dspx_embed_stats(const float *feats_dev, int64_t n_clips, int64_t n_frames, 
     DSPX_REQUIRE(n_clips >= 0 && n_frames > 0 && n_coef > 0, "bad shape");
     if (n_clips == 0) return DSPX_OK;
     return launch_embed(feats_dev, n_clips, n_frames, n_coef, out_dev, static_cast<cudaStream_t>(stream));
+}
+
+int64_t dspx_ragged_layout(const dspx_config *cfg, const int64_t *starts, const int64_t *lengths, int64_t n_clips,
+                           int dtype, dspx_ragged_clip *table_out)
+{
+    DSPX_REQUIRE(cfg && (n_clips == 0 || (starts && lengths && table_out)), "null argument");
+    DSPX_REQUIRE(n_clips >= 0, "negative clip count");
+    DSPX_REQUIRE(cfg->frame_length > 0 && cfg->hop_length > 0, "frame_length and hop_length must be positive");
+    DSPX_REQUIRE(dtype == DSPX_DTYPE_F32 || dtype == DSPX_DTYPE_PCM16, "ragged batches take float32 or PCM16 samples");
+    int64_t frames = 0, pairs = 0;
+    for (int64_t i = 0; i < n_clips; i++) {
+        DSPX_REQUIRE(lengths[i] >= cfg->frame_length, "clip %lld: %lld samples is shorter than one frame (%d)", (long long)i,
+                     (long long)lengths[i], cfg->frame_length);
+        DSPX_REQUIRE(starts[i] >= 0, "clip %lld: negative start %lld", (long long)i, (long long)starts[i]);
+        DSPX_REQUIRE(dtype != DSPX_DTYPE_F32 || !(starts[i] & 1),
+                     "clip %lld: float32 clips must start at an even sample (start %lld)", (long long)i, (long long)starts[i]);
+        dspx_ragged_clip &r = table_out[i];
+        r.start = starts[i];
+        r.length = lengths[i];
+        r.n_frames = 1 + (lengths[i] - cfg->frame_length) / cfg->hop_length;
+        r.first_frame = frames;
+        r.first_pair = pairs;
+        frames += r.n_frames;
+        pairs += (r.n_frames + 1) / 2;
+        DSPX_REQUIRE(pairs < (int64_t)0x7fffffff, "ragged batch of 2^31 frame pairs or more (clip %lld)", (long long)i);
+    }
+    return frames;
+}
+
+size_t dspx_features_ragged_workspace(const dspx_plan *plan, const dspx_ragged_clip *table_host, int64_t n_clips,
+                                      int dtype, int normalize, int want_logmel, int want_mfcc, int want_embed)
+{
+    (void)want_logmel;
+    if (!plan || n_clips < 0 || (n_clips > 0 && !table_host)) return 0;
+    return ragged_ws_carve(plan, table_host, n_clips, dtype, normalize, want_mfcc != 0, want_embed != 0, nullptr, nullptr);
+}
+
+int dspx_features_ragged(const dspx_plan *plan, const void *samples_dev, int dtype, int normalize,
+                         const dspx_ragged_clip *table_dev, const dspx_ragged_clip *table_host, int64_t n_clips,
+                         int64_t total_frames, float *logmel_out_dev, float *mfcc_out_dev, float *embed_out_dev,
+                         void *workspace_dev, size_t workspace_bytes, void *stream)
+{
+    DSPX_REQUIRE(plan, "null plan");
+    DSPX_REQUIRE(dtype == DSPX_DTYPE_F32 || dtype == DSPX_DTYPE_PCM16, "ragged batches take float32 or PCM16 samples");
+    DSPX_REQUIRE(n_clips >= 0, "negative clip count");
+    if (n_clips == 0) return DSPX_OK;
+    DSPX_REQUIRE(samples_dev && table_dev && table_host, "null argument");
+    DSPX_REQUIRE(dtype != DSPX_DTYPE_F32 || !(reinterpret_cast<uintptr_t>(samples_dev) & 7),
+                 "float32 samples must be 8-byte aligned");
+    DSPX_REQUIRE(n_clips < (int64_t)2147483647, "too many clips for one launch");
+    const dspx_ragged_clip &last = table_host[n_clips - 1];
+    DSPX_REQUIRE(last.first_frame + last.n_frames == total_frames, "total_frames %lld does not match the table (%lld)",
+                 (long long)total_frames, (long long)(last.first_frame + last.n_frames));
+    DSPX_REQUIRE(last.first_pair + (last.n_frames + 1) / 2 < (int64_t)0x7fffffff, "ragged batch of 2^31 frame pairs or more");
+    for (int64_t i = 0; i < n_clips; i++)
+        DSPX_REQUIRE(table_host[i].length >= plan->cfg.frame_length, "clip %lld: %lld samples is shorter than one frame (%d)",
+                     (long long)i, (long long)table_host[i].length, plan->cfg.frame_length);
+    const size_t need = dspx_features_ragged_workspace(plan, table_host, n_clips, dtype, normalize, logmel_out_dev != nullptr,
+                                                       mfcc_out_dev != nullptr, embed_out_dev != nullptr);
+    DSPX_REQUIRE(workspace_dev && workspace_bytes >= need, "workspace too small (%zu bytes needed)", need);
+    if (!logmel_out_dev && !mfcc_out_dev && !embed_out_dev) return DSPX_OK;
+    DeviceGuard guard(plan->device);
+    char *ws = static_cast<char *>(workspace_dev);
+    ws += (256 - (reinterpret_cast<uintptr_t>(ws) & 255)) & 255;
+    return features_ragged(plan, samples_dev, dtype, normalize ? 1 : 0, table_dev, table_host, n_clips, logmel_out_dev,
+                           mfcc_out_dev, embed_out_dev, ws, static_cast<cudaStream_t>(stream));
+}
+
+int dspx_embed_stats_ragged(const float *feats_dev, const dspx_ragged_clip *table_dev, int64_t n_clips, int n_coef,
+                            float *out_dev, void *stream)
+{
+    DSPX_REQUIRE(n_clips >= 0 && n_coef > 0, "bad shape");
+    if (n_clips == 0) return DSPX_OK;
+    DSPX_REQUIRE(feats_dev && table_dev && out_dev, "null argument");
+    return launch_embed(feats_dev, n_clips, 1, n_coef, out_dev, static_cast<cudaStream_t>(stream), table_dev);
 }
 
 int dspx_cmvn(float *feats_dev, int64_t n_clips, int64_t n_frames, int n_coef, double eps, void *stream)

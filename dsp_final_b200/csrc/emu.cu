@@ -9,6 +9,7 @@
 // path.
 #include <vector>
 
+#define DSPX_EMU                     // no ragged launcher: its 88 kernel instantiations are not replayed here
 #include "dspx_internal.cuh"
 #include "tables.cuh"
 #include "feat_generic.cuh"
@@ -217,9 +218,11 @@ int emu_warp8_layout(const dspx_config *cfg, int32_t *out)
 }
 
 // Replays feat_warp8_kernel: one "warp" at a time, each phase run for lanes 0..31 in turn
-// (a __syncwarp() separates the phases on the device).
-int emu_features_warp8(const dspx_config *cfg, const float *clips, int64_t n_clips, int64_t clip_len,
-                       int64_t clip_stride, float *logmel, float *mfcc, float *stft_out, int stft_pre)
+// (a __syncwarp() separates the phases on the device).  rtab != NULL replays the RAGGED variant over a
+// dspx_ragged_layout table (clip_len and clip_stride unused).
+static int emu_warp8(const dspx_config *cfg, const float *clips, int64_t n_clips, int64_t clip_len,
+                     int64_t clip_stride, float *logmel, float *mfcc, float *stft_out, int stft_pre,
+                     const dspx_ragged_clip *rtab)
 {
     EmuTables e;
     int rc = emu_build(cfg, e);
@@ -230,15 +233,15 @@ int emu_features_warp8(const dspx_config *cfg, const float *clips, int64_t n_cli
     pl.M = e.M;
     pl.n_bins = e.n_bins;
     pl.host = e.t;
-    if (!warp8_supported(&pl) || clip_len < cfg->frame_length) return DSPX_EUNSUPPORTED;
+    if (!warp8_supported(&pl) || (!rtab && clip_len < cfg->frame_length)) return DSPX_EUNSUPPORTED;
     // frames off the 8-byte grid replay the 4-byte-load variant, like launch_warp8 picks it
-    const bool u4 = (clip_stride & 1) || (cfg->hop_length & 1) || (reinterpret_cast<uintptr_t>(clips) & 7) ||
+    const bool u4 = (!rtab && (clip_stride & 1)) || (cfg->hop_length & 1) || (reinterpret_cast<uintptr_t>(clips) & 7) ||
                     cfg->frame_length != e.P;
     if (u4 && stft_out) return DSPX_EUNSUPPORTED;
     std::vector<float> blob;
     W8Tables tb{};
     warp8_build_tables(&pl, blob, tb);
-    const int64_t T = 1 + (clip_len - cfg->frame_length) / cfg->hop_length;
+    const int64_t T = rtab ? 0 : 1 + (clip_len - cfg->frame_length) / cfg->hop_length;
     W8Params p{};
     p.clips = clips;
     p.n_clips = n_clips;
@@ -246,6 +249,15 @@ int emu_features_warp8(const dspx_config *cfg, const float *clips, int64_t n_cli
     p.n_frames = T;
     p.pairs_per_clip = (uint32_t)((T + 1) / 2);
     p.n_items = (uint32_t)(n_clips * p.pairs_per_clip);
+    std::vector<uint32_t> rpairs;
+    if (rtab) {
+        if (tb.x2 || stft_out) return DSPX_EUNSUPPORTED;
+        for (int64_t i = 0; i < n_clips; i++) rpairs.push_back((uint32_t)rtab[i].first_pair);
+        rpairs.push_back(n_clips ? (uint32_t)(rtab[n_clips - 1].first_pair + (rtab[n_clips - 1].n_frames + 1) / 2) : 0);
+        p.rtab = rtab;
+        p.rpairs = rpairs.data();
+        p.n_items = rpairs.back();
+    }
     p.hop = cfg->hop_length;
     p.n_mels = cfg->n_mels;
     p.n_mfcc = cfg->n_mfcc;
@@ -314,7 +326,8 @@ int emu_features_warp8(const dspx_config *cfg, const float *clips, int64_t n_cli
     // the device kernel computes window / twiddles on the feature path and loads them in STFT mode: replay the same
 #define W8_P1(R, PRE_, SH_) do { if (p.stft) w8_pass1<R, PRE_, SH_, false>(c, lane); else if (u4) w8_pass1<R, PRE_, false, false, true>(c, lane); else w8_pass1<R, PRE_, SH_, true>(c, lane); } while (0)
     for (uint32_t item = 0; item < p.n_items; item++) {
-        w8_set_item(p, c, item);
+        if (rtab) w8_set_item<false, true>(p, c, item);
+        else w8_set_item(p, c, item);
         for (int lane = 0; lane < 32; lane++) {
             const bool share = 2 * cfg->hop_length == e.P && r1 != 16 && !u4;
             if (r1 == 4 && share) { if (pre) W8_P1(4, true, true); else W8_P1(4, false, true); }
@@ -365,6 +378,19 @@ int emu_features_warp8(const dspx_config *cfg, const float *clips, int64_t n_cli
         }
     }
     return DSPX_OK;
+}
+
+int emu_features_warp8(const dspx_config *cfg, const float *clips, int64_t n_clips, int64_t clip_len,
+                       int64_t clip_stride, float *logmel, float *mfcc, float *stft_out, int stft_pre)
+{
+    return emu_warp8(cfg, clips, n_clips, clip_len, clip_stride, logmel, mfcc, stft_out, stft_pre, nullptr);
+}
+
+// The RAGGED variant over a flat float32 buffer and a dspx_ragged_layout table: outputs [total_frames, ...].
+int emu_features_warp8_ragged(const dspx_config *cfg, const float *samples, const dspx_ragged_clip *table, int64_t n_clips,
+                              float *logmel, float *mfcc)
+{
+    return emu_warp8(cfg, samples, n_clips, 0, 0, logmel, mfcc, nullptr, 0, table);
 }
 
 // Exhaustive check of the fused PCM16 normalisation (w8_pcm_to_float): for every peak m in [1, 32768] and every sample

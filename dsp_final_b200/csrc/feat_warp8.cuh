@@ -212,6 +212,9 @@ struct W8Params {
     float2 *stft;            // STFT mode: complex spectrum [n_clips, n_frames, M + 1]
     long long *eacc;         // embedding accumulators [n_clips][2][n_mfcc] (fixed point, see w8_embed_accumulate) or null
     const int *peaks;        // PCM variant: max |sample| of every clip (peak normalisation), null = divide by 32768 only
+    // RAGGED variant (appended: the fields above keep their offsets): items are global frame-pair indices
+    const dspx_ragged_clip *rtab;   // per-clip start, n_frames, first_frame (dspx_ragged_layout)
+    const uint32_t *rpairs;         // [n_clips + 1] first pair of every clip, then the total: the array the search walks
 };
 
 struct W8Ctx {               // everything one warp needs for one frame pair
@@ -879,12 +882,15 @@ DSPX_HD void w8_dct_store(const W8Ctx &c, int lane, int c0, float2 total)
 }
 
 #if defined(__CUDACC__)
-__global__ void embed_finalize_kernel(const long long *eacc, int64_t n_clips, int64_t n_frames, int n_coef, float *out)
+// rtab (ragged batches): every clip's own frame count instead of n_frames
+__global__ void embed_finalize_kernel(const long long *eacc, int64_t n_clips, int64_t n_frames, int n_coef, float *out,
+                                      const dspx_ragged_clip *rtab = nullptr)
 {
     const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n_clips * n_coef) return;
     const int64_t clip = i / n_coef;
     const int q = (int)(i - clip * n_coef);
+    if (rtab) n_frames = rtab[clip].n_frames;
     const long long *e = eacc + clip * 2 * n_coef;
     const double mean = (double)e[q] / W8_EFIX1 / (double)n_frames;
     const double ex2 = (double)e[n_coef + q] / W8_EFIX2 / (double)n_frames;
@@ -894,10 +900,49 @@ __global__ void embed_finalize_kernel(const long long *eacc, int64_t n_clips, in
 }
 #endif
 
-// set the per-item fields of the context (item = clip * pairs_per_clip + pair)
-template <bool PCM = false>
+// RAGGED: the clip that holds global frame pair `item` -- the last one whose first pair is <= item (binary search over
+// rpairs, which is strictly increasing: every clip has at least one frame)
+DSPX_HD uint32_t w8_ragged_clip(const W8Params &p, uint32_t item)
+{
+    uint32_t lo = 0, hi = (uint32_t)p.n_clips;                // rpairs[lo] <= item < rpairs[hi]
+    while (hi - lo > 1) {
+        const uint32_t mid = (lo + hi) >> 1;
+        if (p.rpairs[mid] <= item) lo = mid;
+        else hi = mid;
+    }
+    return lo;
+}
+
+// set the per-item fields of the context (item = clip * pairs_per_clip + pair; RAGGED: item = rpairs[clip] + pair)
+template <bool PCM = false, bool RAGGED = false>
 DSPX_HD void w8_set_item(const W8Params &p, W8Ctx &c, uint32_t item)
 {
+    if (RAGGED) {
+        const uint32_t clip = w8_ragged_clip(p, item), pair = item - p.rpairs[clip];
+        const dspx_ragged_clip &rc = p.rtab[clip];
+        const int64_t tA = 2 * (int64_t)pair, tB = tA + 1;
+        c.validB = tB < rc.n_frames;
+        using S = typename W8Sample<PCM>::type;
+        const S *base = reinterpret_cast<const S *>(p.clips) + rc.start;
+        c.fa = reinterpret_cast<const float *>(base + tA * p.hop);
+        c.fb = c.validB ? reinterpret_cast<const float *>(base + tB * p.hop) : c.fa;
+        if (PCM) {
+            const int m = p.peaks ? p.peaks[clip] : 0;
+            c.pcm_m = (float)m;
+            c.pcm_r = m > 0 ? 1.0f / (float)m : 0.f;
+        }
+        c.firstA = pair == 0;                                 // pre-emphasis restarts at sample 0 of every clip
+        c.firstB = c.validB ? 0 : c.firstA;
+        const int64_t rowA = rc.first_frame + tA, rowB = rowA + 1;
+        c.logmelA = p.logmel ? p.logmel + rowA * p.n_mels : nullptr;
+        c.logmelB = c.logmelA ? c.logmelA + p.n_mels : nullptr;
+        c.lm_fs = 1;
+        c.mfccA = p.mfcc ? p.mfcc + rowA * p.n_mfcc : nullptr;
+        c.mfccB = p.mfcc ? p.mfcc + rowB * p.n_mfcc : nullptr;
+        c.stftA = c.stftB = nullptr;
+        c.eacc = p.eacc ? p.eacc + (int64_t)clip * 2 * p.n_mfcc : nullptr;
+        return;
+    }
     const uint32_t clip = item / p.pairs_per_clip, pair = item - clip * p.pairs_per_clip;
     const int64_t tA = 2 * (int64_t)pair, tB = tA + 1;
     c.validB = tB < p.n_frames;
@@ -927,19 +972,28 @@ DSPX_HD void w8_set_item(const W8Params &p, W8Ctx &c, uint32_t item)
 // the whole per-item sequence; SYNC is __syncwarp() on the device and a no-op in the lane-loop replay
 #if defined(__CUDACC__)
 // pull the next item's samples towards L2 while this one is being transformed
+template <bool RAGGED = false>
 __device__ __forceinline__ void w8_prefetch(const W8Params &p, uint32_t item, int lane, int n_fft, int elem = 4)
 {
     if (item >= p.n_items) return;
-    const uint32_t clip = item / p.pairs_per_clip, pair = item - clip * p.pairs_per_clip;
-    const char *base = reinterpret_cast<const char *>(p.clips) + ((int64_t)clip * p.clip_stride + 2 * (int64_t)pair * p.hop) * elem;
+    const char *base;
+    if (RAGGED) {
+        const uint32_t clip = w8_ragged_clip(p, item);
+        base = reinterpret_cast<const char *>(p.clips) + (p.rtab[clip].start + 2 * (int64_t)(item - p.rpairs[clip]) * p.hop) * elem;
+    } else {
+        const uint32_t clip = item / p.pairs_per_clip, pair = item - clip * p.pairs_per_clip;
+        base = reinterpret_cast<const char *>(p.clips) + ((int64_t)clip * p.clip_stride + 2 * (int64_t)pair * p.hop) * elem;
+    }
     const int span = (p.hop + n_fft) * elem;                   // bytes covered by the frame pair
     for (int off = lane * 128; off < span; off += 32 * 128)
         asm volatile("prefetch.global.L2 [%0];" ::"l"(base + off));
 }
 
 // EMB: accumulate clip embeddings (w8_embed_accumulate); a template switch so that the plain feature kernels keep
-// their register allocation (the extra pointer alone pushed the 96-register headline variant into spills)
-template <int R1, bool PRE, bool STFT, bool SHARE, int NW, bool EMB = false, bool U4 = false, bool PCM = false>
+// their register allocation (the extra pointer alone pushed the 96-register headline variant into spills).
+// RAGGED: clips of different lengths (w8_set_item); a switch for the same reason.
+template <int R1, bool PRE, bool STFT, bool SHARE, int NW, bool EMB = false, bool U4 = false, bool PCM = false,
+          bool RAGGED = false>
 __global__ void __launch_bounds__(NW * 32, (R1 == 16 || NW > 8) ? 1 : 2) feat_warp8_kernel(const W8Params p)
 {
     using G = W8Geo<R1>;
@@ -970,10 +1024,10 @@ __global__ void __launch_bounds__(NW * 32, (R1 == 16 || NW > 8) ? 1 : 2) feat_wa
     c.take = p.take;
     const uint32_t n_warps = gridDim.x * NW;
     for (uint32_t item = blockIdx.x * NW + warp; item < p.n_items; item += n_warps) {
-        w8_set_item<PCM>(p, c, item);
+        w8_set_item<PCM, RAGGED>(p, c, item);
         if (!EMB) c.eacc = nullptr;
         w8_pass1<R1, PRE, SHARE, (!STFT && R1 <= 8 && !U4), U4, PCM>(c, lane);
-        if (p.prefetch) w8_prefetch(p, item + n_warps, lane, G::P, PCM ? 2 : 4);
+        if (p.prefetch) w8_prefetch<RAGGED>(p, item + n_warps, lane, G::P, PCM ? 2 : 4);
         __syncwarp();
 #if !defined(DSPX_ABL) || DSPX_ABL != 5
         w8_pass2<R1>(c, lane);
@@ -1462,17 +1516,18 @@ inline void warp8_release(dspx_plan *pl)
 int launch_generic_fallback(const dspx_plan *pl, const float *clips, int64_t n_clips, int64_t clip_len,
                             int64_t clip_stride, int64_t T, float *logmel, float *mfcc, cudaStream_t st, int nchw);
 
-template <int R1, bool PRE, bool STFT, bool SHARE, int NW, bool EMB = false, bool U4 = false, bool PCM = false>
+template <int R1, bool PRE, bool STFT, bool SHARE, int NW, bool EMB = false, bool U4 = false, bool PCM = false,
+          bool RAGGED = false>
 inline int w8_launch_nw(const W8Params &p, size_t smem, int device, int64_t ctas, cudaStream_t st)
 {
     static std::atomic<unsigned char> optin[64];
-    DSPX_CUDA_CHECK(optin_max_smem(feat_warp8_kernel<R1, PRE, STFT, SHARE, NW, EMB, U4, PCM>, optin, device));
-    feat_warp8_kernel<R1, PRE, STFT, SHARE, NW, EMB, U4, PCM><<<(unsigned)ctas, NW * 32, smem, st>>>(p);
+    DSPX_CUDA_CHECK(optin_max_smem(feat_warp8_kernel<R1, PRE, STFT, SHARE, NW, EMB, U4, PCM, RAGGED>, optin, device));
+    feat_warp8_kernel<R1, PRE, STFT, SHARE, NW, EMB, U4, PCM, RAGGED><<<(unsigned)ctas, NW * 32, smem, st>>>(p);
     DSPX_CUDA_CHECK(cudaGetLastError());
     return DSPX_OK;
 }
 
-template <int R1, bool PRE, bool STFT, bool SHARE>
+template <int R1, bool PRE, bool STFT, bool SHARE, bool RAGGED = false>
 inline int w8_launch_cfg(const W8Params &p, const W8PlanData *pd, int device, int sm_count, cudaStream_t st)
 {
     // persistent grid: warps stride over the items
@@ -1480,62 +1535,62 @@ inline int w8_launch_cfg(const W8Params &p, const W8PlanData *pd, int device, in
         int64_t ctas = ((int64_t)p.n_items + W8_WARPS_WIDE - 1) / W8_WARPS_WIDE;
         if (ctas > sm_count) ctas = sm_count;
         constexpr int NWW = (R1 != 16 && !STFT) ? W8_WARPS_WIDE : W8_WARPS;
-        if (!STFT && p.eacc) return w8_launch_nw<R1, PRE, STFT, SHARE, NWW, !STFT>(p, pd->smem_wide, device, ctas, st);
-        return w8_launch_nw<R1, PRE, STFT, SHARE, NWW>(p, pd->smem_wide, device, ctas, st);
+        if (!STFT && p.eacc) return w8_launch_nw<R1, PRE, STFT, SHARE, NWW, !STFT, false, false, RAGGED>(p, pd->smem_wide, device, ctas, st);
+        return w8_launch_nw<R1, PRE, STFT, SHARE, NWW, false, false, false, RAGGED>(p, pd->smem_wide, device, ctas, st);
     }
     if (!STFT && R1 != 16 && pd->smem_mid) {
         int64_t ctas = ((int64_t)p.n_items + W8_WARPS_MID - 1) / W8_WARPS_MID;
         if (ctas > sm_count) ctas = sm_count;
         constexpr int NWM = (R1 != 16 && !STFT) ? W8_WARPS_MID : W8_WARPS;
-        if (!STFT && p.eacc) return w8_launch_nw<R1, PRE, STFT, SHARE, NWM, !STFT>(p, pd->smem_mid, device, ctas, st);
-        return w8_launch_nw<R1, PRE, STFT, SHARE, NWM>(p, pd->smem_mid, device, ctas, st);
+        if (!STFT && p.eacc) return w8_launch_nw<R1, PRE, STFT, SHARE, NWM, !STFT, false, false, RAGGED>(p, pd->smem_mid, device, ctas, st);
+        return w8_launch_nw<R1, PRE, STFT, SHARE, NWM, false, false, false, RAGGED>(p, pd->smem_mid, device, ctas, st);
     }
     if (!STFT && R1 == 16 && pd->smem_r16) {
         int64_t ctas = ((int64_t)p.n_items + W8_WARPS_R16 - 1) / W8_WARPS_R16;
         if (ctas > sm_count) ctas = sm_count;
         constexpr int NWR = (R1 == 16 && !STFT) ? W8_WARPS_R16 : W8_WARPS;
-        if (p.eacc) return w8_launch_nw<R1, PRE, STFT, SHARE, NWR, !STFT>(p, pd->smem_r16, device, ctas, st);
-        return w8_launch_nw<R1, PRE, STFT, SHARE, NWR>(p, pd->smem_r16, device, ctas, st);
+        if (p.eacc) return w8_launch_nw<R1, PRE, STFT, SHARE, NWR, !STFT, false, false, RAGGED>(p, pd->smem_r16, device, ctas, st);
+        return w8_launch_nw<R1, PRE, STFT, SHARE, NWR, false, false, false, RAGGED>(p, pd->smem_r16, device, ctas, st);
     }
     int64_t ctas = ((int64_t)p.n_items + W8_WARPS - 1) / W8_WARPS;
     const int64_t resident = (int64_t)sm_count * pd->ctas_per_sm;
     if (ctas > resident) ctas = resident;
-    if (!STFT && p.eacc) return w8_launch_nw<R1, PRE, STFT, SHARE, W8_WARPS, !STFT>(p, pd->smem, device, ctas, st);
-    return w8_launch_nw<R1, PRE, STFT, SHARE, W8_WARPS>(p, pd->smem, device, ctas, st);
+    if (!STFT && p.eacc) return w8_launch_nw<R1, PRE, STFT, SHARE, W8_WARPS, !STFT, false, false, RAGGED>(p, pd->smem, device, ctas, st);
+    return w8_launch_nw<R1, PRE, STFT, SHARE, W8_WARPS, false, false, false, RAGGED>(p, pd->smem, device, ctas, st);
 }
 
 // features from frames that are not 8-byte aligned: 4-byte sample loads, no row sharing, no fused embeddings
-template <int R1, bool PRE, bool PCM = false>
+template <int R1, bool PRE, bool PCM = false, bool RAGGED = false>
 inline int w8_launch_u4(const W8Params &p, const W8PlanData *pd, int device, int sm_count, cudaStream_t st)
 {
     if (R1 != 16 && pd->smem_wide) {
         int64_t ctas = ((int64_t)p.n_items + W8_WARPS_WIDE - 1) / W8_WARPS_WIDE;
         if (ctas > sm_count) ctas = sm_count;
-        return w8_launch_nw<R1, PRE, false, false, (R1 != 16) ? W8_WARPS_WIDE : W8_WARPS, false, true, PCM>(p, pd->smem_wide, device, ctas, st);
+        return w8_launch_nw<R1, PRE, false, false, (R1 != 16) ? W8_WARPS_WIDE : W8_WARPS, false, true, PCM, RAGGED>(p, pd->smem_wide, device, ctas, st);
     }
     if (R1 != 16 && pd->smem_mid) {
         int64_t ctas = ((int64_t)p.n_items + W8_WARPS_MID - 1) / W8_WARPS_MID;
         if (ctas > sm_count) ctas = sm_count;
-        return w8_launch_nw<R1, PRE, false, false, (R1 != 16) ? W8_WARPS_MID : W8_WARPS, false, true, PCM>(p, pd->smem_mid, device, ctas, st);
+        return w8_launch_nw<R1, PRE, false, false, (R1 != 16) ? W8_WARPS_MID : W8_WARPS, false, true, PCM, RAGGED>(p, pd->smem_mid, device, ctas, st);
     }
     if (R1 == 16 && pd->smem_r16) {
         int64_t ctas = ((int64_t)p.n_items + W8_WARPS_R16 - 1) / W8_WARPS_R16;
         if (ctas > sm_count) ctas = sm_count;
-        return w8_launch_nw<R1, PRE, false, false, (R1 == 16) ? W8_WARPS_R16 : W8_WARPS, false, true, PCM>(p, pd->smem_r16, device, ctas, st);
+        return w8_launch_nw<R1, PRE, false, false, (R1 == 16) ? W8_WARPS_R16 : W8_WARPS, false, true, PCM, RAGGED>(p, pd->smem_r16, device, ctas, st);
     }
     int64_t ctas = ((int64_t)p.n_items + W8_WARPS - 1) / W8_WARPS;
     const int64_t resident = (int64_t)sm_count * pd->ctas_per_sm;
     if (ctas > resident) ctas = resident;
-    return w8_launch_nw<R1, PRE, false, false, W8_WARPS, false, true, PCM>(p, pd->smem, device, ctas, st);
+    return w8_launch_nw<R1, PRE, false, false, W8_WARPS, false, true, PCM, RAGGED>(p, pd->smem, device, ctas, st);
 }
 
-template <int R1, bool PRE, bool STFT>
+template <int R1, bool PRE, bool STFT, bool RAGGED = false>
 inline int w8_launch_one(const W8Params &p, const W8PlanData *pd, int device, int sm_count, cudaStream_t st)
 {
     // rows are shared between the two frames of a pair when hop == n_fft / 2 (R1 = 16 keeps the plain loads:
     // 24 distinct rows in flight would not fit its register budget)
-    if (R1 != 16 && p.share) return w8_launch_cfg<R1, PRE, STFT, (R1 != 16)>(p, pd, device, sm_count, st);
-    return w8_launch_cfg<R1, PRE, STFT, false>(p, pd, device, sm_count, st);
+    if (R1 != 16 && p.share) return w8_launch_cfg<R1, PRE, STFT, (R1 != 16), RAGGED>(p, pd, device, sm_count, st);
+    return w8_launch_cfg<R1, PRE, STFT, false, RAGGED>(p, pd, device, sm_count, st);
 }
 
 // items are 32-bit
@@ -1552,6 +1607,25 @@ inline bool warp8_aligned(const dspx_plan *pl, const float *clips, int64_t clip_
 {
     return pl->cfg.frame_length == pl->P && !(pl->cfg.hop_length & 1) && !(clip_stride & 1) &&
            !(reinterpret_cast<uintptr_t>(clips) & 7);
+}
+
+// the launch fields that come from the plan alone
+inline W8Params w8_plan_params(const dspx_plan *pl)
+{
+    const W8PlanData *pd = static_cast<const W8PlanData *>(pl->fast_host);
+    W8Params p{};
+    p.hop = pl->cfg.hop_length;
+    p.n_mels = pl->cfg.n_mels;
+    p.n_mfcc = pl->cfg.n_mfcc;
+    p.prefetch = 1;
+    p.take = std::min(pl->cfg.frame_length, pl->P);
+    p.share = pd->share;
+    p.alpha = (float)pl->cfg.pre_emphasis;
+    p.win_a = pl->cfg.window == DSPX_WINDOW_HANN ? 0.25f : (pl->cfg.window == DSPX_WINDOW_HAMMING ? 0.27f : 0.5f);
+    p.win_b = pl->cfg.window == DSPX_WINDOW_HANN ? -0.25f : (pl->cfg.window == DSPX_WINDOW_HAMMING ? -0.23f : 0.f);
+    p.tb = pd->tb;
+    p.tables = static_cast<const float *>(pl->d_fast_tables);
+    return p;
 }
 
 inline int launch_warp8(const dspx_plan *pl, const float *clips, int64_t n_clips, int64_t clip_len,
@@ -1571,24 +1645,13 @@ inline int launch_warp8(const dspx_plan *pl, const float *clips, int64_t n_clips
         return launch_generic_fallback(pl, clips, n_clips, clip_len, clip_stride, T, logmel, mfcc, st, nchw);
     }
     const W8PlanData *pd = static_cast<const W8PlanData *>(pl->fast_host);
-    W8Params p{};
+    W8Params p = w8_plan_params(pl);
     p.clips = clips;
     p.n_clips = n_clips;
     p.clip_stride = clip_stride;
     p.n_frames = T;
     p.pairs_per_clip = (uint32_t)pairs;
     p.n_items = (uint32_t)(n_clips * pairs);
-    p.hop = pl->cfg.hop_length;
-    p.n_mels = pl->cfg.n_mels;
-    p.n_mfcc = pl->cfg.n_mfcc;
-    p.prefetch = 1;
-    p.take = std::min(pl->cfg.frame_length, pl->P);
-    p.share = pd->share;
-    p.alpha = (float)pl->cfg.pre_emphasis;
-    p.win_a = pl->cfg.window == DSPX_WINDOW_HANN ? 0.25f : (pl->cfg.window == DSPX_WINDOW_HAMMING ? 0.27f : 0.5f);
-    p.win_b = pl->cfg.window == DSPX_WINDOW_HANN ? -0.25f : (pl->cfg.window == DSPX_WINDOW_HAMMING ? -0.23f : 0.f);
-    p.tb = pd->tb;
-    p.tables = static_cast<const float *>(pl->d_fast_tables);
     p.logmel = logmel;
     p.mfcc = mfcc;
     p.lm_ts = nchw ? 1 : p.n_mels;
@@ -1633,6 +1696,70 @@ inline int launch_warp8(const dspx_plan *pl, const float *clips, int64_t n_clips
     return DSPX_EUNSUPPORTED;
 #endif
 }
+
+// frames of float32 clips that start at even samples of an 8-byte aligned buffer sit on the 8-byte grid when the hop is
+// even: the aligned variants (row sharing, fused embeddings) apply exactly when they would to each clip alone
+inline bool warp8_ragged_aligned(const dspx_plan *pl, int pcm)
+{
+    return !pcm && pl->cfg.frame_length == pl->P && !(pl->cfg.hop_length & 1);
+}
+
+// [n_clips + 1] first frame pair of every clip, then the total: the compact array w8_ragged_clip searches
+__global__ void ragged_pairs_kernel(const dspx_ragged_clip *rtab, int64_t n_clips, uint32_t *rpairs)
+{
+    const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i < n_clips) rpairs[i] = (uint32_t)rtab[i].first_pair;
+    else if (i == n_clips) rpairs[i] = (uint32_t)(rtab[i - 1].first_pair + (rtab[i - 1].n_frames + 1) / 2);
+}
+
+#if !defined(DSPX_W8_LAB) && !defined(DSPX_EMU)
+// Ragged batch, one launch: items are the n_items frame pairs of all clips (RAGGED variants; not the STFT mode).
+// samples: float32 (8-byte aligned, even starts) or int16 (pcm); eacc needs warp8_ragged_aligned.
+inline int launch_warp8_ragged(const dspx_plan *pl, const void *samples, int pcm, const dspx_ragged_clip *rtab,
+                               const uint32_t *rpairs, int64_t n_clips, uint32_t n_items, float *logmel, float *mfcc,
+                               long long *eacc, const int *peaks, cudaStream_t st)
+{
+    const bool aligned = warp8_ragged_aligned(pl, pcm);
+    if (eacc && !aligned) { set_error("warp8 fused embeddings: frames off the 8-byte grid"); return DSPX_EUNSUPPORTED; }
+    const W8PlanData *pd = static_cast<const W8PlanData *>(pl->fast_host);
+    W8Params p = w8_plan_params(pl);
+    p.clips = static_cast<const float *>(samples);
+    p.n_clips = n_clips;
+    p.n_items = n_items;
+    p.logmel = logmel;
+    p.mfcc = mfcc;
+    p.lm_ts = p.n_mels;
+    p.lm_fs = 1;
+    p.eacc = eacc;
+    p.peaks = peaks;
+    p.rtab = rtab;
+    p.rpairs = rpairs;
+    const int ctas = pl->sm_count;
+    const bool pre = pl->cfg.pre_emphasis > 0.0;
+#define W8R_SWITCH(CALL4, CALL8, CALL16)                                     \
+    switch (pd->tb.r1) {                                                   \
+        case 4: return CALL4;                                              \
+        case 8: return CALL8;                                              \
+        case 16: return CALL16;                                            \
+    }
+    if (pcm) {
+        W8R_SWITCH((pre ? w8_launch_u4<4, true, true, true>(p, pd, pl->device, ctas, st) : w8_launch_u4<4, false, true, true>(p, pd, pl->device, ctas, st)),
+                   (pre ? w8_launch_u4<8, true, true, true>(p, pd, pl->device, ctas, st) : w8_launch_u4<8, false, true, true>(p, pd, pl->device, ctas, st)),
+                   (pre ? w8_launch_u4<16, true, true, true>(p, pd, pl->device, ctas, st) : w8_launch_u4<16, false, true, true>(p, pd, pl->device, ctas, st)))
+    } else if (!aligned) {
+        W8R_SWITCH((pre ? w8_launch_u4<4, true, false, true>(p, pd, pl->device, ctas, st) : w8_launch_u4<4, false, false, true>(p, pd, pl->device, ctas, st)),
+                   (pre ? w8_launch_u4<8, true, false, true>(p, pd, pl->device, ctas, st) : w8_launch_u4<8, false, false, true>(p, pd, pl->device, ctas, st)),
+                   (pre ? w8_launch_u4<16, true, false, true>(p, pd, pl->device, ctas, st) : w8_launch_u4<16, false, false, true>(p, pd, pl->device, ctas, st)))
+    } else {
+        W8R_SWITCH((pre ? w8_launch_one<4, true, false, true>(p, pd, pl->device, ctas, st) : w8_launch_one<4, false, false, true>(p, pd, pl->device, ctas, st)),
+                   (pre ? w8_launch_one<8, true, false, true>(p, pd, pl->device, ctas, st) : w8_launch_one<8, false, false, true>(p, pd, pl->device, ctas, st)),
+                   (pre ? w8_launch_one<16, true, false, true>(p, pd, pl->device, ctas, st) : w8_launch_one<16, false, false, true>(p, pd, pl->device, ctas, st)))
+    }
+#undef W8R_SWITCH
+    set_error("warp8: bad radix");
+    return DSPX_EUNSUPPORTED;
+}
+#endif
 #endif
 
 }  // namespace dspx

@@ -43,9 +43,12 @@ __global__ void __launch_bounds__(256) pcm16_to_float_kernel(const int16_t *pcm,
 }
 // max |sample| of every clip: all the fused PCM16 path needs before the feature kernel converts the samples in its
 // own loads (w8_pcm_to_float).  One CTA per clip; the clip was just copied to the device, so this read is L2-warm.
-__global__ void __launch_bounds__(256) pcm16_peak_kernel(const int16_t *pcm, int64_t clip_len, int64_t pcm_stride, int *peaks)
+// rtab (ragged batches): clip b is rtab[b].length samples from rtab[b].start instead of clip_len from b * pcm_stride.
+__global__ void __launch_bounds__(256) pcm16_peak_kernel(const int16_t *pcm, int64_t clip_len, int64_t pcm_stride, int *peaks,
+                                                         const dspx_ragged_clip *rtab = nullptr)
 {
-    const int16_t *src = pcm + (size_t)blockIdx.x * pcm_stride;
+    const int16_t *src = pcm + (rtab ? rtab[blockIdx.x].start : (int64_t)blockIdx.x * pcm_stride);
+    if (rtab) clip_len = rtab[blockIdx.x].length;
     __shared__ int s_peak[8];
     int m = 0;
     const int64_t pairs = ((reinterpret_cast<uintptr_t>(src) & 3) == 0) ? clip_len / 2 : 0;      // 32-bit loads when aligned

@@ -28,12 +28,14 @@ constexpr int TK_MAX_SPLITS = 32;
 #if defined(__CUDACC__)
 
 // ---- embedding statistics ---------------------------------------------------
+// rtab (ragged batches): clip i is rtab[i].n_frames rows from row rtab[i].first_frame; the same summation order
 __global__ void __launch_bounds__(128) embed_stats_kernel(const float *feats, int64_t n_frames, int n_coef,
-                                                         float *out)
+                                                         float *out, const dspx_ragged_clip *rtab = nullptr)
 {
     extern __shared__ double es_sm[];                  // [groups][n_coef] partials, then [n_coef] means
     const int64_t clip = blockIdx.x;
-    const float *f = feats + (size_t)clip * n_frames * n_coef;
+    const float *f = feats + (size_t)(rtab ? rtab[clip].first_frame : clip * n_frames) * n_coef;
+    if (rtab) n_frames = rtab[clip].n_frames;
     const int cw = n_coef < 128 ? n_coef : 128;        // coefficient lanes per pass
     const int groups = 128 / cw;
     const int tid = threadIdx.x;

@@ -38,6 +38,12 @@ def config_key(cfg: Any) -> tuple:
     )
 
 
+def config_struct(key: tuple, kernel: str = "auto") -> _lib.DspxConfig:
+    """struct dspx_config of a config_key tuple."""
+    sr, fl, hop, n_fft, n_mels, n_mfcc, f_min, f_max, pre, window = key
+    return _lib.DspxConfig(sr, fl, hop, n_fft, n_mels, n_mfcc, f_min, f_max, pre, _lib.WINDOWS[window], _lib.KERNELS[kernel])
+
+
 def current_device() -> int:
     """The CUDA device of this process (torch's current device when torch has CUDA up)."""
     try:
@@ -60,8 +66,7 @@ class Plan:
         if fl <= 0 or hop <= 0:
             raise ValueError("frame_length and hop_length must be positive")   # stft.py:29-30
         self.key, self.device, self.kernel_request = key, device, kernel
-        c = _lib.DspxConfig(sr, fl, hop, n_fft, n_mels, n_mfcc, f_min, f_max, pre, _lib.WINDOWS[window],
-                            _lib.KERNELS[kernel])
+        c = config_struct(key, kernel)
         handle = C.c_void_p()
         _lib.check(lib.dspx_plan_create(C.byref(c), device, C.byref(handle)), "dspx_plan_create")
         self._h = handle

@@ -17,7 +17,7 @@ from typing import Any, Iterable, List
 import numpy as np
 
 from . import _lib
-from .batch import _is_cuda_tensor, embed_stats, features_batch
+from .batch import _is_cuda_tensor, embed_stats, features_batch, features_ragged
 from .dsp.mfcc import MfccConfig
 
 
@@ -51,11 +51,8 @@ def _load_clips(items: List[Any], cfg: MfccConfig, loader) -> list:
     return clips
 
 
-def _by_length(arrays: list) -> dict:
-    groups: dict = {}
-    for i, a in enumerate(arrays):
-        groups.setdefault(a.shape, []).append(i)
-    return groups
+def _equal_shapes(arrays: list) -> bool:
+    return len({a.shape for a in arrays}) == 1
 
 
 def compute_embeddings(items: List[Any], cfg: MfccConfig, feature_cache=None, loader=None) -> np.ndarray:
@@ -63,9 +60,10 @@ def compute_embeddings(items: List[Any], cfg: MfccConfig, feature_cache=None, lo
 
     Reference signature (items, cfg, feature_cache=None); `loader(item) -> samples` optionally replaces the
     audio decoding.  Without a cache the clips are read from item.path (load_audio + normalize_audio
-    semantics) and clips of equal length go through the fused kernel as one batch.  With a cache the
-    float32 MFCCs come from it (any object with the reference's get_feature; BatchFeatureCache fills its
-    misses in GPU batches) and are reduced on the GPU -- the path scripts/tasks/run_retrieval.py takes.
+    semantics) and go through the fused kernel as one batch (one ragged launch when their lengths differ).
+    With a cache the float32 MFCCs come from it (any object with the reference's get_feature; BatchFeatureCache
+    fills its misses in GPU batches) and are reduced on the GPU in one launch -- the path
+    scripts/tasks/run_retrieval.py takes.
     """
     items = list(items)
     if not items:
@@ -76,15 +74,11 @@ def compute_embeddings(items: List[Any], cfg: MfccConfig, feature_cache=None, lo
         else:
             feats = [feature_cache.get_feature(item, "mfcc", cfg) for item in items]
         feats = [np.asarray(f, dtype=np.float32) for f in feats]
-        out = np.empty((len(items), 2 * feats[0].shape[1]), np.float32)
-        for shape, rows in _by_length(feats).items():
-            out[rows] = embed_stats(np.stack([feats[i] for i in rows], axis=0))
-        return out
+        return embed_stats(np.stack(feats, axis=0) if _equal_shapes(feats) else feats)
     clips = _load_clips(items, cfg, loader)
-    out = np.empty((len(items), 2 * cfg.n_mfcc), np.float32)
-    for shape, rows in _by_length(clips).items():
-        out[rows] = features_batch(np.stack([clips[i] for i in rows], axis=0), cfg, ("embed",))["embed"]
-    return out
+    if _equal_shapes(clips):
+        return features_batch(np.stack(clips, axis=0), cfg, ("embed",))["embed"]
+    return features_ragged(clips, cfg, ("embed",))["embed"]
 
 
 def _dev_matrix(x):

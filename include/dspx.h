@@ -172,6 +172,43 @@ int dspx_features_host_pcm16(const dspx_plan *plan, const int16_t *pcm_host, int
                              int64_t clip_len, int64_t pcm_stride, int normalize,
                              float *logmel_out_host, float *mfcc_out_host, float *embed_out_host);
 
+/* ---- ragged batches: clips of different lengths in one call ----
+ * The clips lie back to back in one flat buffer of float32 or int16 samples.  dspx_ragged_layout (host only, no
+ * device needed) validates their starts and lengths and fills one table row per clip; the outputs are the per-clip
+ * outputs of dspx_features stacked along the frame axis: logmel [total_frames, n_mels], mfcc [total_frames, n_mfcc],
+ * embed [n_clips, 2*n_mfcc]; clip i owns rows first_frame .. first_frame + n_frames - 1.  Every clip gets exactly
+ * the values dspx_features / dspx_features_pcm16 give it alone (pre-emphasis restarts at its sample 0). */
+#define DSPX_DTYPE_PCM16 2
+typedef struct dspx_ragged_clip {
+    int64_t start;        /* first sample of the clip in the flat buffer (samples of the buffer's type) */
+    int64_t length;       /* samples */
+    int64_t n_frames;     /* 1 + (length - frame_length) / hop_length */
+    int64_t first_frame;  /* row of its first frame in the [total_frames, ...] outputs */
+    int64_t first_pair;   /* exclusive prefix sum of (n_frames + 1) / 2 */
+} dspx_ragged_clip;
+/* Returns total_frames (>= 0), or DSPX_EINVAL naming the first clip shorter than frame_length, a float32 clip that
+ * starts at an odd sample, a negative start, or a batch of 2^31 frame pairs or more.  dtype: DSPX_DTYPE_F32 or
+ * DSPX_DTYPE_PCM16. */
+int64_t dspx_ragged_layout(const dspx_config *cfg, const int64_t *starts, const int64_t *lengths, int64_t n_clips,
+                           int dtype, dspx_ragged_clip *table_out);
+/* Device scratch for one dspx_features_ragged call with these outputs requested (flags 0 / 1). */
+size_t dspx_features_ragged_workspace(const dspx_plan *plan, const dspx_ragged_clip *table_host, int64_t n_clips,
+                                      int dtype, int normalize, int want_logmel, int want_mfcc, int want_embed);
+/* samples_dev: the flat buffer (float32: 8-byte aligned), dtype DSPX_DTYPE_F32 or DSPX_DTYPE_PCM16 (normalize as in
+ * dspx_features_pcm16).  table_dev and table_host hold the same dspx_ragged_layout table, on the device and on the
+ * host.  Any of the three outputs may be NULL.  Warp8 plans with n_fft 512 / 1024 / 2048 run one launch for the
+ * whole batch (with embed alone on aligned float32 frames, the fused embeddings of dspx_embeddings).  Plans without
+ * a ragged kernel (the generic kernel, n_fft 4096) loop over the clips on the host and enqueue one feature call per
+ * clip: correct, but as slow as one call per clip. */
+int dspx_features_ragged(const dspx_plan *plan, const void *samples_dev, int dtype, int normalize,
+                         const dspx_ragged_clip *table_dev, const dspx_ragged_clip *table_host, int64_t n_clips,
+                         int64_t total_frames, float *logmel_out_dev, float *mfcc_out_dev, float *embed_out_dev,
+                         void *workspace_dev, size_t workspace_bytes, void *stream);
+/* dspx_embed_stats over stacked features: feats [total_frames, n_coef], clip i = rows first_frame .. + n_frames;
+ * out [n_clips, 2*n_coef].  Same per-clip summation order as dspx_embed_stats. */
+int dspx_embed_stats_ragged(const float *feats_dev, const dspx_ragged_clip *table_dev, int64_t n_clips, int n_coef,
+                            float *out_dev, void *stream);
+
 /* ---- fft / ifft / rfft  src/dsp/fft.py:27-77 ----
  * in_dev [batch, n_in] interleaved complex64; the first min(n_in, n) samples are used,
  * zero-padded to P = next_pow2(n).  out_dev and work_dev each hold [batch, P] complex64.

@@ -3,8 +3,7 @@
 #include "../../dsp_final_b200/csrc/dspx_internal.cuh"
 #include "../../dsp_final_b200/csrc/tables.cuh"
 #include "../../dsp_final_b200/csrc/feat_warp8.cuh"
-namespace dspx { void set_error(const char*, ...) {} const char* get_error(){return "";}
-int launch_generic_fallback(const dspx_plan *, const float *, int64_t, int64_t, int64_t, int64_t, float *, float *, cudaStream_t, int){return -1;} }
+namespace dspx { void set_error(const char*, ...) {} const char* get_error(){return "";} }
 using namespace dspx;
 int main(){
   for (int P : {512,1024,2048}) for (int nm : {40,64,128}) {

@@ -26,12 +26,6 @@ void set_error(const char *fmt, ...)
     va_end(ap);
 }
 const char *get_error() { return g_err; }
-int launch_generic_fallback(const dspx_plan *, const float *, int64_t, int64_t, int64_t, int64_t, float *, float *,
-                            cudaStream_t, int)
-{
-    set_error("lab: generic fallback not built");
-    return DSPX_EUNSUPPORTED;
-}
 }  // namespace dspx
 
 __global__ void synth_kernel(float *x, int64_t n_clips, int64_t len)
@@ -83,13 +77,14 @@ int main(int argc, char **argv)
     CK(cudaMalloc(&cs, 16));
     synth_kernel<<<(unsigned)n_clips, 256>>>(clips, n_clips, len);
     CK(cudaDeviceSynchronize());
+    const W8Params p = w8_batch_params(&pl, clips, n_clips, len, T, mfcc_only ? nullptr : lm, mf, 0);
     for (int i = 0; i < 3; i++)
-        if (launch_warp8(&pl, clips, n_clips, len, len, T, mfcc_only ? nullptr : lm, mf, 0) != DSPX_OK) { printf("launch failed: %s\n", get_error()); return 1; }
+        if (launch_warp8(&pl, W8_SHARE, p, true, 0) != DSPX_OK) { printf("launch failed: %s\n", get_error()); return 1; }
     CK(cudaDeviceSynchronize());
     cudaEvent_t e0, e1;
     cudaEventCreate(&e0); cudaEventCreate(&e1);
     cudaEventRecord(e0);
-    for (int i = 0; i < reps; i++) launch_warp8(&pl, clips, n_clips, len, len, T, mfcc_only ? nullptr : lm, mf, 0);
+    for (int i = 0; i < reps; i++) launch_warp8(&pl, W8_SHARE, p, true, 0);
     cudaEventRecord(e1);
     CK(cudaDeviceSynchronize());
     float ms = 0;

@@ -60,6 +60,11 @@ def _is_pcm16(clips) -> bool:
     return dt is not None and str(dt) in ("int16", "torch.int16")
 
 
+def _ran(rc: int, what: str) -> bool:
+    """False when the entry point does not apply (DSPX_EUNSUPPORTED, nothing enqueued); raises on any other error."""
+    return rc != _lib.EUNSUPPORTED and _lib.check(rc, what) >= 0
+
+
 def pcm16_to_float(pcm, normalize: bool = True):
     """int16 PCM [B, L] on the GPU -> float32 [B, L]: x/32768, then x/max|x| (src/utils/audio.py:19-38)."""
     import torch
@@ -91,64 +96,54 @@ def features_batch(clips, cfg: Any, want: Iterable[str] = ("mfcc",), device: int
     if _is_cuda_tensor(clips):
         import torch
 
-        if _is_pcm16(clips):
-            pcm = clips if clips.dim() == 2 else clips[None, :]
-            pcm = pcm if pcm.stride(1) == 1 else pcm.contiguous()
-            dev = pcm.device.index if device is None else device
-            plan = get_plan(cfg, dev, kernel)
-            if plan.kernel == "warp8" and plan.n_fft != 4096:
-                # conversion and peak normalisation inside the feature kernel's loads: no float32 copy of the clips
-                b, length = pcm.shape
-                t = plan.num_frames(length)
-                need_mfcc = "mfcc" in want or "embed" in want
-                with torch.cuda.device(dev):
-                    lm = torch.empty((b, t, plan.n_mels), dtype=torch.float32, device=pcm.device) if "log_mel" in want else None
-                    mf = torch.empty((b, t, plan.n_mfcc), dtype=torch.float32, device=pcm.device) if need_mfcc else None
-                    em = torch.empty((b, 2 * plan.n_mfcc), dtype=torch.float32, device=pcm.device) if "embed" in want else None
-                    ws_bytes = int(lib.dspx_features_pcm16_workspace(b))
-                    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=pcm.device)
-                    _lib.check(lib.dspx_features_pcm16(plan.handle, pcm.data_ptr(), b, length, pcm.stride(0), 1 if normalize else 0,
-                                                       lm.data_ptr() if lm is not None else None,
-                                                       mf.data_ptr() if mf is not None else None,
-                                                       em.data_ptr() if em is not None else None, ws.data_ptr(), ws_bytes,
-                                                       torch.cuda.current_stream(dev).cuda_stream), "dspx_features_pcm16")
-                out = {}
-                if lm is not None:
-                    out["log_mel"] = lm
-                if "mfcc" in want:
-                    out["mfcc"] = mf
-                if em is not None:
-                    out["embed"] = em
-                return out
-            clips = pcm16_to_float(clips, normalize)
         x = clips if clips.dim() == 2 else clips[None, :]
-        if x.dtype != torch.float32 or x.stride(1) != 1:
+        pcm = _is_pcm16(x)
+        if pcm:
+            x = x if x.stride(1) == 1 else x.contiguous()
+        elif x.dtype != torch.float32 or x.stride(1) != 1:
             x = x.to(torch.float32).contiguous()
         dev = x.device.index if device is None else device
         plan = get_plan(cfg, dev, kernel)
         b, length = x.shape
         t = plan.num_frames(length)
-        # embeddings without MFCCs: accumulated inside the feature kernel (no [B, T, n_mfcc] tensor at all)
-        fused = ("embed" in want and "mfcc" not in want and plan.kernel == "warp8" and plan.n_fft != 4096
-                 and x.data_ptr() % 8 == 0 and x.stride(0) % 2 == 0 and plan.hop_length % 2 == 0)
-        need_mfcc = "mfcc" in want or ("embed" in want and not fused)
+
+        def new(*shape):
+            return torch.empty(shape, dtype=torch.float32, device=x.device)
+
+        def ptr(a):
+            return a.data_ptr() if a is not None else None
+
+        # The fused entry points return DSPX_EUNSUPPORTED, having enqueued nothing, where they do not apply (plan, batch
+        # size, alignment); dspx_features then computes the same values through an MFCC tensor.
         with torch.cuda.device(dev):
-            out = {}
-            lm = torch.empty((b, t, plan.n_mels), dtype=torch.float32, device=x.device) if "log_mel" in want else None
-            mf = torch.empty((b, t, plan.n_mfcc), dtype=torch.float32, device=x.device) if need_mfcc else None
-            em = torch.empty((b, 2 * plan.n_mfcc), dtype=torch.float32, device=x.device) if "embed" in want else None
             stream = torch.cuda.current_stream(dev).cuda_stream
-            if fused:
+            lm = new(b, t, plan.n_mels) if "log_mel" in want else None
+            mf = new(b, t, plan.n_mfcc) if "mfcc" in want else None
+            em = new(b, 2 * plan.n_mfcc) if "embed" in want else None
+            done = False
+            if pcm:
+                # conversion and peak normalisation inside the feature kernel's loads: no float32 copy of the clips
+                if em is not None and mf is None:
+                    mf = new(b, t, plan.n_mfcc)
+                ws_bytes = int(lib.dspx_features_pcm16_workspace(b))
+                ws = torch.empty(ws_bytes, dtype=torch.uint8, device=x.device)
+                done = _ran(lib.dspx_features_pcm16(plan.handle, x.data_ptr(), b, length, x.stride(0), 1 if normalize else 0,
+                                                    ptr(lm), ptr(mf), ptr(em), ws.data_ptr(), ws_bytes, stream),
+                            "dspx_features_pcm16")
+                if not done:
+                    x = pcm16_to_float(x, normalize)
+            elif em is not None and mf is None:
+                # embeddings without MFCCs: accumulated inside the feature kernel (no [B, T, n_mfcc] tensor at all)
                 ws_bytes = int(lib.dspx_embeddings_workspace(plan.handle, b))
                 ws = torch.empty(ws_bytes, dtype=torch.uint8, device=x.device)
-                _lib.check(lib.dspx_embeddings(plan.handle, x.data_ptr(), b, length, x.stride(0), em.data_ptr(),
-                                               lm.data_ptr() if lm is not None else None, ws.data_ptr(), ws_bytes, stream),
-                           "dspx_embeddings")
-            else:
-                _lib.check(lib.dspx_features(plan.handle, x.data_ptr(), b, length, x.stride(0),
-                                             lm.data_ptr() if lm is not None else None,
-                                             mf.data_ptr() if mf is not None else None,
-                                             em.data_ptr() if em is not None else None, stream), "dspx_features")
+                done = _ran(lib.dspx_embeddings(plan.handle, x.data_ptr(), b, length, x.stride(0), em.data_ptr(), ptr(lm),
+                                                ws.data_ptr(), ws_bytes, stream), "dspx_embeddings")
+            if not done:
+                if em is not None and mf is None:
+                    mf = new(b, t, plan.n_mfcc)
+                _lib.check(lib.dspx_features(plan.handle, x.data_ptr(), b, length, x.stride(0), ptr(lm), ptr(mf), ptr(em),
+                                             stream), "dspx_features")
+        out = {}
         if lm is not None:
             out["log_mel"] = lm
         if "mfcc" in want:

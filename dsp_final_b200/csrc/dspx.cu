@@ -3,6 +3,7 @@
 // kernels included below; this file only validates arguments and launches.
 #include <cstdarg>
 #include <cstddef>
+#include <cstdlib>
 #include <cstring>
 #include <mutex>
 #include <new>
@@ -171,11 +172,21 @@ static int launch_generic(const dspx_plan *pl, const float *clips, int64_t n_cli
     return DSPX_OK;
 }
 
-int launch_generic_fallback(const dspx_plan *pl, const float *clips, int64_t n_clips, int64_t clip_len,
-                            int64_t clip_stride, int64_t T, float *logmel, float *mfcc, cudaStream_t st, int nchw)
+// Features of an equal-length batch on the path warp8_select chose (PCM16: int16 rows, peaks per clip or null).
+static int launch_features(const dspx_plan *pl, W8Path path, const void *clips, int64_t n_clips, int64_t clip_len,
+                           int64_t clip_stride, int64_t T, float *logmel, float *mfcc, cudaStream_t st, int nchw = 0,
+                           long long *eacc = nullptr, const int *peaks = nullptr)
 {
-    return launch_generic(pl, clips, n_clips, clip_len, clip_stride, T, pl->take_feat,
-                          pl->cfg.pre_emphasis > 0.0 ? 1 : 0, logmel, mfcc, nullptr, st, nchw);
+    const bool pre = pl->cfg.pre_emphasis > 0.0;
+    const float *x = static_cast<const float *>(clips);
+    if (path == W8_GENERIC)
+        return launch_generic(pl, x, n_clips, clip_len, clip_stride, T, pl->take_feat, pre ? 1 : 0, logmel, mfcc, nullptr, st, nchw);
+    if (path == W8_X2 || path == W8_X2_AL4)
+        return launch_warp8_x2(pl, path == W8_X2_AL4, x, n_clips, clip_stride, T, logmel, mfcc, st, nchw);
+    W8Params p = w8_batch_params(pl, clips, n_clips, clip_stride, T, logmel, mfcc, nchw);
+    p.eacc = eacc;
+    p.peaks = peaks;
+    return launch_warp8(pl, path, p, pre, st);
 }
 
 static int launch_embed(const float *feats, int64_t n_clips, int64_t T, int C, float *out, cudaStream_t st,
@@ -199,31 +210,25 @@ static int features_device(const dspx_plan *pl, const float *clips, int64_t n_cl
 {
     const int64_t T = dspx_num_frames(pl, clip_len);
     if (T < 0) return DSPX_EINVAL;
-    int rc;
-    if (embed && !mfcc) {
-        if (!eacc || pl->kernel != DSPX_KERNEL_WARP8 || warp8_x2(pl) || !warp8_can_launch(clips, n_clips, clip_stride, T) ||
-            !warp8_aligned(pl, clips, clip_stride)) {
-            set_error("embeddings without an MFCC buffer need the warp8 kernel and 8-byte aligned clips with an even stride");
-            return DSPX_EUNSUPPORTED;
-        }
-        const int C = pl->cfg.n_mfcc;
-        DSPX_CUDA_CHECK(cudaMemsetAsync(eacc, 0, (size_t)n_clips * 2 * C * sizeof(long long), st));
-        rc = launch_warp8(pl, clips, n_clips, clip_len, clip_stride, T, logmel, nullptr, st, nchw, nullptr, 0, eacc);
-        if (rc != DSPX_OK) return rc;
+    const bool fused = embed && !mfcc;
+    const W8Path path = warp8_select(pl, clips, clip_stride, DSPX_DTYPE_F32, false, n_clips, T,
+                                     fused ? W8_WANT_EMBED : W8_WANT_FEATURES);
+    if (path == W8_UNSUPPORTED) {
+        set_error("embeddings without an MFCC buffer need the warp8 kernel (n_fft 512 / 1024 / 2048), frame_length = "
+                  "n_fft, an even hop and row stride and 8-byte aligned clips");
+        return DSPX_EUNSUPPORTED;
+    }
+    const int C = pl->cfg.n_mfcc;
+    if (fused) DSPX_CUDA_CHECK(cudaMemsetAsync(eacc, 0, (size_t)n_clips * 2 * C * sizeof(long long), st));
+    int rc = launch_features(pl, path, clips, n_clips, clip_len, clip_stride, T, logmel, mfcc, st, nchw, fused ? eacc : nullptr);
+    if (rc != DSPX_OK) return rc;
+    if (fused) {
         const int64_t total = n_clips * C;
         embed_finalize_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(eacc, n_clips, T, C, embed);
         DSPX_CUDA_CHECK(cudaGetLastError());
         return DSPX_OK;
     }
-    if (pl->kernel == DSPX_KERNEL_WARP8 && warp8_x2(pl))
-        rc = launch_warp8_x2(pl, clips, n_clips, clip_len, clip_stride, T, logmel, mfcc, st, nchw);
-    else if (pl->kernel == DSPX_KERNEL_WARP8)
-        rc = launch_warp8(pl, clips, n_clips, clip_len, clip_stride, T, logmel, mfcc, st, nchw);
-    else
-        rc = launch_generic(pl, clips, n_clips, clip_len, clip_stride, T, pl->take_feat,
-                            pl->cfg.pre_emphasis > 0.0 ? 1 : 0, logmel, mfcc, nullptr, st, nchw);
-    if (rc != DSPX_OK) return rc;
-    if (embed) rc = launch_embed(mfcc, n_clips, T, pl->cfg.n_mfcc, embed, st);
+    if (embed) rc = launch_embed(mfcc, n_clips, T, C, embed, st);
     return rc;
 }
 
@@ -234,8 +239,10 @@ static int features_device_pcm16(const dspx_plan *pl, const int16_t *pcm, int64_
 {
     const int64_t T = dspx_num_frames(pl, clip_len);
     if (T < 0) return DSPX_EINVAL;
-    if (pl->kernel != DSPX_KERNEL_WARP8 || warp8_x2(pl)) {
-        set_error("fused PCM16 ingest needs the warp8 kernel (n_fft 512 / 1024 / 2048): convert with dspx_pcm16_to_float first");
+    const W8Path path = warp8_select(pl, pcm, pcm_stride, DSPX_DTYPE_PCM16, false, n_clips, T, W8_WANT_FEATURES);
+    if (path == W8_UNSUPPORTED) {
+        set_error("fused PCM16 ingest needs the warp8 kernel (n_fft 512 / 1024 / 2048) and fewer than 2^31 frame pairs: "
+                  "convert with dspx_pcm16_to_float first");
         return DSPX_EUNSUPPORTED;
     }
     DSPX_REQUIRE(!embed || mfcc, "embed_out needs mfcc_out on the PCM16 path");
@@ -245,8 +252,8 @@ static int features_device_pcm16(const dspx_plan *pl, const int16_t *pcm, int64_
         pcm16_peak_kernel<<<(unsigned)n_clips, 256, 0, st>>>(pcm, clip_len, pcm_stride, peaks_ws);
         DSPX_CUDA_CHECK(cudaGetLastError());
     }
-    int rc = launch_warp8(pl, reinterpret_cast<const float *>(pcm), n_clips, clip_len, pcm_stride, T, logmel, mfcc, st, 0,
-                          nullptr, 0, nullptr, 1, normalize ? peaks_ws : nullptr);
+    int rc = launch_features(pl, path, pcm, n_clips, clip_len, pcm_stride, T, logmel, mfcc, st, 0, nullptr,
+                             normalize ? peaks_ws : nullptr);
     if (rc != DSPX_OK) return rc;
     if (embed) rc = launch_embed(mfcc, n_clips, T, pl->cfg.n_mfcc, embed, st);
     return rc;
@@ -256,10 +263,12 @@ static int features_device_pcm16(const dspx_plan *pl, const int16_t *pcm, int64_
 static int stft_device(const dspx_plan *pl, const float *clips, int64_t n_clips, int64_t clip_len, int64_t clip_stride,
                        int64_t T, int pre, float2 *out, cudaStream_t st)
 {
-    if (pl->kernel == DSPX_KERNEL_WARP8 && !warp8_x2(pl) && pl->take_stft == pl->P &&
-        warp8_can_launch(clips, n_clips, clip_stride, T) && warp8_aligned(pl, clips, clip_stride))
-        return launch_warp8(pl, clips, n_clips, clip_len, clip_stride, T, nullptr, nullptr, st, 0, out, pre);
-    return launch_generic(pl, clips, n_clips, clip_len, clip_stride, T, pl->take_stft, pre, nullptr, nullptr, out, st);
+    const W8Path path = warp8_select(pl, clips, clip_stride, DSPX_DTYPE_F32, false, n_clips, T, W8_WANT_STFT);
+    if (path == W8_GENERIC)
+        return launch_generic(pl, clips, n_clips, clip_len, clip_stride, T, pl->take_stft, pre, nullptr, nullptr, out, st);
+    W8Params p = w8_batch_params(pl, clips, n_clips, clip_stride, T, nullptr, nullptr, 0);
+    p.stft = out;
+    return launch_warp8(pl, path, p, pre != 0, st);
 }
 
 // ---- ragged batches (dspx_features_ragged) ------------------------------------------------------------
@@ -275,13 +284,16 @@ struct RaggedWs {
     float *f32 = nullptr;
 };
 
-static bool ragged_kernel(const dspx_plan *pl) { return pl->kernel == DSPX_KERNEL_WARP8 && !warp8_x2(pl); }
+static W8Path ragged_path(const dspx_plan *pl, int dtype, W8Want want)
+{
+    return warp8_select(pl, nullptr, 0, dtype, true, 0, 0, want);
+}
 
 static size_t ragged_ws_carve(const dspx_plan *pl, const dspx_ragged_clip *tab, int64_t n_clips, int dtype, int normalize,
                               bool want_mfcc, bool want_embed, char *base, RaggedWs *ws)
 {
-    const bool pcm = dtype == DSPX_DTYPE_PCM16, rk = ragged_kernel(pl);
-    const bool fused = want_embed && !want_mfcc && rk && warp8_ragged_aligned(pl, pcm);
+    const bool pcm = dtype == DSPX_DTYPE_PCM16, rk = ragged_path(pl, dtype, W8_WANT_FEATURES) != W8_UNSUPPORTED;
+    const bool fused = want_embed && !want_mfcc && ragged_path(pl, dtype, W8_WANT_EMBED) != W8_UNSUPPORTED;
     int64_t total_frames = 0, max_len = 0;
     if (n_clips > 0) total_frames = tab[n_clips - 1].first_frame + tab[n_clips - 1].n_frames;
     for (int64_t i = 0; i < n_clips; i++) max_len = std::max(max_len, tab[i].length);
@@ -336,7 +348,9 @@ static int features_ragged(const dspx_plan *pl, const void *samples, int dtype, 
     const int pcm = dtype == DSPX_DTYPE_PCM16 ? 1 : 0;
     RaggedWs ws;
     ragged_ws_carve(pl, tab, n_clips, dtype, normalize, mfcc != nullptr, embed != nullptr, ws_base, &ws);
-    if (!ragged_kernel(pl))
+    const bool fused = ws.eacc != nullptr;                   // embeddings alone, accumulated inside the feature kernel
+    const W8Path path = ragged_path(pl, dtype, fused ? W8_WANT_EMBED : W8_WANT_FEATURES);
+    if (path == W8_UNSUPPORTED)
         return features_ragged_per_clip(pl, samples, pcm, normalize, tab_dev, tab, n_clips, logmel, mfcc, embed, ws, st);
     const int C = pl->cfg.n_mfcc;
     const uint32_t n_items = (uint32_t)(tab[n_clips - 1].first_pair + (tab[n_clips - 1].n_frames + 1) / 2);
@@ -346,19 +360,22 @@ static int features_ragged(const dspx_plan *pl, const void *samples, int dtype, 
         pcm16_peak_kernel<<<(unsigned)n_clips, 256, 0, st>>>(static_cast<const int16_t *>(samples), 0, 0, ws.peaks, tab_dev);
         DSPX_CUDA_CHECK(cudaGetLastError());
     }
-    if (ws.eacc) {                                   // embeddings alone, accumulated inside the feature kernel
-        DSPX_CUDA_CHECK(cudaMemsetAsync(ws.eacc, 0, (size_t)n_clips * 2 * C * sizeof(long long), st));
-        int rc = launch_warp8_ragged(pl, samples, pcm, tab_dev, ws.rpairs, n_clips, n_items, logmel, nullptr, ws.eacc,
-                                     nullptr, st);
-        if (rc != DSPX_OK) return rc;
+    if (fused) DSPX_CUDA_CHECK(cudaMemsetAsync(ws.eacc, 0, (size_t)n_clips * 2 * C * sizeof(long long), st));
+    float *mf = mfcc ? mfcc : ws.mfcc;                      // ws.mfcc: scratch for embeddings that are not fused, else null
+    W8Params p = w8_batch_params(pl, samples, n_clips, 0, 0, logmel, mf, 0);
+    p.rtab = tab_dev;
+    p.rpairs = ws.rpairs;
+    p.n_items = n_items;
+    p.eacc = ws.eacc;
+    p.peaks = ws.peaks;
+    int rc = launch_warp8(pl, path, p, pl->cfg.pre_emphasis > 0.0, st);
+    if (rc != DSPX_OK) return rc;
+    if (fused) {
         const int64_t total = n_clips * C;
         embed_finalize_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(ws.eacc, n_clips, 1, C, embed, tab_dev);
         DSPX_CUDA_CHECK(cudaGetLastError());
         return DSPX_OK;
     }
-    float *mf = mfcc ? mfcc : (embed ? ws.mfcc : nullptr);
-    int rc = launch_warp8_ragged(pl, samples, pcm, tab_dev, ws.rpairs, n_clips, n_items, logmel, mf, nullptr, ws.peaks, st);
-    if (rc != DSPX_OK) return rc;
     return embed ? launch_embed(mf, n_clips, 1, C, embed, st, tab_dev) : DSPX_OK;
 }
 
@@ -465,21 +482,24 @@ static int host_pipeline(dspx_plan *pl, int mode, const void *clips_v, int64_t n
     if (!guard.ok) { set_error("cudaSetDevice(%d) failed", pl->device); return DSPX_ECUDA; }
     const size_t clip_bytes = (size_t)clip_len * elem;
     const size_t lm_b = (mode == 0 && o_logmel) ? (size_t)T * pl->cfg.n_mels * 4 : 0;
-    // embeddings alone: accumulated inside the feature kernel (16 bytes of scratch per coefficient instead of an
-    // MFCC tensor); otherwise they are the statistics of the MFCCs that are written anyway
-    const bool fused_embed = mode == 0 && elem == 4 && o_embed && !o_mfcc && pl->kernel == DSPX_KERNEL_WARP8 && !warp8_x2(pl) &&
-                             !(clip_len & 1) && !(pl->cfg.hop_length & 1);
+    // chunk: ~48 MiB of input or ~96 MiB of output, whichever is hit first
+    int64_t chunk = std::min<int64_t>(n_clips, (int64_t)((48u << 20) / (clip_bytes ? clip_bytes : 1)));
+    if (chunk < 1) chunk = 1;
+    // the kernels read a chunk's device copy: rows of clip_len samples in a cudaMalloc'd, so aligned, buffer (the null
+    // pointer below)
+    const int dtype = elem == 2 ? DSPX_DTYPE_PCM16 : DSPX_DTYPE_F32;
+    // embeddings alone: accumulated inside the feature kernel when it can (16 bytes of scratch per coefficient instead
+    // of an MFCC tensor); otherwise they are the statistics of the MFCCs that are written anyway
+    const bool fused_embed = mode == 0 && o_embed && !o_mfcc &&
+                             warp8_select(pl, nullptr, clip_len, dtype, false, chunk, T, W8_WANT_EMBED) != W8_UNSUPPORTED;
     const bool need_mfcc = mode == 0 && (o_mfcc || (o_embed && !fused_embed));
     const size_t mf_b = need_mfcc ? (size_t)T * pl->cfg.n_mfcc * 4 : (fused_embed ? (size_t)pl->cfg.n_mfcc * 16 : 0);
     const size_t em_b = (mode == 0 && o_embed) ? (size_t)2 * pl->cfg.n_mfcc * 4 : 0;
     const size_t st_b = mode == 1 ? (size_t)T * pl->n_bins * 8 : 0;
     const size_t out_per_clip = lm_b + mf_b + em_b + st_b;
-    // chunk: ~48 MiB of input or ~96 MiB of output, whichever is hit first
-    int64_t chunk = (int64_t)((48u << 20) / (clip_bytes ? clip_bytes : 1));
     const int64_t chunk_o = (int64_t)((96u << 20) / (out_per_clip ? out_per_clip : 1));
     if (chunk_o < chunk) chunk = chunk_o;
     if (chunk < 1) chunk = 1;
-    if (chunk > n_clips) chunk = n_clips;
     const bool in_pinned = is_pinned(clips);
     const bool out_pinned = is_pinned(o_logmel) && is_pinned(o_mfcc) && is_pinned(o_embed) && is_pinned(o_stft);
     const size_t off_mf = align256(lm_b * chunk), off_em = off_mf + align256(mf_b * chunk);
@@ -490,9 +510,10 @@ static int host_pipeline(dspx_plan *pl, int mode, const void *clips_v, int64_t n
     HostPipe *hp = static_cast<HostPipe *>(pl->host_pipe);
     DSPX_REQUIRE(hp, "plan has no host pipeline state");
     std::lock_guard<std::mutex> lock(hp->mu);
-    // PCM16 on a warp8 plan: the feature kernel converts in its own loads (no float32 copy of the clips); the scratch
-    // buffer then only holds one int per clip.  Other plans convert first (pcm16_to_float_kernel) and need the copy.
-    const bool fused_pcm = elem == 2 && mode == 0 && pl->kernel == DSPX_KERNEL_WARP8 && !warp8_x2(pl);
+    // PCM16: the feature kernel converts in its own loads when it can (no float32 copy of the clips); the scratch
+    // buffer then only holds one int per clip.  Otherwise pcm16_to_float_kernel converts first and needs the copy.
+    const bool fused_pcm = elem == 2 && mode == 0 &&
+                           warp8_select(pl, nullptr, clip_len, dtype, false, chunk, T, W8_WANT_FEATURES) != W8_UNSUPPORTED;
     int rc = ensure_pipe(pl, clip_bytes * chunk, out_bytes, !in_pinned, !out_pinned, &hp,
                          elem == 2 ? (fused_pcm ? (size_t)chunk * sizeof(int) : (size_t)clip_len * 4 * chunk) : 0);
     if (rc != DSPX_OK) return rc;

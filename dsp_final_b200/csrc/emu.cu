@@ -9,7 +9,7 @@
 // path.
 #include <vector>
 
-#define DSPX_EMU                     // no ragged launcher: its 88 kernel instantiations are not replayed here
+#define DSPX_EMU                     // no launchers, so no feature-kernel instantiations: only their phase functions run here
 #include "dspx_internal.cuh"
 #include "tables.cuh"
 #include "feat_generic.cuh"
@@ -233,15 +233,18 @@ static int emu_warp8(const dspx_config *cfg, const float *clips, int64_t n_clips
     pl.M = e.M;
     pl.n_bins = e.n_bins;
     pl.host = e.t;
+    pl.take_stft = e.take_stft;
+    pl.kernel = DSPX_KERNEL_WARP8;
     if (!warp8_supported(&pl) || (!rtab && clip_len < cfg->frame_length)) return DSPX_EUNSUPPORTED;
-    // frames off the 8-byte grid replay the 4-byte-load variant, like launch_warp8 picks it
-    const bool u4 = (!rtab && (clip_stride & 1)) || (cfg->hop_length & 1) || (reinterpret_cast<uintptr_t>(clips) & 7) ||
-                    cfg->frame_length != e.P;
-    if (u4 && stft_out) return DSPX_EUNSUPPORTED;
+    const int64_t T = rtab ? 0 : 1 + (clip_len - cfg->frame_length) / cfg->hop_length;
+    // the variant the library would launch
+    const W8Path path = warp8_select(&pl, clips, clip_stride, DSPX_DTYPE_F32, rtab != nullptr, n_clips, T,
+                                     stft_out ? W8_WANT_STFT : W8_WANT_FEATURES);
+    if (path == W8_GENERIC || path == W8_UNSUPPORTED) return DSPX_EUNSUPPORTED;
+    const bool u4 = path == W8_U4, share = path == W8_SHARE;
     std::vector<float> blob;
     W8Tables tb{};
     warp8_build_tables(&pl, blob, tb);
-    const int64_t T = rtab ? 0 : 1 + (clip_len - cfg->frame_length) / cfg->hop_length;
     W8Params p{};
     p.clips = clips;
     p.n_clips = n_clips;
@@ -251,7 +254,6 @@ static int emu_warp8(const dspx_config *cfg, const float *clips, int64_t n_clips
     p.n_items = (uint32_t)(n_clips * p.pairs_per_clip);
     std::vector<uint32_t> rpairs;
     if (rtab) {
-        if (tb.x2 || stft_out) return DSPX_EUNSUPPORTED;
         for (int64_t i = 0; i < n_clips; i++) rpairs.push_back((uint32_t)rtab[i].first_pair);
         rpairs.push_back(n_clips ? (uint32_t)(rtab[n_clips - 1].first_pair + (rtab[n_clips - 1].n_frames + 1) / 2) : 0);
         p.rtab = rtab;
@@ -290,10 +292,9 @@ static int emu_warp8(const dspx_config *cfg, const float *clips, int64_t n_clips
     const int units = r1 >= 8 ? r1 / 8 : 1;
     if (tb.x2) {
         // n_fft 4096 (feat_warp8_x2.cuh): one frame per item, the same phase order as feat_warp8_x2_kernel
-        if (stft_out) return DSPX_EUNSUPPORTED;
         p.pairs_per_clip = (uint32_t)T;
         p.n_items = (uint32_t)(n_clips * T);
-        const bool al4 = cfg->frame_length >= e.P && !(cfg->hop_length & 3) && !(clip_stride & 3) && !(reinterpret_cast<uintptr_t>(clips) & 15);
+        const bool al4 = path == W8_X2_AL4;
         std::vector<W8Power4> pw4(32 * 2);
         for (uint32_t item = 0; item < p.n_items; item++) {
             w8x2_set_item(p, c, item);
@@ -329,7 +330,6 @@ static int emu_warp8(const dspx_config *cfg, const float *clips, int64_t n_clips
         if (rtab) w8_set_item<false, true>(p, c, item);
         else w8_set_item(p, c, item);
         for (int lane = 0; lane < 32; lane++) {
-            const bool share = 2 * cfg->hop_length == e.P && r1 != 16 && !u4;
             if (r1 == 4 && share) { if (pre) W8_P1(4, true, true); else W8_P1(4, false, true); }
             else if (r1 == 4) { if (pre) W8_P1(4, true, false); else W8_P1(4, false, false); }
             else if (r1 == 8 && share) { if (pre) W8_P1(8, true, true); else W8_P1(8, false, true); }

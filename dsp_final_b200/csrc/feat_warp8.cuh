@@ -27,7 +27,6 @@
 #pragma once
 
 #include <algorithm>
-#include <cstdlib>
 
 #include "dspx_internal.cuh"
 
@@ -1101,6 +1100,51 @@ inline bool warp8_supported(const dspx_plan *pl)
            pl->cfg.n_mels <= 256 && pl->cfg.n_mfcc <= 128 && pl->host.two_band_ok;
 }
 
+// ---- which kernel runs a call ------------------------------------------------------------------------------------
+// What the call asks for: log-mel / MFCC, embeddings without an MFCC output (accumulated inside the kernel, EMB), or
+// the complex STFT.
+enum W8Want { W8_WANT_FEATURES, W8_WANT_EMBED, W8_WANT_STFT };
+
+enum W8Path {
+    W8_GENERIC,       // feat_generic_kernel
+    W8_X2,            // feat_warp8_x2_kernel (n_fft 4096)
+    W8_X2_AL4,        //   with 16-byte loads: frame_length >= n_fft, hop and row stride multiples of 4, 16-byte aligned base
+    W8_ALIGNED,       // feat_warp8_kernel with 8-byte loads: frame_length = n_fft, every frame on the 8-byte grid
+    W8_SHARE,         //   and the two frames of a pair share rows: hop = n_fft / 2 (not at radix 16, whose 24 distinct
+                      //   rows in flight would not fit its register budget)
+    W8_U4,            // feat_warp8_kernel with 4-byte loads: frames off the 8-byte grid or shorter than n_fft
+    W8_PCM16,         // feat_warp8_kernel on int16 samples (4-byte loads, conversion in the loads)
+    W8_UNSUPPORTED,   // no kernel does this: the entry point returns DSPX_EUNSUPPORTED before it enqueues anything
+};
+
+// The one place that picks the kernel of a call.  samples, row_stride (in samples of `dtype`), n_clips and T (frames
+// per clip) describe an equal-length batch; a ragged batch ignores them: its layout holds fewer than 2^31 frame pairs
+// and starts float32 clips on the 8-byte grid (dspx_ragged_layout, dspx_features_ragged).  A ragged batch on a plan
+// without a ragged kernel (the generic kernel, n_fft 4096) gets W8_UNSUPPORTED and runs one clip at a time.
+inline W8Path warp8_select(const dspx_plan *pl, const void *samples, int64_t row_stride, int dtype, bool ragged,
+                           int64_t n_clips, int64_t T, W8Want want)
+{
+    const bool pcm = dtype == DSPX_DTYPE_PCM16, warp8 = pl->kernel == DSPX_KERNEL_WARP8 && !warp8_x2(pl);
+    if (ragged && (!warp8 || want == W8_WANT_STFT)) return W8_UNSUPPORTED;        // the RAGGED variants have no STFT mode
+    if (!warp8) {
+        if (pcm || want == W8_WANT_EMBED) return W8_UNSUPPORTED;
+        // x2 items are single frames, 32-bit
+        if (pl->kernel != DSPX_KERNEL_WARP8 || want == W8_WANT_STFT || n_clips * T >= (int64_t)0x7fffffff) return W8_GENERIC;
+        const bool al4 = pl->cfg.frame_length >= pl->P && !(pl->cfg.hop_length & 3) && !(row_stride & 3) &&
+                         !(reinterpret_cast<uintptr_t>(samples) & 15);
+        return al4 ? W8_X2_AL4 : W8_X2;
+    }
+    const bool fits = ragged || n_clips * ((T + 1) / 2) < (int64_t)0x7fffffff;      // items are 32-bit frame pairs
+    if (pcm) return fits && want == W8_WANT_FEATURES ? W8_PCM16 : W8_UNSUPPORTED;
+    // frames on the 8-byte grid: even hop, even row stride, 8-byte aligned base
+    const bool aligned = fits && pl->cfg.frame_length == pl->P && !(pl->cfg.hop_length & 1) &&
+                         (ragged || (!(row_stride & 1) && !(reinterpret_cast<uintptr_t>(samples) & 7)));
+    const W8Path fast = 2 * pl->cfg.hop_length == pl->P && warp8_radix(pl) != 16 ? W8_SHARE : W8_ALIGNED;
+    if (want == W8_WANT_EMBED) return aligned ? fast : W8_UNSUPPORTED;
+    if (want == W8_WANT_STFT) return aligned && pl->take_stft == pl->P ? fast : W8_GENERIC;
+    return aligned ? fast : (fits ? W8_U4 : W8_GENERIC);
+}
+
 
 // ---- bank-conflict-free table layouts (host side) -------------------------------------------------------
 // 64-bit shared-memory accesses are served per half-warp, one wavefront per set of lanes that touch 16 different
@@ -1471,7 +1515,8 @@ inline size_t warp8_smem_bytes(const W8Tables &tb, int n_mels, int n_warps = W8_
     return ((size_t)tb.total + (size_t)n_warps * w8_warp_floats(tb, n_mels)) * sizeof(float);
 }
 
-#if defined(__CUDACC__)
+// ---- launch (not in csrc/emu.cu, which replays the phase functions on the host and instantiates no kernel) --------
+#if defined(__CUDACC__) && !defined(DSPX_EMU)
 struct W8PlanData {
     W8Tables tb;
     int ctas_per_sm;
@@ -1479,7 +1524,6 @@ struct W8PlanData {
     size_t smem_wide;        // 0 when the 20-warp configuration does not fit
     size_t smem_mid;         // shared memory of the W8_WARPS_MID-warp configuration (used when the wide one does not fit), or 0
     size_t smem_r16;         // n_fft 2048: shared memory of the W8_WARPS_R16-warp configuration, 0 when it does not fit
-    bool share;              // hop == n_fft / 2: the two frames of a pair share rows (DSPX_W8_NOSHARE=1 at plan creation disables)
 };
 
 inline int warp8_prepare(dspx_plan *pl)
@@ -1494,12 +1538,11 @@ inline int warp8_prepare(dspx_plan *pl)
     pd->smem = smem;
     pd->ctas_per_sm = (tb.r1 != 16 && smem * 2 + 2048 <= 227 * 1024) ? 2 : 1;   // (x2 plans have r1 = 16: one CTA)
     const size_t wide = warp8_smem_bytes(tb, pl->cfg.n_mels, W8_WARPS_WIDE);
-    pd->smem_wide = (tb.r1 != 16 && wide + 1024 <= 227 * 1024 && !getenv("DSPX_W8_NARROW")) ? wide : 0;
+    pd->smem_wide = (tb.r1 != 16 && wide + 1024 <= 227 * 1024) ? wide : 0;
     const size_t mid = warp8_smem_bytes(tb, pl->cfg.n_mels, W8_WARPS_MID);
-    pd->smem_mid = (tb.r1 != 16 && !pd->smem_wide && pd->ctas_per_sm == 1 && mid + 1024 <= 227 * 1024 && !getenv("DSPX_W8_NARROW")) ? mid : 0;
+    pd->smem_mid = (tb.r1 != 16 && !pd->smem_wide && pd->ctas_per_sm == 1 && mid + 1024 <= 227 * 1024) ? mid : 0;
     const size_t r16 = warp8_smem_bytes(tb, pl->cfg.n_mels, W8_WARPS_R16);
     pd->smem_r16 = (tb.r1 == 16 && !tb.x2 && W8_WARPS_R16 > W8_WARPS && r16 + 1024 <= 227 * 1024) ? r16 : 0;
-    pd->share = (2 * pl->cfg.hop_length == pl->P) && pl->cfg.frame_length == pl->P && !getenv("DSPX_W8_NOSHARE");
     pl->fast_host = pd;
     DSPX_CUDA_CHECK(cudaMalloc(&pl->d_fast_tables, blob.size() * sizeof(float)));
     DSPX_CUDA_CHECK(cudaMemcpy(pl->d_fast_tables, blob.data(), blob.size() * sizeof(float), cudaMemcpyHostToDevice));
@@ -1513,102 +1556,6 @@ inline void warp8_release(dspx_plan *pl)
     pl->fast_host = nullptr;
 }
 
-int launch_generic_fallback(const dspx_plan *pl, const float *clips, int64_t n_clips, int64_t clip_len,
-                            int64_t clip_stride, int64_t T, float *logmel, float *mfcc, cudaStream_t st, int nchw);
-
-template <int R1, bool PRE, bool STFT, bool SHARE, int NW, bool EMB = false, bool U4 = false, bool PCM = false,
-          bool RAGGED = false>
-inline int w8_launch_nw(const W8Params &p, size_t smem, int device, int64_t ctas, cudaStream_t st)
-{
-    static std::atomic<unsigned char> optin[64];
-    DSPX_CUDA_CHECK(optin_max_smem(feat_warp8_kernel<R1, PRE, STFT, SHARE, NW, EMB, U4, PCM, RAGGED>, optin, device));
-    feat_warp8_kernel<R1, PRE, STFT, SHARE, NW, EMB, U4, PCM, RAGGED><<<(unsigned)ctas, NW * 32, smem, st>>>(p);
-    DSPX_CUDA_CHECK(cudaGetLastError());
-    return DSPX_OK;
-}
-
-template <int R1, bool PRE, bool STFT, bool SHARE, bool RAGGED = false>
-inline int w8_launch_cfg(const W8Params &p, const W8PlanData *pd, int device, int sm_count, cudaStream_t st)
-{
-    // persistent grid: warps stride over the items
-    if (!STFT && R1 != 16 && pd->smem_wide) {
-        int64_t ctas = ((int64_t)p.n_items + W8_WARPS_WIDE - 1) / W8_WARPS_WIDE;
-        if (ctas > sm_count) ctas = sm_count;
-        constexpr int NWW = (R1 != 16 && !STFT) ? W8_WARPS_WIDE : W8_WARPS;
-        if (!STFT && p.eacc) return w8_launch_nw<R1, PRE, STFT, SHARE, NWW, !STFT, false, false, RAGGED>(p, pd->smem_wide, device, ctas, st);
-        return w8_launch_nw<R1, PRE, STFT, SHARE, NWW, false, false, false, RAGGED>(p, pd->smem_wide, device, ctas, st);
-    }
-    if (!STFT && R1 != 16 && pd->smem_mid) {
-        int64_t ctas = ((int64_t)p.n_items + W8_WARPS_MID - 1) / W8_WARPS_MID;
-        if (ctas > sm_count) ctas = sm_count;
-        constexpr int NWM = (R1 != 16 && !STFT) ? W8_WARPS_MID : W8_WARPS;
-        if (!STFT && p.eacc) return w8_launch_nw<R1, PRE, STFT, SHARE, NWM, !STFT, false, false, RAGGED>(p, pd->smem_mid, device, ctas, st);
-        return w8_launch_nw<R1, PRE, STFT, SHARE, NWM, false, false, false, RAGGED>(p, pd->smem_mid, device, ctas, st);
-    }
-    if (!STFT && R1 == 16 && pd->smem_r16) {
-        int64_t ctas = ((int64_t)p.n_items + W8_WARPS_R16 - 1) / W8_WARPS_R16;
-        if (ctas > sm_count) ctas = sm_count;
-        constexpr int NWR = (R1 == 16 && !STFT) ? W8_WARPS_R16 : W8_WARPS;
-        if (p.eacc) return w8_launch_nw<R1, PRE, STFT, SHARE, NWR, !STFT, false, false, RAGGED>(p, pd->smem_r16, device, ctas, st);
-        return w8_launch_nw<R1, PRE, STFT, SHARE, NWR, false, false, false, RAGGED>(p, pd->smem_r16, device, ctas, st);
-    }
-    int64_t ctas = ((int64_t)p.n_items + W8_WARPS - 1) / W8_WARPS;
-    const int64_t resident = (int64_t)sm_count * pd->ctas_per_sm;
-    if (ctas > resident) ctas = resident;
-    if (!STFT && p.eacc) return w8_launch_nw<R1, PRE, STFT, SHARE, W8_WARPS, !STFT, false, false, RAGGED>(p, pd->smem, device, ctas, st);
-    return w8_launch_nw<R1, PRE, STFT, SHARE, W8_WARPS, false, false, false, RAGGED>(p, pd->smem, device, ctas, st);
-}
-
-// features from frames that are not 8-byte aligned: 4-byte sample loads, no row sharing, no fused embeddings
-template <int R1, bool PRE, bool PCM = false, bool RAGGED = false>
-inline int w8_launch_u4(const W8Params &p, const W8PlanData *pd, int device, int sm_count, cudaStream_t st)
-{
-    if (R1 != 16 && pd->smem_wide) {
-        int64_t ctas = ((int64_t)p.n_items + W8_WARPS_WIDE - 1) / W8_WARPS_WIDE;
-        if (ctas > sm_count) ctas = sm_count;
-        return w8_launch_nw<R1, PRE, false, false, (R1 != 16) ? W8_WARPS_WIDE : W8_WARPS, false, true, PCM, RAGGED>(p, pd->smem_wide, device, ctas, st);
-    }
-    if (R1 != 16 && pd->smem_mid) {
-        int64_t ctas = ((int64_t)p.n_items + W8_WARPS_MID - 1) / W8_WARPS_MID;
-        if (ctas > sm_count) ctas = sm_count;
-        return w8_launch_nw<R1, PRE, false, false, (R1 != 16) ? W8_WARPS_MID : W8_WARPS, false, true, PCM, RAGGED>(p, pd->smem_mid, device, ctas, st);
-    }
-    if (R1 == 16 && pd->smem_r16) {
-        int64_t ctas = ((int64_t)p.n_items + W8_WARPS_R16 - 1) / W8_WARPS_R16;
-        if (ctas > sm_count) ctas = sm_count;
-        return w8_launch_nw<R1, PRE, false, false, (R1 == 16) ? W8_WARPS_R16 : W8_WARPS, false, true, PCM, RAGGED>(p, pd->smem_r16, device, ctas, st);
-    }
-    int64_t ctas = ((int64_t)p.n_items + W8_WARPS - 1) / W8_WARPS;
-    const int64_t resident = (int64_t)sm_count * pd->ctas_per_sm;
-    if (ctas > resident) ctas = resident;
-    return w8_launch_nw<R1, PRE, false, false, W8_WARPS, false, true, PCM, RAGGED>(p, pd->smem, device, ctas, st);
-}
-
-template <int R1, bool PRE, bool STFT, bool RAGGED = false>
-inline int w8_launch_one(const W8Params &p, const W8PlanData *pd, int device, int sm_count, cudaStream_t st)
-{
-    // rows are shared between the two frames of a pair when hop == n_fft / 2 (R1 = 16 keeps the plain loads:
-    // 24 distinct rows in flight would not fit its register budget)
-    if (R1 != 16 && p.share) return w8_launch_cfg<R1, PRE, STFT, (R1 != 16), RAGGED>(p, pd, device, sm_count, st);
-    return w8_launch_cfg<R1, PRE, STFT, false, RAGGED>(p, pd, device, sm_count, st);
-}
-
-// items are 32-bit
-inline bool warp8_can_launch(const float *clips, int64_t n_clips, int64_t clip_stride, int64_t T)
-{
-    (void)clips;
-    (void)clip_stride;
-    return n_clips * ((T + 1) / 2) < (int64_t)0x7fffffff;
-}
-
-// 8-byte vector loads (and with them row sharing, the STFT mode and the fused embeddings) need every frame to start on
-// an 8-byte boundary: even hop, even row stride, aligned base
-inline bool warp8_aligned(const dspx_plan *pl, const float *clips, int64_t clip_stride)
-{
-    return pl->cfg.frame_length == pl->P && !(pl->cfg.hop_length & 1) && !(clip_stride & 1) &&
-           !(reinterpret_cast<uintptr_t>(clips) & 7);
-}
-
 // the launch fields that come from the plan alone
 inline W8Params w8_plan_params(const dspx_plan *pl)
 {
@@ -1619,7 +1566,6 @@ inline W8Params w8_plan_params(const dspx_plan *pl)
     p.n_mfcc = pl->cfg.n_mfcc;
     p.prefetch = 1;
     p.take = std::min(pl->cfg.frame_length, pl->P);
-    p.share = pd->share;
     p.alpha = (float)pl->cfg.pre_emphasis;
     p.win_a = pl->cfg.window == DSPX_WINDOW_HANN ? 0.25f : (pl->cfg.window == DSPX_WINDOW_HAMMING ? 0.27f : 0.5f);
     p.win_b = pl->cfg.window == DSPX_WINDOW_HANN ? -0.25f : (pl->cfg.window == DSPX_WINDOW_HAMMING ? -0.23f : 0.f);
@@ -1628,25 +1574,14 @@ inline W8Params w8_plan_params(const dspx_plan *pl)
     return p;
 }
 
-inline int launch_warp8(const dspx_plan *pl, const float *clips, int64_t n_clips, int64_t clip_len,
-                        int64_t clip_stride, int64_t T, float *logmel, float *mfcc, cudaStream_t st, int nchw = 0,
-                        float2 *stft = nullptr, int stft_pre = 0, long long *eacc = nullptr, int pcm = 0,
-                        const int *peaks = nullptr)
+// ... and those of an equal-length batch: n_clips rows of clip_stride samples, T frames each, one frame pair per item.
+// A ragged batch sets rtab, rpairs and n_items on top.
+inline W8Params w8_batch_params(const dspx_plan *pl, const void *samples, int64_t n_clips, int64_t clip_stride, int64_t T,
+                                float *logmel, float *mfcc, int nchw)
 {
-    const int64_t pairs = (T + 1) / 2;
-    // pcm: `clips` points at int16 samples (strides in samples); always the general variant
-    const bool aligned = !pcm && warp8_aligned(pl, clips, clip_stride);
-    if (pcm && (stft || eacc || !warp8_can_launch(clips, n_clips, clip_stride, T))) {
-        set_error("warp8 pcm16 ingest: features only, at most 2^31 frame pairs per launch");
-        return DSPX_EUNSUPPORTED;
-    }
-    if (!warp8_can_launch(clips, n_clips, clip_stride, T) || (!aligned && (stft || eacc))) {
-        if (stft || eacc) { set_error("warp8 stft / fused embeddings: unaligned clips or batch too large"); return DSPX_EUNSUPPORTED; }
-        return launch_generic_fallback(pl, clips, n_clips, clip_len, clip_stride, T, logmel, mfcc, st, nchw);
-    }
-    const W8PlanData *pd = static_cast<const W8PlanData *>(pl->fast_host);
     W8Params p = w8_plan_params(pl);
-    p.clips = clips;
+    const int64_t pairs = (T + 1) / 2;
+    p.clips = static_cast<const float *>(samples);
     p.n_clips = n_clips;
     p.clip_stride = clip_stride;
     p.n_frames = T;
@@ -1656,52 +1591,92 @@ inline int launch_warp8(const dspx_plan *pl, const float *clips, int64_t n_clips
     p.mfcc = mfcc;
     p.lm_ts = nchw ? 1 : p.n_mels;
     p.lm_fs = nchw ? T : 1;
-    p.stft = stft;
-    p.eacc = eacc;
-    p.peaks = peaks;
-    const int ctas = pl->sm_count;                           // grid size is derived per configuration in w8_launch_cfg
-#ifdef DSPX_W8_LAB
-    // benchmarks/lab/w8_lab.cu: only the headline instantiation, for quick builds of kernel variants
-    return w8_launch_nw<8, true, false, true, W8_WARPS_WIDE>(p, pd->smem_wide, pl->device, std::min<int64_t>(ctas, (p.n_items + W8_WARPS_WIDE - 1) / W8_WARPS_WIDE), st);
-#else
-    if (stft) {
-        const bool pre = stft_pre && pl->cfg.pre_emphasis > 0.0;
-        switch (pd->tb.r1) {
-            case 4: return pre ? w8_launch_one<4, true, true>(p, pd, pl->device, ctas, st) : w8_launch_one<4, false, true>(p, pd, pl->device, ctas, st);
-            case 8: return pre ? w8_launch_one<8, true, true>(p, pd, pl->device, ctas, st) : w8_launch_one<8, false, true>(p, pd, pl->device, ctas, st);
-            case 16: return pre ? w8_launch_one<16, true, true>(p, pd, pl->device, ctas, st) : w8_launch_one<16, false, true>(p, pd, pl->device, ctas, st);
-        }
+    return p;
+}
+
+// persistent grid: at most max_ctas CTAs, whose warps stride over the items
+template <int R1, bool PRE, bool STFT, bool SHARE, int NW, bool EMB = false, bool U4 = false, bool PCM = false,
+          bool RAGGED = false>
+inline int w8_launch_nw(const W8Params &p, size_t smem, int device, int64_t max_ctas, cudaStream_t st)
+{
+    const int64_t ctas = std::min<int64_t>(((int64_t)p.n_items + NW - 1) / NW, max_ctas);
+    static std::atomic<unsigned char> optin[64];
+    DSPX_CUDA_CHECK(optin_max_smem(feat_warp8_kernel<R1, PRE, STFT, SHARE, NW, EMB, U4, PCM, RAGGED>, optin, device));
+    feat_warp8_kernel<R1, PRE, STFT, SHARE, NW, EMB, U4, PCM, RAGGED><<<(unsigned)ctas, NW * 32, smem, st>>>(p);
+    DSPX_CUDA_CHECK(cudaGetLastError());
+    return DSPX_OK;
+}
+
+// warps per CTA: on the feature path one CTA of 20 (or 12) warps per SM when it fits beside the tables (radix 4 / 8) or
+// of 10 warps (radix 16); otherwise 8-warp CTAs, as many per SM as fit
+template <int R1, bool PRE, bool STFT, bool SHARE, bool EMB, bool U4, bool PCM, bool RAGGED>
+inline int w8_launch_cfg(const W8Params &p, const W8PlanData *pd, int device, int sm_count, cudaStream_t st)
+{
+    if constexpr (!STFT && R1 != 16) {
+        if (pd->smem_wide)
+            return w8_launch_nw<R1, PRE, STFT, SHARE, W8_WARPS_WIDE, EMB, U4, PCM, RAGGED>(p, pd->smem_wide, device, sm_count, st);
+        if (pd->smem_mid)
+            return w8_launch_nw<R1, PRE, STFT, SHARE, W8_WARPS_MID, EMB, U4, PCM, RAGGED>(p, pd->smem_mid, device, sm_count, st);
     }
-    const bool pre = pl->cfg.pre_emphasis > 0.0;
-    if (pcm) {
-        switch (pd->tb.r1) {
-            case 4: return pre ? w8_launch_u4<4, true, true>(p, pd, pl->device, ctas, st) : w8_launch_u4<4, false, true>(p, pd, pl->device, ctas, st);
-            case 8: return pre ? w8_launch_u4<8, true, true>(p, pd, pl->device, ctas, st) : w8_launch_u4<8, false, true>(p, pd, pl->device, ctas, st);
-            case 16: return pre ? w8_launch_u4<16, true, true>(p, pd, pl->device, ctas, st) : w8_launch_u4<16, false, true>(p, pd, pl->device, ctas, st);
-        }
+    if constexpr (!STFT && R1 == 16) {
+        if (pd->smem_r16)
+            return w8_launch_nw<R1, PRE, STFT, SHARE, W8_WARPS_R16, EMB, U4, PCM, RAGGED>(p, pd->smem_r16, device, sm_count, st);
     }
-    if (!aligned) {
-        switch (pd->tb.r1) {
-            case 4: return pre ? w8_launch_u4<4, true>(p, pd, pl->device, ctas, st) : w8_launch_u4<4, false>(p, pd, pl->device, ctas, st);
-            case 8: return pre ? w8_launch_u4<8, true>(p, pd, pl->device, ctas, st) : w8_launch_u4<8, false>(p, pd, pl->device, ctas, st);
-            case 16: return pre ? w8_launch_u4<16, true>(p, pd, pl->device, ctas, st) : w8_launch_u4<16, false>(p, pd, pl->device, ctas, st);
-        }
-    }
+    return w8_launch_nw<R1, PRE, STFT, SHARE, W8_WARPS, EMB, U4, PCM, RAGGED>(p, pd->smem, device,
+                                                                              (int64_t)sm_count * pd->ctas_per_sm, st);
+}
+
+// the radix and pre-emphasis switch over one variant <STFT, SHARE, EMB, U4, PCM, RAGGED> (radix 16 never shares rows,
+// see W8_SHARE)
+template <bool STFT, bool SHARE, bool EMB, bool U4, bool PCM, bool RAGGED>
+inline int w8_launch_variant(const dspx_plan *pl, const W8Params &p, bool pre, cudaStream_t st)
+{
+    const W8PlanData *pd = static_cast<const W8PlanData *>(pl->fast_host);
+    const int dev = pl->device, sms = pl->sm_count;
     switch (pd->tb.r1) {
-        case 4: return pre ? w8_launch_one<4, true, false>(p, pd, pl->device, ctas, st) : w8_launch_one<4, false, false>(p, pd, pl->device, ctas, st);
-        case 8: return pre ? w8_launch_one<8, true, false>(p, pd, pl->device, ctas, st) : w8_launch_one<8, false, false>(p, pd, pl->device, ctas, st);
-        case 16: return pre ? w8_launch_one<16, true, false>(p, pd, pl->device, ctas, st) : w8_launch_one<16, false, false>(p, pd, pl->device, ctas, st);
+        case 4: return pre ? w8_launch_cfg<4, true, STFT, SHARE, EMB, U4, PCM, RAGGED>(p, pd, dev, sms, st)
+                           : w8_launch_cfg<4, false, STFT, SHARE, EMB, U4, PCM, RAGGED>(p, pd, dev, sms, st);
+        case 8: return pre ? w8_launch_cfg<8, true, STFT, SHARE, EMB, U4, PCM, RAGGED>(p, pd, dev, sms, st)
+                           : w8_launch_cfg<8, false, STFT, SHARE, EMB, U4, PCM, RAGGED>(p, pd, dev, sms, st);
+        case 16: return pre ? w8_launch_cfg<16, true, STFT, false, EMB, U4, PCM, RAGGED>(p, pd, dev, sms, st)
+                            : w8_launch_cfg<16, false, STFT, false, EMB, U4, PCM, RAGGED>(p, pd, dev, sms, st);
     }
     set_error("warp8: bad radix");
     return DSPX_EUNSUPPORTED;
-#endif
 }
 
-// frames of float32 clips that start at even samples of an 8-byte aligned buffer sit on the 8-byte grid when the hop is
-// even: the aligned variants (row sharing, fused embeddings) apply exactly when they would to each clip alone
-inline bool warp8_ragged_aligned(const dspx_plan *pl, int pcm)
+// a path's variant; fused embeddings (EMB) when p.eacc is set
+template <bool RAGGED>
+inline int w8_launch_path(const dspx_plan *pl, W8Path path, const W8Params &p, bool pre, cudaStream_t st)
 {
-    return !pcm && pl->cfg.frame_length == pl->P && !(pl->cfg.hop_length & 1);
+    const bool emb = p.eacc != nullptr;
+    switch (path) {
+        case W8_SHARE: return emb ? w8_launch_variant<false, true, true, false, false, RAGGED>(pl, p, pre, st)
+                                  : w8_launch_variant<false, true, false, false, false, RAGGED>(pl, p, pre, st);
+        case W8_ALIGNED: return emb ? w8_launch_variant<false, false, true, false, false, RAGGED>(pl, p, pre, st)
+                                    : w8_launch_variant<false, false, false, false, false, RAGGED>(pl, p, pre, st);
+        case W8_U4: return w8_launch_variant<false, false, false, true, false, RAGGED>(pl, p, pre, st);
+        case W8_PCM16: return w8_launch_variant<false, false, false, true, true, RAGGED>(pl, p, pre, st);
+        default: set_error("warp8: path %d is not a feat_warp8_kernel variant", (int)path); return DSPX_EUNSUPPORTED;
+    }
+}
+
+// Launches feat_warp8_kernel on a path warp8_select chose: W8_ALIGNED, W8_SHARE, W8_U4 or W8_PCM16.  p.stft selects the
+// STFT mode, p.eacc the fused embeddings, p.rtab a ragged batch; pre: apply pre-emphasis.
+inline int launch_warp8(const dspx_plan *pl, W8Path path, W8Params p, bool pre, cudaStream_t st)
+{
+    p.share = path == W8_SHARE;
+#ifdef DSPX_W8_LAB
+    // benchmarks/lab/w8_lab.cu: only the headline instantiation, for quick builds of kernel variants
+    (void)pre;
+    return w8_launch_nw<8, true, false, true, W8_WARPS_WIDE>(p, static_cast<const W8PlanData *>(pl->fast_host)->smem_wide,
+                                                             pl->device, pl->sm_count, st);
+#else
+    if (p.stft)
+        return p.share ? w8_launch_variant<true, true, false, false, false, false>(pl, p, pre, st)
+                       : w8_launch_variant<true, false, false, false, false, false>(pl, p, pre, st);
+    return p.rtab ? w8_launch_path<true>(pl, path, p, pre, st) : w8_launch_path<false>(pl, path, p, pre, st);
+#endif
 }
 
 // [n_clips + 1] first frame pair of every clip, then the total: the compact array w8_ragged_clip searches
@@ -1711,55 +1686,6 @@ __global__ void ragged_pairs_kernel(const dspx_ragged_clip *rtab, int64_t n_clip
     if (i < n_clips) rpairs[i] = (uint32_t)rtab[i].first_pair;
     else if (i == n_clips) rpairs[i] = (uint32_t)(rtab[i - 1].first_pair + (rtab[i - 1].n_frames + 1) / 2);
 }
-
-#if !defined(DSPX_W8_LAB) && !defined(DSPX_EMU)
-// Ragged batch, one launch: items are the n_items frame pairs of all clips (RAGGED variants; not the STFT mode).
-// samples: float32 (8-byte aligned, even starts) or int16 (pcm); eacc needs warp8_ragged_aligned.
-inline int launch_warp8_ragged(const dspx_plan *pl, const void *samples, int pcm, const dspx_ragged_clip *rtab,
-                               const uint32_t *rpairs, int64_t n_clips, uint32_t n_items, float *logmel, float *mfcc,
-                               long long *eacc, const int *peaks, cudaStream_t st)
-{
-    const bool aligned = warp8_ragged_aligned(pl, pcm);
-    if (eacc && !aligned) { set_error("warp8 fused embeddings: frames off the 8-byte grid"); return DSPX_EUNSUPPORTED; }
-    const W8PlanData *pd = static_cast<const W8PlanData *>(pl->fast_host);
-    W8Params p = w8_plan_params(pl);
-    p.clips = static_cast<const float *>(samples);
-    p.n_clips = n_clips;
-    p.n_items = n_items;
-    p.logmel = logmel;
-    p.mfcc = mfcc;
-    p.lm_ts = p.n_mels;
-    p.lm_fs = 1;
-    p.eacc = eacc;
-    p.peaks = peaks;
-    p.rtab = rtab;
-    p.rpairs = rpairs;
-    const int ctas = pl->sm_count;
-    const bool pre = pl->cfg.pre_emphasis > 0.0;
-#define W8R_SWITCH(CALL4, CALL8, CALL16)                                     \
-    switch (pd->tb.r1) {                                                   \
-        case 4: return CALL4;                                              \
-        case 8: return CALL8;                                              \
-        case 16: return CALL16;                                            \
-    }
-    if (pcm) {
-        W8R_SWITCH((pre ? w8_launch_u4<4, true, true, true>(p, pd, pl->device, ctas, st) : w8_launch_u4<4, false, true, true>(p, pd, pl->device, ctas, st)),
-                   (pre ? w8_launch_u4<8, true, true, true>(p, pd, pl->device, ctas, st) : w8_launch_u4<8, false, true, true>(p, pd, pl->device, ctas, st)),
-                   (pre ? w8_launch_u4<16, true, true, true>(p, pd, pl->device, ctas, st) : w8_launch_u4<16, false, true, true>(p, pd, pl->device, ctas, st)))
-    } else if (!aligned) {
-        W8R_SWITCH((pre ? w8_launch_u4<4, true, false, true>(p, pd, pl->device, ctas, st) : w8_launch_u4<4, false, false, true>(p, pd, pl->device, ctas, st)),
-                   (pre ? w8_launch_u4<8, true, false, true>(p, pd, pl->device, ctas, st) : w8_launch_u4<8, false, false, true>(p, pd, pl->device, ctas, st)),
-                   (pre ? w8_launch_u4<16, true, false, true>(p, pd, pl->device, ctas, st) : w8_launch_u4<16, false, false, true>(p, pd, pl->device, ctas, st)))
-    } else {
-        W8R_SWITCH((pre ? w8_launch_one<4, true, false, true>(p, pd, pl->device, ctas, st) : w8_launch_one<4, false, false, true>(p, pd, pl->device, ctas, st)),
-                   (pre ? w8_launch_one<8, true, false, true>(p, pd, pl->device, ctas, st) : w8_launch_one<8, false, false, true>(p, pd, pl->device, ctas, st)),
-                   (pre ? w8_launch_one<16, true, false, true>(p, pd, pl->device, ctas, st) : w8_launch_one<16, false, false, true>(p, pd, pl->device, ctas, st)))
-    }
-#undef W8R_SWITCH
-    set_error("warp8: bad radix");
-    return DSPX_EUNSUPPORTED;
-}
-#endif
 #endif
 
 }  // namespace dspx

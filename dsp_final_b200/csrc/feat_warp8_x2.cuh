@@ -200,7 +200,7 @@ DSPX_HD void w8x2_set_item(const W8Params &p, W8Ctx &c, uint32_t item)
     c.eacc = nullptr;
 }
 
-#if defined(__CUDACC__)
+#if defined(__CUDACC__) && !defined(DSPX_EMU)
 template <bool PRE, bool AL4>
 __global__ void __launch_bounds__(W8_WARPS * 32, 1) feat_warp8_x2_kernel(const W8Params p)
 {
@@ -272,33 +272,14 @@ inline int w8x2_launch(const W8Params &p, const W8PlanData *pd, int device, int 
     return DSPX_OK;
 }
 
-// features of 4096-point frames; one launch, n_clips * n_frames items
-inline int launch_warp8_x2(const dspx_plan *pl, const float *clips, int64_t n_clips, int64_t clip_len, int64_t clip_stride,
-                           int64_t T, float *logmel, float *mfcc, cudaStream_t st, int nchw)
+// features of 4096-point frames; one launch, n_clips * n_frames items (al4: the W8_X2_AL4 path)
+inline int launch_warp8_x2(const dspx_plan *pl, bool al4, const float *clips, int64_t n_clips, int64_t clip_stride, int64_t T,
+                           float *logmel, float *mfcc, cudaStream_t st, int nchw)
 {
-    if (n_clips * T >= (int64_t)0x7fffffff)
-        return launch_generic_fallback(pl, clips, n_clips, clip_len, clip_stride, T, logmel, mfcc, st, nchw);
     const W8PlanData *pd = static_cast<const W8PlanData *>(pl->fast_host);
-    W8Params p{};
-    p.clips = clips;
-    p.n_clips = n_clips;
-    p.clip_stride = clip_stride;
-    p.n_frames = T;
-    p.pairs_per_clip = (uint32_t)T;
+    W8Params p = w8_batch_params(pl, clips, n_clips, clip_stride, T, logmel, mfcc, nchw);
+    p.pairs_per_clip = (uint32_t)T;                          // one frame per item
     p.n_items = (uint32_t)(n_clips * T);
-    p.hop = pl->cfg.hop_length;
-    p.n_mels = pl->cfg.n_mels;
-    p.n_mfcc = pl->cfg.n_mfcc;
-    p.take = std::min(pl->cfg.frame_length, pl->P);
-    p.alpha = (float)pl->cfg.pre_emphasis;
-    p.tb = pd->tb;
-    p.tables = static_cast<const float *>(pl->d_fast_tables);
-    p.logmel = logmel;
-    p.mfcc = mfcc;
-    p.lm_ts = nchw ? 1 : p.n_mels;
-    p.lm_fs = nchw ? T : 1;
-    const bool al4 = pl->cfg.frame_length >= pl->P && !(pl->cfg.hop_length & 3) && !(clip_stride & 3) &&
-                     !(reinterpret_cast<uintptr_t>(clips) & 15);
     const bool pre = pl->cfg.pre_emphasis > 0.0;
     if (al4) return pre ? w8x2_launch<true, true>(p, pd, pl->device, pl->sm_count, st) : w8x2_launch<false, true>(p, pd, pl->device, pl->sm_count, st);
     return pre ? w8x2_launch<true, false>(p, pd, pl->device, pl->sm_count, st) : w8x2_launch<false, false>(p, pd, pl->device, pl->sm_count, st);

@@ -13,6 +13,8 @@
  *   - extern "C", plain pointers and sizes, no C++/torch types.
  *   - return 0 on success, a negative DSPX_E* code otherwise; never throws.
  *     dspx_last_error() returns a thread-local message for the last failure.
+ *     A call that returns DSPX_EUNSUPPORTED has enqueued nothing, so the
+ *     caller may fall back to another entry point on the same buffers.
  *   - "_dev" pointers are device memory owned by the caller; all device work is
  *     enqueued on the caller's stream (cudaStream_t passed as void*), with no
  *     hidden synchronisation and no allocation in the launch path.
@@ -117,7 +119,9 @@ int dspx_features(const dspx_plan *plan, const float *clips_dev, int64_t n_clips
  * the feature kernel adds every frame's coefficients and their squares to per-clip fixed-point accumulators in
  * workspace_dev (order-independent, so results are reproducible) and a finalize step writes
  * embed [n_clips, 2*n_mfcc] f32.  No MFCC tensor is written or read.  logmel_out_dev may be NULL.
- * Needs the warp8 kernel (DSPX_EUNSUPPORTED otherwise: use dspx_features with an MFCC buffer). */
+ * Runs when the plan uses the warp8 kernel, frame_length equals the transform length (n_fft_pow2) and that is 512,
+ * 1024 or 2048, hop_length and clip_stride are even, clips_dev is 8-byte aligned and n_clips * ceil(n_frames / 2)
+ * < 2^31.  Otherwise DSPX_EUNSUPPORTED: use dspx_features with an MFCC buffer. */
 size_t dspx_embeddings_workspace(const dspx_plan *plan, int64_t n_clips);
 int dspx_embeddings(const dspx_plan *plan, const float *clips_dev, int64_t n_clips, int64_t clip_len,
                     int64_t clip_stride, float *embed_out_dev, float *logmel_out_dev, void *workspace_dev,
@@ -160,8 +164,9 @@ int dspx_stft_host(const dspx_plan *plan, const float *clips_host, int64_t n_cli
  * to NumPy.  The _host form ships int16 over PCIe (half the bytes of float32 clips). */
 int dspx_pcm16_to_float(const int16_t *pcm_dev, int64_t n_clips, int64_t clip_len, int64_t pcm_stride,
                         int normalize, float *out_dev, int64_t out_stride, void *stream);
-/* Device-pointer form with the conversion FUSED into the feature kernel's sample loads (warp8 plans: n_fft 512 / 1024 /
- * 2048; DSPX_EUNSUPPORTED otherwise): no float32 copy of the clips exists.  q = s * (1/m), one fma refinement -- the
+/* Device-pointer form with the conversion FUSED into the feature kernel's sample loads: no float32 copy of the clips
+ * exists.  Runs when the plan uses the warp8 kernel with a transform length (n_fft_pow2) of 512, 1024 or 2048 and
+ * n_clips * ceil(n_frames / 2) < 2^31; otherwise DSPX_EUNSUPPORTED: convert with dspx_pcm16_to_float first.  q = s * (1/m), one fma refinement -- the
  * correctly rounded s / m for every |s| <= m <= 32768 (checked exhaustively), i.e. the same samples as above.
  * workspace_dev (dspx_features_pcm16_workspace bytes) holds one peak per clip; unused when normalize == 0. */
 size_t dspx_features_pcm16_workspace(int64_t n_clips);

@@ -334,8 +334,8 @@ def test_fused_embeddings_without_mfcc(torch_cuda, clips_5s):
     from dsp_final_b200.dsp.mfcc import MfccConfig
     from oracle import oracle as O
 
-    for fl, hop in ((1024, 512), (512, 256), (2048, 1024), (1024, 300)):
-        cfg = MfccConfig(sample_rate=44100, frame_length=fl, hop_length=hop)
+    for fl, hop, n_fft in ((1024, 512, None), (512, 256, None), (2048, 1024, None), (1024, 300, None), (400, 160, 512)):
+        cfg = MfccConfig(sample_rate=44100, frame_length=fl, hop_length=hop, n_fft=n_fft)
         x = clips_5s[:96]
         both = features_batch(x, cfg, ("mfcc", "embed"))                 # embed = statistics of the MFCC tensor
         alone = features_batch(x, cfg, ("embed",))["embed"]              # fused: no MFCC tensor
@@ -344,7 +344,7 @@ def test_fused_embeddings_without_mfcc(torch_cuda, clips_5s):
         scale = float(both["embed"].abs().max())
         assert float((alone - both["embed"]).abs().max()) <= 2e-6 * scale, (fl, hop)
         assert torch.equal(again["log_mel"], features_batch(x, cfg, ("log_mel",))["log_mel"])
-        ref = O.features_batch(x[:3].cpu().numpy(), O.OracleConfig(44100, fl, hop), want=("embed",))["embed"]
+        ref = O.features_batch(x[:3].cpu().numpy(), O.OracleConfig(44100, fl, hop, n_fft), want=("embed",))["embed"]
         assert rel_err(alone[:3].cpu().numpy(), ref) < TOL, (fl, hop)
         host = features_batch(x[:40].cpu().numpy(), cfg, ("embed",))["embed"]      # host pipeline takes the same path
         assert np.array_equal(host, alone[:40].cpu().numpy()), (fl, hop)

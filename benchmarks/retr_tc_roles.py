@@ -13,14 +13,13 @@ import torch
 from dsp_final_b200 import retrieval as R
 g = torch.Generator(device="cuda"); g.manual_seed(0)
 names = ["mma wait acc_empty", "mma wait full_b", "mma issue+commit", "prod wait empty", "prod store", "epi wait acc_full", "epi masks", "epi enqueue+drain", "tiles", "mma total"]
-for nq, ndb, sp in ((8192, 262144, 1), (8192, 262144, 9), (20000, 1000000, 9)):
-    os.environ["DSPX_TOPK_SPLITS"] = str(sp)
+for nq, ndb in ((8192, 262144), (20000, 1000000)):
     q = torch.randn((nq, 26), generator=g, device="cuda"); db = torch.randn((ndb, 26), generator=g, device="cuda")
     R.cosine_topk(q, db, 20); torch.cuda.synchronize()
     out = (ctypes.c_longlong * 16)()
     h = ctypes.CDLL(os.environ["DSPX_LIBRARY"])
     rc = h.dspx_debug_tc_prof(out)
     tiles = out[8]
-    print(nq, ndb, "splits", sp, "rc", rc, "tiles", tiles)
+    print(nq, ndb, "rc", rc, "tiles", tiles)
     for i, n in enumerate(names):
         if i != 8: print(f"   {n:22s} {out[i]/max(tiles,1):9.0f} cycles/tile")

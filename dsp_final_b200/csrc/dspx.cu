@@ -600,6 +600,160 @@ static int host_pipeline(dspx_plan *pl, int mode, const void *clips_v, int64_t n
     return DSPX_OK;
 }
 
+// ---- ranking (dspx_cosine_topk, dspx_cosine_matrix) ------------------------------
+
+// The three ranking kernels return the same lists: each scores every row it keeps exactly in float64.  The two filters
+// first screen the database with a cheaper score (split fp16 on the tensor cores, packed FP32) against the running k-th
+// score, minus a bound on that score's error.
+enum TopkKernel { TOPK_TC, TOPK_F32, TOPK_F64 };
+
+struct TopkLaunch {
+    TopkKernel kernel;
+    int cw;                     // template argument: 26 (MFCC embeddings, 2 x 13), else 0 (TOPK_TC) or 32
+    dim3 grid;                  // (query tiles, database splits)
+    int threads;
+    size_t smem;                // dynamic shared memory
+    int n_splits;
+    int64_t rows_per_split;     // multiple of TK_ROWS
+};
+
+// float64 kernel: about two CTAs per SM, at least 4 tiles per split
+static int topk_splits(int64_t nq, int64_t ndb, int sm_count)
+{
+    const int64_t qtiles = (nq + TK_QPC - 1) / TK_QPC;
+    int64_t s = (2 * (int64_t)sm_count + qtiles - 1) / qtiles;
+    const int64_t max_by_rows = (ndb + 4 * TK_ROWS - 1) / (4 * TK_ROWS);       // at least 4 tiles per split
+    if (s > max_by_rows) s = max_by_rows;
+    if (s > TK_MAX_SPLITS) s = TK_MAX_SPLITS;
+    if (s < 1) s = 1;
+    return (int)s;
+}
+
+// filter kernels, one CTA per SM: the split count whose grid fills whole waves (every extra split also restarts the
+// running lists, which costs insertions -- the per-split penalty), at most 16, at least 8 tiles per split
+static int64_t topk_wave_splits(int64_t qtiles, int64_t ndb, int sm_count)
+{
+    int64_t max_sp = (ndb + 8 * TK_ROWS - 1) / (8 * TK_ROWS);
+    if (max_sp > 16) max_sp = 16;
+    if (max_sp < 1) max_sp = 1;
+    int64_t sp = 1;
+    double best = 1e30;
+    for (int64_t c = 1; c <= max_sp; c++) {
+        const double waves = (double)((qtiles * c + sm_count - 1) / sm_count);
+        const double cost = waves / (double)c * (1.0 + 0.02 * (double)c);
+        if (cost < best - 1e-12) { best = cost; sp = c; }
+    }
+    return sp;
+}
+
+// The kernel of a call and its launch, from the shape alone:
+//   dim <= 32 and k <= TC_MAX_K                                   tensor-core filter
+//   dim <= 32 and the FP32 filter's lists fit in 200 KB of smem   FP32 filter (k <= 55 at dim 26, k <= 37 at dim 32)
+//   otherwise                                                     float64 kernel
+static TopkLaunch topk_select(int64_t nq, int64_t ndb, int dim, int k, int sm_count)
+{
+    TopkLaunch L{};
+    const int cw = dim == 26 ? 26 : 32;
+    int64_t qtiles;
+    if (dim <= 32 && k <= TC_MAX_K) {
+        L.kernel = TOPK_TC;
+        L.cw = dim == 26 ? 26 : 0;
+        L.threads = TC_THREADS;
+        L.smem = topk_tc_smem_bytes(k);
+        qtiles = (nq + TC_QT - 1) / TC_QT;
+    } else if (dim <= 32 && topk_f32_smem_bytes(dim, k, cw) <= 200 * 1024) {
+        L.kernel = TOPK_F32;
+        L.cw = cw;
+        L.threads = TKF_WARPS * 32;
+        L.smem = topk_f32_smem_bytes(dim, k, cw);
+        qtiles = (nq + TKF_QPC - 1) / TKF_QPC;
+    } else {
+        L.kernel = TOPK_F64;
+        L.cw = cw;
+        L.threads = TK_WARPS * 32;
+        L.smem = topk_smem_bytes(dim, k, cw);
+        qtiles = (nq + TK_QPC - 1) / TK_QPC;
+    }
+    const int64_t sp = L.kernel == TOPK_F64 ? topk_splits(nq, ndb, sm_count) : topk_wave_splits(qtiles, ndb, sm_count);
+    int64_t rows = (ndb + sp - 1) / sp;
+    rows = (rows + TK_ROWS - 1) / TK_ROWS * TK_ROWS;
+    L.rows_per_split = rows;
+    L.n_splits = (int)((ndb + rows - 1) / rows);
+    L.grid = dim3((unsigned)qtiles, (unsigned)L.n_splits);
+    return L;
+}
+
+struct TopkWs {
+    double *qn, *dbn;                   // [nq, dim], [ndb, dim] normalised rows
+    double *pscore;                     // per-split lists [nq, n_splits, k], n_splits <= TK_MAX_SPLITS
+    int32_t *pidx;
+    float *qf, *dbf;                    // operand images of the filter kernels: 32 floats per row covers both layouts (dim <= 32 there)
+    size_t qf_bytes, dbf_bytes;
+    unsigned long long *shared_thr;     // [nq] thresholds shared between splits
+    int *split_done;                    // per (query tile, split): lists written
+};
+
+// One layout of the ranking workspace for the size query and the launches.  Returns its size; with base, also the pointers.
+static size_t topk_ws_carve(int64_t nq, int64_t ndb, int dim, int k, char *base, TopkWs *ws)
+{
+    TopkWs w;
+    w.qf_bytes = (size_t)((nq + TC_QT - 1) / TC_QT) * TC_QT * TC_KPAD * 4;
+    w.dbf_bytes = (size_t)((ndb + TK_ROWS - 1) / TK_ROWS) * TK_ROWS * TC_KPAD * 4;
+    size_t off = 0;
+    auto take = [&](size_t bytes) -> char * {
+        char *p = base ? base + off : nullptr;
+        off += align256(bytes);
+        return p;
+    };
+    w.qn = reinterpret_cast<double *>(take((size_t)nq * dim * 8));
+    w.dbn = reinterpret_cast<double *>(take((size_t)ndb * dim * 8));
+    w.pscore = reinterpret_cast<double *>(take((size_t)nq * TK_MAX_SPLITS * k * 8));
+    w.pidx = reinterpret_cast<int32_t *>(take((size_t)nq * TK_MAX_SPLITS * k * 4));
+    w.qf = reinterpret_cast<float *>(take(w.qf_bytes));
+    w.dbf = reinterpret_cast<float *>(take(w.dbf_bytes));
+    w.shared_thr = reinterpret_cast<unsigned long long *>(take((size_t)nq * 8));
+    w.split_done = reinterpret_cast<int *>(take((size_t)((nq + TC_QT - 1) / TC_QT) * TK_MAX_SPLITS * 4));
+    if (ws) *ws = w;
+    return off + 1024;
+}
+
+// Normalised float64 rows of x into out64, plus the operand image that kernel `kern` reads, in tiles of `tile` rows: the
+// fp16 split of the tensor-core filter (including its zero padding), the float copy of the FP32 filter, none for TOPK_F64.
+template <typename T>
+static void launch_normalize(TopkKernel kern, const T *x, int64_t n, int dim, int tile, double *out64, float *img,
+                             cudaStream_t st)
+{
+    if (kern == TOPK_TC) {
+        const int64_t n_pad = (n + tile - 1) / tile * tile;
+        normalize_rows_split16_kernel<T><<<(unsigned)((n_pad + NR_ROWS - 1) / NR_ROWS), 128, 0, st>>>(
+            x, n, n_pad, dim, out64, reinterpret_cast<unsigned char *>(img));
+    } else if (kern == TOPK_F32) {
+        normalize_rows_tiled_kernel<T><<<(unsigned)((n + 127) / 128), 128, 0, st>>>(x, n, dim, out64, img, tile);
+    } else {
+        normalize_rows_kernel<T><<<(unsigned)((n + 127) / 128), 128, 0, st>>>(x, n, dim, out64);
+    }
+}
+
+static void normalize_rows(TopkKernel kern, const void *x, int dtype, int64_t n, int dim, int tile, double *out64,
+                           float *img, cudaStream_t st)
+{
+    if (dtype == DSPX_DTYPE_F32)
+        launch_normalize(kern, static_cast<const float *>(x), n, dim, tile, out64, img, st);
+    else
+        launch_normalize(kern, static_cast<const double *>(x), n, dim, tile, out64, img, st);
+}
+
+// each kernel instantiation has its own opt-in flags
+template <auto Kernel, class Params>
+static int topk_launch(const TopkLaunch &L, const Params &p, int device, cudaStream_t st)
+{
+    static std::atomic<unsigned char> optin[64];
+    DSPX_CUDA_CHECK(optin_max_smem(Kernel, optin, device));
+    Kernel<<<L.grid, L.threads, L.smem, st>>>(p);
+    DSPX_CUDA_CHECK(cudaGetLastError());
+    return DSPX_OK;
+}
+
 }  // namespace dspx
 
 using namespace dspx;
@@ -1034,48 +1188,10 @@ int dspx_fft_c2c(const float *in_dev, int64_t batch, int64_t n_in, int64_t n, in
     return DSPX_OK;
 }
 
-// Tuning / test knobs of the ranking path, read from the environment once per process (never in the launch
-// path): DSPX_TOPK = tc | f32 | f64 forces a kernel, DSPX_TOPK_SPLITS fixes the database split count.
-struct TopkKnobs {
-    const char *force;
-    bool f64;
-    long long splits;
-};
-static const TopkKnobs &topk_knobs()
-{
-    static const TopkKnobs k = [] {
-        TopkKnobs t{};
-        t.force = getenv("DSPX_TOPK");
-        t.f64 = getenv("DSPX_TOPK_F64") != nullptr;
-        const char *e = getenv("DSPX_TOPK_SPLITS");
-        t.splits = e ? atoll(e) : 0;
-        return t;
-    }();
-    return k;
-}
-
-static int topk_splits(int64_t nq, int64_t ndb, int sm_count)
-{
-    const int64_t qtiles = (nq + TK_QPC - 1) / TK_QPC;
-    int64_t s = (2 * (int64_t)sm_count + qtiles - 1) / qtiles;
-    const int64_t max_by_rows = (ndb + 4 * TK_ROWS - 1) / (4 * TK_ROWS);       // at least 4 tiles per split
-    if (s > max_by_rows) s = max_by_rows;
-    if (s > TK_MAX_SPLITS) s = TK_MAX_SPLITS;
-    if (s < 1) s = 1;
-    return (int)s;
-}
-
 size_t dspx_cosine_topk_workspace(int64_t nq, int64_t ndb, int dim, int k)
 {
     if (nq < 0 || ndb < 0 || dim <= 0 || k <= 0) return 0;
-    size_t b = align256((size_t)nq * dim * 8) + align256((size_t)ndb * dim * 8);
-    b += align256((size_t)nq * TK_MAX_SPLITS * k * 8) + align256((size_t)nq * TK_MAX_SPLITS * k * 4);
-    // float copies for the filter kernels: 32 floats per row covers both layouts (dim <= 32 there)
-    b += align256((size_t)((nq + TC_QT - 1) / TC_QT) * TC_QT * TC_KPAD * 4);
-    b += align256((size_t)((ndb + TK_ROWS - 1) / TK_ROWS) * TK_ROWS * TC_KPAD * 4);
-    b += align256((size_t)nq * 8);                                                // thresholds shared between splits
-    b += align256((size_t)((nq + TC_QT - 1) / TC_QT) * TK_MAX_SPLITS * 4);      // per (query tile, split): lists written
-    return b + 1024;
+    return topk_ws_carve(nq, ndb, dim, k, nullptr, nullptr);
 }
 
 int dspx_cosine_topk(const void *q_dev, int64_t nq, const void *db_dev, int64_t ndb, int dim, int dtype, int k,
@@ -1093,154 +1209,60 @@ int dspx_cosine_topk(const void *q_dev, int64_t nq, const void *db_dev, int64_t 
     int dev = 0, sm = 148;
     DSPX_CUDA_CHECK(cudaGetDevice(&dev));
     DSPX_CUDA_CHECK(cudaDeviceGetAttribute(&sm, cudaDevAttrMultiProcessorCount, dev));
-    char *ws = static_cast<char *>(workspace_dev);
-    double *qn = reinterpret_cast<double *>(ws);
-    ws += align256((size_t)nq * dim * 8);
-    double *dbn = reinterpret_cast<double *>(ws);
-    ws += align256((size_t)ndb * dim * 8);
-    double *pscore = reinterpret_cast<double *>(ws);
-    ws += align256((size_t)nq * TK_MAX_SPLITS * k * 8);
-    int32_t *pidx = reinterpret_cast<int32_t *>(ws);
-    ws += align256((size_t)nq * TK_MAX_SPLITS * k * 4);
-    float *qf_t = reinterpret_cast<float *>(ws);
-    const size_t qf_bytes = (size_t)((nq + TC_QT - 1) / TC_QT) * TC_QT * TC_KPAD * 4;
-    ws += align256(qf_bytes);
-    float *dbf_t = reinterpret_cast<float *>(ws);
-    const size_t dbf_bytes = (size_t)((ndb + TK_ROWS - 1) / TK_ROWS) * TK_ROWS * TC_KPAD * 4;
-    ws += align256(dbf_bytes);
-    unsigned long long *shared_thr = reinterpret_cast<unsigned long long *>(ws);
-    ws += align256((size_t)nq * 8);
-    int *split_done = reinterpret_cast<int *>(ws);
-    // Filter kernels (single-chunk dimensions, lists that fit beside the tiles), all with exact float64 re-scoring:
-    // tensor-core (split fp16) filter, else packed-FP32 filter, else the all-float64 kernel.  DSPX_TOPK = tc | f32 | f64 forces one.
-    const TopkKnobs &knobs = topk_knobs();
-    const char *force = knobs.force;
-    const bool want_f64 = knobs.f64 || (force && !strcmp(force, "f64"));
-    const bool tc_ok = dim <= 32 && k <= TC_MAX_K;
-    const bool f32_ok = dim <= 32 && topk_f32_smem_bytes(dim, k, dim == 26 ? 26 : 32) <= 200 * 1024;
-    const bool use_tc = !want_f64 && tc_ok && !(force && !strcmp(force, "f32") && f32_ok);
-    const bool prefilter = !want_f64 && !use_tc && f32_ok;
-
-    if (use_tc) {
-        // fp16 operand images (128 bytes per row, same size as the float copies of the other filter); the kernel writes the
-        // zero padding too (columns >= dim, rows up to the tile multiple): no memset pass
-        const int64_t nq_pad = (nq + TC_QT - 1) / TC_QT * TC_QT, ndb_pad = (ndb + TK_ROWS - 1) / TK_ROWS * TK_ROWS;
-        const unsigned gq = (unsigned)((nq_pad + NR_ROWS - 1) / NR_ROWS), gd = (unsigned)((ndb_pad + NR_ROWS - 1) / NR_ROWS);
-        if (dtype == DSPX_DTYPE_F32) {
-            normalize_rows_split16_kernel<float><<<gq, 128, 0, st>>>((const float *)q_dev, nq, nq_pad, dim, qn, (unsigned char *)qf_t);
-            normalize_rows_split16_kernel<float><<<gd, 128, 0, st>>>((const float *)db_dev, ndb, ndb_pad, dim, dbn, (unsigned char *)dbf_t);
-        } else {
-            normalize_rows_split16_kernel<double><<<gq, 128, 0, st>>>((const double *)q_dev, nq, nq_pad, dim, qn, (unsigned char *)qf_t);
-            normalize_rows_split16_kernel<double><<<gd, 128, 0, st>>>((const double *)db_dev, ndb, ndb_pad, dim, dbn, (unsigned char *)dbf_t);
-        }
-    } else
-    if (prefilter) {
-        DSPX_CUDA_CHECK(cudaMemsetAsync(qf_t, 0, qf_bytes, st));              // zero padding of the last tiles
-        DSPX_CUDA_CHECK(cudaMemsetAsync(dbf_t, 0, dbf_bytes, st));
-        if (dtype == DSPX_DTYPE_F32) {
-            normalize_rows_tiled_kernel<float><<<(unsigned)((nq + 127) / 128), 128, 0, st>>>((const float *)q_dev, nq, dim, qn, qf_t, TKF_QPC);
-            normalize_rows_tiled_kernel<float><<<(unsigned)((ndb + 127) / 128), 128, 0, st>>>((const float *)db_dev, ndb, dim, dbn, dbf_t, TK_ROWS);
-        } else {
-            normalize_rows_tiled_kernel<double><<<(unsigned)((nq + 127) / 128), 128, 0, st>>>((const double *)q_dev, nq, dim, qn, qf_t, TKF_QPC);
-            normalize_rows_tiled_kernel<double><<<(unsigned)((ndb + 127) / 128), 128, 0, st>>>((const double *)db_dev, ndb, dim, dbn, dbf_t, TK_ROWS);
-        }
-    } else if (dtype == DSPX_DTYPE_F32) {
-        normalize_rows_kernel<float><<<(unsigned)((nq + 127) / 128), 128, 0, st>>>((const float *)q_dev, nq, dim, qn);
-        normalize_rows_kernel<float><<<(unsigned)((ndb + 127) / 128), 128, 0, st>>>((const float *)db_dev, ndb, dim, dbn);
-    } else {
-        normalize_rows_kernel<double><<<(unsigned)((nq + 127) / 128), 128, 0, st>>>((const double *)q_dev, nq, dim, qn);
-        normalize_rows_kernel<double><<<(unsigned)((ndb + 127) / 128), 128, 0, st>>>((const double *)db_dev, ndb, dim, dbn);
+    const TopkLaunch L = topk_select(nq, ndb, dim, k, sm);
+    TopkWs ws;
+    topk_ws_carve(nq, ndb, dim, k, static_cast<char *>(workspace_dev), &ws);
+    if (L.kernel == TOPK_F32) {                        // zero padding of the last tiles (the fp16 split writes its own)
+        DSPX_CUDA_CHECK(cudaMemsetAsync(ws.qf, 0, ws.qf_bytes, st));
+        DSPX_CUDA_CHECK(cudaMemsetAsync(ws.dbf, 0, ws.dbf_bytes, st));
     }
+    normalize_rows(L.kernel, q_dev, dtype, nq, dim, L.kernel == TOPK_TC ? TC_QT : TKF_QPC, ws.qn, ws.qf, st);
+    normalize_rows(L.kernel, db_dev, dtype, ndb, dim, TK_ROWS, ws.dbn, ws.dbf, st);
     DSPX_CUDA_CHECK(cudaGetLastError());
 
     TopkParams tp{};
-    tp.qn = qn;
-    tp.dbn = dbn;
+    tp.qn = ws.qn;
+    tp.dbn = ws.dbn;
     tp.nq = nq;
     tp.ndb = ndb;
     tp.dim = dim;
     tp.k = k;
-    tp.n_splits = topk_splits(nq, ndb, sm);
-    int64_t rps = (ndb + tp.n_splits - 1) / tp.n_splits;
-    rps = (rps + TK_ROWS - 1) / TK_ROWS * TK_ROWS;
-    tp.rows_per_split = rps;
-    tp.n_splits = (int)((ndb + rps - 1) / rps);
-    tp.idx_out = tp.n_splits == 1 ? idx_out_dev : pidx;
-    tp.score_out = tp.n_splits == 1 ? score_out_dev : pscore;
-    dim3 grid((unsigned)((nq + TK_QPC - 1) / TK_QPC), (unsigned)tp.n_splits);
-    if (use_tc || prefilter) {
-        // one CTA per SM: pick the split count whose grid fills whole waves (every extra split also restarts
-        // the running lists, which costs insertions -- the per-split penalty)
-        const int64_t qtiles = use_tc ? (nq + TC_QT - 1) / TC_QT : (nq + TKF_QPC - 1) / TKF_QPC;
-        int64_t max_sp = (ndb + 8 * TK_ROWS - 1) / (8 * TK_ROWS);
-        if (max_sp > 16) max_sp = 16;
-        if (max_sp < 1) max_sp = 1;
-        int64_t sp = 1;
-        double best = 1e30;
-        for (int64_t c = 1; c <= max_sp; c++) {
-            const double waves = (double)((qtiles * c + sm - 1) / sm);
-            const double cost = waves / (double)c * (1.0 + 0.02 * (double)c);
-            if (cost < best - 1e-12) { best = cost; sp = c; }
-        }
-        if (knobs.splits >= 1 && knobs.splits <= TK_MAX_SPLITS) sp = knobs.splits;      // tuning knob
-        int64_t rows = (ndb + sp - 1) / sp;
-        rows = (rows + TK_ROWS - 1) / TK_ROWS * TK_ROWS;
-        tp.rows_per_split = rows;
-        tp.n_splits = (int)((ndb + rows - 1) / rows);
-        tp.idx_out = tp.n_splits == 1 ? idx_out_dev : pidx;
-        tp.score_out = tp.n_splits == 1 ? score_out_dev : pscore;
-        if (use_tc) {
-            TopkTcParams cp{};
-            cp.base = tp;
-            cp.qx = reinterpret_cast<const unsigned char *>(qf_t);
-            cp.dbx = reinterpret_cast<const unsigned char *>(dbf_t);
-            cp.shared_thr = tp.n_splits > 1 ? shared_thr : nullptr;
-            cp.done = tp.n_splits > 1 ? split_done : nullptr;
-            if (cp.done) DSPX_CUDA_CHECK(cudaMemsetAsync(split_done, 0, (size_t)qtiles * tp.n_splits * 4, st));
+    tp.n_splits = L.n_splits;
+    tp.rows_per_split = L.rows_per_split;
+    tp.idx_out = L.n_splits == 1 ? idx_out_dev : ws.pidx;
+    tp.score_out = L.n_splits == 1 ? score_out_dev : ws.pscore;
+    int rc;
+    if (L.kernel == TOPK_TC) {
+        TopkTcParams cp{};
+        cp.base = tp;
+        cp.qx = reinterpret_cast<const unsigned char *>(ws.qf);
+        cp.dbx = reinterpret_cast<const unsigned char *>(ws.dbf);
+        if (L.n_splits > 1) {
+            cp.shared_thr = ws.shared_thr;
+            cp.done = ws.split_done;
+            DSPX_CUDA_CHECK(cudaMemsetAsync(ws.split_done, 0, (size_t)L.grid.x * L.n_splits * 4, st));
 #ifdef DSPX_TC_PROFILE                  // profiling builds only: DSPX_EXPERIMENT_KEEP_THR=1 keeps the thresholds of the previous call (steady-state per-role cycles)
-            if (cp.shared_thr && !getenv("DSPX_EXPERIMENT_KEEP_THR"))
-#else
-            if (cp.shared_thr)
+            if (!getenv("DSPX_EXPERIMENT_KEEP_THR"))
 #endif
-                DSPX_CUDA_CHECK(cudaMemsetAsync(shared_thr, 0, (size_t)nq * 8, st));
-            dim3 cgrid((unsigned)qtiles, (unsigned)tp.n_splits);
-            const size_t smem = topk_tc_smem_bytes(k);
-            if (dim == 26) {
-                { static std::atomic<unsigned char> optin[64]; DSPX_CUDA_CHECK(optin_max_smem(cosine_topk_tc_kernel<26>, optin, dev)); }
-                cosine_topk_tc_kernel<26><<<cgrid, TC_THREADS, smem, st>>>(cp);
-            } else {
-                { static std::atomic<unsigned char> optin[64]; DSPX_CUDA_CHECK(optin_max_smem(cosine_topk_tc_kernel<0>, optin, dev)); }
-                cosine_topk_tc_kernel<0><<<cgrid, TC_THREADS, smem, st>>>(cp);
-            }
-        } else {
+                DSPX_CUDA_CHECK(cudaMemsetAsync(ws.shared_thr, 0, (size_t)nq * 8, st));
+        }
+        rc = L.cw == 26 ? topk_launch<cosine_topk_tc_kernel<26>>(L, cp, dev, st)
+                        : topk_launch<cosine_topk_tc_kernel<0>>(L, cp, dev, st);
+    } else if (L.kernel == TOPK_F32) {
         TopkF32Params fp{};
         fp.base = tp;
-        fp.qf_t = qf_t;
-        fp.dbf_t = dbf_t;
+        fp.qf_t = ws.qf;
+        fp.dbf_t = ws.dbf;
         fp.eps = 4e-6f + (float)dim * 1.2e-7f;         // > 2 * 2^-24 * (dim + 2): bound on |s32 - s64| for unit vectors
-        dim3 fgrid((unsigned)qtiles, (unsigned)tp.n_splits);
-        if (dim == 26) {
-            const size_t smem = topk_f32_smem_bytes(dim, k, 26);
-            { static std::atomic<unsigned char> optin[64]; DSPX_CUDA_CHECK(optin_max_smem(cosine_topk_f32_kernel<26>, optin, dev)); }
-            cosine_topk_f32_kernel<26><<<fgrid, TKF_WARPS * 32, smem, st>>>(fp);
-        } else {
-            const size_t smem = topk_f32_smem_bytes(dim, k, 32);
-            { static std::atomic<unsigned char> optin[64]; DSPX_CUDA_CHECK(optin_max_smem(cosine_topk_f32_kernel<32>, optin, dev)); }
-            cosine_topk_f32_kernel<32><<<fgrid, TKF_WARPS * 32, smem, st>>>(fp);
-        }
-        }
-    } else if (dim == 26) {                            // MFCC embeddings: 2 x 13, the whole vector in one chunk
-        const size_t smem = topk_smem_bytes(dim, k, 26);
-        { static std::atomic<unsigned char> optin[64]; DSPX_CUDA_CHECK(optin_max_smem(cosine_topk_kernel<26>, optin, dev)); }
-        cosine_topk_kernel<26><<<grid, TK_WARPS * 32, smem, st>>>(tp);
+        rc = L.cw == 26 ? topk_launch<cosine_topk_f32_kernel<26>>(L, fp, dev, st)
+                        : topk_launch<cosine_topk_f32_kernel<32>>(L, fp, dev, st);
     } else {
-        const size_t smem = topk_smem_bytes(dim, k, 32);
-        { static std::atomic<unsigned char> optin[64]; DSPX_CUDA_CHECK(optin_max_smem(cosine_topk_kernel<32>, optin, dev)); }
-        cosine_topk_kernel<32><<<grid, TK_WARPS * 32, smem, st>>>(tp);
+        rc = L.cw == 26 ? topk_launch<cosine_topk_kernel<26>>(L, tp, dev, st)
+                        : topk_launch<cosine_topk_kernel<32>>(L, tp, dev, st);
     }
-    DSPX_CUDA_CHECK(cudaGetLastError());
-    if (tp.n_splits > 1) {
-        topk_merge_kernel<<<(unsigned)((nq + 3) / 4), 128, 0, st>>>(pidx, pscore, nq, tp.n_splits, k, idx_out_dev, score_out_dev);
+    if (rc != DSPX_OK) return rc;
+    if (L.n_splits > 1) {
+        topk_merge_kernel<<<(unsigned)((nq + 3) / 4), 128, 0, st>>>(ws.pidx, ws.pscore, nq, L.n_splits, k, idx_out_dev, score_out_dev);
         DSPX_CUDA_CHECK(cudaGetLastError());
     }
     return DSPX_OK;
@@ -1267,18 +1289,12 @@ int dspx_cosine_matrix(const void *q_dev, int64_t nq, const void *db_dev, int64_
     DSPX_REQUIRE(workspace_bytes >= dspx_cosine_topk_workspace(nq, ndb, dim, 1), "workspace too small");
     if (nq == 0 || ndb == 0) return DSPX_OK;
     cudaStream_t st = static_cast<cudaStream_t>(stream);
-    char *ws = static_cast<char *>(workspace_dev);
-    double *qn = reinterpret_cast<double *>(ws);
-    double *dbn = reinterpret_cast<double *>(ws + align256((size_t)nq * dim * 8));
-    if (dtype == DSPX_DTYPE_F32) {
-        normalize_rows_kernel<float><<<(unsigned)((nq + 127) / 128), 128, 0, st>>>((const float *)q_dev, nq, dim, qn);
-        normalize_rows_kernel<float><<<(unsigned)((ndb + 127) / 128), 128, 0, st>>>((const float *)db_dev, ndb, dim, dbn);
-    } else {
-        normalize_rows_kernel<double><<<(unsigned)((nq + 127) / 128), 128, 0, st>>>((const double *)q_dev, nq, dim, qn);
-        normalize_rows_kernel<double><<<(unsigned)((ndb + 127) / 128), 128, 0, st>>>((const double *)db_dev, ndb, dim, dbn);
-    }
+    TopkWs ws;
+    topk_ws_carve(nq, ndb, dim, 1, static_cast<char *>(workspace_dev), &ws);
+    normalize_rows(TOPK_F64, q_dev, dtype, nq, dim, 0, ws.qn, nullptr, st);
+    normalize_rows(TOPK_F64, db_dev, dtype, ndb, dim, 0, ws.dbn, nullptr, st);
     dim3 grid((unsigned)((ndb + 255) / 256), (unsigned)nq);
-    cosine_matrix_kernel<<<grid, 256, 0, st>>>(qn, dbn, nq, ndb, dim, sims_out_dev);
+    cosine_matrix_kernel<<<grid, 256, 0, st>>>(ws.qn, ws.dbn, nq, ndb, dim, sims_out_dev);
     DSPX_CUDA_CHECK(cudaGetLastError());
     return DSPX_OK;
 }

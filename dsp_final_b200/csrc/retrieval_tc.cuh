@@ -78,25 +78,13 @@ constexpr int TC_EPI_THREADS = 256;
 constexpr int TC_THREADS = TC_EPI_THREADS + 32 + 64;      // + bulk-copy warp + two tensor-core issue warps (one per query half)
 constexpr int TC_KPAD = 32;           // padded embedding dimension: 32 hi + 32 lo halves = one 128-byte swizzle row
 constexpr int TC_TILE_BYTES = 128 * 128;                  // operand image of 128 rows
-#ifndef DSPX_TC_EPS
-#define DSPX_TC_EPS 6e-6
-#endif
-constexpr double TC_EPS = DSPX_TC_EPS;
+constexpr double TC_EPS = 6e-6;
 constexpr float TC_S = 2048.f;                            // operand scale S = 2^11
 constexpr float TC_SCALE = TC_S * TC_S;                   // the accumulator holds S^2 * score
-#ifndef DSPX_TC_TRIGGER_LANE
-#define DSPX_TC_TRIGGER_LANE 8
-#endif
-#ifndef DSPX_TC_TRIGGER_WARP
-#define DSPX_TC_TRIGGER_WARP 64
-#endif
-// pending candidates per query: ring size; the warp re-scores when one ring holds TRIGGER_LANE rows or all 32 rings together
-// hold TRIGGER_WARP (one full scoring pass)
-constexpr int TC_FIFO = 8, TC_FIFO_TRIGGER = DSPX_TC_TRIGGER_LANE, TC_WARP_TRIGGER = DSPX_TC_TRIGGER_WARP;
-#ifndef DSPX_TC_IDLE_CYCLES
-#define DSPX_TC_IDLE_CYCLES 3500
-#endif
-constexpr long long TC_IDLE_CYCLES = DSPX_TC_IDLE_CYCLES;   // wait on acc_full after which an epilogue warp uses the stall to re-score
+// pending candidates per query: ring size; the warp re-scores when one ring holds TC_FIFO_TRIGGER rows or all 32 rings
+// together hold TC_WARP_TRIGGER (one full scoring pass)
+constexpr int TC_FIFO = 8, TC_FIFO_TRIGGER = 8, TC_WARP_TRIGGER = 64;
+constexpr long long TC_IDLE_CYCLES = 3500;   // wait on acc_full after which an epilogue warp uses the stall to re-score
 constexpr int TC_MAX_K = 24;          // the per-thread lists ([k][256] doubles + ints) share smem with the tiles
 
 // Rows scaled by 1 / (||row|| + 1e-10) in float64 (src/retrieval/retrieval.py:46-48: the division, not a multiply by
@@ -210,15 +198,10 @@ __device__ __forceinline__ void tc_mbar_wait(uint64_t *bar, uint32_t parity)
 {
     for (uint32_t spin = 0;; spin++) {
         uint32_t ok;
-#ifdef DSPX_TC_TESTWAIT
-        asm volatile("{ .reg .pred p; mbarrier.test_wait.parity.shared::cta.b64 p, [%1], %2; selp.u32 %0, 1, 0, p; }"
-                     : "=r"(ok) : "r"(tc_smem_u32(bar)), "r"(parity) : "memory");
-#else
         // the suspend-time hint lets the hardware park the thread instead of re-issuing the wait: the two single-thread
         // roles share their schedulers with epilogue warps 0/4 and 1/5, which the issue thread ends up waiting for
         asm volatile("{ .reg .pred p; mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2, %3; selp.u32 %0, 1, 0, p; }"
                      : "=r"(ok) : "r"(tc_smem_u32(bar)), "r"(parity), "r"(0x989680u) : "memory");
-#endif
         if (ok) return;
         if (spin > (1u << 28)) __trap();
     }
@@ -399,9 +382,6 @@ __global__ void __launch_bounds__(TC_THREADS, 1) cosine_topk_tc_kernel(const Top
         // the rounds.  Each lane sees its rows in increasing order.
         int f_head = 0, f_cnt = 0, wpos = 0;
         bool thr_dirty = false;                                    // the list's k-th score or fill count changed since thr32c was formed
-#ifdef DSPX_TC_EXPERIMENT_NODRAIN
-        bool t_nodrain_skip = false;
-#endif
         int32_t *fifo = s_fifo + ql;
         // One exactly scored row into the thread's list.  Rows reach a list in an order in which every entry already there
         // with the same score has a lower index (own rows: increasing index; rows taken over from finished splits: see below).
@@ -505,9 +485,6 @@ __global__ void __launch_bounds__(TC_THREADS, 1) cosine_topk_tc_kernel(const Top
         // some lane has a hit or 'force': every exit leaves all rings below their trigger (drain() empties them), so a tile
         // without a hit has nothing to do here.
         auto enqueue = [&](uint32_t (&m)[4], int64_t tile, bool force) {
-#ifdef DSPX_TC_EXPERIMENT_NODRAIN        // timing only (results are wrong): the scan + tensor-core pipeline without re-scoring
-            if (t_nodrain_skip) { m[0] = m[1] = m[2] = m[3] = 0u; }
-#endif
             for (;;) {
 #pragma unroll
                 for (int cb = 0; cb < 4; cb++) {
@@ -636,13 +613,8 @@ __global__ void __launch_bounds__(TC_THREADS, 1) cosine_topk_tc_kernel(const Top
                 if (lane == 0) tc_mbar_arrive(&my_empty[buf]);
                 if (lane == 0) TC_TRACE(t, 10 + warp);
                 released = true;
-#ifdef DSPX_TC_EXPERIMENT_NOSCAN         // timing only (results are wrong): TMEM read-out and hand-off without the scan
-                const float t0 = __uint_as_float(v0[5] ^ v1[9] ^ v2[17] ^ v3[31]), t1 = t0, t2 = t0, t3 = t0;
-                any_hit = __any_sync(0xffffffffu, t >= 4 ? (t0 == 123.456f) : (t0 > thr32));
-#else
                 const float t0 = tc_top32(v0), t1 = tc_top32(v1), t2 = tc_top32(v2), t3 = tc_top32(v3);
                 any_hit = __any_sync(0xffffffffu, fmaxf(fmaxf(t0, t1), fmaxf(t2, t3)) > thr32);
-#endif
                 if (any_hit) {
                     if (__any_sync(0xffffffffu, t0 > thr32)) m[0] = tc_bits32(v0, thr32);
                     if (__any_sync(0xffffffffu, t1 > thr32)) m[1] = tc_bits32(v1, thr32);
@@ -657,9 +629,6 @@ __global__ void __launch_bounds__(TC_THREADS, 1) cosine_topk_tc_kernel(const Top
                 if (lane == 0) TC_TRACE(t, 10 + warp);
             }
             TC_PROF_ADD(6);
-#ifdef DSPX_TC_EXPERIMENT_NODRAIN
-            t_nodrain_skip = t >= 4;
-#endif
             {
                 const bool force = t < 4 || t == n_tiles - 1;
                 if (any_hit || force) enqueue(m, tile, force);

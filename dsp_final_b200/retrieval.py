@@ -100,6 +100,20 @@ def _dev_matrix(x):
     return t, (_lib.DTYPE_F32 if t.dtype == torch.float32 else _lib.DTYPE_F64)
 
 
+def _dev_pair(a, b):
+    """-> (a, b, dtype code): both as _dev_matrix, in float64 when their dtypes differ; their dimensions must match."""
+    import torch
+
+    q, dq = _dev_matrix(a)
+    db, dd = _dev_matrix(b)
+    if dq != dd:
+        q, db = q.to(torch.float64), db.to(torch.float64)
+        dq = _lib.DTYPE_F64
+    if q.shape[1] != db.shape[1]:
+        raise ValueError("query and database embeddings differ in dimension")
+    return q, db, dq
+
+
 def cosine_topk(query_embeddings, db_embeddings, k: int, return_scores: bool = False):
     """Indices [nq, k] (int32) of the k most similar database rows per query, best first.
 
@@ -111,13 +125,7 @@ def cosine_topk(query_embeddings, db_embeddings, k: int, return_scores: bool = F
     _lib.require_device()
     lib = _lib.load()
     host = not _is_cuda_tensor(query_embeddings)
-    q, dq = _dev_matrix(query_embeddings)
-    db, dd = _dev_matrix(db_embeddings)
-    if dq != dd:
-        q, db = q.to(torch.float64), db.to(torch.float64)
-        dq = _lib.DTYPE_F64
-    if q.shape[1] != db.shape[1]:
-        raise ValueError("query and database embeddings differ in dimension")
+    q, db, dq = _dev_pair(query_embeddings, db_embeddings)
     nq, dim = q.shape
     ndb = db.shape[0]
     k = int(min(k, ndb))
@@ -150,11 +158,7 @@ def cosine_similarity(a: np.ndarray, b: np.ndarray) -> np.ndarray:
     _lib.require_device()
     lib = _lib.load()
     host = not _is_cuda_tensor(a)
-    q, dq = _dev_matrix(a)
-    db, dd = _dev_matrix(b)
-    if dq != dd:
-        q, db = q.to(torch.float64), db.to(torch.float64)
-        dq = _lib.DTYPE_F64
+    q, db, dq = _dev_pair(a, b)
     nq, dim = q.shape
     ndb = db.shape[0]
     dev = q.device.index
@@ -198,18 +202,10 @@ def hits_at_k(topk_idx, k: int, targets_db, targets_query) -> int:
 
     _lib.require_device()
     idx = topk_idx if _is_cuda_tensor(topk_idx) else torch.as_tensor(np.ascontiguousarray(topk_idx, dtype=np.int32)).cuda()
-    idx = idx.to(torch.int32).contiguous()
     dev = idx.device
     tdb = torch.as_tensor(np.asarray(targets_db.cpu() if _is_cuda_tensor(targets_db) else targets_db, dtype=np.int32)).to(dev)
     tq = torch.as_tensor(np.asarray(targets_query.cpu() if _is_cuda_tensor(targets_query) else targets_query, dtype=np.int32)).to(dev)
-    if k > idx.shape[1]:
-        raise ValueError("k exceeds the width of topk_idx")
-    with torch.cuda.device(dev.index):
-        hits = torch.zeros(1, dtype=torch.int64, device=dev)
-        _lib.check(_lib.load().dspx_hits_at_k(idx.data_ptr(), idx.shape[0], idx.shape[1], int(k), tdb.data_ptr(),
-                                              tq.data_ptr(), hits.data_ptr(),
-                                              torch.cuda.current_stream(dev.index).cuda_stream), "dspx_hits_at_k")
-    return int(hits.item())
+    return int(hits_at_k_device(idx, [k], tdb, tq).item())
 
 
 def evaluate_retrieval(db_items: List[Any], query_items: List[Any], db_embeddings, query_embeddings,

@@ -262,6 +262,8 @@ def test_retrieval_golden_bit_exact(torch_cuda, golden_retrieval):
     np.testing.assert_allclose(sims, qn @ dn.T, rtol=0, atol=1e-14)
     idx, sc = R.cosine_topk(q.astype(np.float64), db.astype(np.float64), 20, return_scores=True)
     assert np.array_equal(np.take_along_axis(sims, idx.astype(np.int64), axis=1), sc)
+    with pytest.raises(ValueError):
+        R.cosine_similarity(q, db[:, :13])
 
 
 @pytest.mark.parametrize("nq,ndb,dim,k", [(1, 20, 26, 20), (63, 129, 26, 1), (400, 1600, 26, 20), (130, 40_000, 26, 20),

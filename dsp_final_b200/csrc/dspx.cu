@@ -215,7 +215,8 @@ static int features_device(const dspx_plan *pl, const float *clips, int64_t n_cl
                                      fused ? W8_WANT_EMBED : W8_WANT_FEATURES);
     if (path == W8_UNSUPPORTED) {
         set_error("embeddings without an MFCC buffer need the warp8 kernel (n_fft 512 / 1024 / 2048), frame_length = "
-                  "n_fft, an even hop and row stride and 8-byte aligned clips");
+                  "n_fft, an even hop and row stride, 8-byte aligned clips and at most %lld frames per clip",
+                  (long long)w8_embed_max_frames(pl->cfg.n_mels));
         return DSPX_EUNSUPPORTED;
     }
     const int C = pl->cfg.n_mfcc;
@@ -284,16 +285,25 @@ struct RaggedWs {
     float *f32 = nullptr;
 };
 
-static W8Path ragged_path(const dspx_plan *pl, int dtype, W8Want want)
+// the path of a ragged batch whose longest clip has max_frames frames
+static W8Path ragged_path(const dspx_plan *pl, int dtype, W8Want want, int64_t max_frames)
 {
-    return warp8_select(pl, nullptr, 0, dtype, true, 0, 0, want);
+    return warp8_select(pl, nullptr, 0, dtype, true, 0, max_frames, want);
+}
+
+static int64_t ragged_max_frames(const dspx_ragged_clip *tab, int64_t n_clips)
+{
+    int64_t m = 0;
+    for (int64_t i = 0; i < n_clips; i++) m = std::max(m, tab[i].n_frames);
+    return m;
 }
 
 static size_t ragged_ws_carve(const dspx_plan *pl, const dspx_ragged_clip *tab, int64_t n_clips, int dtype, int normalize,
                               bool want_mfcc, bool want_embed, char *base, RaggedWs *ws)
 {
-    const bool pcm = dtype == DSPX_DTYPE_PCM16, rk = ragged_path(pl, dtype, W8_WANT_FEATURES) != W8_UNSUPPORTED;
-    const bool fused = want_embed && !want_mfcc && ragged_path(pl, dtype, W8_WANT_EMBED) != W8_UNSUPPORTED;
+    const int64_t max_frames = ragged_max_frames(tab, n_clips);
+    const bool pcm = dtype == DSPX_DTYPE_PCM16, rk = ragged_path(pl, dtype, W8_WANT_FEATURES, max_frames) != W8_UNSUPPORTED;
+    const bool fused = want_embed && !want_mfcc && ragged_path(pl, dtype, W8_WANT_EMBED, max_frames) != W8_UNSUPPORTED;
     int64_t total_frames = 0, max_len = 0;
     if (n_clips > 0) total_frames = tab[n_clips - 1].first_frame + tab[n_clips - 1].n_frames;
     for (int64_t i = 0; i < n_clips; i++) max_len = std::max(max_len, tab[i].length);
@@ -349,7 +359,7 @@ static int features_ragged(const dspx_plan *pl, const void *samples, int dtype, 
     RaggedWs ws;
     ragged_ws_carve(pl, tab, n_clips, dtype, normalize, mfcc != nullptr, embed != nullptr, ws_base, &ws);
     const bool fused = ws.eacc != nullptr;                   // embeddings alone, accumulated inside the feature kernel
-    const W8Path path = ragged_path(pl, dtype, fused ? W8_WANT_EMBED : W8_WANT_FEATURES);
+    const W8Path path = ragged_path(pl, dtype, fused ? W8_WANT_EMBED : W8_WANT_FEATURES, ragged_max_frames(tab, n_clips));
     if (path == W8_UNSUPPORTED)
         return features_ragged_per_clip(pl, samples, pcm, normalize, tab_dev, tab, n_clips, logmel, mfcc, embed, ws, st);
     const int C = pl->cfg.n_mfcc;
@@ -850,6 +860,8 @@ int dspx_plan_create(const dspx_config *cfg, int device, dspx_plan **out)
         } else if (ok) {
             rc = warp8_prepare(p);
             if (rc == DSPX_OK) p->kernel = DSPX_KERNEL_WARP8;
+            // tables too large for shared memory (e.g. 256 mels at n_fft 1024, 128 mels at 4096): the generic kernel
+            else if (rc == DSPX_EUNSUPPORTED && cfg->kernel != DSPX_KERNEL_WARP8) rc = DSPX_OK;
         }
     }
     if (rc != DSPX_OK) {

@@ -217,6 +217,29 @@ int emu_warp8_layout(const dspx_config *cfg, int32_t *out)
     return DSPX_OK;
 }
 
+// The CTA shapes a plan of feat_warp8_kernel can launch (warp8_shapes): out = {table bytes, shared memory of the 8-,
+// 20-, 12- and 10-warp configurations (0 where one does not fit), 8-warp CTAs per SM, first-pass radix, x2 (n_fft 4096)}
+int emu_warp8_shapes(const dspx_config *cfg, int64_t *out)
+{
+    EmuTables e;
+    int rc = emu_build(cfg, e);
+    if (rc != DSPX_OK) return rc;
+    dspx_plan pl;
+    pl.cfg = *cfg;
+    pl.P = e.P;
+    pl.M = e.M;
+    pl.n_bins = e.n_bins;
+    pl.host = e.t;
+    if (!warp8_supported(&pl)) return DSPX_EUNSUPPORTED;
+    std::vector<float> blob;
+    W8Tables tb{};
+    warp8_build_tables(&pl, blob, tb);
+    const W8Shapes s = warp8_shapes(tb, cfg->n_mels);
+    out[0] = (int64_t)tb.total * 4; out[1] = s.smem; out[2] = s.smem_wide; out[3] = s.smem_mid; out[4] = s.smem_r16;
+    out[5] = s.ctas_per_sm; out[6] = tb.r1; out[7] = tb.x2;
+    return DSPX_OK;
+}
+
 // Replays feat_warp8_kernel: one "warp" at a time, each phase run for lanes 0..31 in turn
 // (a __syncwarp() separates the phases on the device).  rtab != NULL replays the RAGGED variant over a
 // dspx_ragged_layout table (clip_len and clip_stride unused).

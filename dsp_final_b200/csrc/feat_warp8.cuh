@@ -843,8 +843,26 @@ DSPX_HD float2 w8_dct_partial(const W8Ctx &c, int lane, int c0)
 // without an MFCC round trip through HBM: every frame adds x and x^2 to per-clip accumulators.  The sums are kept
 // in 64-bit FIXED POINT (x * 2^32, x^2 * 2^20) so that the atomic adds commute exactly -- the result does not
 // depend on the order in which warps finish -- and embed_finalize_kernel turns them into mean / std in float64.
-// Range: |x| < 2^15 over 2^15 frames; resolution 2^-33 per x, 2^-21 per x^2 (std error < 1e-6 for std > 0.01).
+// Resolution 2^-33 per x, 2^-21 per x^2 (std error < 1e-6 for std > 0.01).  Range: a frame adds at most
+// |x| 2^32 + 1/2 and x^2 2^20 + 1/2 to a sum, so a clip of n frames stays exact while n (x^2 2^20 + 1/2) < 2^63 and
+// n (|x| 2^32 + 1/2) < 2^63 (|x| < 2^15 allows 2^11 frames, not 2^15).  w8_embed_max_frames bounds n from a bound on
+// |x|; warp8_select refuses the fused path beyond it.
 constexpr double W8_EFIX1 = 4294967296.0, W8_EFIX2 = 1048576.0;
+
+// The bound on |x|.  A coefficient is C_k = sum_f 2 cos(pi k (f + 1/2) / n_mels) lm_f, so |C_k| <= 2 n_mels max|lm|.
+// A log-mel value is at least ln 1e-10 = -23.03.  From above: the triangles weigh every bin by at most 1 and the
+// one-sided power spectrum of a frame sums to at most n_fft sum_n (w_n y_n)^2 <= (2 n_fft max|x|)^2 (Parseval, window
+// <= 1, pre-emphasis y_n = x_n - alpha x_{n-1} with alpha <= 1), so lm <= ln(4 n_fft^2 max|x|^2) = 38.8 for samples
+// within +-2^16 at n_fft 2048.  Hence |lm| <= 40 and |C_k| <= 80 n_mels for such input.
+constexpr double W8_EMBED_LOGMEL_MAX = 40.0;
+
+// The most frames a clip may have for the fused sums to stay exact (n_mels 40: 671 087, 128: 83 885, 256: 20 970).
+inline int64_t w8_embed_max_frames(int n_mels)
+{
+    const double c = 2.0 * n_mels * W8_EMBED_LOGMEL_MAX;
+    const double per_frame = std::max(c * W8_EFIX1, c * c * W8_EFIX2) + 0.5;
+    return (int64_t)(9223372036854775808.0 / per_frame) - 1;
+}
 
 // Out of line on the device: the float64 / 64-bit integer code must not take part in the register allocation of
 // the main loop (inlined it cost the headline kernel 36 bytes of spills); it runs once per frame pair on 13 lanes.
@@ -1118,9 +1136,10 @@ enum W8Path {
 };
 
 // The one place that picks the kernel of a call.  samples, row_stride (in samples of `dtype`), n_clips and T (frames
-// per clip) describe an equal-length batch; a ragged batch ignores them: its layout holds fewer than 2^31 frame pairs
-// and starts float32 clips on the 8-byte grid (dspx_ragged_layout, dspx_features_ragged).  A ragged batch on a plan
-// without a ragged kernel (the generic kernel, n_fft 4096) gets W8_UNSUPPORTED and runs one clip at a time.
+// per clip) describe an equal-length batch; a ragged batch ignores all but T, the frame count of its longest clip: its
+// layout holds fewer than 2^31 frame pairs and starts float32 clips on the 8-byte grid (dspx_ragged_layout,
+// dspx_features_ragged).  A ragged batch on a plan without a ragged kernel (the generic kernel, n_fft 4096) gets
+// W8_UNSUPPORTED and runs one clip at a time.  Fused embeddings need clips of at most w8_embed_max_frames frames.
 inline W8Path warp8_select(const dspx_plan *pl, const void *samples, int64_t row_stride, int dtype, bool ragged,
                            int64_t n_clips, int64_t T, W8Want want)
 {
@@ -1140,7 +1159,7 @@ inline W8Path warp8_select(const dspx_plan *pl, const void *samples, int64_t row
     const bool aligned = fits && pl->cfg.frame_length == pl->P && !(pl->cfg.hop_length & 1) &&
                          (ragged || (!(row_stride & 1) && !(reinterpret_cast<uintptr_t>(samples) & 7)));
     const W8Path fast = 2 * pl->cfg.hop_length == pl->P && warp8_radix(pl) != 16 ? W8_SHARE : W8_ALIGNED;
-    if (want == W8_WANT_EMBED) return aligned ? fast : W8_UNSUPPORTED;
+    if (want == W8_WANT_EMBED) return aligned && T <= w8_embed_max_frames(pl->cfg.n_mels) ? fast : W8_UNSUPPORTED;
     if (want == W8_WANT_STFT) return aligned && pl->take_stft == pl->P ? fast : W8_GENERIC;
     return aligned ? fast : (fits ? W8_U4 : W8_GENERIC);
 }
@@ -1515,15 +1534,33 @@ inline size_t warp8_smem_bytes(const W8Tables &tb, int n_mels, int n_warps = W8_
     return ((size_t)tb.total + (size_t)n_warps * w8_warp_floats(tb, n_mels)) * sizeof(float);
 }
 
-// ---- launch (not in csrc/emu.cu, which replays the phase functions on the host and instantiates no kernel) --------
-#if defined(__CUDACC__) && !defined(DSPX_EMU)
-struct W8PlanData {
-    W8Tables tb;
+// The CTA shapes a plan can launch, chosen from its table size when it is built (w8_launch_cfg picks among them)
+struct W8Shapes {
     int ctas_per_sm;
-    size_t smem;
+    size_t smem;             // the W8_WARPS-warp configuration; more than 227 KB: the plan cannot use warp8
     size_t smem_wide;        // 0 when the 20-warp configuration does not fit
     size_t smem_mid;         // shared memory of the W8_WARPS_MID-warp configuration (used when the wide one does not fit), or 0
     size_t smem_r16;         // n_fft 2048: shared memory of the W8_WARPS_R16-warp configuration, 0 when it does not fit
+};
+
+inline W8Shapes warp8_shapes(const W8Tables &tb, int n_mels)
+{
+    W8Shapes s{};
+    s.smem = warp8_smem_bytes(tb, n_mels);
+    s.ctas_per_sm = (tb.r1 != 16 && s.smem * 2 + 2048 <= 227 * 1024) ? 2 : 1;   // (x2 plans have r1 = 16: one CTA)
+    const size_t wide = warp8_smem_bytes(tb, n_mels, W8_WARPS_WIDE);
+    s.smem_wide = (tb.r1 != 16 && wide + 1024 <= 227 * 1024) ? wide : 0;
+    const size_t mid = warp8_smem_bytes(tb, n_mels, W8_WARPS_MID);
+    s.smem_mid = (tb.r1 != 16 && !s.smem_wide && s.ctas_per_sm == 1 && mid + 1024 <= 227 * 1024) ? mid : 0;
+    const size_t r16 = warp8_smem_bytes(tb, n_mels, W8_WARPS_R16);
+    s.smem_r16 = (tb.r1 == 16 && !tb.x2 && W8_WARPS_R16 > W8_WARPS && r16 + 1024 <= 227 * 1024) ? r16 : 0;
+    return s;
+}
+
+// ---- launch (not in csrc/emu.cu, which replays the phase functions on the host and instantiates no kernel) --------
+#if defined(__CUDACC__) && !defined(DSPX_EMU)
+struct W8PlanData : W8Shapes {
+    W8Tables tb;
 };
 
 inline int warp8_prepare(dspx_plan *pl)
@@ -1531,18 +1568,11 @@ inline int warp8_prepare(dspx_plan *pl)
     std::vector<float> blob;
     W8Tables tb{};
     warp8_build_tables(pl, blob, tb);
-    const size_t smem = warp8_smem_bytes(tb, pl->cfg.n_mels);
-    if (smem > 227 * 1024) { set_error("warp8: tables too large for shared memory"); return DSPX_EUNSUPPORTED; }
+    const W8Shapes shapes = warp8_shapes(tb, pl->cfg.n_mels);
+    if (shapes.smem > 227 * 1024) { set_error("warp8: tables too large for shared memory"); return DSPX_EUNSUPPORTED; }
     auto *pd = new W8PlanData();
+    static_cast<W8Shapes &>(*pd) = shapes;
     pd->tb = tb;
-    pd->smem = smem;
-    pd->ctas_per_sm = (tb.r1 != 16 && smem * 2 + 2048 <= 227 * 1024) ? 2 : 1;   // (x2 plans have r1 = 16: one CTA)
-    const size_t wide = warp8_smem_bytes(tb, pl->cfg.n_mels, W8_WARPS_WIDE);
-    pd->smem_wide = (tb.r1 != 16 && wide + 1024 <= 227 * 1024) ? wide : 0;
-    const size_t mid = warp8_smem_bytes(tb, pl->cfg.n_mels, W8_WARPS_MID);
-    pd->smem_mid = (tb.r1 != 16 && !pd->smem_wide && pd->ctas_per_sm == 1 && mid + 1024 <= 227 * 1024) ? mid : 0;
-    const size_t r16 = warp8_smem_bytes(tb, pl->cfg.n_mels, W8_WARPS_R16);
-    pd->smem_r16 = (tb.r1 == 16 && !tb.x2 && W8_WARPS_R16 > W8_WARPS && r16 + 1024 <= 227 * 1024) ? r16 : 0;
     pl->fast_host = pd;
     DSPX_CUDA_CHECK(cudaMalloc(&pl->d_fast_tables, blob.size() * sizeof(float)));
     DSPX_CUDA_CHECK(cudaMemcpy(pl->d_fast_tables, blob.data(), blob.size() * sizeof(float), cudaMemcpyHostToDevice));

@@ -120,8 +120,13 @@ int dspx_features(const dspx_plan *plan, const float *clips_dev, int64_t n_clips
  * workspace_dev (order-independent, so results are reproducible) and a finalize step writes
  * embed [n_clips, 2*n_mfcc] f32.  No MFCC tensor is written or read.  logmel_out_dev may be NULL.
  * Runs when the plan uses the warp8 kernel, frame_length equals the transform length (n_fft_pow2) and that is 512,
- * 1024 or 2048, hop_length and clip_stride are even, clips_dev is 8-byte aligned and n_clips * ceil(n_frames / 2)
- * < 2^31.  Otherwise DSPX_EUNSUPPORTED: use dspx_features with an MFCC buffer. */
+ * 1024 or 2048, hop_length and clip_stride are even, clips_dev is 8-byte aligned, n_clips * ceil(n_frames / 2)
+ * < 2^31 and n_frames < floor(2^63 / (max(C 2^32, C^2 2^20) + 1/2)) with C = 80 n_mels (at most 20 970 frames at
+ * 256 mels, 83 885 at 128, 671 087 at 40).  Otherwise DSPX_EUNSUPPORTED: use dspx_features with an MFCC buffer.
+ * That frame bound keeps the 64-bit sums of x 2^32 and x^2 2^20 from overflowing: C bounds every coefficient,
+ * |C_k| <= 2 n_mels max|log-mel|, for log-mel values in [ln 1e-10, 40] = [-23.03, 40], i.e. for samples within
+ * +-2^16 (a log-mel value is at most ln(4 n_fft^2 max|x|^2) = 38.8 there).  Louder input may overflow them on clips
+ * near the bound. */
 size_t dspx_embeddings_workspace(const dspx_plan *plan, int64_t n_clips);
 int dspx_embeddings(const dspx_plan *plan, const float *clips_dev, int64_t n_clips, int64_t clip_len,
                     int64_t clip_stride, float *embed_out_dev, float *logmel_out_dev, void *workspace_dev,

@@ -99,6 +99,13 @@ _SIGNATURES = {
     "dspx_features_ragged_workspace": (_SZ, [_VP, _VP, _I64, _I32, _I32, _I32, _I32, _I32]),
     "dspx_features_ragged": (_I32, [_VP, _VP, _I32, _I32, _VP, _VP, _I64, _I64, _VP, _VP, _VP, _VP, _SZ, _VP]),
     "dspx_embed_stats_ragged": (_I32, [_VP, _VP, _I64, _I32, _VP, _VP]),
+    "dspx_resampler_create": (_I32, [_I64, _I64, _VP, _I64, _I32, C.POINTER(_VP)]),
+    "dspx_resampler_destroy": (_I32, [_VP]),
+    "dspx_resample_len": (_I64, [_VP, _I64]),
+    "dspx_resample_workspace": (_SZ, [_I64]),
+    "dspx_resample": (_I32, [_VP, _VP, _I32, _I64, _I64, _I64, _I32, _VP, _I64, _VP, _SZ, _VP]),
+    "dspx_resample_layout": (_I64, [_I64, _I64, _VP, _VP, _I64, _VP]),
+    "dspx_resample_ragged": (_I32, [_VP, _VP, _I32, _I32, _VP, _VP, _I64, _VP, _VP, _SZ, _VP]),
     "dspx_next_pow_two": (_I64, [_I64]),
     "dspx_fft_c2c": (_I32, [_VP, _I64, _I64, _I64, _I32, _VP, _VP, _VP]),
     "dspx_cosine_topk_workspace": (_SZ, [_I64, _I64, _I32, _I32]),

@@ -114,3 +114,18 @@ def load_pcm16(path: str | Path, target_sr: int | None = None) -> np.ndarray | N
     if tag != ((1 << 8) | 16) or x.shape[1] != 1 or (target_sr is not None and rate != target_sr):
         return None
     return np.ascontiguousarray(x[:, 0])
+
+
+def read_pcm16(path: str | Path) -> Tuple[np.ndarray, int] | None:
+    """(int16 samples, sample_rate) when the file is mono 16-bit PCM at any rate, else None.
+
+    Clips at another rate than the config's can still take the GPU path: features_batch(..., sample_rate=rate)
+    resamples them on the device, bit-identically to load_audio's resample_poly.
+    """
+    try:
+        x, rate, tag = read_wav_raw(path)
+    except ValueError:
+        return None
+    if tag != ((1 << 8) | 16) or x.shape[1] != 1:
+        return None
+    return np.ascontiguousarray(x[:, 0]), rate

@@ -14,6 +14,10 @@ over them and keep the reference signatures.
 
 features_ragged takes clips of different lengths in one call (dspx_features_ragged):
 outputs are stacked along the frame axis and split per clip with "frame_offsets".
+
+resample_poly is scipy.signal.resample_poly on the GPU, bit for bit (dspx_resample).  With sample_rate= the
+clips' own rate, features_batch and features_ragged resample on the device first when it differs from
+cfg.sample_rate (src/utils/audio.py:27-30 resamples on the host there).
 """
 from __future__ import annotations
 
@@ -23,7 +27,7 @@ from typing import Any, Iterable
 import numpy as np
 
 from . import _lib
-from .plan import Plan, config_key, config_struct, get_plan
+from .plan import Plan, Resampler, config_key, config_struct, get_plan, get_resampler, reduce_ratio
 
 FEATURES = ("log_mel", "mfcc", "embed")
 
@@ -82,16 +86,160 @@ def pcm16_to_float(pcm, normalize: bool = True):
     return out
 
 
+def _resample_dtype(x) -> bool:
+    """True for int16 PCM, False for float32; ValueError for anything else (scipy would filter float64 in float64)."""
+    if _is_pcm16(x):
+        return True
+    if str(getattr(x, "dtype", None)) not in ("float32", "torch.float32"):
+        raise ValueError(f"resample_poly takes float32 or int16 samples, not {getattr(x, 'dtype', type(x).__name__)}")
+    return False
+
+
+def _resample_2d(x, rs: Resampler, normalize: bool):
+    """[B, L] torch CUDA float32 / int16 (unit stride) -> [B, n_out] float32 on torch's current stream."""
+    import torch
+
+    lib = _lib.load()
+    pcm = _is_pcm16(x)
+    b, n_in = x.shape
+    if n_in < 1:
+        raise ValueError("resample_poly of an empty clip")
+    n_out = rs.out_len(n_in)
+    dev = x.device.index
+    with torch.cuda.device(dev):
+        out = torch.empty((b, n_out), dtype=torch.float32, device=x.device)
+        ws_bytes = int(lib.dspx_resample_workspace(b))
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=x.device)
+        _lib.check(lib.dspx_resample(rs.handle, x.data_ptr(), _lib.DTYPE_PCM16 if pcm else _lib.DTYPE_F32, b, n_in,
+                                     x.stride(0), 1 if normalize else 0, out.data_ptr(), n_out, ws.data_ptr(), ws_bytes,
+                                     torch.cuda.current_stream(dev).cuda_stream), "dspx_resample")
+    return out
+
+
+def _resample_ragged(xs: list, rs: Resampler, normalize: bool):
+    """1-D torch CUDA clips of one dtype -> (packed float32 output, table int64 [n, 4]): one launch.  Clip i is
+    out[table[i, 2]:table[i, 2] + table[i, 3]]; starts are multiples of RAGGED_ALIGN and the gaps are zero."""
+    import torch
+
+    lib = _lib.load()
+    pcm = _is_pcm16(xs[0])
+    lengths = np.array([len(x) for x in xs], np.int64)
+    starts = np.concatenate(([0], np.cumsum(lengths)[:-1])).astype(np.int64)
+    table = np.zeros((len(xs), 4), np.int64)
+    total = _lib.check(int(lib.dspx_resample_layout(rs.up, rs.down, starts.ctypes.data, lengths.ctypes.data, len(xs),
+                                                    table.ctypes.data)), "dspx_resample_layout")
+    dev = xs[0].device
+    with torch.cuda.device(dev.index):
+        samples = torch.cat(xs)
+        table_dev = torch.from_numpy(table).to(dev)
+        out = torch.zeros(total, dtype=torch.float32, device=dev)
+        ws_bytes = int(lib.dspx_resample_workspace(len(xs)))
+        ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+        _lib.check(lib.dspx_resample_ragged(rs.handle, samples.data_ptr(), _lib.DTYPE_PCM16 if pcm else _lib.DTYPE_F32,
+                                            1 if normalize else 0, table_dev.data_ptr(), table.ctypes.data, len(xs),
+                                            out.data_ptr(), ws.data_ptr(), ws_bytes,
+                                            torch.cuda.current_stream(dev.index).cuda_stream), "dspx_resample_ragged")
+    return out, table
+
+
+def _to_device(x, device: int | None):
+    """A torch CUDA tensor as it is; NumPy (or a CPU tensor) uploaded with torch to `device` (default: current)."""
+    import torch
+
+    if _is_cuda_tensor(x):
+        return x
+    if type(x).__module__.startswith("torch"):
+        x = x.detach().numpy()
+    dev = torch.cuda.current_device() if device is None else int(device)
+    x = np.ascontiguousarray(x)
+    if not x.flags.writeable:                  # decoded WAV data is a read-only view; torch.from_numpy wants writable
+        x = x.copy()
+    return torch.from_numpy(x).to(torch.device("cuda", dev))
+
+
+def resample_poly(x, up: int, down: int, normalize: bool = False, device: int | None = None):
+    """scipy.signal.resample_poly(x, up, down) with its default filter, on the GPU, bit for bit.
+
+    x: a 1-D array, a [B, L] array (each row resampled) or a list of 1-D arrays of any lengths (one launch), as
+    NumPy or torch CUDA, float32 or int16 PCM (read as int16 / 32768, what load_audio decodes).  The result comes
+    back float32 in the same kind of container.  normalize=True then divides each clip by its peak, like
+    normalize_audio.  Other dtypes raise ValueError: scipy filters float64 in float64, which this does not do.
+    """
+    up, down = reduce_ratio(up, down)
+    if isinstance(x, (list, tuple)):
+        if not x:
+            return []
+        on_gpu = [_is_cuda_tensor(c) for c in x]
+        if any(on_gpu) and not all(on_gpu):
+            raise ValueError("clips must be all NumPy arrays or all torch CUDA tensors")
+        if len({_resample_dtype(c) for c in x}) > 1:
+            raise ValueError("clips must all be float32 or all be int16 PCM")
+        _lib.require_device()
+        xs = [_to_device(c, device).reshape(-1) for c in x]
+        if any(len(c) < 1 for c in xs):
+            raise ValueError("resample_poly of an empty clip")
+        if len({c.device for c in xs}) > 1:
+            raise ValueError("clips must be on one device")
+        out, table = _resample_ragged(xs, get_resampler(up, down, xs[0].device.index), normalize)
+        if all(on_gpu):
+            return [out[s:s + n] for s, n in zip(table[:, 2], table[:, 3])]
+        host = out.cpu().numpy()
+        return [host[s:s + n].copy() for s, n in zip(table[:, 2], table[:, 3])]
+    _resample_dtype(x)
+    if len(getattr(x, "shape", ())) not in (1, 2):
+        raise ValueError("resample_poly takes a 1-D array, a [B, L] array or a list of 1-D arrays")
+    _lib.require_device()
+    on_gpu = _is_cuda_tensor(x)
+    t = _to_device(x, device)
+    t2 = t if t.dim() == 2 else t[None, :]
+    if t2.stride(1) != 1:
+        t2 = t2.contiguous()
+    out = _resample_2d(t2, get_resampler(up, down, t2.device.index), normalize)
+    out = out if t.dim() == 2 else out[0]
+    return out if on_gpu else out.cpu().numpy()
+
+
+def _resample_ratio(cfg: Any, sample_rate) -> tuple[int, int] | None:
+    """(up, down) from the clips' rate to cfg.sample_rate, or None when no rate is given or the two are equal."""
+    if sample_rate is None or int(sample_rate) == config_key(cfg)[0]:
+        return None
+    return reduce_ratio(config_key(cfg)[0], int(sample_rate))
+
+
+def _features_resampled(clips, cfg: Any, want, device, kernel: str, normalize: bool, ratio) -> dict:
+    """features_batch of clips at another rate: resampled on the device first, PCM16 peak-normalised after the
+    resample when `normalize` (the reference's order: load_audio, then normalize_audio)."""
+    on_gpu = _is_cuda_tensor(clips)
+    pcm = _resample_dtype(clips)
+    t = _to_device(clips, device)
+    t = t if t.dim() == 2 else t[None, :]
+    if t.stride(1) != 1:
+        t = t.contiguous()
+    y = _resample_2d(t, get_resampler(*ratio, t.device.index), normalize and pcm)
+    out = features_batch(y, cfg, want, device, kernel, normalize)
+    return out if on_gpu else _as_host(out)
+
+
+def _as_host(out: dict) -> dict:
+    return {k: (v.cpu().numpy() if _is_cuda_tensor(v) else v) for k, v in out.items()}
+
+
 def features_batch(clips, cfg: Any, want: Iterable[str] = ("mfcc",), device: int | None = None,
-                   kernel: str = "auto", normalize: bool = True) -> dict:
+                   kernel: str = "auto", normalize: bool = True, sample_rate: int | None = None) -> dict:
     """log-mel / MFCC / clip embeddings of a batch of equal-length clips.
 
     Follows src/dsp/mfcc.py:86-109 (+ src/retrieval/retrieval.py:19-23 for "embed").
     Returns {"log_mel": [B,T,n_mels], "mfcc": [B,T,n_mfcc], "embed": [B,2*n_mfcc]} (float32)
     restricted to `want`.  int16 input is taken as PCM16 and converted on the GPU like
     load_audio (+ normalize_audio when `normalize`), src/utils/audio.py:19-38, cache.py:66-67.
+    `sample_rate`: the clips' own rate.  When it differs from cfg.sample_rate the clips are first resampled on the
+    GPU, bit-identically to load_audio's scipy.signal.resample_poly (int16 PCM is normalised after the resample);
+    NumPy input is uploaded with torch.  float32 or int16 clips only on that path.
     """
     want = _want(want)
+    ratio = _resample_ratio(cfg, sample_rate)
+    if ratio is not None:
+        return _features_resampled(clips, cfg, want, device, kernel, normalize, ratio)
     lib = _lib.load()
     if _is_cuda_tensor(clips):
         import torch
@@ -265,7 +413,7 @@ def ragged_launch(plan: Plan, samples, pcm: bool, table: np.ndarray, table_dev, 
 
 
 def features_ragged(clips, cfg: Any, want: Iterable[str] = ("mfcc",), device: int | None = None,
-                    normalize: bool = True) -> dict:
+                    normalize: bool = True, sample_rate: int | None = None) -> dict:
     """log-mel / MFCC / clip embeddings of clips of different lengths, in one launch.
 
     `clips` is a sequence of 1-D arrays: all NumPy (float32, or int16 PCM converted like features_batch does), or all
@@ -273,11 +421,17 @@ def features_ragged(clips, cfg: Any, want: Iterable[str] = ("mfcc",), device: in
     "embed": [B, 2*n_mfcc]} restricted to `want`, plus "frame_offsets" (int64 [B+1]): clip i owns rows
     frame_offsets[i]:frame_offsets[i+1].  Every clip gets the values features_batch gives it alone.  NumPy in ->
     NumPy out (one pinned staging buffer, one copy each way); torch CUDA in -> torch CUDA out on torch's current
-    stream.  A clip shorter than frame_length raises ValueError naming its index.
+    stream.  A clip shorter than frame_length raises ValueError naming its index.  `sample_rate` as in
+    features_batch: clips at another rate are resampled on the GPU in one launch first.
     """
     import torch
 
     want = _want(want)
+    ratio = _resample_ratio(cfg, sample_rate)
+    if ratio is not None:
+        clips = list(clips)
+        if clips:
+            return _features_ragged_resampled(clips, cfg, want, device, normalize, ratio)
     xs, on_gpu, pcm = _ragged_inputs(clips)
     starts, table, total = ragged_layout([len(x) for x in xs], cfg, np.int16 if pcm else np.float32)
     offsets = np.concatenate((table[:, 3], [total])).astype(np.int64) if len(xs) else np.zeros(1, np.int64)
@@ -327,6 +481,36 @@ def features_ragged(clips, cfg: Any, want: Iterable[str] = ("mfcc",), device: in
             off += m
     out["frame_offsets"] = offsets
     return out
+
+
+def _features_ragged_resampled(clips: list, cfg: Any, want, device, normalize: bool, ratio) -> dict:
+    """features_ragged of clips at another rate: one resample launch into a packed buffer whose layout is a valid
+    ragged feature batch, then one feature launch."""
+    import torch
+
+    on_gpu = [_is_cuda_tensor(c) for c in clips]
+    if any(on_gpu) and not all(on_gpu):
+        raise ValueError("clips must be all NumPy arrays or all torch CUDA tensors")
+    pcm = {_resample_dtype(c) for c in clips}
+    if len(pcm) > 1:
+        raise ValueError("clips must all be float32 or all be int16 PCM")
+    xs = [_to_device(c, device).reshape(-1) for c in clips]
+    if len({c.device for c in xs}) > 1:
+        raise ValueError("clips must be on one device")
+    dev = xs[0].device
+    samples, rtable = _resample_ragged(xs, get_resampler(*ratio, dev.index), normalize and pcm.pop())
+    starts, table, total = ragged_layout(rtable[:, 3], cfg, np.float32, rtable[:, 2])
+    plan = get_plan(cfg, dev.index if device is None else device)
+    with torch.cuda.device(dev.index):
+        table_dev = torch.from_numpy(table).to(dev)
+        res, _ = ragged_launch(plan, samples, False, table, table_dev, total, want, normalize)
+    offsets = np.concatenate((table[:, 3], [total])).astype(np.int64)
+    if all(on_gpu):
+        res["frame_offsets"] = torch.from_numpy(offsets).to(dev)
+        return res
+    res = _as_host(res)
+    res["frame_offsets"] = offsets
+    return res
 
 
 def split_ragged(stacked, frame_offsets) -> list:

@@ -77,15 +77,16 @@ def read_npy_shape(path: Path) -> tuple:
         return tuple(reader(handle)[0])
 
 
-def _features_per_clip(clips: list, cfg: Any, feature_types: tuple, normalize: bool = True) -> dict:
+def _features_per_clip(clips: list, cfg: Any, feature_types: tuple, normalize: bool = True,
+                       sample_rate: int | None = None) -> dict:
     """{feature_type: one [n_frames, n_coef] array per clip}: one batch when the clips have one length, else one
-    ragged launch."""
+    ragged launch.  Clips at another `sample_rate` than cfg's are resampled on the GPU first."""
     from .batch import features_batch, features_ragged, split_ragged
 
     if len({c.shape for c in clips}) == 1:
-        out = features_batch(np.stack(clips, axis=0), cfg, feature_types, normalize=normalize)
+        out = features_batch(np.stack(clips, axis=0), cfg, feature_types, normalize=normalize, sample_rate=sample_rate)
         return {ft: list(out[ft]) for ft in feature_types}
-    out = features_ragged(clips, cfg, feature_types, normalize=normalize)
+    out = features_ragged(clips, cfg, feature_types, normalize=normalize, sample_rate=sample_rate)
     return {ft: split_ragged(out[ft], out["frame_offsets"]) for ft in feature_types}
 
 
@@ -145,7 +146,8 @@ class BatchFeatureCache:
             raise ValueError(f"Unsupported feature_type: {feature_type}")
         if isinstance(cfg, Mapping):
             raise ValueError("get_feature requires MfccConfig for mfcc/log_mel")      # cache.py:83
-        return _features_per_clip(_load_clips(list(items), cfg, loader), cfg, (feature_type,))[feature_type]
+        clips, rate = _load_clips(list(items), cfg, loader)
+        return _features_per_clip(clips, cfg, (feature_type,), sample_rate=rate)[feature_type]
 
     def get_features(self, items: Sequence[Any], feature_type: str, cfg: Any, loader=None, batch: int = 256,
                      workers: int = 8) -> list:
@@ -202,13 +204,16 @@ class BatchFeatureCache:
     # ---- batched precompute (GPU) --------------------------------------------------------------------
     def precompute(self, items: Sequence[Any], cfg: Any, feature_types: Iterable[str] = FEATURE_TYPES,
                    clips: np.ndarray | None = None, loader: Callable[[Any], np.ndarray] | None = None,
-                   batch: int = 256, workers: int = 8, normalize: bool = True, skip_existing: bool = True) -> dict:
+                   batch: int = 256, workers: int = 8, normalize: bool = True, skip_existing: bool = True,
+                   sample_rate: int | None = None) -> dict:
         """Fill the cache for `items`: the batched twin of precompute_features.py:62-113.
 
         Audio comes from `clips` ([N, L] float32 already loaded/normalised, or int16 PCM which is
         converted and peak-normalised on the GPU; or a list of N clips of different lengths) or from
         `loader(item)` (decoding files is out of scope here).  A batch of clips of different lengths is
-        one ragged launch.  Returns {feature_type: manifest path}.
+        one ragged launch.  `sample_rate`: the clips' own rate; when it differs from cfg.sample_rate they are
+        resampled on the GPU first (int16 PCM is normalised after the resample).  Returns {feature_type: manifest
+        path}.
         """
         feature_types = tuple(feature_types)
         for ft in feature_types:
@@ -229,7 +234,7 @@ class BatchFeatureCache:
                     x = [np.asarray(clips[s + i]) for i in todo]
                 else:
                     x = [np.asarray(loader(chunk[i])) for i in todo]
-                out = _features_per_clip(x, cfg, feature_types, normalize=normalize)
+                out = _features_per_clip(x, cfg, feature_types, normalize=normalize, sample_rate=sample_rate)
                 for ft in feature_types:
                     self.save_features([chunk[i] for i in todo], out[ft], ft, cfg, workers=workers)
             for ft in feature_types:

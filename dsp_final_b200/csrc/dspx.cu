@@ -19,6 +19,7 @@
 #include "retrieval_f32.cuh"
 #include "retrieval_tc.cuh"
 #include "ingest.cuh"
+#include "resample.cuh"
 
 // the ctypes binding (dsp_final_b200/_lib.py) mirrors these layouts; tests assert the same numbers
 static_assert(sizeof(dspx_config) == 56 && offsetof(dspx_config, f_min) == 24 && offsetof(dspx_config, window) == 48,
@@ -764,6 +765,43 @@ static int topk_launch(const TopkLaunch &L, const Params &p, int device, cudaStr
     return DSPX_OK;
 }
 
+// ---- resampling (resample.cuh) --------------------------------------------------
+
+// One batch: zero the per-clip peaks, resample (or copy, for up == down == 1), then divide by the peaks.  Grids are
+// split every 65535 clips (grid.y).  max_out: output length of the longest clip.
+static int resample_launch(const dspx_resampler *rs, RsBatch b, int64_t n_clips, int64_t max_out, int normalize,
+                           unsigned *peaks, cudaStream_t st)
+{
+    static std::atomic<unsigned char> optin[64];
+    const RsGeom &g = rs->g;
+    const int64_t tiles = rs->identity ? 0 : rs_tiles(g, max_out);
+    DSPX_REQUIRE(tiles < (int64_t)0x7fffffff, "clip too long for one launch");
+    if (!rs->identity && g.smem > 48 * 1024) DSPX_CUDA_CHECK(optin_max_smem(resample_poly_kernel, optin, rs->device));
+    if (normalize) DSPX_CUDA_CHECK(cudaMemsetAsync(peaks, 0, (size_t)n_clips * sizeof(unsigned), st));
+    const int64_t elem_blocks = std::min<int64_t>(rs_ceil_div(max_out, 256), 4096);
+    for (int64_t c0 = 0; c0 < n_clips; c0 += 65535) {
+        const unsigned nc = (unsigned)std::min<int64_t>(n_clips - c0, 65535);
+        RsBatch bc = b;
+        if (b.rtab) {
+            bc.rtab = b.rtab + c0;
+        } else {
+            bc.in = static_cast<const char *>(b.in) + (size_t)(c0 * b.in_stride) * (b.pcm ? sizeof(int16_t) : sizeof(float));
+            bc.out = b.out + c0 * b.out_stride;
+        }
+        unsigned *pk = normalize ? peaks + c0 : nullptr;
+        if (rs->identity)
+            resample_copy_kernel<<<dim3((unsigned)elem_blocks, nc), 256, 0, st>>>(g, bc, pk);
+        else
+            resample_poly_kernel<<<dim3((unsigned)tiles, nc), RS_THREADS, g.smem, st>>>(g, bc, rs->d_tab, pk);
+        DSPX_CUDA_CHECK(cudaGetLastError());
+        if (normalize) {
+            resample_normalize_kernel<<<dim3((unsigned)elem_blocks, nc), 256, 0, st>>>(g, bc, pk);
+            DSPX_CUDA_CHECK(cudaGetLastError());
+        }
+    }
+    return DSPX_OK;
+}
+
 }  // namespace dspx
 
 using namespace dspx;
@@ -1332,6 +1370,145 @@ int dspx_hits_at_k(const int32_t *topk_idx_dev, int64_t nq, int k_stride, int k,
         topk_idx_dev, nq, k_stride, k, targets_db_dev, targets_q_dev, reinterpret_cast<unsigned long long *>(hits_dev));
     DSPX_CUDA_CHECK(cudaGetLastError());
     return DSPX_OK;
+}
+
+// ---- resampling ----
+
+int dspx_resampler_create(int64_t up, int64_t down, const float *window_host, int64_t n_window, int device,
+                          dspx_resampler **out)
+{
+    DSPX_REQUIRE(out, "null argument");
+    *out = nullptr;
+    DSPX_REQUIRE(up >= 1 && down >= 1, "up and down must be >= 1 (got %lld, %lld)", (long long)up, (long long)down);
+    int64_t a = up, b = down;
+    while (b) { const int64_t r = a % b; a = b; b = r; }
+    up /= a;
+    down /= a;
+    DSPX_REQUIRE(up <= RS_MAX_FACTOR && down <= RS_MAX_FACTOR, "reduced ratio %lld/%lld: factors above 2^20 are not supported",
+                 (long long)up, (long long)down);
+    const bool identity = up == 1 && down == 1;
+    DSPX_REQUIRE(identity || (window_host && n_window >= 1), "a filter window is required");
+    const int ndev = dspx_device_count();
+    if (ndev <= 0) { set_error("no CUDA device: libdspx has no CPU fallback"); return DSPX_ENODEVICE; }
+    DSPX_REQUIRE(device >= 0 && device < ndev, "device %d out of range (%d devices)", device, ndev);
+    dspx_resampler *rs = new (std::nothrow) dspx_resampler();
+    if (!rs) { set_error("out of host memory"); return DSPX_ENOMEM; }
+    rs->identity = identity;
+    rs->device = device;
+    rs->g.up = up;
+    rs->g.down = down;
+    if (!identity) {
+        std::vector<float> tab;
+        int P = 0;
+        int64_t remove = 0;
+        if (!rs_build_table(up, down, window_host, n_window, tab, &P, &remove)) {
+            delete rs;
+            set_error("window of %lld taps is too short for up = %lld (need n_window - (n_window - 1) / 2 >= up)",
+                      (long long)n_window, (long long)up);
+            return DSPX_EINVAL;
+        }
+        if (!rs_geometry(up, down, P, remove, MAX_OPTIN_SMEM, &rs->g)) {
+            delete rs;
+            set_error("ratio %lld/%lld needs %d taps per phase: too many for one tile in shared memory", (long long)up,
+                      (long long)down, P);
+            return DSPX_EINVAL;
+        }
+        DeviceGuard guard(device);
+        if (!guard.ok) { delete rs; set_error("cudaSetDevice(%d) failed", device); return DSPX_ECUDA; }
+        const int rc = upload(tab, &rs->d_tab);
+        if (rc != DSPX_OK) { cudaFree(rs->d_tab); delete rs; return rc; }
+    }
+    *out = rs;
+    return DSPX_OK;
+}
+
+int dspx_resampler_destroy(dspx_resampler *rs)
+{
+    if (!rs) return DSPX_OK;
+    DeviceGuard guard(rs->device);
+    cudaFree(rs->d_tab);
+    delete rs;
+    return DSPX_OK;
+}
+
+int64_t dspx_resample_len(const dspx_resampler *rs, int64_t n_in)
+{
+    DSPX_REQUIRE(rs, "null resampler");
+    DSPX_REQUIRE(n_in >= 0 && n_in <= ((int64_t)1 << 40), "input length %lld out of range", (long long)n_in);
+    return rs_out_len(n_in, rs->g.up, rs->g.down);
+}
+
+size_t dspx_resample_workspace(int64_t n_clips) { return n_clips > 0 ? (size_t)n_clips * sizeof(unsigned) + 256 : 256; }
+
+int dspx_resample(const dspx_resampler *rs, const void *in_dev, int dtype, int64_t n_clips, int64_t n_in, int64_t in_stride,
+                  int normalize, float *out_dev, int64_t out_stride, void *workspace_dev, size_t workspace_bytes, void *stream)
+{
+    DSPX_REQUIRE(rs && in_dev && out_dev, "null argument");
+    DSPX_REQUIRE(dtype == DSPX_DTYPE_F32 || dtype == DSPX_DTYPE_PCM16, "resampling takes float32 or PCM16 samples");
+    DSPX_REQUIRE(n_clips >= 0 && n_in >= 1 && n_in <= ((int64_t)1 << 40) && in_stride >= n_in, "bad input buffer arguments");
+    const int64_t n_out = rs_out_len(n_in, rs->g.up, rs->g.down);
+    DSPX_REQUIRE(out_stride >= n_out, "out_stride %lld is shorter than the output (%lld)", (long long)out_stride, (long long)n_out);
+    DSPX_REQUIRE(!normalize || (workspace_dev && workspace_bytes >= dspx_resample_workspace(n_clips)), "workspace too small");
+    if (n_clips == 0) return DSPX_OK;
+    DeviceGuard guard(rs->device);
+    char *ws = static_cast<char *>(workspace_dev);
+    if (ws) ws += (256 - (reinterpret_cast<uintptr_t>(ws) & 255)) & 255;
+    const RsBatch b{in_dev, dtype == DSPX_DTYPE_PCM16, n_in, in_stride, out_dev, out_stride, nullptr};
+    return resample_launch(rs, b, n_clips, n_out, normalize ? 1 : 0, reinterpret_cast<unsigned *>(ws),
+                           static_cast<cudaStream_t>(stream));
+}
+
+int64_t dspx_resample_layout(int64_t up, int64_t down, const int64_t *in_starts, const int64_t *in_lengths, int64_t n_clips,
+                             dspx_resample_clip *table_out)
+{
+    DSPX_REQUIRE(n_clips == 0 || (in_starts && in_lengths && table_out), "null argument");
+    DSPX_REQUIRE(n_clips >= 0, "negative clip count");
+    DSPX_REQUIRE(up >= 1 && down >= 1, "up and down must be >= 1 (got %lld, %lld)", (long long)up, (long long)down);
+    int64_t a = up, b = down;
+    while (b) { const int64_t r = a % b; a = b; b = r; }
+    up /= a;
+    down /= a;
+    int64_t at = 0;
+    for (int64_t i = 0; i < n_clips; i++) {
+        DSPX_REQUIRE(in_lengths[i] >= 1 && in_lengths[i] <= ((int64_t)1 << 40), "clip %lld: length %lld out of range",
+                     (long long)i, (long long)in_lengths[i]);
+        DSPX_REQUIRE(in_starts[i] >= 0, "clip %lld: negative start %lld", (long long)i, (long long)in_starts[i]);
+        dspx_resample_clip &r = table_out[i];
+        r.in_start = in_starts[i];
+        r.in_length = in_lengths[i];
+        r.out_start = at;
+        r.out_length = rs_out_len(in_lengths[i], up, down);
+        at += (r.out_length + 3) & ~(int64_t)3;      // RAGGED_ALIGN: the packed output is a valid ragged feature batch
+    }
+    return n_clips ? table_out[n_clips - 1].out_start + table_out[n_clips - 1].out_length : 0;
+}
+
+int dspx_resample_ragged(const dspx_resampler *rs, const void *in_dev, int dtype, int normalize,
+                         const dspx_resample_clip *table_dev, const dspx_resample_clip *table_host, int64_t n_clips,
+                         float *out_dev, void *workspace_dev, size_t workspace_bytes, void *stream)
+{
+    DSPX_REQUIRE(rs, "null resampler");
+    DSPX_REQUIRE(dtype == DSPX_DTYPE_F32 || dtype == DSPX_DTYPE_PCM16, "resampling takes float32 or PCM16 samples");
+    DSPX_REQUIRE(n_clips >= 0, "negative clip count");
+    if (n_clips == 0) return DSPX_OK;
+    DSPX_REQUIRE(in_dev && out_dev && table_dev && table_host, "null argument");
+    DSPX_REQUIRE(!normalize || (workspace_dev && workspace_bytes >= dspx_resample_workspace(n_clips)), "workspace too small");
+    int64_t max_out = 0;
+    for (int64_t i = 0; i < n_clips; i++) {
+        const dspx_resample_clip &r = table_host[i];
+        DSPX_REQUIRE(r.in_start >= 0 && r.in_length >= 1 && r.in_length <= ((int64_t)1 << 40) && r.out_start >= 0,
+                     "clip %lld: bad table row", (long long)i);
+        DSPX_REQUIRE(r.out_length == rs_out_len(r.in_length, rs->g.up, rs->g.down),
+                     "clip %lld: output length %lld does not match this ratio (%lld)", (long long)i, (long long)r.out_length,
+                     (long long)rs_out_len(r.in_length, rs->g.up, rs->g.down));
+        max_out = std::max(max_out, r.out_length);
+    }
+    DeviceGuard guard(rs->device);
+    char *ws = static_cast<char *>(workspace_dev);
+    if (ws) ws += (256 - (reinterpret_cast<uintptr_t>(ws) & 255)) & 255;
+    const RsBatch b{in_dev, dtype == DSPX_DTYPE_PCM16, 0, 0, out_dev, 0, table_dev};
+    return resample_launch(rs, b, n_clips, max_out, normalize ? 1 : 0, reinterpret_cast<unsigned *>(ws),
+                           static_cast<cudaStream_t>(stream));
 }
 
 }  // extern "C"

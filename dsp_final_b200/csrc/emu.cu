@@ -15,6 +15,7 @@
 #include "feat_generic.cuh"
 #include "feat_warp8.cuh"
 #include "feat_warp8_x2.cuh"
+#include "resample.cuh"
 
 namespace dspx {
 void set_error(const char *, ...) {}
@@ -434,6 +435,77 @@ long long emu_pcm16_quotient_mismatches(long long *total)
     }
     if (total) *total = n;
     return bad;
+}
+
+static int emu_resampler(int64_t up, int64_t down, const float *window, int64_t n_window, RsGeom &g, std::vector<float> &tab,
+                         bool &identity)
+{
+    if (up < 1 || down < 1) return DSPX_EINVAL;
+    int64_t a = up, b = down;
+    while (b) { const int64_t r = a % b; a = b; b = r; }
+    up /= a;
+    down /= a;
+    identity = up == 1 && down == 1;
+    g.up = up;
+    g.down = down;
+    if (identity) return DSPX_OK;
+    int P = 0;
+    int64_t remove = 0;
+    if (!rs_build_table(up, down, window, n_window, tab, &P, &remove)) return DSPX_EINVAL;
+    if (!rs_geometry(up, down, P, remove, MAX_OPTIN_SMEM, &g)) return DSPX_EINVAL;
+    return DSPX_OK;
+}
+
+// Tile geometry of a ratio: out[0..7] = P, S, NR, W, RS, smem bytes, U, remove.
+int emu_resample_shape(int64_t up, int64_t down, const float *window, int64_t n_window, int64_t *out)
+{
+    RsGeom g;
+    std::vector<float> tab;
+    bool identity = false;
+    const int rc = emu_resampler(up, down, window, n_window, g, tab, identity);
+    if (rc != DSPX_OK) return rc;
+    const int64_t v[8] = {g.P, g.S, g.NR, g.W, g.RS, (int64_t)g.smem, g.U, g.remove};
+    for (int i = 0; i < 8; i++) out[i] = v[i];
+    return DSPX_OK;
+}
+
+// Replays resample_poly_kernel (or resample_copy_kernel) and resample_normalize_kernel through the kernel's tile
+// decomposition: each tile's inputs and table rows are staged (rs_stage_row, rs_stage_phase) into a buffer of exactly the
+// kernel's dynamic shared-memory size, then every (work item, lane) runs rs_group.  table != NULL: ragged batch (n_in, in_stride, out_stride unused).
+int emu_resample(int64_t up, int64_t down, const float *window, int64_t n_window, const void *in, int dtype, int64_t n_clips,
+                 int64_t n_in, int64_t in_stride, int normalize, float *out, int64_t out_stride, const dspx_resample_clip *table)
+{
+    RsGeom g;
+    std::vector<float> tab;
+    bool identity = false;
+    const int rc = emu_resampler(up, down, window, n_window, g, tab, identity);
+    if (rc != DSPX_OK) return rc;
+    if (dtype != DSPX_DTYPE_F32 && dtype != DSPX_DTYPE_PCM16) return DSPX_EINVAL;
+    const RsBatch b{in, dtype == DSPX_DTYPE_PCM16, n_in, in_stride, out, out_stride, table};
+    for (int64_t clip = 0; clip < n_clips; clip++) {
+        const RsClip c = rs_clip(b, g, clip);
+        unsigned peak = 0;
+        if (identity) {
+            for (int64_t i = 0; i < c.n_out; i++) {
+                c.out[i] = rs_load(c.in, b.pcm, i);
+                peak = std::max(peak, rs_abs_bits(c.out[i]));
+            }
+        } else {
+            const int64_t tiles = rs_tiles(g, c.n_out);
+            for (int64_t tile = 0; tile < tiles; tile++) {
+                const RsTile t = rs_tile(g, tile);
+                std::vector<float> smem(g.smem / sizeof(float));
+                float *ts = smem.data() + (int64_t)g.NR * g.RS;
+                for (int r = 0; r < g.NR; r++) rs_stage_row(g, t, c, b.pcm, r, smem.data() + (int64_t)r * g.RS, 0, 1);
+                for (int s = 0; s < t.S; s++) rs_stage_phase(g, t, tab.data(), s, ts + (int64_t)s * g.P, 0, 1);
+                for (int item = 0; item < rs_items(g, t); item++)
+                    for (int lane = 0; lane < 32; lane++) peak = std::max(peak, rs_group(g, t, c, smem.data(), ts, item, lane));
+            }
+        }
+        if (normalize)
+            for (int64_t i = 0; i < c.n_out; i++) c.out[i] = rs_normalize(c.out[i], peak);
+    }
+    return DSPX_OK;
 }
 
 }  // extern "C"

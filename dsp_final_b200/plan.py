@@ -7,6 +7,7 @@ unhashable, so plans are keyed on the tuple of its fields instead.
 from __future__ import annotations
 
 import ctypes as C
+import math
 import threading
 from typing import Any
 
@@ -124,3 +125,73 @@ def clear_plans() -> None:
         for p in _plans.values():
             p.close()
         _plans.clear()
+        for r in _resamplers.values():
+            r.close()
+        _resamplers.clear()
+
+
+# ---- resamplers: one immutable dspx_resampler (device phase table) per reduced ratio and device ----
+_resamplers: dict[tuple, "Resampler"] = {}
+
+
+def reduce_ratio(up, down) -> tuple[int, int]:
+    """(up, down) reduced by their gcd; ValueError unless both are integers >= 1 (as scipy.signal.resample_poly)."""
+    if isinstance(up, bool) or isinstance(down, bool) or int(up) != up or int(down) != down:
+        raise ValueError("up and down must be integers")
+    up, down = int(up), int(down)
+    if up < 1 or down < 1:
+        raise ValueError("up and down must be >= 1")
+    g = math.gcd(up, down)
+    return up // g, down // g
+
+
+def default_window(up: int, down: int) -> np.ndarray:
+    """scipy.signal.resample_poly's default filter design, cast to float32 as it is for float32 input."""
+    from scipy.signal import firwin
+
+    max_rate = max(up, down)
+    return np.ascontiguousarray(firwin(2 * 10 * max_rate + 1, 1.0 / max_rate, window=("kaiser", 5.0)), dtype=np.float32)
+
+
+class Resampler:
+    """Owns a dspx_resampler* for a reduced ratio.  Immutable after creation; safe to share between threads."""
+
+    def __init__(self, up: int, down: int, device: int):
+        lib = _lib.load()
+        _lib.require_device()
+        self.up, self.down, self.device = up, down, device
+        w = default_window(up, down) if (up, down) != (1, 1) else np.zeros(1, np.float32)
+        handle = C.c_void_p()
+        _lib.check(lib.dspx_resampler_create(up, down, w.ctypes.data, len(w), device, C.byref(handle)),
+                   "dspx_resampler_create")
+        self._h = handle
+
+    @property
+    def handle(self) -> C.c_void_p:
+        return self._h
+
+    def out_len(self, n_in: int) -> int:
+        return _lib.check(int(_lib.load().dspx_resample_len(self._h, int(n_in))), "dspx_resample_len")
+
+    def close(self) -> None:
+        if getattr(self, "_h", None) is not None and self._h.value:
+            _lib.load().dspx_resampler_destroy(self._h)
+            self._h = C.c_void_p()
+
+    def __del__(self):                                               # best effort
+        try:
+            self.close()
+        except Exception:
+            pass
+
+
+def get_resampler(up, down, device: int | None = None) -> Resampler:
+    up, down = reduce_ratio(up, down)
+    dev = current_device() if device is None else int(device)
+    key = (up, down, dev)
+    with _lock:
+        rs = _resamplers.get(key)
+        if rs is None:
+            rs = Resampler(up, down, dev)
+            _resamplers[key] = rs
+        return rs

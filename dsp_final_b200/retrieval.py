@@ -33,22 +33,25 @@ def _mfcc_embedding(signal: np.ndarray, cfg: MfccConfig) -> np.ndarray:
     return features_batch(sig, cfg, ("embed",))["embed"][0].astype(np.float64)
 
 
-def _load_clips(items: List[Any], cfg: MfccConfig, loader) -> list:
-    """One array per item: what the reference's load_audio + normalize_audio return (float32), or -- when every
-    file is mono 16-bit PCM at cfg.sample_rate, the ESC-50 case -- the raw int16 samples, which the GPU converts
-    and peak-normalises with bit-identical results (src/utils/audio.py:19-38 as used by retrieval.py:35-36)."""
-    from .audio import load_audio, load_pcm16, normalize_audio
+def _load_clips(items: List[Any], cfg: MfccConfig, loader) -> tuple[list, int | None]:
+    """(one array per item, their sample rate; None for float32 clips, which are already at cfg.sample_rate).
+
+    The arrays are what the reference's load_audio + normalize_audio return (float32), or -- when every file is mono
+    16-bit PCM at one common rate -- the raw int16 samples and that rate.  The GPU then resamples them when that rate
+    is not cfg.sample_rate, converts and peak-normalises, with bit-identical results (src/utils/audio.py:19-38 as used
+    by retrieval.py:35-36).  Mixed rates and other encodings take the host path."""
+    from .audio import load_audio, normalize_audio, read_pcm16
 
     if loader is not None:
-        return [np.asarray(loader(item), dtype=np.float32).reshape(-1) for item in items]
-    pcm = [load_pcm16(item.path, cfg.sample_rate) for item in items]
-    if all(p is not None for p in pcm):
-        return pcm
+        return [np.asarray(loader(item), dtype=np.float32).reshape(-1) for item in items], None
+    pcm = [read_pcm16(item.path) for item in items]
+    if all(p is not None for p in pcm) and len({rate for _, rate in pcm}) == 1:
+        return [x for x, _ in pcm], pcm[0][1]
     clips = []
     for item in items:
         audio, _ = load_audio(item.path, target_sr=cfg.sample_rate)
         clips.append(normalize_audio(audio).astype(np.float32))
-    return clips
+    return clips, None
 
 
 def _equal_shapes(arrays: list) -> bool:
@@ -75,10 +78,10 @@ def compute_embeddings(items: List[Any], cfg: MfccConfig, feature_cache=None, lo
             feats = [feature_cache.get_feature(item, "mfcc", cfg) for item in items]
         feats = [np.asarray(f, dtype=np.float32) for f in feats]
         return embed_stats(np.stack(feats, axis=0) if _equal_shapes(feats) else feats)
-    clips = _load_clips(items, cfg, loader)
+    clips, rate = _load_clips(items, cfg, loader)
     if _equal_shapes(clips):
-        return features_batch(np.stack(clips, axis=0), cfg, ("embed",))["embed"]
-    return features_ragged(clips, cfg, ("embed",))["embed"]
+        return features_batch(np.stack(clips, axis=0), cfg, ("embed",), sample_rate=rate)["embed"]
+    return features_ragged(clips, cfg, ("embed",), sample_rate=rate)["embed"]
 
 
 def _dev_matrix(x):

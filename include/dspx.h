@@ -219,6 +219,48 @@ int dspx_features_ragged(const dspx_plan *plan, const void *samples_dev, int dty
 int dspx_embed_stats_ragged(const float *feats_dev, const dspx_ragged_clip *table_dev, int64_t n_clips, int n_coef,
                             float *out_dev, void *stream);
 
+/* ---- resample_poly(x, up, down)  src/utils/audio.py:27-30 (scipy.signal.resample_poly, default design) ----
+ * Bit-identical to scipy 1.18.1's resample_poly on float32 input (which filters in float32; DESIGN.md 4.5), and
+ * to it on int16 / 32768 for PCM16 input: output i = sum over the filter's taps in ascending input order, each
+ * product and each partial sum rounded to float32, starting from +0.  up and down are reduced by their gcd; for
+ * up == down == 1 the output is a copy of the input.  window_host: the float32 FIR window w (scipy's default is
+ * firwin(2 * 10 * max(up, down) + 1, 1 / max(up, down), window=("kaiser", 5.0))), taken as h = w * float32(up);
+ * it must satisfy n_window - (n_window - 1) / 2 >= up (the default does).  Ratios whose reduced factors exceed
+ * 2^20, or that need more than ~1700 taps per phase (down / up above ~85), give DSPX_EINVAL.
+ * The resampler owns the device phase table; it is immutable after creation and may be shared between threads. */
+typedef struct dspx_resampler dspx_resampler;
+int dspx_resampler_create(int64_t up, int64_t down, const float *window_host, int64_t n_window, int device,
+                          dspx_resampler **out);
+int dspx_resampler_destroy(dspx_resampler *rs);
+/* n_out = ceil(n_in * up / down) */
+int64_t dspx_resample_len(const dspx_resampler *rs, int64_t n_in);
+/* Device scratch: one peak per clip (used when normalize != 0). */
+size_t dspx_resample_workspace(int64_t n_clips);
+/* in_dev [n_clips][in_stride] float32 or int16 (dtype DSPX_DTYPE_F32 / DSPX_DTYPE_PCM16; PCM16 is read as s / 32768),
+ * first n_in samples of each row used; out_dev [n_clips][out_stride] float32, first dspx_resample_len(n_in) samples
+ * written.  normalize != 0 then divides each clip by its max |y| as normalize_audio does (the correctly rounded
+ * float32 quotient; an all-zero clip is left as it is). */
+int dspx_resample(const dspx_resampler *rs, const void *in_dev, int dtype, int64_t n_clips, int64_t n_in, int64_t in_stride,
+                  int normalize, float *out_dev, int64_t out_stride, void *workspace_dev, size_t workspace_bytes, void *stream);
+/* Ragged batches.  dspx_resample_layout (host only, no device needed) fills one row per clip from the input starts
+ * and lengths (samples of the input's type); the outputs are packed back to back with starts aligned to 4 samples,
+ * so (out_start, out_length) can go straight to dspx_ragged_layout and dspx_features_ragged.  Returns the packed
+ * output length (the last out_start + out_length), or DSPX_EINVAL for a length outside [1, 2^40], a negative start or
+ * a bad ratio. */
+typedef struct dspx_resample_clip {
+    int64_t in_start;
+    int64_t in_length;
+    int64_t out_start;
+    int64_t out_length;   /* dspx_resample_len(in_length) */
+} dspx_resample_clip;
+int64_t dspx_resample_layout(int64_t up, int64_t down, const int64_t *in_starts, const int64_t *in_lengths, int64_t n_clips,
+                             dspx_resample_clip *table_out);
+/* One launch for the whole batch; every clip gets exactly what dspx_resample gives it alone.  table_dev and
+ * table_host hold the same table. */
+int dspx_resample_ragged(const dspx_resampler *rs, const void *in_dev, int dtype, int normalize,
+                         const dspx_resample_clip *table_dev, const dspx_resample_clip *table_host, int64_t n_clips,
+                         float *out_dev, void *workspace_dev, size_t workspace_bytes, void *stream);
+
 /* ---- fft / ifft / rfft  src/dsp/fft.py:27-77 ----
  * in_dev [batch, n_in] interleaved complex64; the first min(n_in, n) samples are used,
  * zero-padded to P = next_pow2(n).  out_dev and work_dev each hold [batch, P] complex64.

@@ -54,6 +54,8 @@ const char *get_error();
         }                                       \
     } while (0)
 
+inline size_t align256(size_t x) { return (x + 255) & ~(size_t)255; }
+
 // Opt-in dynamic shared memory: a per-function, per-device attribute shared by every plan and thread.  It is
 // set once per (kernel, device) to the architectural maximum and never lowered, so launches of plans with
 // different shared-memory sizes cannot race on it (the size actually used is a launch argument).

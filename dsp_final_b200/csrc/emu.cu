@@ -16,6 +16,7 @@
 #include "feat_warp8.cuh"
 #include "feat_warp8_x2.cuh"
 #include "resample.cuh"
+#include "retrieval_select.cuh"
 
 namespace dspx {
 void set_error(const char *, ...) {}
@@ -505,6 +506,35 @@ int emu_resample(int64_t up, int64_t down, const float *window, int64_t n_window
         if (normalize)
             for (int64_t i = 0; i < c.n_out; i++) c.out[i] = rs_normalize(c.out[i], peak);
     }
+    return DSPX_OK;
+}
+
+// The launch of a dspx_cosine_topk call (topk_select): out = {kernel (0 tensor-core filter, 1 FP32 filter, 2 float64),
+// template argument, grid.x, grid.y, threads, dynamic shared memory, n_splits, rows_per_split}
+int emu_topk_select(int64_t nq, int64_t ndb, int dim, int k, int sm_count, int64_t *out)
+{
+    if (nq < 0 || ndb < 1 || dim < 1 || k < 1 || sm_count < 1) return DSPX_EINVAL;
+    const TopkLaunch L = topk_select(nq, ndb, dim, k, sm_count);
+    const int64_t v[8] = {(int64_t)L.kernel, L.cw, L.grid.x, L.grid.y, L.threads, (int64_t)L.smem, L.n_splits, L.rows_per_split};
+    for (int i = 0; i < 8; i++) out[i] = v[i];
+    return DSPX_OK;
+}
+
+// The ranking workspace (topk_ws_carve): out = {offset, extent} of qn, dbn, pscore, pidx, qf, dbf, shared_thr and
+// split_done, then the total (dspx_cosine_topk_workspace).  A region's extent runs to the next region's offset.
+int emu_topk_workspace(int64_t nq, int64_t ndb, int dim, int k, int64_t *out)
+{
+    if (nq < 0 || ndb < 0 || dim < 1 || k < 1) return DSPX_EINVAL;
+    char *const base = reinterpret_cast<char *>((uintptr_t)1 << 44);   // never dereferenced: only offsets are read
+    TopkWs w;
+    const size_t total = topk_ws_carve(nq, ndb, dim, k, base, &w);
+    const char *p[9] = {(char *)w.qn, (char *)w.dbn, (char *)w.pscore, (char *)w.pidx, (char *)w.qf, (char *)w.dbf,
+                        (char *)w.shared_thr, (char *)w.split_done, base + (total - 1024)};
+    for (int i = 0; i < 8; i++) {
+        out[2 * i] = p[i] - base;
+        out[2 * i + 1] = p[i + 1] - p[i];
+    }
+    out[16] = (int64_t)total;
     return DSPX_OK;
 }
 

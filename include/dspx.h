@@ -272,7 +272,8 @@ int dspx_fft_c2c(const float *in_dev, int64_t batch, int64_t n_in, int64_t n, in
 /* ---- cosine_similarity + argsort(-sims)[:, :k]  src/retrieval/retrieval.py:46-49,65 ----
  * q [nq, dim], db [ndb, dim] of dtype DSPX_DTYPE_*.  Scores are float64, rows scaled by
  * 1/(||row|| + 1e-10); idx_out [nq, k] int32 in descending score order, ties broken by
- * the lower database index (np.argsort(..., kind="stable")).  score_out may be NULL.
+ * the lower database index (np.argsort(..., kind="stable")).  score_out may be NULL, and so may q and idx_out when
+ * nq == 0.
  * workspace_dev must hold dspx_cosine_topk_workspace() bytes.  k <= DSPX_MAX_K. */
 #define DSPX_MAX_K 128
 size_t dspx_cosine_topk_workspace(int64_t nq, int64_t ndb, int dim, int k);
@@ -281,7 +282,8 @@ int dspx_cosine_topk(const void *q_dev, int64_t nq, const void *db_dev, int64_t 
                      void *workspace_dev, size_t workspace_bytes, void *stream);
 
 /* The dense matrix itself (cosine_similarity, retrieval.py:46-49), float64 [nq, ndb];
- * same scores, bit for bit, as the ones dspx_cosine_topk ranks.  Same workspace. */
+ * same scores, bit for bit, as the ones dspx_cosine_topk ranks.  Same workspace.  q, db and sims_out may be NULL when
+ * nq or ndb is 0. */
 int dspx_cosine_matrix(const void *q_dev, int64_t nq, const void *db_dev, int64_t ndb, int dim,
                        int dtype, double *sims_out_dev, void *workspace_dev, size_t workspace_bytes,
                        void *stream);

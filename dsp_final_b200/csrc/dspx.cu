@@ -1,6 +1,8 @@
 // dspx.cu -- C ABI of libdspx.so (include/dspx.h): plan management, kernel
 // launches and the host-buffer pipeline.  All numerical work is in the .cuh
-// kernels included below; this file only validates arguments and launches.
+// kernels included below, and what a plan and a call run is chosen in the host
+// headers (feat_select.cuh, retrieval_select.cuh); this file validates
+// arguments and launches what they choose.
 #include <cstdarg>
 #include <cstddef>
 #include <cstdlib>
@@ -14,6 +16,7 @@
 #include "feat_generic.cuh"
 #include "feat_warp8.cuh"
 #include "feat_warp8_x2.cuh"
+#include "feat_select.cuh"
 #include "fft_generic.cuh"
 #include "retrieval.cuh"
 #include "retrieval_f32.cuh"
@@ -73,8 +76,8 @@ struct HostPipe {
     void *d_out[PIPE_SLOTS] = {nullptr, nullptr, nullptr};
     void *h_in[PIPE_SLOTS] = {nullptr, nullptr, nullptr};    // pinned staging (pageable callers)
     void *h_out[PIPE_SLOTS] = {nullptr, nullptr, nullptr};
-    void *d_f32[PIPE_SLOTS] = {nullptr, nullptr, nullptr};   // float32 clips converted from PCM16
-    size_t in_bytes = 0, out_bytes = 0, hin_bytes = 0, hout_bytes = 0, f32_bytes = 0;
+    void *d_ws[PIPE_SLOTS] = {nullptr, nullptr, nullptr};    // scratch of the feature call (feat_ws_carve)
+    size_t in_bytes = 0, out_bytes = 0, hin_bytes = 0, hout_bytes = 0, ws_bytes = 0;
     void release()
     {
         for (int i = 0; i < PIPE_SLOTS; i++) {
@@ -82,13 +85,13 @@ struct HostPipe {
             if (d_out[i]) cudaFree(d_out[i]);
             if (h_in[i]) cudaFreeHost(h_in[i]);
             if (h_out[i]) cudaFreeHost(h_out[i]);
-            if (d_f32[i]) cudaFree(d_f32[i]);
-            d_f32[i] = nullptr;
+            if (d_ws[i]) cudaFree(d_ws[i]);
+            d_ws[i] = nullptr;
             if (stream[i]) cudaStreamDestroy(stream[i]);
             d_in[i] = d_out[i] = h_in[i] = h_out[i] = nullptr;
             stream[i] = nullptr;
         }
-        in_bytes = out_bytes = hin_bytes = hout_bytes = f32_bytes = 0;
+        in_bytes = out_bytes = hin_bytes = hout_bytes = ws_bytes = 0;
     }
 };
 
@@ -172,23 +175,6 @@ static int launch_generic(const dspx_plan *pl, const float *clips, int64_t n_cli
     return DSPX_OK;
 }
 
-// Features of an equal-length batch on the path warp8_select chose (PCM16: int16 rows, peaks per clip or null).
-static int launch_features(const dspx_plan *pl, W8Path path, const void *clips, int64_t n_clips, int64_t clip_len,
-                           int64_t clip_stride, int64_t T, float *logmel, float *mfcc, cudaStream_t st, int nchw = 0,
-                           long long *eacc = nullptr, const int *peaks = nullptr)
-{
-    const bool pre = pl->cfg.pre_emphasis > 0.0;
-    const float *x = static_cast<const float *>(clips);
-    if (path == W8_GENERIC)
-        return launch_generic(pl, x, n_clips, clip_len, clip_stride, T, pl->take_feat, pre ? 1 : 0, logmel, mfcc, nullptr, st, nchw);
-    if (path == W8_X2 || path == W8_X2_AL4)
-        return launch_warp8_x2(pl, path == W8_X2_AL4, x, n_clips, clip_stride, T, logmel, mfcc, st, nchw);
-    W8Params p = w8_batch_params(pl, clips, n_clips, clip_stride, T, logmel, mfcc, nchw);
-    p.eacc = eacc;
-    p.peaks = peaks;
-    return launch_warp8(pl, path, p, pre, st);
-}
-
 static int launch_embed(const float *feats, int64_t n_clips, int64_t T, int C, float *out, cudaStream_t st,
                         const dspx_ragged_clip *rtab = nullptr)
 {
@@ -200,64 +186,6 @@ static int launch_embed(const float *feats, int64_t n_clips, int64_t T, int C, f
     embed_stats_kernel<<<(unsigned)n_clips, 128, smem, st>>>(feats, T, C, out, rtab);
     DSPX_CUDA_CHECK(cudaGetLastError());
     return DSPX_OK;
-}
-
-// embed without mfcc: the fused path -- the kernel accumulates per-clip sums into `eacc` ([n_clips][2][n_mfcc]
-// int64, caller-provided scratch) and embed_finalize_kernel writes mean / std; no MFCC tensor exists anywhere.
-static int features_device(const dspx_plan *pl, const float *clips, int64_t n_clips, int64_t clip_len,
-                           int64_t clip_stride, float *logmel, float *mfcc, float *embed, cudaStream_t st, int nchw = 0,
-                           long long *eacc = nullptr)
-{
-    const int64_t T = dspx_num_frames(pl, clip_len);
-    if (T < 0) return DSPX_EINVAL;
-    const bool fused = embed && !mfcc;
-    const W8Path path = warp8_select(pl, clips, clip_stride, DSPX_DTYPE_F32, false, n_clips, T,
-                                     fused ? W8_WANT_EMBED : W8_WANT_FEATURES);
-    if (path == W8_UNSUPPORTED) {
-        set_error("embeddings without an MFCC buffer need the warp8 kernel (n_fft 512 / 1024 / 2048), frame_length = "
-                  "n_fft, an even hop and row stride, 8-byte aligned clips and at most %lld frames per clip",
-                  (long long)w8_embed_max_frames(pl->cfg.n_mels));
-        return DSPX_EUNSUPPORTED;
-    }
-    const int C = pl->cfg.n_mfcc;
-    if (fused) DSPX_CUDA_CHECK(cudaMemsetAsync(eacc, 0, (size_t)n_clips * 2 * C * sizeof(long long), st));
-    int rc = launch_features(pl, path, clips, n_clips, clip_len, clip_stride, T, logmel, mfcc, st, nchw, fused ? eacc : nullptr);
-    if (rc != DSPX_OK) return rc;
-    if (fused) {
-        const int64_t total = n_clips * C;
-        embed_finalize_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(eacc, n_clips, T, C, embed);
-        DSPX_CUDA_CHECK(cudaGetLastError());
-        return DSPX_OK;
-    }
-    if (embed) rc = launch_embed(mfcc, n_clips, T, C, embed, st);
-    return rc;
-}
-
-// PCM16 clips on the device -> features, conversion and peak normalisation inside the feature kernel's sample loads.
-// peaks_ws: n_clips ints of scratch (only touched when normalize).  warp8 plans only.
-static int features_device_pcm16(const dspx_plan *pl, const int16_t *pcm, int64_t n_clips, int64_t clip_len, int64_t pcm_stride,
-                                 int normalize, float *logmel, float *mfcc, float *embed, int *peaks_ws, cudaStream_t st)
-{
-    const int64_t T = dspx_num_frames(pl, clip_len);
-    if (T < 0) return DSPX_EINVAL;
-    const W8Path path = warp8_select(pl, pcm, pcm_stride, DSPX_DTYPE_PCM16, false, n_clips, T, W8_WANT_FEATURES);
-    if (path == W8_UNSUPPORTED) {
-        set_error("fused PCM16 ingest needs the warp8 kernel (n_fft 512 / 1024 / 2048) and fewer than 2^31 frame pairs: "
-                  "convert with dspx_pcm16_to_float first");
-        return DSPX_EUNSUPPORTED;
-    }
-    DSPX_REQUIRE(!embed || mfcc, "embed_out needs mfcc_out on the PCM16 path");
-    DSPX_REQUIRE(n_clips < (int64_t)2147483647, "too many clips for one launch");
-    if (normalize) {
-        DSPX_REQUIRE(peaks_ws, "peak normalisation needs the workspace");
-        pcm16_peak_kernel<<<(unsigned)n_clips, 256, 0, st>>>(pcm, clip_len, pcm_stride, peaks_ws);
-        DSPX_CUDA_CHECK(cudaGetLastError());
-    }
-    int rc = launch_features(pl, path, pcm, n_clips, clip_len, pcm_stride, T, logmel, mfcc, st, 0, nullptr,
-                             normalize ? peaks_ws : nullptr);
-    if (rc != DSPX_OK) return rc;
-    if (embed) rc = launch_embed(mfcc, n_clips, T, pl->cfg.n_mfcc, embed, st);
-    return rc;
 }
 
 // complex STFT: the warp8 kernel when frame_length == n_fft in {512, 1024, 2048} and the rows are aligned
@@ -272,125 +200,82 @@ static int stft_device(const dspx_plan *pl, const float *clips, int64_t n_clips,
     return launch_warp8(pl, path, p, pre != 0, st);
 }
 
-// ---- ragged batches (dspx_features_ragged) ------------------------------------------------------------
-// Workspace of one call, carved the same way by the size query and the launch (offsets from a 256-byte aligned base):
-// the compact first-pair array the ragged kernel searches, PCM16 peaks, fixed-point embedding sums, MFCC scratch for
-// embeddings without an MFCC output (when the fused path does not apply), and on plans without a ragged kernel a
-// float32 copy of one PCM16 clip at a time.
-struct RaggedWs {
-    uint32_t *rpairs = nullptr;
-    int *peaks = nullptr;
-    long long *eacc = nullptr;
-    float *mfcc = nullptr;
-    float *f32 = nullptr;
+// ---- feature calls (dspx_features, dspx_embeddings, dspx_log_mel_nchw, dspx_features_pcm16, dspx_features_ragged and
+// the host pipeline): feat_steps (feat_select.cuh) chooses the steps, run_features enqueues them ---------------------
+struct FeatOut {
+    float *logmel, *mfcc, *embed;
+    int nchw;                 // log-mel as [B, 1, n_mels, T]
 };
 
-// the path of a ragged batch whose longest clip has max_frames frames
-static W8Path ragged_path(const dspx_plan *pl, int dtype, W8Want want, int64_t max_frames)
+static int run_features(const dspx_plan *pl, const FeatBatch &b, const FeatSteps &s, const FeatOut &o, const FeatWs &ws,
+                        cudaStream_t st)
 {
-    return warp8_select(pl, nullptr, 0, dtype, true, 0, max_frames, want);
-}
-
-static int64_t ragged_max_frames(const dspx_ragged_clip *tab, int64_t n_clips)
-{
-    int64_t m = 0;
-    for (int64_t i = 0; i < n_clips; i++) m = std::max(m, tab[i].n_frames);
-    return m;
-}
-
-static size_t ragged_ws_carve(const dspx_plan *pl, const dspx_ragged_clip *tab, int64_t n_clips, int dtype, int normalize,
-                              bool want_mfcc, bool want_embed, char *base, RaggedWs *ws)
-{
-    const int64_t max_frames = ragged_max_frames(tab, n_clips);
-    const bool pcm = dtype == DSPX_DTYPE_PCM16, rk = ragged_path(pl, dtype, W8_WANT_FEATURES, max_frames) != W8_UNSUPPORTED;
-    const bool fused = want_embed && !want_mfcc && ragged_path(pl, dtype, W8_WANT_EMBED, max_frames) != W8_UNSUPPORTED;
-    int64_t total_frames = 0, max_len = 0;
-    if (n_clips > 0) total_frames = tab[n_clips - 1].first_frame + tab[n_clips - 1].n_frames;
-    for (int64_t i = 0; i < n_clips; i++) max_len = std::max(max_len, tab[i].length);
-    const size_t b_pairs = rk ? (size_t)(n_clips + 1) * sizeof(uint32_t) : 0;
-    const size_t b_peaks = rk && pcm && normalize ? (size_t)n_clips * sizeof(int) : 0;
-    const size_t b_eacc = fused ? (size_t)n_clips * 2 * pl->cfg.n_mfcc * sizeof(long long) : 0;
-    const size_t b_mfcc = want_embed && !want_mfcc && !fused ? (size_t)total_frames * pl->cfg.n_mfcc * sizeof(float) : 0;
-    const size_t b_f32 = !rk && pcm ? (size_t)max_len * sizeof(float) : 0;
-    size_t off = 0;
-    auto take = [&](size_t bytes) -> char * {
-        char *p = bytes && base ? base + off : nullptr;
-        off += align256(bytes);
-        return p;
-    };
-    RaggedWs w;
-    w.rpairs = reinterpret_cast<uint32_t *>(take(b_pairs));
-    w.peaks = reinterpret_cast<int *>(take(b_peaks));
-    w.eacc = reinterpret_cast<long long *>(take(b_eacc));
-    w.mfcc = reinterpret_cast<float *>(take(b_mfcc));
-    w.f32 = reinterpret_cast<float *>(take(b_f32));
-    if (ws) *ws = w;
-    return off + 256;
-}
-
-// Plans without a ragged kernel: one stream-ordered feature call per clip into its rows of the stacked outputs, the
-// embeddings from the stacked MFCCs at the end.  Each clip is computed exactly as a [1, length] call computes it.
-static int features_ragged_per_clip(const dspx_plan *pl, const void *samples, int pcm, int normalize,
-                                    const dspx_ragged_clip *tab_dev, const dspx_ragged_clip *tab, int64_t n_clips,
-                                    float *logmel, float *mfcc, float *embed, const RaggedWs &ws, cudaStream_t st)
-{
-    float *mf = mfcc ? mfcc : (embed ? ws.mfcc : nullptr);
-    for (int64_t i = 0; i < n_clips; i++) {
-        const int64_t len = tab[i].length, ff = tab[i].first_frame;
-        const float *x = static_cast<const float *>(samples) + tab[i].start;
-        if (pcm) {
-            pcm16_to_float_kernel<<<1, 256, 0, st>>>(static_cast<const int16_t *>(samples) + tab[i].start, len, len,
-                                                     normalize ? 1 : 0, ws.f32, len);
-            DSPX_CUDA_CHECK(cudaGetLastError());
-            x = ws.f32;
-        }
-        const int rc = features_device(pl, x, 1, len, len, logmel ? logmel + ff * pl->cfg.n_mels : nullptr,
-                                       mf ? mf + ff * pl->cfg.n_mfcc : nullptr, nullptr, st);
-        if (rc != DSPX_OK) return rc;
-    }
-    return embed ? launch_embed(mf, n_clips, 1, pl->cfg.n_mfcc, embed, st, tab_dev) : DSPX_OK;
-}
-
-static int features_ragged(const dspx_plan *pl, const void *samples, int dtype, int normalize, const dspx_ragged_clip *tab_dev,
-                           const dspx_ragged_clip *tab, int64_t n_clips, float *logmel, float *mfcc, float *embed,
-                           char *ws_base, cudaStream_t st)
-{
-    const int pcm = dtype == DSPX_DTYPE_PCM16 ? 1 : 0;
-    RaggedWs ws;
-    ragged_ws_carve(pl, tab, n_clips, dtype, normalize, mfcc != nullptr, embed != nullptr, ws_base, &ws);
-    const bool fused = ws.eacc != nullptr;                   // embeddings alone, accumulated inside the feature kernel
-    const W8Path path = ragged_path(pl, dtype, fused ? W8_WANT_EMBED : W8_WANT_FEATURES, ragged_max_frames(tab, n_clips));
-    if (path == W8_UNSUPPORTED)
-        return features_ragged_per_clip(pl, samples, pcm, normalize, tab_dev, tab, n_clips, logmel, mfcc, embed, ws, st);
     const int C = pl->cfg.n_mfcc;
-    const uint32_t n_items = (uint32_t)(tab[n_clips - 1].first_pair + (tab[n_clips - 1].n_frames + 1) / 2);
-    ragged_pairs_kernel<<<(unsigned)((n_clips + 256) / 256), 256, 0, st>>>(tab_dev, n_clips, ws.rpairs);
-    DSPX_CUDA_CHECK(cudaGetLastError());
-    if (ws.peaks) {
-        pcm16_peak_kernel<<<(unsigned)n_clips, 256, 0, st>>>(static_cast<const int16_t *>(samples), 0, 0, ws.peaks, tab_dev);
+    const int64_t n = b.n_clips;
+    float *mf = o.mfcc ? o.mfcc : ws.mfcc;
+    if (s.per_clip) {
+        // one stream-ordered call per clip into its rows of the stacked outputs, each computed exactly as a [1, length]
+        // call computes it; the embeddings from the stacked MFCCs at the end
+        const size_t elem = b.dtype == DSPX_DTYPE_PCM16 ? sizeof(int16_t) : sizeof(float);
+        for (int64_t i = 0; i < n; i++) {
+            const dspx_ragged_clip &c = b.tab[i];
+            const FeatBatch row{static_cast<const char *>(b.samples) + c.start * elem, b.dtype, b.normalize, 1, c.length,
+                                c.length, nullptr, nullptr};
+            const FeatOut ro{o.logmel ? o.logmel + c.first_frame * pl->cfg.n_mels : nullptr,
+                             mf ? mf + c.first_frame * C : nullptr, nullptr, 0};
+            const int rc = run_features(pl, row, feat_steps(pl, row, mf != nullptr, false), ro, ws, st);
+            if (rc != DSPX_OK) return rc;
+        }
+        return o.embed ? launch_embed(mf, n, 1, C, o.embed, st, b.tab_dev) : DSPX_OK;
+    }
+    const bool ragged = b.tab != nullptr, pre = pl->cfg.pre_emphasis > 0.0;
+    if (ragged) {
+        ragged_pairs_kernel<<<(unsigned)((n + 256) / 256), 256, 0, st>>>(b.tab_dev, n, ws.rpairs);
         DSPX_CUDA_CHECK(cudaGetLastError());
     }
-    if (fused) DSPX_CUDA_CHECK(cudaMemsetAsync(ws.eacc, 0, (size_t)n_clips * 2 * C * sizeof(long long), st));
-    float *mf = mfcc ? mfcc : ws.mfcc;                      // ws.mfcc: scratch for embeddings that are not fused, else null
-    W8Params p = w8_batch_params(pl, samples, n_clips, 0, 0, logmel, mf, 0);
-    p.rtab = tab_dev;
-    p.rpairs = ws.rpairs;
-    p.n_items = n_items;
-    p.eacc = ws.eacc;
-    p.peaks = ws.peaks;
-    int rc = launch_warp8(pl, path, p, pl->cfg.pre_emphasis > 0.0, st);
+    const void *x = b.samples;
+    int64_t stride = b.stride;
+    if (s.peaks) {
+        pcm16_peak_kernel<<<(unsigned)n, 256, 0, st>>>(static_cast<const int16_t *>(b.samples), b.clip_len, b.stride, ws.peaks,
+                                                       b.tab_dev);
+        DSPX_CUDA_CHECK(cudaGetLastError());
+    } else if (s.convert) {
+        pcm16_to_float_kernel<<<(unsigned)n, 256, 0, st>>>(static_cast<const int16_t *>(b.samples), b.clip_len, b.stride,
+                                                           b.normalize, ws.f32, b.clip_len);
+        DSPX_CUDA_CHECK(cudaGetLastError());
+        x = ws.f32;
+        stride = b.clip_len;
+    }
+    if (s.fused) DSPX_CUDA_CHECK(cudaMemsetAsync(ws.eacc, 0, (size_t)n * 2 * C * sizeof(long long), st));
+    const float *xf = static_cast<const float *>(x);
+    int rc;
+    if (s.path == W8_GENERIC) {
+        rc = launch_generic(pl, xf, n, b.clip_len, stride, s.T, pl->take_feat, pre ? 1 : 0, o.logmel, mf, nullptr, st, o.nchw);
+    } else if (s.path == W8_X2 || s.path == W8_X2_AL4) {
+        rc = launch_warp8_x2(pl, s.path == W8_X2_AL4, xf, n, stride, s.T, o.logmel, mf, st, o.nchw);
+    } else {
+        W8Params p = w8_batch_params(pl, x, n, stride, ragged ? 0 : s.T, o.logmel, mf, o.nchw);
+        if (ragged) {
+            p.rtab = b.tab_dev;
+            p.rpairs = ws.rpairs;
+            p.n_items = (uint32_t)(b.tab[n - 1].first_pair + (b.tab[n - 1].n_frames + 1) / 2);
+        }
+        p.eacc = ws.eacc;
+        p.peaks = ws.peaks;
+        rc = launch_warp8(pl, s.path, p, pre, st);
+    }
     if (rc != DSPX_OK) return rc;
-    if (fused) {
-        const int64_t total = n_clips * C;
-        embed_finalize_kernel<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(ws.eacc, n_clips, 1, C, embed, tab_dev);
+    const int64_t frames = ragged ? 1 : s.T;          // a ragged batch takes each clip's frames from its table
+    if (s.fused) {
+        embed_finalize_kernel<<<(unsigned)((n * C + 255) / 256), 256, 0, st>>>(ws.eacc, n, frames, C, o.embed, b.tab_dev);
         DSPX_CUDA_CHECK(cudaGetLastError());
         return DSPX_OK;
     }
-    return embed ? launch_embed(mf, n_clips, 1, C, embed, st, tab_dev) : DSPX_OK;
+    return o.embed ? launch_embed(mf, n, frames, C, o.embed, st, b.tab_dev) : DSPX_OK;
 }
 
-static int ensure_pipe(dspx_plan *pl, size_t in_bytes, size_t out_bytes, bool stage_in, bool stage_out, HostPipe **out,
-                       size_t f32_bytes = 0)
+static int ensure_pipe(dspx_plan *pl, size_t in_bytes, size_t out_bytes, size_t ws_bytes, bool stage_in, bool stage_out,
+                       HostPipe **out)
 {
     // the HostPipe object itself is created with the plan; its streams and buffers are (re)sized here, with
     // hp->mu held by the caller for the whole pipelined call
@@ -415,13 +300,13 @@ static int ensure_pipe(dspx_plan *pl, size_t in_bytes, size_t out_bytes, bool st
         }
         hp->out_bytes = out_bytes;
     }
-    if (f32_bytes > hp->f32_bytes) {
+    if (ws_bytes > hp->ws_bytes) {
         for (int i = 0; i < PIPE_SLOTS; i++) {
-            if (hp->d_f32[i]) cudaFree(hp->d_f32[i]);
-            hp->d_f32[i] = nullptr;
-            DSPX_CUDA_CHECK(cudaMalloc(&hp->d_f32[i], f32_bytes));
+            if (hp->d_ws[i]) cudaFree(hp->d_ws[i]);
+            hp->d_ws[i] = nullptr;
+            DSPX_CUDA_CHECK(cudaMalloc(&hp->d_ws[i], ws_bytes));
         }
-        hp->f32_bytes = f32_bytes;
+        hp->ws_bytes = ws_bytes;
     }
     if (stage_in && in_bytes > hp->hin_bytes) {
         for (int i = 0; i < PIPE_SLOTS; i++) {
@@ -495,18 +380,18 @@ static int host_pipeline(dspx_plan *pl, int mode, const void *clips_v, int64_t n
     // chunk: ~48 MiB of input or ~96 MiB of output, whichever is hit first
     int64_t chunk = std::min<int64_t>(n_clips, (int64_t)((48u << 20) / (clip_bytes ? clip_bytes : 1)));
     if (chunk < 1) chunk = 1;
-    // the kernels read a chunk's device copy: rows of clip_len samples in a cudaMalloc'd, so aligned, buffer (the null
-    // pointer below)
-    const int dtype = elem == 2 ? DSPX_DTYPE_PCM16 : DSPX_DTYPE_F32;
-    // embeddings alone: accumulated inside the feature kernel when it can (16 bytes of scratch per coefficient instead
-    // of an MFCC tensor); otherwise they are the statistics of the MFCCs that are written anyway
-    const bool fused_embed = mode == 0 && o_embed && !o_mfcc &&
-                             warp8_select(pl, nullptr, clip_len, dtype, false, chunk, T, W8_WANT_EMBED) != W8_UNSUPPORTED;
-    const bool need_mfcc = mode == 0 && (o_mfcc || (o_embed && !fused_embed));
-    const size_t mf_b = need_mfcc ? (size_t)T * pl->cfg.n_mfcc * 4 : (fused_embed ? (size_t)pl->cfg.n_mfcc * 16 : 0);
+    // the kernels read a chunk's device copy: rows of clip_len samples at the start of a cudaMalloc'd, so aligned,
+    // buffer.  The steps do not depend on the chunk's clip count: 48 MiB of input hold fewer than 2^31 frames, and a
+    // chunk of one clip stays one.
+    const FeatBatch batch{nullptr, elem == 2 ? DSPX_DTYPE_PCM16 : DSPX_DTYPE_F32, normalize, chunk, clip_len, clip_len,
+                          nullptr, nullptr};
+    const FeatSteps steps = mode == 0 ? feat_steps(pl, batch, o_mfcc != nullptr, o_embed != nullptr) : FeatSteps{};
+    const size_t mf_b = o_mfcc ? (size_t)T * pl->cfg.n_mfcc * 4 : 0;
     const size_t em_b = (mode == 0 && o_embed) ? (size_t)2 * pl->cfg.n_mfcc * 4 : 0;
     const size_t st_b = mode == 1 ? (size_t)T * pl->n_bins * 8 : 0;
-    const size_t out_per_clip = lm_b + mf_b + em_b + st_b;
+    // the chunk counts an MFCC tensor for embeddings that do not fuse and 16 bytes per coefficient for fused sums
+    const size_t scratch_b = steps.mfcc_scratch ? (size_t)T * pl->cfg.n_mfcc * 4 : (steps.fused ? (size_t)pl->cfg.n_mfcc * 16 : 0);
+    const size_t out_per_clip = lm_b + mf_b + scratch_b + em_b + st_b;
     const int64_t chunk_o = (int64_t)((96u << 20) / (out_per_clip ? out_per_clip : 1));
     if (chunk_o < chunk) chunk = chunk_o;
     if (chunk < 1) chunk = 1;
@@ -520,12 +405,10 @@ static int host_pipeline(dspx_plan *pl, int mode, const void *clips_v, int64_t n
     HostPipe *hp = static_cast<HostPipe *>(pl->host_pipe);
     DSPX_REQUIRE(hp, "plan has no host pipeline state");
     std::lock_guard<std::mutex> lock(hp->mu);
-    // PCM16: the feature kernel converts in its own loads when it can (no float32 copy of the clips); the scratch
-    // buffer then only holds one int per clip.  Otherwise pcm16_to_float_kernel converts first and needs the copy.
-    const bool fused_pcm = elem == 2 && mode == 0 &&
-                           warp8_select(pl, nullptr, clip_len, dtype, false, chunk, T, W8_WANT_FEATURES) != W8_UNSUPPORTED;
-    int rc = ensure_pipe(pl, clip_bytes * chunk, out_bytes, !in_pinned, !out_pinned, &hp,
-                         elem == 2 ? (fused_pcm ? (size_t)chunk * sizeof(int) : (size_t)clip_len * 4 * chunk) : 0);
+    FeatBatch sized = batch;
+    sized.n_clips = chunk;
+    const size_t ws_bytes = mode == 0 ? feat_ws_carve(pl, sized, steps, nullptr, nullptr) : 0;
+    int rc = ensure_pipe(pl, clip_bytes * chunk, out_bytes, ws_bytes, !in_pinned, !out_pinned, &hp);
     if (rc != DSPX_OK) return rc;
     // "_host" contract: nothing may still be reading the caller's input or writing the caller's output when
     // the call returns, also on the error paths below
@@ -546,7 +429,7 @@ static int host_pipeline(dspx_plan *pl, int mode, const void *clips_v, int64_t n
             const int64_t f = pend[s].first, c = pend[s].count;
             const char *h = static_cast<const char *>(hp->h_out[s]);
             if (lm_b) parallel_rows_copy((char *)(o_logmel + (size_t)f * (lm_b / 4)), lm_b, h, lm_b, lm_b, c);
-            if (mf_b && o_mfcc) parallel_rows_copy((char *)(o_mfcc + (size_t)f * (mf_b / 4)), mf_b, h + off_mf, mf_b, mf_b, c);
+            if (mf_b) parallel_rows_copy((char *)(o_mfcc + (size_t)f * (mf_b / 4)), mf_b, h + off_mf, mf_b, mf_b, c);
             if (em_b) memcpy(o_embed + (size_t)f * (em_b / 4), h + off_em, em_b * c);
             if (st_b) parallel_rows_copy((char *)(o_stft + (size_t)f * (st_b / 4)), st_b, h + off_st, st_b, st_b, c);
         }
@@ -570,26 +453,21 @@ static int host_pipeline(dspx_plan *pl, int mode, const void *clips_v, int64_t n
             parallel_rows_copy(h, clip_bytes, src, (size_t)clip_stride * elem, clip_bytes, cnt);
             DSPX_CUDA_CHECK(cudaMemcpyAsync(d_raw, h, clip_bytes * cnt, cudaMemcpyHostToDevice, st));
         }
-        float *d_clips = static_cast<float *>(d_raw);
-        if (elem == 2 && !fused_pcm) {
-            d_clips = static_cast<float *>(hp->d_f32[slot]);
-            pcm16_to_float_kernel<<<(unsigned)cnt, 256, 0, st>>>(static_cast<const int16_t *>(d_raw), clip_len, clip_len,
-                                                                 normalize, d_clips, clip_len);
-            DSPX_CUDA_CHECK(cudaGetLastError());
-        }
         float *d_lm = lm_b ? reinterpret_cast<float *>(d_o) : nullptr;
         float *d_mf = mf_b ? reinterpret_cast<float *>(d_o + off_mf) : nullptr;
         float *d_em = em_b ? reinterpret_cast<float *>(d_o + off_em) : nullptr;
         float *d_st = st_b ? reinterpret_cast<float *>(d_o + off_st) : nullptr;
-        if (fused_pcm)
-            rc = features_device_pcm16(pl, static_cast<const int16_t *>(d_raw), cnt, clip_len, clip_len, normalize, d_lm, d_mf,
-                                       d_em, static_cast<int *>(hp->d_f32[slot]), st);
-        else if (mode == 0)
-            rc = fused_embed ? features_device(pl, d_clips, cnt, clip_len, clip_len, d_lm, nullptr, d_em, st, 0,
-                                               reinterpret_cast<long long *>(d_mf))
-                             : features_device(pl, d_clips, cnt, clip_len, clip_len, d_lm, d_mf, d_em, st);
-        else
-            rc = stft_device(pl, d_clips, cnt, clip_len, clip_len, T, pre, reinterpret_cast<float2 *>(d_st), st);
+        if (mode == 0) {
+            FeatBatch b = batch;
+            b.samples = d_raw;
+            b.n_clips = cnt;
+            FeatWs ws;
+            feat_ws_carve(pl, b, steps, static_cast<char *>(hp->d_ws[slot]), &ws);
+            rc = run_features(pl, b, steps, FeatOut{d_lm, d_mf, d_em, 0}, ws, st);
+        } else {
+            rc = stft_device(pl, static_cast<const float *>(d_raw), cnt, clip_len, clip_len, T, pre,
+                             reinterpret_cast<float2 *>(d_st), st);
+        }
         if (rc != DSPX_OK) return rc;
         char *h_o = out_pinned ? nullptr : static_cast<char *>(hp->h_out[slot]);
         auto d2h = [&](float *user, size_t per, size_t off, const void *dsrc) -> int {
@@ -599,7 +477,7 @@ static int host_pipeline(dspx_plan *pl, int mode, const void *clips_v, int64_t n
             return DSPX_OK;
         };
         if ((rc = d2h(o_logmel, lm_b, 0, d_lm)) != DSPX_OK) return rc;
-        if (o_mfcc && (rc = d2h(o_mfcc, mf_b, off_mf, d_mf)) != DSPX_OK) return rc;
+        if ((rc = d2h(o_mfcc, mf_b, off_mf, d_mf)) != DSPX_OK) return rc;
         if ((rc = d2h(o_embed, em_b, off_em, d_em)) != DSPX_OK) return rc;
         if ((rc = d2h(o_stft, st_b, off_st, d_st)) != DSPX_OK) return rc;
         pend[slot].first = first;
@@ -721,34 +599,15 @@ int dspx_plan_create(const dspx_config *cfg, int device, dspx_plan **out)
 
     dspx_plan *p = new (std::nothrow) dspx_plan();
     if (!p) { set_error("out of host memory"); return DSPX_ENOMEM; }
-    p->cfg = *cfg;
     p->device = device;
     p->host_pipe = new (std::nothrow) HostPipe();
     if (!p->host_pipe) { set_error("out of host memory"); delete p; return DSPX_ENOMEM; }
-    const int nfft_raw = cfg->n_fft > 0 ? cfg->n_fft : cfg->frame_length;
-    const int64_t P = next_pow_two(nfft_raw);
-    if (P < 16 || P > 8192) {
-        set_error("transform length %lld unsupported (power of two in [16, 8192])", (long long)P);
+    int rc = plan_derive(cfg, p);
+    if (rc != DSPX_OK) {
         plan_free_device(p);
         delete p;
-        return DSPX_EUNSUPPORTED;
+        return rc;
     }
-    p->P = (int)P;
-    p->M = p->P / 2;
-    p->n_bins = p->P / 2 + 1;
-    p->take_feat = cfg->frame_length < p->P ? cfg->frame_length : p->P;       // mfcc.py:89-98
-    p->take_stft = cfg->frame_length < nfft_raw ? cfg->frame_length : nfft_raw; // fft.py:32-33
-    int m = p->M, ns = 0;
-    while (m > 1) {
-        if (m % 4 == 0) { p->radix[ns++] = 4; m /= 4; }
-        else { p->radix[ns++] = 2; m /= 2; }
-    }
-    p->n_stages = ns;
-
-    build_window(cfg->window, cfg->frame_length, p->host.window);
-    const double f_max = cfg->f_max < 0.0 ? (double)cfg->sample_rate / 2.0 : cfg->f_max;
-    build_filterbank(cfg->n_mels, p->P, cfg->sample_rate, cfg->f_min, f_max, p->host);
-    build_dct2(cfg->n_mfcc, cfg->n_mels, p->host.dct2);
 
     DeviceGuard guard(device);
     if (!guard.ok) { set_error("cudaSetDevice(%d) failed", device); plan_free_device(p); delete p; return DSPX_ECUDA; }
@@ -756,38 +615,17 @@ int dspx_plan_create(const dspx_config *cfg, int device, dspx_plan **out)
     if (cudaGetDeviceProperties(&prop, device) != cudaSuccess) { set_error("cudaGetDeviceProperties failed"); plan_free_device(p); delete p; return DSPX_ECUDA; }
     p->sm_count = prop.multiProcessorCount;
 
-    std::vector<float> w32(p->host.window.begin(), p->host.window.end());
-    std::vector<float> d32(p->host.dct2.begin(), p->host.dct2.end());
-    std::vector<float2> tw(p->P);
-    for (int j = 0; j < p->P; j++) {
-        const double a = -2.0 * M_PI * (double)j / (double)p->P;
-        tw[j] = make_float2((float)std::cos(a), (float)std::sin(a));
-    }
-    int rc = DSPX_OK;
-    if (rc == DSPX_OK) rc = upload(w32, &p->d_window);
-    if (rc == DSPX_OK) rc = upload(tw, &p->d_tw);
+    rc = upload(p->host.window32, &p->d_window);
+    if (rc == DSPX_OK) rc = upload(p->host.tw, &p->d_tw);
     if (rc == DSPX_OK) rc = upload(p->host.fb_start, &p->d_fb_start);
     if (rc == DSPX_OK) rc = upload(p->host.fb_cnt, &p->d_fb_cnt);
     if (rc == DSPX_OK) rc = upload(p->host.fb_off, &p->d_fb_off);
     if (rc == DSPX_OK) rc = upload(p->host.fb_w, &p->d_fb_w);
-    if (rc == DSPX_OK) rc = upload(d32, &p->d_dct2);
+    if (rc == DSPX_OK) rc = upload(p->host.dct2_32, &p->d_dct2);
     if (rc == DSPX_OK) rc = upload(p->host.bin_filt, &p->d_bin_filt);
     if (rc == DSPX_OK) rc = upload(p->host.bin_wfall, &p->d_bin_wfall);
     if (rc == DSPX_OK) rc = upload(p->host.bin_wrise, &p->d_bin_wrise);
-
-    p->kernel = DSPX_KERNEL_GENERIC;
-    if (rc == DSPX_OK && cfg->kernel != DSPX_KERNEL_GENERIC) {
-        const bool ok = warp8_supported(p);
-        if (cfg->kernel == DSPX_KERNEL_WARP8 && !ok) {
-            set_error("warp8 kernel does not support this configuration");
-            rc = DSPX_EUNSUPPORTED;
-        } else if (ok) {
-            rc = warp8_prepare(p);
-            if (rc == DSPX_OK) p->kernel = DSPX_KERNEL_WARP8;
-            // tables too large for shared memory (e.g. 256 mels at n_fft 1024, 128 mels at 4096): the generic kernel
-            else if (rc == DSPX_EUNSUPPORTED && cfg->kernel != DSPX_KERNEL_WARP8) rc = DSPX_OK;
-        }
-    }
+    if (rc == DSPX_OK && p->kernel == DSPX_KERNEL_WARP8) rc = warp8_prepare(p);
     if (rc != DSPX_OK) {
         plan_free_device(p);
         delete p;
@@ -881,8 +719,9 @@ int dspx_features(const dspx_plan *plan, const float *clips_dev, int64_t n_clips
     if (dspx_num_frames(plan, clip_len) < 0) return DSPX_EINVAL;
     if (n_clips == 0) return DSPX_OK;
     DeviceGuard guard(plan->device);
-    return features_device(plan, clips_dev, n_clips, clip_len, clip_stride, logmel_out_dev, mfcc_out_dev, embed_out_dev,
-                           static_cast<cudaStream_t>(stream));
+    const FeatBatch b{clips_dev, DSPX_DTYPE_F32, 0, n_clips, clip_len, clip_stride, nullptr, nullptr};
+    return run_features(plan, b, feat_steps(plan, b, mfcc_out_dev != nullptr, embed_out_dev != nullptr),
+                        FeatOut{logmel_out_dev, mfcc_out_dev, embed_out_dev, 0}, FeatWs{}, static_cast<cudaStream_t>(stream));
 }
 
 size_t dspx_embeddings_workspace(const dspx_plan *plan, int64_t n_clips)
@@ -900,10 +739,17 @@ int dspx_embeddings(const dspx_plan *plan, const float *clips_dev, int64_t n_cli
     if (dspx_num_frames(plan, clip_len) < 0) return DSPX_EINVAL;
     if (n_clips == 0) return DSPX_OK;
     DeviceGuard guard(plan->device);
-    char *ws = static_cast<char *>(workspace_dev);
-    ws += (256 - (reinterpret_cast<uintptr_t>(ws) & 255)) & 255;
-    return features_device(plan, clips_dev, n_clips, clip_len, clip_stride, logmel_out_dev, nullptr, embed_out_dev,
-                           static_cast<cudaStream_t>(stream), 0, reinterpret_cast<long long *>(ws));
+    const FeatBatch b{clips_dev, DSPX_DTYPE_F32, 0, n_clips, clip_len, clip_stride, nullptr, nullptr};
+    const FeatSteps s = feat_steps(plan, b, false, true);
+    if (!s.fused) {
+        set_error("embeddings without an MFCC buffer need the warp8 kernel (n_fft 512 / 1024 / 2048), frame_length = "
+                  "n_fft, an even hop and row stride, 8-byte aligned clips and at most %lld frames per clip",
+                  (long long)w8_embed_max_frames(plan->cfg.n_mels));
+        return DSPX_EUNSUPPORTED;
+    }
+    FeatWs ws;
+    feat_ws_carve(plan, b, s, ws_align(workspace_dev), &ws);
+    return run_features(plan, b, s, FeatOut{logmel_out_dev, nullptr, embed_out_dev, 0}, ws, static_cast<cudaStream_t>(stream));
 }
 
 int dspx_log_mel_nchw(const dspx_plan *plan, const float *clips_dev, int64_t n_clips, int64_t clip_len,
@@ -914,8 +760,9 @@ int dspx_log_mel_nchw(const dspx_plan *plan, const float *clips_dev, int64_t n_c
     if (dspx_num_frames(plan, clip_len) < 0) return DSPX_EINVAL;
     if (n_clips == 0) return DSPX_OK;
     DeviceGuard guard(plan->device);
-    return features_device(plan, clips_dev, n_clips, clip_len, clip_stride, out_dev, nullptr, nullptr,
-                           static_cast<cudaStream_t>(stream), 1);
+    const FeatBatch b{clips_dev, DSPX_DTYPE_F32, 0, n_clips, clip_len, clip_stride, nullptr, nullptr};
+    return run_features(plan, b, feat_steps(plan, b, false, false), FeatOut{out_dev, nullptr, nullptr, 1}, FeatWs{},
+                        static_cast<cudaStream_t>(stream));
 }
 
 int dspx_embed_stats(const float *feats_dev, int64_t n_clips, int64_t n_frames, int n_coef, float *out_dev, void *stream)
@@ -958,7 +805,8 @@ size_t dspx_features_ragged_workspace(const dspx_plan *plan, const dspx_ragged_c
 {
     (void)want_logmel;
     if (!plan || n_clips < 0 || (n_clips > 0 && !table_host)) return 0;
-    return ragged_ws_carve(plan, table_host, n_clips, dtype, normalize, want_mfcc != 0, want_embed != 0, nullptr, nullptr);
+    const FeatBatch b{nullptr, dtype, normalize ? 1 : 0, n_clips, 0, 0, table_host, nullptr};
+    return feat_ws_carve(plan, b, feat_steps(plan, b, want_mfcc != 0, want_embed != 0), nullptr, nullptr);
 }
 
 int dspx_features_ragged(const dspx_plan *plan, const void *samples_dev, int dtype, int normalize,
@@ -981,15 +829,16 @@ int dspx_features_ragged(const dspx_plan *plan, const void *samples_dev, int dty
     for (int64_t i = 0; i < n_clips; i++)
         DSPX_REQUIRE(table_host[i].length >= plan->cfg.frame_length, "clip %lld: %lld samples is shorter than one frame (%d)",
                      (long long)i, (long long)table_host[i].length, plan->cfg.frame_length);
-    const size_t need = dspx_features_ragged_workspace(plan, table_host, n_clips, dtype, normalize, logmel_out_dev != nullptr,
-                                                       mfcc_out_dev != nullptr, embed_out_dev != nullptr);
+    const FeatBatch b{samples_dev, dtype, normalize ? 1 : 0, n_clips, 0, 0, table_host, table_dev};
+    const FeatSteps s = feat_steps(plan, b, mfcc_out_dev != nullptr, embed_out_dev != nullptr);
+    const size_t need = feat_ws_carve(plan, b, s, nullptr, nullptr);
     DSPX_REQUIRE(workspace_dev && workspace_bytes >= need, "workspace too small (%zu bytes needed)", need);
     if (!logmel_out_dev && !mfcc_out_dev && !embed_out_dev) return DSPX_OK;
     DeviceGuard guard(plan->device);
-    char *ws = static_cast<char *>(workspace_dev);
-    ws += (256 - (reinterpret_cast<uintptr_t>(ws) & 255)) & 255;
-    return features_ragged(plan, samples_dev, dtype, normalize ? 1 : 0, table_dev, table_host, n_clips, logmel_out_dev,
-                           mfcc_out_dev, embed_out_dev, ws, static_cast<cudaStream_t>(stream));
+    FeatWs ws;
+    feat_ws_carve(plan, b, s, ws_align(workspace_dev), &ws);
+    return run_features(plan, b, s, FeatOut{logmel_out_dev, mfcc_out_dev, embed_out_dev, 0}, ws,
+                        static_cast<cudaStream_t>(stream));
 }
 
 int dspx_embed_stats_ragged(const float *feats_dev, const dspx_ragged_clip *table_dev, int64_t n_clips, int n_coef,
@@ -1050,10 +899,19 @@ int dspx_features_pcm16(const dspx_plan *plan, const int16_t *pcm_dev, int64_t n
     if (dspx_num_frames(plan, clip_len) < 0) return DSPX_EINVAL;
     if (n_clips == 0) return DSPX_OK;
     DeviceGuard guard(plan->device);
-    char *ws = static_cast<char *>(workspace_dev);
-    if (ws) ws += (256 - (reinterpret_cast<uintptr_t>(ws) & 255)) & 255;
-    return features_device_pcm16(plan, pcm_dev, n_clips, clip_len, pcm_stride, normalize ? 1 : 0, logmel_out_dev, mfcc_out_dev,
-                                 embed_out_dev, reinterpret_cast<int *>(ws), static_cast<cudaStream_t>(stream));
+    const FeatBatch b{pcm_dev, DSPX_DTYPE_PCM16, normalize ? 1 : 0, n_clips, clip_len, pcm_stride, nullptr, nullptr};
+    const FeatSteps s = feat_steps(plan, b, mfcc_out_dev != nullptr, embed_out_dev != nullptr);
+    if (s.convert) {
+        set_error("fused PCM16 ingest needs the warp8 kernel (n_fft 512 / 1024 / 2048) and fewer than 2^31 frame pairs: "
+                  "convert with dspx_pcm16_to_float first");
+        return DSPX_EUNSUPPORTED;
+    }
+    DSPX_REQUIRE(!embed_out_dev || mfcc_out_dev, "embed_out needs mfcc_out on the PCM16 path");
+    DSPX_REQUIRE(n_clips < (int64_t)2147483647, "too many clips for one launch");
+    FeatWs ws;
+    feat_ws_carve(plan, b, s, ws_align(workspace_dev), &ws);
+    return run_features(plan, b, s, FeatOut{logmel_out_dev, mfcc_out_dev, embed_out_dev, 0}, ws,
+                        static_cast<cudaStream_t>(stream));
 }
 
 int dspx_features_host_pcm16(const dspx_plan *plan, const int16_t *pcm_host, int64_t n_clips, int64_t clip_len,
@@ -1337,10 +1195,8 @@ int dspx_resample(const dspx_resampler *rs, const void *in_dev, int dtype, int64
     DSPX_REQUIRE(!normalize || (workspace_dev && workspace_bytes >= dspx_resample_workspace(n_clips)), "workspace too small");
     if (n_clips == 0) return DSPX_OK;
     DeviceGuard guard(rs->device);
-    char *ws = static_cast<char *>(workspace_dev);
-    if (ws) ws += (256 - (reinterpret_cast<uintptr_t>(ws) & 255)) & 255;
     const RsBatch b{in_dev, dtype == DSPX_DTYPE_PCM16, n_in, in_stride, out_dev, out_stride, nullptr};
-    return resample_launch(rs, b, n_clips, n_out, normalize ? 1 : 0, reinterpret_cast<unsigned *>(ws),
+    return resample_launch(rs, b, n_clips, n_out, normalize ? 1 : 0, reinterpret_cast<unsigned *>(ws_align(workspace_dev)),
                            static_cast<cudaStream_t>(stream));
 }
 
@@ -1390,10 +1246,8 @@ int dspx_resample_ragged(const dspx_resampler *rs, const void *in_dev, int dtype
         max_out = std::max(max_out, r.out_length);
     }
     DeviceGuard guard(rs->device);
-    char *ws = static_cast<char *>(workspace_dev);
-    if (ws) ws += (256 - (reinterpret_cast<uintptr_t>(ws) & 255)) & 255;
     const RsBatch b{in_dev, dtype == DSPX_DTYPE_PCM16, 0, 0, out_dev, 0, table_dev};
-    return resample_launch(rs, b, n_clips, max_out, normalize ? 1 : 0, reinterpret_cast<unsigned *>(ws),
+    return resample_launch(rs, b, n_clips, max_out, normalize ? 1 : 0, reinterpret_cast<unsigned *>(ws_align(workspace_dev)),
                            static_cast<cudaStream_t>(stream));
 }
 

@@ -56,6 +56,13 @@ const char *get_error();
 
 inline size_t align256(size_t x) { return (x + 255) & ~(size_t)255; }
 
+// A caller's workspace moved up to the next 256-byte boundary: the workspace size queries leave 256 bytes for this
+inline char *ws_align(void *p)
+{
+    char *c = static_cast<char *>(p);
+    return c ? c + ((256 - (reinterpret_cast<uintptr_t>(c) & 255)) & 255) : nullptr;
+}
+
 // Opt-in dynamic shared memory: a per-function, per-device attribute shared by every plan and thread.  It is
 // set once per (kernel, device) to the architectural maximum and never lowered, so launches of plans with
 // different shared-memory sizes cannot race on it (the size actually used is a launch argument).
@@ -89,6 +96,9 @@ struct HostTables {
     std::vector<float> bin_wfall;      // [n_bins]
     std::vector<float> bin_wrise;      // [n_bins]
     bool two_band_ok = false;          // per-bin form is exact for this filterbank
+    // float32 tables the generic kernel reads besides fb_*: window, DCT, twiddles exp(-2 pi i j / P)
+    std::vector<float> window32, dct2_32;
+    std::vector<float2> tw;
 };
 
 }  // namespace dspx

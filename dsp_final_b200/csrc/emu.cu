@@ -17,6 +17,7 @@
 #include "feat_warp8_x2.cuh"
 #include "resample.cuh"
 #include "retrieval_select.cuh"
+#include "feat_select.cuh"
 
 namespace dspx {
 void set_error(const char *, ...) {}
@@ -25,39 +26,21 @@ const char *get_error() { return ""; }
 
 using namespace dspx;
 
-struct EmuTables {
-    HostTables t;
-    std::vector<float> window, dct2;
-    std::vector<float2> tw;
-    int P = 0, M = 0, n_bins = 0, take_feat = 0, take_stft = 0, n_stages = 0;
-    int radix[16] = {0};
+// A plan as dspx_plan_create derives it (plan_derive), without the device uploads
+struct EmuPlan : dspx_plan {
+    ~EmuPlan() { warp8_release(this); }
 };
 
-static int emu_build(const dspx_config *cfg, EmuTables &e)
+// The warp8 tables of a configuration, also where they do not fit in shared memory (the plan then uses the generic kernel)
+static int emu_warp8_tables(const dspx_config *cfg, std::vector<float> &blob, W8Tables &tb)
 {
-    const int nfft_raw = cfg->n_fft > 0 ? cfg->n_fft : cfg->frame_length;
-    e.P = (int)next_pow_two(nfft_raw);
-    if (e.P < 16 || e.P > 8192) return DSPX_EUNSUPPORTED;
-    e.M = e.P / 2;
-    e.n_bins = e.M + 1;
-    e.take_feat = cfg->frame_length < e.P ? cfg->frame_length : e.P;
-    e.take_stft = cfg->frame_length < nfft_raw ? cfg->frame_length : nfft_raw;
-    int m = e.M;
-    while (m > 1) {
-        if (m % 4 == 0) { e.radix[e.n_stages++] = 4; m /= 4; }
-        else { e.radix[e.n_stages++] = 2; m /= 2; }
-    }
-    if (!build_window(cfg->window, cfg->frame_length, e.t.window)) return DSPX_EINVAL;
-    const double f_max = cfg->f_max < 0.0 ? cfg->sample_rate / 2.0 : cfg->f_max;
-    build_filterbank(cfg->n_mels, e.P, cfg->sample_rate, cfg->f_min, f_max, e.t);
-    build_dct2(cfg->n_mfcc, cfg->n_mels, e.t.dct2);
-    e.window.assign(e.t.window.begin(), e.t.window.end());
-    e.dct2.assign(e.t.dct2.begin(), e.t.dct2.end());
-    e.tw.resize(e.P);
-    for (int j = 0; j < e.P; j++) {
-        const double a = -2.0 * M_PI * (double)j / (double)e.P;
-        e.tw[j] = make_float2((float)std::cos(a), (float)std::sin(a));
-    }
+    dspx_config gc = *cfg;
+    gc.kernel = DSPX_KERNEL_GENERIC;
+    EmuPlan pl;
+    const int rc = plan_derive(&gc, &pl);
+    if (rc != DSPX_OK) return rc;
+    if (!warp8_supported(&pl)) return DSPX_EUNSUPPORTED;
+    warp8_build_tables(&pl, blob, tb);
     return DSPX_OK;
 }
 
@@ -68,9 +51,12 @@ int emu_features_generic(const dspx_config *cfg, const float *clips, int64_t n_c
                          int64_t clip_stride, int stft_mode, int stft_pre, float *logmel, float *mfcc, float *stft_out,
                          int frames_per_cta_override)
 {
-    EmuTables e;
-    int rc = emu_build(cfg, e);
+    dspx_config gc = *cfg;
+    gc.kernel = DSPX_KERNEL_GENERIC;
+    EmuPlan pl;
+    int rc = plan_derive(&gc, &pl);
     if (rc != DSPX_OK) return rc;
+    const HostTables &h = pl.host;
     if (clip_len < cfg->frame_length) return DSPX_EINVAL;
     const int64_t T = 1 + (clip_len - cfg->frame_length) / cfg->hop_length;
     GenParams p{};
@@ -81,15 +67,15 @@ int emu_features_generic(const dspx_config *cfg, const float *clips, int64_t n_c
     p.n_frames = T;
     p.frame_length = cfg->frame_length;
     p.hop = cfg->hop_length;
-    p.take = stft_mode ? e.take_stft : e.take_feat;
-    p.P = e.P;
-    p.M = e.M;
-    p.n_bins = e.n_bins;
-    p.n_stages = e.n_stages;
-    for (int i = 0; i < 16; i++) p.radix[i] = e.radix[i];
+    p.take = stft_mode ? pl.take_stft : pl.take_feat;
+    p.P = pl.P;
+    p.M = pl.M;
+    p.n_bins = pl.n_bins;
+    p.n_stages = pl.n_stages;
+    for (int i = 0; i < 16; i++) p.radix[i] = pl.radix[i];
     p.n_mels = cfg->n_mels;
     p.n_mfcc = cfg->n_mfcc;
-    int G = 1024 / e.M;
+    int G = 1024 / pl.M;
     if (G < 1) G = 1;
     if (G > 16) G = 16;
     p.G = G;
@@ -99,13 +85,13 @@ int emu_features_generic(const dspx_config *cfg, const float *clips, int64_t n_c
     p.ctas_per_clip = (int)((T + p.frames_per_cta - 1) / p.frames_per_cta);
     p.pre = stft_mode ? (stft_pre && cfg->pre_emphasis > 0.0) : (cfg->pre_emphasis > 0.0);
     p.alpha = (float)cfg->pre_emphasis;
-    p.window = e.window.data();
-    p.tw = e.tw.data();
-    p.fb_start = e.t.fb_start.data();
-    p.fb_cnt = e.t.fb_cnt.data();
-    p.fb_off = e.t.fb_off.data();
-    p.fb_w = e.t.fb_w.data();
-    p.dct2 = e.dct2.data();
+    p.window = h.window32.data();
+    p.tw = h.tw.data();
+    p.fb_start = h.fb_start.data();
+    p.fb_cnt = h.fb_cnt.data();
+    p.fb_off = h.fb_off.data();
+    p.fb_w = h.fb_w.data();
+    p.dct2 = h.dct2_32.data();
     p.logmel = logmel;
     p.lm_ts = p.n_mels;
     p.lm_fs = 1;
@@ -148,19 +134,10 @@ int emu_features_generic(const dspx_config *cfg, const float *clips, int64_t n_c
 //        bins that share a tile slot with another bin (must be 0)}
 int emu_warp8_layout(const dspx_config *cfg, int32_t *out)
 {
-    EmuTables e;
-    int rc = emu_build(cfg, e);
-    if (rc != DSPX_OK) return rc;
-    dspx_plan pl;
-    pl.cfg = *cfg;
-    pl.P = e.P;
-    pl.M = e.M;
-    pl.n_bins = e.n_bins;
-    pl.host = e.t;
-    if (!warp8_supported(&pl)) return DSPX_EUNSUPPORTED;
     std::vector<float> blob;
     W8Tables tb{};
-    warp8_build_tables(&pl, blob, tb);
+    const int rc = emu_warp8_tables(cfg, blob, tb);
+    if (rc != DSPX_OK) return rc;
     if (tb.x2) return DSPX_EUNSUPPORTED;
     const int units = tb.r1 >= 8 ? tb.r1 / 8 : 1, active = tb.r1 >= 8 ? 32 : 16, M = 64 * tb.r1, J = 8 * tb.r1;
     const int32_t *ppos = reinterpret_cast<const int32_t *>(blob.data() + tb.ppos);
@@ -223,19 +200,10 @@ int emu_warp8_layout(const dspx_config *cfg, int32_t *out)
 // 20-, 12- and 10-warp configurations (0 where one does not fit), 8-warp CTAs per SM, first-pass radix, x2 (n_fft 4096)}
 int emu_warp8_shapes(const dspx_config *cfg, int64_t *out)
 {
-    EmuTables e;
-    int rc = emu_build(cfg, e);
-    if (rc != DSPX_OK) return rc;
-    dspx_plan pl;
-    pl.cfg = *cfg;
-    pl.P = e.P;
-    pl.M = e.M;
-    pl.n_bins = e.n_bins;
-    pl.host = e.t;
-    if (!warp8_supported(&pl)) return DSPX_EUNSUPPORTED;
     std::vector<float> blob;
     W8Tables tb{};
-    warp8_build_tables(&pl, blob, tb);
+    const int rc = emu_warp8_tables(cfg, blob, tb);
+    if (rc != DSPX_OK) return rc;
     const W8Shapes s = warp8_shapes(tb, cfg->n_mels);
     out[0] = (int64_t)tb.total * 4; out[1] = s.smem; out[2] = s.smem_wide; out[3] = s.smem_mid; out[4] = s.smem_r16;
     out[5] = s.ctas_per_sm; out[6] = tb.r1; out[7] = tb.x2;
@@ -249,27 +217,17 @@ static int emu_warp8(const dspx_config *cfg, const float *clips, int64_t n_clips
                      int64_t clip_stride, float *logmel, float *mfcc, float *stft_out, int stft_pre,
                      const dspx_ragged_clip *rtab)
 {
-    EmuTables e;
-    int rc = emu_build(cfg, e);
-    if (rc != DSPX_OK) return rc;
-    dspx_plan pl;
-    pl.cfg = *cfg;
-    pl.P = e.P;
-    pl.M = e.M;
-    pl.n_bins = e.n_bins;
-    pl.host = e.t;
-    pl.take_stft = e.take_stft;
-    pl.kernel = DSPX_KERNEL_WARP8;
-    if (!warp8_supported(&pl) || (!rtab && clip_len < cfg->frame_length)) return DSPX_EUNSUPPORTED;
+    EmuPlan pl;
+    if (plan_derive(cfg, &pl) != DSPX_OK || pl.kernel != DSPX_KERNEL_WARP8 || (!rtab && clip_len < cfg->frame_length))
+        return DSPX_EUNSUPPORTED;
     const int64_t T = rtab ? 0 : 1 + (clip_len - cfg->frame_length) / cfg->hop_length;
     // the variant the library would launch
     const W8Path path = warp8_select(&pl, clips, clip_stride, DSPX_DTYPE_F32, rtab != nullptr, n_clips, T,
                                      stft_out ? W8_WANT_STFT : W8_WANT_FEATURES);
     if (path == W8_GENERIC || path == W8_UNSUPPORTED) return DSPX_EUNSUPPORTED;
     const bool u4 = path == W8_U4, share = path == W8_SHARE;
-    std::vector<float> blob;
-    W8Tables tb{};
-    warp8_build_tables(&pl, blob, tb);
+    W8PlanData &pd = *static_cast<W8PlanData *>(pl.fast_host);
+    const W8Tables &tb = pd.tb;
     W8Params p{};
     p.clips = clips;
     p.n_clips = n_clips;
@@ -290,7 +248,7 @@ static int emu_warp8(const dspx_config *cfg, const float *clips, int64_t n_clips
     p.n_mfcc = cfg->n_mfcc;
     p.alpha = (float)cfg->pre_emphasis;
     p.tb = tb;
-    p.tables = blob.data();
+    p.tables = pd.blob.data();
     p.logmel = logmel;
     p.mfcc = mfcc;
     p.lm_ts = p.n_mels;
@@ -302,7 +260,7 @@ static int emu_warp8(const dspx_config *cfg, const float *clips, int64_t n_clips
     // 16-byte align the warp tile like the device carve-up does
     float *ws = warp_smem.data();
     while (reinterpret_cast<uintptr_t>(ws) & 15) ws++;
-    w8_carve(blob.data(), ws, tb, p.n_mels, c);
+    w8_carve(pd.blob.data(), ws, tb, p.n_mels, c);
     c.alpha = p.alpha;
     c.win_a = cfg->window == DSPX_WINDOW_HANN ? 0.25f : (cfg->window == DSPX_WINDOW_HAMMING ? 0.27f : 0.5f);
     c.win_b = cfg->window == DSPX_WINDOW_HANN ? -0.25f : (cfg->window == DSPX_WINDOW_HAMMING ? -0.23f : 0.f);
@@ -312,7 +270,7 @@ static int emu_warp8(const dspx_config *cfg, const float *clips, int64_t n_clips
     c.cw_lanes = tb.cw_lanes;
     c.dct_row = tb.dct_row;
     c.lm_part = tb.lm_part;
-    c.take = cfg->frame_length < e.P ? cfg->frame_length : e.P;
+    c.take = pl.take_feat;
     const int r1 = tb.r1;
     const int units = r1 >= 8 ? r1 / 8 : 1;
     if (tb.x2) {
@@ -535,6 +493,57 @@ int emu_topk_workspace(int64_t nq, int64_t ndb, int dim, int k, int64_t *out)
         out[2 * i + 1] = p[i + 1] - p[i];
     }
     out[16] = (int64_t)total;
+    return DSPX_OK;
+}
+
+// A plan as dspx_plan_create derives it; *kernel: the DSPX_KERNEL_* it runs
+int emu_plan_create(const dspx_config *cfg, int *kernel, dspx_plan **out)
+{
+    EmuPlan *pl = new EmuPlan();
+    const int rc = plan_derive(cfg, pl);
+    if (rc != DSPX_OK) { delete pl; return rc; }
+    *kernel = pl->kernel;
+    *out = pl;
+    return DSPX_OK;
+}
+
+void emu_plan_destroy(dspx_plan *pl) { delete static_cast<EmuPlan *>(pl); }
+
+static FeatBatch emu_batch(const void *samples, int dtype, int normalize, int64_t n_clips, int64_t clip_len, int64_t stride,
+                           const dspx_ragged_clip *table)
+{
+    return table ? FeatBatch{samples, dtype, normalize, n_clips, 0, 0, table, nullptr}
+                 : FeatBatch{samples, dtype, normalize, n_clips, clip_len, stride, nullptr, nullptr};
+}
+
+// The steps of a feature call (feat_steps): out = {path (W8Path), convert, peaks, fused, mfcc_scratch, per_clip, T}.
+// samples is only compared for alignment; table != NULL: a ragged batch (clip_len and stride unused).
+int emu_feat_steps(const dspx_plan *pl, const void *samples, int dtype, int normalize, int64_t n_clips, int64_t clip_len,
+                   int64_t stride, const dspx_ragged_clip *table, int want_mfcc, int want_embed, int64_t *out)
+{
+    const FeatSteps s = feat_steps(pl, emu_batch(samples, dtype, normalize, n_clips, clip_len, stride, table), want_mfcc != 0,
+                                   want_embed != 0);
+    const int64_t v[7] = {s.path, s.convert, s.peaks, s.fused, s.mfcc_scratch, s.per_clip, s.T};
+    for (int i = 0; i < 7; i++) out[i] = v[i];
+    return DSPX_OK;
+}
+
+// The workspace of that call (feat_ws_carve) in a buffer that starts base_offset bytes past a 256-byte boundary, moved
+// up to the next one as the entry points do (ws_align): out = offsets from the buffer's start of rpairs, peaks, eacc,
+// mfcc and f32 (-1 where a step needs none), then the carve's size (dspx_features_ragged_workspace).
+int emu_feat_workspace(const dspx_plan *pl, const void *samples, int dtype, int normalize, int64_t n_clips, int64_t clip_len,
+                       int64_t stride, const dspx_ragged_clip *table, int want_mfcc, int want_embed, int64_t base_offset,
+                       int64_t *out)
+{
+    if (base_offset < 0) return DSPX_EINVAL;
+    const FeatBatch b = emu_batch(samples, dtype, normalize, n_clips, clip_len, stride, table);
+    const FeatSteps s = feat_steps(pl, b, want_mfcc != 0, want_embed != 0);
+    char *const buf = reinterpret_cast<char *>(((uintptr_t)1 << 44) + base_offset);   // never dereferenced
+    FeatWs w;
+    const size_t total = feat_ws_carve(pl, b, s, ws_align(buf), &w);
+    const char *p[5] = {(char *)w.rpairs, (char *)w.peaks, (char *)w.eacc, (char *)w.mfcc, (char *)w.f32};
+    for (int i = 0; i < 5; i++) out[i] = p[i] ? p[i] - buf : -1;
+    out[5] = (int64_t)total;
     return DSPX_OK;
 }
 

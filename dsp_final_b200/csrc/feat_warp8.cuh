@@ -1557,33 +1557,27 @@ inline W8Shapes warp8_shapes(const W8Tables &tb, int n_mels)
     return s;
 }
 
-// ---- launch (not in csrc/emu.cu, which replays the phase functions on the host and instantiates no kernel) --------
-#if defined(__CUDACC__) && !defined(DSPX_EMU)
+// The warp8 tables of a plan (plan_derive builds them on the host, warp8_prepare uploads the blob)
 struct W8PlanData : W8Shapes {
     W8Tables tb;
-};
-
-inline int warp8_prepare(dspx_plan *pl)
-{
     std::vector<float> blob;
-    W8Tables tb{};
-    warp8_build_tables(pl, blob, tb);
-    const W8Shapes shapes = warp8_shapes(tb, pl->cfg.n_mels);
-    if (shapes.smem > 227 * 1024) { set_error("warp8: tables too large for shared memory"); return DSPX_EUNSUPPORTED; }
-    auto *pd = new W8PlanData();
-    static_cast<W8Shapes &>(*pd) = shapes;
-    pd->tb = tb;
-    pl->fast_host = pd;
-    DSPX_CUDA_CHECK(cudaMalloc(&pl->d_fast_tables, blob.size() * sizeof(float)));
-    DSPX_CUDA_CHECK(cudaMemcpy(pl->d_fast_tables, blob.data(), blob.size() * sizeof(float), cudaMemcpyHostToDevice));
-    pl->fast_tables_bytes = blob.size() * sizeof(float);
-    return DSPX_OK;
-}
+};
 
 inline void warp8_release(dspx_plan *pl)
 {
     delete static_cast<W8PlanData *>(pl->fast_host);
     pl->fast_host = nullptr;
+}
+
+// ---- launch (not in csrc/emu.cu, which replays the phase functions on the host and instantiates no kernel) --------
+#if defined(__CUDACC__) && !defined(DSPX_EMU)
+inline int warp8_prepare(dspx_plan *pl)
+{
+    const std::vector<float> &blob = static_cast<const W8PlanData *>(pl->fast_host)->blob;
+    DSPX_CUDA_CHECK(cudaMalloc(&pl->d_fast_tables, blob.size() * sizeof(float)));
+    DSPX_CUDA_CHECK(cudaMemcpy(pl->d_fast_tables, blob.data(), blob.size() * sizeof(float), cudaMemcpyHostToDevice));
+    pl->fast_tables_bytes = blob.size() * sizeof(float);
+    return DSPX_OK;
 }
 
 // the launch fields that come from the plan alone

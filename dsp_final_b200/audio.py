@@ -34,8 +34,8 @@ def _riff_chunks(blob: bytes):
         pos += 8 + size + (size & 1)
 
 
-def read_wav_raw(path: str | Path) -> Tuple[np.ndarray, int, int]:
-    """(samples [n, channels] in the file's own dtype, sample_rate, format tag) of a WAV file."""
+def _wav_chunks(path: str | Path) -> Tuple[int, int, int, int, bytes]:
+    """(format code, channels, sample_rate, bits per sample, data chunk) of a WAV file."""
     fmt = data = None
     for tag, body in _riff_chunks(Path(path).read_bytes()):
         if tag == b"fmt ":
@@ -47,6 +47,12 @@ def read_wav_raw(path: str | Path) -> Tuple[np.ndarray, int, int]:
     code, channels, rate, _bps, _align, bits = struct.unpack_from("<HHIIHH", fmt, 0)
     if code == 0xFFFE and len(fmt) >= 26:                       # WAVE_FORMAT_EXTENSIBLE: real tag in the GUID
         code = struct.unpack_from("<H", fmt, 24)[0]
+    return code, channels, rate, bits, data
+
+
+def read_wav_raw(path: str | Path) -> Tuple[np.ndarray, int, int]:
+    """(samples [n, channels] in the file's own dtype, sample_rate, format tag) of a WAV file."""
+    code, channels, rate, bits, data = _wav_chunks(path)
     if code == 1 and bits == 16:
         x = np.frombuffer(data, dtype="<i2")
     elif code == 1 and bits == 8:
@@ -76,6 +82,30 @@ def read_wav(path: str | Path) -> Tuple[np.ndarray, int]:
     else:
         y = (x.astype(np.float64) / float(1 << (bits - 1))).astype(np.float32)
     return (y[:, 0] if y.shape[1] == 1 else y), rate
+
+
+# (format code, bits) -> (dtype code of include/dspx.h, bytes per sample)
+_DEVICE_ENCODINGS = {(1, 8): (3, 1), (1, 16): (2, 2), (1, 24): (4, 3), (1, 32): (5, 4), (3, 32): (0, 4), (3, 64): (1, 8)}
+MAX_DEVICE_CHANNELS = 32
+
+
+def read_wav_data(path: str | Path) -> Tuple[np.ndarray, int, int, int, int] | None:
+    """(data chunk as uint8, sample_rate, channels, dtype code, n_frames) with no conversion, for the device decoder.
+
+    The dtype code is one of include/dspx.h's DSPX_DTYPE_PCM8 / PCM16 / PCM24 / PCM32 / F32 / F64.  n_frames follows
+    read_wav_raw: whole samples, then whole frames, and the bytes returned are exactly those frames.  None when the
+    file is not a WAV file of one of those six encodings with 1 to 32 channels.
+    """
+    try:
+        code, channels, rate, bits, data = _wav_chunks(path)
+    except (ValueError, struct.error):
+        return None
+    enc = _DEVICE_ENCODINGS.get((code, bits))
+    if enc is None or not 1 <= channels <= MAX_DEVICE_CHANNELS:
+        return None
+    dtype, size = enc
+    n_frames = len(data) // size // channels
+    return np.frombuffer(data, np.uint8, n_frames * channels * size), int(rate), int(channels), dtype, n_frames
 
 
 def load_audio(path: str | Path, target_sr: int | None = None) -> Tuple[np.ndarray, int]:

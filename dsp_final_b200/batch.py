@@ -18,11 +18,14 @@ outputs are stacked along the frame axis and split per clip with "frame_offsets"
 resample_poly is scipy.signal.resample_poly on the GPU, bit for bit (dspx_resample).  With sample_rate= the
 clips' own rate, features_batch and features_ragged resample on the device first when it differs from
 cfg.sample_rate (src/utils/audio.py:27-30 resamples on the host there).
+
+load_audio_batch is load_audio (+ normalize_audio) for many WAV files at once: the files' data chunks go to the GPU
+as stored and are decoded, downmixed and resampled there, bit for bit (dspx_decode_ragged, dspx_resample_ragged).
 """
 from __future__ import annotations
 
 import ctypes as C
-from typing import Any, Iterable
+from typing import Any, Iterable, NamedTuple
 
 import numpy as np
 
@@ -510,6 +513,166 @@ def _features_ragged_resampled(clips: list, cfg: Any, want, device, normalize: b
         return res
     res = _as_host(res)
     res["frame_offsets"] = offsets
+    return res
+
+
+# struct dspx_decode_clip
+DECODE_CLIP = np.dtype([("in_offset", "<i8"), ("n_frames", "<i8"), ("channels", "<i4"), ("dtype", "<i4"),
+                        ("out_start", "<i8"), ("out_length", "<i8")])
+
+
+class PackedClips(NamedTuple):
+    """Clips of one packed float32 torch CUDA buffer: clip i is samples[starts[i]:starts[i] + lengths[i]], every start a
+    multiple of RAGGED_ALIGN, so the buffer is a valid ragged feature batch as it is."""
+    samples: Any
+    starts: np.ndarray
+    lengths: np.ndarray
+
+
+def _decode_layout(lib, offsets, parsed, idx) -> tuple[np.ndarray, int]:
+    """dspx_decode_layout of the files `idx` of `parsed` (read_wav_data tuples) at byte `offsets`."""
+    table = np.zeros(len(idx), DECODE_CLIP)
+    cols = [np.ascontiguousarray(np.asarray(v, dt)) for v, dt in (
+        ([offsets[i] for i in idx], np.int64), ([parsed[i][4] for i in idx], np.int64),
+        ([parsed[i][2] for i in idx], np.int32), ([parsed[i][3] for i in idx], np.int32))]
+    total = _lib.check(int(lib.dspx_decode_layout(*(c.ctypes.data for c in cols), len(idx), table.ctypes.data)),
+                       "dspx_decode_layout")
+    return table, int(total)
+
+
+def _decode(lib, data, table: np.ndarray, normalize: bool, out, dev) -> None:
+    """One dspx_decode_ragged call on torch's current stream into `out` (a float32 CUDA tensor)."""
+    import torch
+
+    if not len(table):
+        return
+    table_dev = torch.from_numpy(table.view(np.uint8)).to(dev)
+    ws_bytes = int(lib.dspx_decode_workspace(len(table)))
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+    _lib.check(lib.dspx_decode_ragged(data.data_ptr(), table_dev.data_ptr(), table.ctypes.data, len(table),
+                                      1 if normalize else 0, out.data_ptr(), ws.data_ptr(), ws_bytes,
+                                      torch.cuda.current_stream(dev.index).cuda_stream), "dspx_decode_ragged")
+
+
+def pack_files(parsed: list) -> tuple[Any, np.ndarray]:
+    """(pinned uint8 tensor holding the data chunks of read_wav_data tuples, their byte offsets: multiples of 16)."""
+    import torch
+
+    sizes = np.array([len(p[0]) for p in parsed], np.int64)
+    offsets = np.zeros(len(parsed), np.int64)
+    offsets[1:] = np.cumsum((sizes + 15) // 16 * 16)[:-1]
+    staging = torch.empty(max(int(offsets[-1] + sizes[-1]) if len(parsed) else 0, 1), dtype=torch.uint8, pin_memory=True)
+    host = staging.numpy()
+    for o, p in zip(offsets, parsed):
+        host[o:o + len(p[0])] = p[0]
+    return staging, offsets
+
+
+def decode_device(data, offsets: np.ndarray, parsed: list, target_sr: int | None, normalize: bool) -> PackedClips:
+    """The device part of decode_packed: `data` (a uint8 torch CUDA tensor) holds the data chunks of the read_wav_data
+    tuples `parsed` at byte `offsets`; work is enqueued on torch's current stream of data's device."""
+    import torch
+
+    lib = _lib.load()
+    dev = data.device
+    n = len(parsed)
+    direct = [i for i in range(n) if target_sr is None or parsed[i][1] == target_sr]
+    others = [i for i in range(n) if not (target_sr is None or parsed[i][1] == target_sr)]
+    starts, lengths = np.zeros(n, np.int64), np.array([p[4] for p in parsed], np.int64)
+    dtab, at = _decode_layout(lib, offsets, parsed, direct)
+    starts[direct] = dtab["out_start"]
+    rtab, r_total = _decode_layout(lib, offsets, parsed, others)
+    groups = []
+    for rate in sorted({parsed[i][1] for i in others}):
+        rows = [j for j, i in enumerate(others) if parsed[i][1] == rate]
+        up, down = reduce_ratio(target_sr, rate)
+        in_starts = np.ascontiguousarray(rtab["out_start"][rows])
+        in_lengths = np.ascontiguousarray(rtab["n_frames"][rows])
+        table = np.zeros((len(rows), 4), np.int64)
+        total = _lib.check(int(lib.dspx_resample_layout(up, down, in_starts.ctypes.data, in_lengths.ctypes.data, len(rows),
+                                                        table.ctypes.data)), "dspx_resample_layout")
+        base = (at + RAGGED_ALIGN - 1) // RAGGED_ALIGN * RAGGED_ALIGN
+        idx = [others[j] for j in rows]
+        starts[idx] = base + table[:, 2]
+        lengths[idx] = table[:, 3]
+        groups.append((up, down, table, base))
+        at = base + int(total)
+    with torch.cuda.device(dev.index):
+        out = torch.zeros(max(at, 1), dtype=torch.float32, device=dev)
+        _decode(lib, data, dtab, normalize, out, dev)
+        if groups:
+            scratch = torch.empty(max(r_total, 1), dtype=torch.float32, device=dev)
+            _decode(lib, data, rtab, False, scratch, dev)
+            stream = torch.cuda.current_stream(dev.index).cuda_stream
+            for up, down, table, base in groups:
+                table_dev = torch.from_numpy(table).to(dev)
+                ws_bytes = int(lib.dspx_resample_workspace(len(table)))
+                ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+                _lib.check(lib.dspx_resample_ragged(get_resampler(up, down, dev.index).handle, scratch.data_ptr(),
+                                                    _lib.DTYPE_F32, 1 if normalize else 0, table_dev.data_ptr(),
+                                                    table.ctypes.data, len(table), out[base:].data_ptr(), ws.data_ptr(),
+                                                    ws_bytes, stream), "dspx_resample_ragged")
+    return PackedClips(out, starts, lengths)
+
+
+def decode_packed(parsed: list, target_sr: int | None, normalize: bool, device: int | None = None) -> PackedClips:
+    """load_audio(path, target_sr)[0] (normalize_audio of it when `normalize`) of every file, from its read_wav_data
+    tuple, into one packed buffer on the GPU.
+
+    The data chunks travel as stored, at 16-byte offsets of one pinned buffer, in one host-to-device copy.  Files at
+    target_sr (or all of them when it is None) are decoded with the normalisation in one launch, straight into the
+    output buffer; the others are decoded without it into a scratch buffer (one launch), then resampled with it, one
+    dspx_resample_ragged launch per rate, each group of outputs at its own offset of the output buffer -- the
+    reference's order: decode, downmix, resample, normalise.
+    """
+    import torch
+
+    _lib.require_device()
+    dev = torch.device("cuda", torch.cuda.current_device() if device is None else int(device))
+    staging, offsets = pack_files(parsed)
+    with torch.cuda.device(dev.index):
+        data = staging.to(dev, non_blocking=True)
+    return decode_device(data, offsets, parsed, target_sr, normalize)
+
+
+def load_audio_batch(paths, target_sr: int | None = None, normalize: bool = False, device: int | None = None) -> list:
+    """[load_audio(p, target_sr)[0] for p in paths] (normalize_audio of each when `normalize`), decoded on the GPU.
+
+    Returns float32 torch CUDA tensors, views into one packed buffer, bit-identical to the host functions.  The files
+    may mix PCM 8/16/24/32-bit and IEEE float 32/64 WAV encodings, 1 to 32 channels, lengths and rates; each is
+    decoded and downmixed on the device, then resampled there when its rate is not target_sr.  A file of another
+    kind, or without audio frames, raises ValueError naming it.
+    """
+    from .audio import read_wav_data
+
+    parsed = []
+    for p in paths:
+        d = read_wav_data(p)
+        if d is None:
+            raise ValueError(f"{p}: not a WAV file of PCM 8/16/24/32-bit or IEEE float 32/64 samples with 1 to 32 channels")
+        if d[4] < 1:
+            raise ValueError(f"{p}: no audio frames")
+        parsed.append(d)
+    if not parsed:
+        return []
+    packed = decode_packed(parsed, None if target_sr is None else int(target_sr), normalize, device)
+    return [packed.samples[s:s + n] for s, n in zip(packed.starts.tolist(), packed.lengths.tolist())]
+
+
+def features_packed(packed: PackedClips, cfg: Any, want: Iterable[str] = ("mfcc",)) -> dict:
+    """features_ragged of the float32 clips of a PackedClips buffer, with no copy of the samples: NumPy outputs plus
+    "frame_offsets", as features_ragged returns for NumPy input."""
+    import torch
+
+    want = _want(want)
+    dev = packed.samples.device
+    starts, table, total = ragged_layout(packed.lengths, cfg, np.float32, packed.starts)
+    plan = get_plan(cfg, dev.index)
+    with torch.cuda.device(dev.index):
+        table_dev = torch.from_numpy(table).to(dev)
+        res, _ = ragged_launch(plan, packed.samples, False, table, table_dev, total, want)
+    res = _as_host(res)
+    res["frame_offsets"] = np.concatenate((table[:, 3], [total])).astype(np.int64)
     return res
 
 

@@ -80,9 +80,13 @@ def read_npy_shape(path: Path) -> tuple:
 def _features_per_clip(clips: list, cfg: Any, feature_types: tuple, normalize: bool = True,
                        sample_rate: int | None = None) -> dict:
     """{feature_type: one [n_frames, n_coef] array per clip}: one batch when the clips have one length, else one
-    ragged launch.  Clips at another `sample_rate` than cfg's are resampled on the GPU first."""
-    from .batch import features_batch, features_ragged, split_ragged
+    ragged launch.  Clips at another `sample_rate` than cfg's are resampled on the GPU first.  A PackedClips buffer
+    (already at cfg's rate and normalised) is one ragged launch on it as it is."""
+    from .batch import PackedClips, features_batch, features_packed, features_ragged, split_ragged
 
+    if isinstance(clips, PackedClips):
+        out = features_packed(clips, cfg, feature_types)
+        return {ft: split_ragged(out[ft], out["frame_offsets"]) for ft in feature_types}
     if len({c.shape for c in clips}) == 1:
         out = features_batch(np.stack(clips, axis=0), cfg, feature_types, normalize=normalize, sample_rate=sample_rate)
         return {ft: list(out[ft]) for ft in feature_types}

@@ -24,11 +24,14 @@
 #include "retrieval_select.cuh"
 #include "ingest.cuh"
 #include "resample.cuh"
+#include "decode.cuh"
 
 // the ctypes binding (dsp_final_b200/_lib.py) mirrors these layouts; tests assert the same numbers
 static_assert(sizeof(dspx_config) == 56 && offsetof(dspx_config, f_min) == 24 && offsetof(dspx_config, window) == 48,
               "dspx_config layout changed: update _lib.DspxConfig");
 static_assert(sizeof(dspx_plan_info) == 32, "dspx_plan_info layout changed: update _lib.DspxPlanInfo");
+static_assert(sizeof(dspx_decode_clip) == 40 && offsetof(dspx_decode_clip, out_start) == 24,
+              "dspx_decode_clip layout changed: update batch.py");
 
 namespace dspx {
 
@@ -563,6 +566,35 @@ static int resample_launch(const dspx_resampler *rs, RsBatch b, int64_t n_clips,
             DSPX_CUDA_CHECK(cudaGetLastError());
         }
     }
+    return DSPX_OK;
+}
+
+// ---- WAV decoding (decode.cuh) ---------------------------------------------------
+
+// A decode table row as dspx_decode_layout writes it; returns an error message or nullptr.
+static const char *decode_row_error(const dspx_decode_clip &r)
+{
+    if (dec_bytes(r.dtype) == 0) return "unknown dtype";
+    if (r.channels < 1 || r.channels > DSPX_MAX_CHANNELS) return "channels outside 1 .. 32";
+    if (r.n_frames < 1 || r.n_frames > DEC_MAX_LEN) return "n_frames outside 1 .. 2^40";
+    if (r.in_offset < 0 || r.in_offset % 16) return "in_offset negative or not a multiple of 16";
+    return nullptr;
+}
+
+// One launch per pass, split every 65535 clips (grid.y): decode (and fold the peaks), then, when normalising, the
+// divide pass.
+static int decode_launch(const void *in, const dspx_decode_clip *tab, int64_t n_clips, int64_t max_tiles, int normalize,
+                         float *out, unsigned *peaks, cudaStream_t st)
+{
+    if (normalize) DSPX_CUDA_CHECK(cudaMemsetAsync(peaks, 0, (size_t)n_clips * sizeof(unsigned), st));
+    const int passes[2] = {normalize ? DEC_PEAK : DEC_STORE, DEC_NORM};
+    for (int p = 0; p < (normalize ? 2 : 1); p++)
+        for (int64_t c0 = 0; c0 < n_clips; c0 += 65535) {
+            const unsigned nc = (unsigned)std::min<int64_t>(n_clips - c0, 65535);
+            wav_decode_kernel<<<dim3((unsigned)max_tiles, nc), DEC_THREADS, DEC_SMEM, st>>>(
+                static_cast<const unsigned char *>(in), tab + c0, out, normalize ? peaks + c0 : nullptr, passes[p]);
+            DSPX_CUDA_CHECK(cudaGetLastError());
+        }
     return DSPX_OK;
 }
 
@@ -1249,6 +1281,50 @@ int dspx_resample_ragged(const dspx_resampler *rs, const void *in_dev, int dtype
     const RsBatch b{in_dev, dtype == DSPX_DTYPE_PCM16, 0, 0, out_dev, 0, table_dev};
     return resample_launch(rs, b, n_clips, max_out, normalize ? 1 : 0, reinterpret_cast<unsigned *>(ws_align(workspace_dev)),
                            static_cast<cudaStream_t>(stream));
+}
+
+// ---- WAV decoding ----
+
+int64_t dspx_decode_layout(const int64_t *in_offsets, const int64_t *n_frames, const int32_t *channels, const int32_t *dtypes,
+                           int64_t n_clips, dspx_decode_clip *table_out)
+{
+    DSPX_REQUIRE(n_clips >= 0, "negative clip count");
+    DSPX_REQUIRE(n_clips == 0 || (in_offsets && n_frames && channels && dtypes && table_out), "null argument");
+    int64_t at = 0;
+    for (int64_t i = 0; i < n_clips; i++) {
+        const dspx_decode_clip r{in_offsets[i], n_frames[i], channels[i], dtypes[i], at, n_frames[i]};
+        const char *bad = decode_row_error(r);
+        DSPX_REQUIRE(!bad, "clip %lld: %s (in_offset %lld, n_frames %lld, channels %d, dtype %d)", (long long)i, bad,
+                     (long long)r.in_offset, (long long)r.n_frames, (int)r.channels, (int)r.dtype);
+        table_out[i] = r;
+        at += (r.out_length + 3) & ~(int64_t)3;      // RAGGED_ALIGN: the packed output is a valid ragged batch
+    }
+    return n_clips ? table_out[n_clips - 1].out_start + table_out[n_clips - 1].out_length : 0;
+}
+
+size_t dspx_decode_workspace(int64_t n_clips) { return n_clips > 0 ? (size_t)n_clips * sizeof(unsigned) + 256 : 256; }
+
+int dspx_decode_ragged(const void *in_dev, const dspx_decode_clip *table_dev, const dspx_decode_clip *table_host,
+                       int64_t n_clips, int normalize, float *out_dev, void *workspace_dev, size_t workspace_bytes, void *stream)
+{
+    DSPX_REQUIRE(n_clips >= 0, "negative clip count");
+    if (n_clips == 0) return DSPX_OK;
+    DSPX_REQUIRE(in_dev && out_dev && table_dev && table_host, "null argument");
+    DSPX_REQUIRE(reinterpret_cast<uintptr_t>(in_dev) % 16 == 0 && reinterpret_cast<uintptr_t>(out_dev) % 16 == 0,
+                 "in_dev and out_dev must be 16-byte aligned");
+    DSPX_REQUIRE(!normalize || (workspace_dev && workspace_bytes >= dspx_decode_workspace(n_clips)), "workspace too small");
+    int64_t max_tiles = 0;
+    for (int64_t i = 0; i < n_clips; i++) {
+        const dspx_decode_clip &r = table_host[i];
+        const char *bad = decode_row_error(r);
+        DSPX_REQUIRE(!bad, "clip %lld: bad table row: %s", (long long)i, bad);
+        DSPX_REQUIRE(r.out_start >= 0 && r.out_start % 4 == 0 && r.out_length == r.n_frames,
+                     "clip %lld: out_start must be a non-negative multiple of 4 and out_length equal n_frames", (long long)i);
+        max_tiles = std::max(max_tiles, dec_tiles(r));
+    }
+    DSPX_REQUIRE(max_tiles < (int64_t)0x7fffffff, "clip too long for one launch");
+    return decode_launch(in_dev, table_dev, n_clips, max_tiles, normalize ? 1 : 0, out_dev,
+                         reinterpret_cast<unsigned *>(ws_align(workspace_dev)), static_cast<cudaStream_t>(stream));
 }
 
 }  // extern "C"

@@ -16,6 +16,7 @@
 #include "feat_warp8.cuh"
 #include "feat_warp8_x2.cuh"
 #include "resample.cuh"
+#include "decode.cuh"
 #include "retrieval_select.cuh"
 #include "feat_select.cuh"
 
@@ -464,6 +465,41 @@ int emu_resample(int64_t up, int64_t down, const float *window, int64_t n_window
         if (normalize)
             for (int64_t i = 0; i < c.n_out; i++) c.out[i] = rs_normalize(c.out[i], peak);
     }
+    return DSPX_OK;
+}
+
+// Replays wav_decode_kernel through the kernel's tile decomposition: each tile's input bytes are staged (dec_stage) into
+// a buffer of exactly the kernel's dynamic shared-memory size, decoded frame by frame (dec_frames) into the output
+// staging part of that buffer and stored (dec_store); with normalize, the peak pass over every tile of the batch
+// comes first, as on the device.  table: a dspx_decode_layout table; in / out as for dspx_decode_ragged.
+int emu_decode(const void *in, const dspx_decode_clip *table, int64_t n_clips, int normalize, float *out)
+{
+    for (int64_t i = 0; i < n_clips; i++)
+        if (dec_bytes(table[i].dtype) == 0 || table[i].channels < 1 || table[i].channels > DSPX_MAX_CHANNELS ||
+            table[i].n_frames < 1 || table[i].in_offset % 16 || table[i].out_start % 4)
+            return DSPX_EINVAL;
+    const unsigned char *src = static_cast<const unsigned char *>(in);
+    std::vector<unsigned> peaks(n_clips, 0u);
+    const int passes[2] = {normalize ? DEC_PEAK : DEC_STORE, DEC_NORM};
+    for (int p = 0; p < (normalize ? 2 : 1); p++)
+        for (int64_t i = 0; i < n_clips; i++) {
+            const dspx_decode_clip &r = table[i];
+            const DecWork w = dec_work(r, passes[p]);
+            for (int64_t tile = 0; tile < dec_tiles(r); tile++) {
+                const DecTile t = dec_tile(r, src, out, tile);
+                if (w.divide) {
+                    dec_divide(t, peaks[i], 0, 1);
+                    continue;
+                }
+                std::vector<unsigned char> smem(DEC_SMEM);
+                unsigned char *xs = smem.data();
+                float *ys = reinterpret_cast<float *>(xs + DEC_IN_BYTES);
+                dec_stage(t, xs, 0, 1);
+                const unsigned pk = dec_frames(r, t, xs, ys, w.store, w.normalize, peaks[i], 0, 1);
+                if (w.peak) peaks[i] = std::max(peaks[i], pk);
+                if (w.store) dec_store(t, ys, 0, 1);
+            }
+        }
     return DSPX_OK;
 }
 

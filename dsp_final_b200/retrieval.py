@@ -17,7 +17,7 @@ from typing import Any, Iterable, List
 import numpy as np
 
 from . import _lib
-from .batch import _is_cuda_tensor, embed_stats, features_batch, features_ragged
+from .batch import PackedClips, _is_cuda_tensor, decode_packed, embed_stats, features_batch, features_packed, features_ragged
 from .dsp.mfcc import MfccConfig
 
 
@@ -33,20 +33,26 @@ def _mfcc_embedding(signal: np.ndarray, cfg: MfccConfig) -> np.ndarray:
     return features_batch(sig, cfg, ("embed",))["embed"][0].astype(np.float64)
 
 
-def _load_clips(items: List[Any], cfg: MfccConfig, loader) -> tuple[list, int | None]:
-    """(one array per item, their sample rate; None for float32 clips, which are already at cfg.sample_rate).
+def _load_clips(items: List[Any], cfg: MfccConfig, loader) -> tuple[list | PackedClips, int | None]:
+    """(the clips, their sample rate; None for float32 clips, which are already at cfg.sample_rate).
 
-    The arrays are what the reference's load_audio + normalize_audio return (float32), or -- when every file is mono
-    16-bit PCM at one common rate -- the raw int16 samples and that rate.  The GPU then resamples them when that rate
-    is not cfg.sample_rate, converts and peak-normalises, with bit-identical results (src/utils/audio.py:19-38 as used
-    by retrieval.py:35-36).  Mixed rates and other encodings take the host path."""
-    from .audio import load_audio, normalize_audio, read_pcm16
+    The clips are what the reference's load_audio + normalize_audio return (src/utils/audio.py:19-38 as used by
+    retrieval.py:35-36), bit for bit, taken in this order:
+      1. every file is mono 16-bit PCM at one common rate: the raw int16 samples and that rate.  The GPU resamples
+         them when that rate is not cfg.sample_rate, converts and peak-normalises inside the feature launch;
+      2. otherwise, when read_wav_data accepts every file (PCM 8/16/24/32-bit or IEEE float 32/64, 1 to 32 channels,
+         any rates): a PackedClips buffer, decoded, downmixed, resampled and normalised on the GPU (decode_packed);
+      3. otherwise: float32 arrays from load_audio + normalize_audio on the host."""
+    from .audio import load_audio, normalize_audio, read_pcm16, read_wav_data
 
     if loader is not None:
         return [np.asarray(loader(item), dtype=np.float32).reshape(-1) for item in items], None
     pcm = [read_pcm16(item.path) for item in items]
     if all(p is not None for p in pcm) and len({rate for _, rate in pcm}) == 1:
         return [x for x, _ in pcm], pcm[0][1]
+    data = [read_wav_data(item.path) for item in items]
+    if all(d is not None and d[4] >= 1 for d in data):
+        return decode_packed(data, int(cfg.sample_rate), True), None
     clips = []
     for item in items:
         audio, _ = load_audio(item.path, target_sr=cfg.sample_rate)
@@ -79,6 +85,8 @@ def compute_embeddings(items: List[Any], cfg: MfccConfig, feature_cache=None, lo
         feats = [np.asarray(f, dtype=np.float32) for f in feats]
         return embed_stats(np.stack(feats, axis=0) if _equal_shapes(feats) else feats)
     clips, rate = _load_clips(items, cfg, loader)
+    if isinstance(clips, PackedClips):
+        return features_packed(clips, cfg, ("embed",))["embed"]
     if _equal_shapes(clips):
         return features_batch(np.stack(clips, axis=0), cfg, ("embed",), sample_rate=rate)["embed"]
     return features_ragged(clips, cfg, ("embed",), sample_rate=rate)["embed"]

@@ -261,6 +261,42 @@ int dspx_resample_ragged(const dspx_resampler *rs, const void *in_dev, int dtype
                          const dspx_resample_clip *table_dev, const dspx_resample_clip *table_host, int64_t n_clips,
                          float *out_dev, void *workspace_dev, size_t workspace_bytes, void *stream);
 
+/* ---- WAV decode + downmix: load_audio's decoding, src/utils/audio.py:19-31 (+ normalize_audio, 34-38) ----
+ * The data chunks of WAV files as stored go to the device; one launch writes, per file, the float32 mono clip
+ * load_audio returns (before any resample), bit for bit (DESIGN.md 4.6): each sample as read_wav scales it, then
+ * np.mean over the channels in numpy's float32 pairwise order (no mean for one channel).  Encodings: DSPX_DTYPE_PCM8
+ * (unsigned), DSPX_DTYPE_PCM16, DSPX_DTYPE_PCM24 (packed 3-byte little-endian), DSPX_DTYPE_PCM32, DSPX_DTYPE_F32 and
+ * DSPX_DTYPE_F64 (rounded to float32, NaN payloads truncated as an x86 conversion does), 1 to DSPX_MAX_CHANNELS
+ * channels interleaved.  A batch may mix encodings, channel counts and lengths. */
+#define DSPX_DTYPE_PCM8 3
+#define DSPX_DTYPE_PCM24 4
+#define DSPX_DTYPE_PCM32 5
+#define DSPX_MAX_CHANNELS 32
+typedef struct dspx_decode_clip {
+    int64_t in_offset;    /* byte offset of the clip's first frame in the input buffer: a multiple of 16 */
+    int64_t n_frames;     /* frames (samples per channel), 1 .. 2^40 */
+    int32_t channels;
+    int32_t dtype;        /* DSPX_DTYPE_PCM8 / PCM16 / PCM24 / PCM32 / F32 / F64 */
+    int64_t out_start;    /* first float32 sample of the clip's output: a multiple of 4 */
+    int64_t out_length;   /* n_frames */
+} dspx_decode_clip;
+/* Host only, no device needed: fills one row per clip, outputs packed back to back with starts aligned to 4 samples,
+ * so (out_start, out_length) can go straight to dspx_resample_layout (as in_start / in_length) and to
+ * dspx_ragged_layout.  Returns the packed output length (the last out_start + out_length; 0 for no clips), or
+ * DSPX_EINVAL naming the first clip with an unknown dtype, channels outside 1 .. DSPX_MAX_CHANNELS, n_frames outside
+ * 1 .. 2^40, or a negative or unaligned in_offset. */
+int64_t dspx_decode_layout(const int64_t *in_offsets, const int64_t *n_frames, const int32_t *channels,
+                           const int32_t *dtypes, int64_t n_clips, dspx_decode_clip *table_out);
+/* Device scratch of one dspx_decode_ragged call: one peak per clip (used when normalize != 0). */
+size_t dspx_decode_workspace(int64_t n_clips);
+/* in_dev: the input bytes (16-byte aligned); table_dev and table_host hold the same dspx_decode_layout table, on the
+ * device and on the host; out_dev: float32, 16-byte aligned.  normalize != 0 then divides each clip by its max |y|
+ * as normalize_audio does (the correctly rounded float32 quotient; a clip that is all zero or holds a NaN is left as
+ * it is).  Runs on the current device; n_clips == 0 enqueues nothing. */
+int dspx_decode_ragged(const void *in_dev, const dspx_decode_clip *table_dev, const dspx_decode_clip *table_host,
+                       int64_t n_clips, int normalize, float *out_dev, void *workspace_dev, size_t workspace_bytes,
+                       void *stream);
+
 /* ---- fft / ifft / rfft  src/dsp/fft.py:27-77 ----
  * in_dev [batch, n_in] interleaved complex64; the first min(n_in, n) samples are used,
  * zero-padded to P = next_pow2(n).  out_dev and work_dev each hold [batch, P] complex64.

@@ -22,6 +22,7 @@ KERNEL_NAMES = {v: k for k, v in KERNELS.items()}
 DTYPE_F32, DTYPE_F64, DTYPE_PCM16 = 0, 1, 2
 DTYPE_PCM8, DTYPE_PCM24, DTYPE_PCM32 = 3, 4, 5
 MAX_CHANNELS = 32
+DTYPE_FLAC = 6                  # a FLAC stream: read_flac_data's dtype code (not a dspx.h sample type)
 MAX_K = 128
 
 
@@ -111,6 +112,9 @@ _SIGNATURES = {
     "dspx_decode_layout": (_I64, [_VP, _VP, _VP, _VP, _I64, _VP]),
     "dspx_decode_workspace": (_SZ, [_I64]),
     "dspx_decode_ragged": (_I32, [_VP, _VP, _VP, _I64, _I32, _VP, _VP, _SZ, _VP]),
+    "dspx_flac_layout": (_I64, [_VP, _VP, _VP, _I64, _VP, _VP, _I64, _VP]),
+    "dspx_flac_workspace": (_SZ, [_VP, _I64]),
+    "dspx_flac_decode": (_I32, [_VP, _VP, _VP, _I64, _VP, _VP, _I64, _I32, _VP, _VP, _VP, _SZ, _VP]),
     "dspx_next_pow_two": (_I64, [_I64]),
     "dspx_fft_c2c": (_I32, [_VP, _I64, _I64, _I64, _I32, _VP, _VP, _VP]),
     "dspx_cosine_topk_workspace": (_SZ, [_I64, _I64, _I32, _I32]),

@@ -8,7 +8,8 @@ which yields int16 / 32768 exactly; `read_wav` below does the same with the stan
 parsing (PCM 8/16/24/32-bit and IEEE float), so the package has no hard dependency on soundfile.  When
 soundfile is importable it is used, like in the reference.  Decoding is host work (file I/O); the batched
 GPU path takes the raw int16 samples instead (`load_pcm16`, dspx_features_host_pcm16: the conversion and
-the peak normalisation then run on the device and PCIe carries half the bytes).
+the peak normalisation then run on the device and PCIe carries half the bytes).  FLAC files are decoded on the
+GPU (`read_flac_data`, batch.load_audio_batch); without soundfile, load_audio reads them that way too.
 """
 from __future__ import annotations
 
@@ -108,12 +109,52 @@ def read_wav_data(path: str | Path) -> Tuple[np.ndarray, int, int, int, int] | N
     return np.frombuffer(data, np.uint8, n_frames * channels * size), int(rate), int(channels), dtype, n_frames
 
 
+def _is_flac(path: str | Path) -> bool:
+    """Whether the file is a native FLAC stream ("fLaC" after an optional ID3v2 tag), from its first bytes only."""
+    with open(path, "rb") as f:
+        head = f.read(10)
+        pos = 0
+        if len(head) == 10 and head[:3] == b"ID3":
+            pos = 10 + (head[6] << 21 | head[7] << 14 | head[8] << 7 | head[9]) + (10 if head[5] & 0x10 else 0)
+        f.seek(pos)
+        return f.read(4) == b"fLaC"
+
+
+def read_flac_data(path: str | Path) -> Tuple[np.ndarray, int, int, int, int, tuple] | None:
+    """(the file's bytes as uint8, sample_rate, channels, DTYPE_FLAC, samples per channel, (file row, frame table)) for
+    the device decoder, or None when the file is not a native FLAC stream (judged by its content, not its name).
+
+    The stream is parsed and its frames found on the host once (batch.flac_parse: dspx_flac_layout, no device
+    needed); decode_packed reuses those tables.  A FLAC file that does not parse raises batch.FlacError (a ValueError)
+    naming it and the byte offset of the problem.
+    """
+    from . import _lib
+    from .batch import flac_parse
+
+    if not _is_flac(path):
+        return None
+    data = np.fromfile(path, np.uint8)
+    row, frames = flac_parse(data, str(path))
+    return data, int(row["sample_rate"]), int(row["channels"]), _lib.DTYPE_FLAC, int(row["out_length"]), (row, frames)
+
+
 def load_audio(path: str | Path, target_sr: int | None = None) -> Tuple[np.ndarray, int]:
-    """src/utils/audio.py:19-31: decode, average channels, resample when the rates differ."""
+    """src/utils/audio.py:19-31: decode, average channels, resample when the rates differ.
+
+    Without soundfile, a FLAC file is decoded, downmixed and resampled on the GPU (batch.decode_packed), which gives
+    the same bits; there is no CPU decoder for it, so without a device that raises."""
     path = Path(path)
     if _sf is not None:
         audio, sr = _sf.read(path, dtype="float32")
     else:
+        flac = read_flac_data(path)
+        if flac is not None:
+            from .batch import decode_packed
+
+            target = None if target_sr is None else int(target_sr)
+            packed = decode_packed([flac], target, False, names=[str(path)])
+            audio = packed.samples[int(packed.starts[0]):int(packed.starts[0] + packed.lengths[0])].cpu().numpy()
+            return audio, flac[1] if target is None else target
         audio, sr = read_wav(path)
     if audio.ndim > 1:
         audio = np.mean(audio, axis=1)

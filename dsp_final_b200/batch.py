@@ -19,8 +19,9 @@ resample_poly is scipy.signal.resample_poly on the GPU, bit for bit (dspx_resamp
 clips' own rate, features_batch and features_ragged resample on the device first when it differs from
 cfg.sample_rate (src/utils/audio.py:27-30 resamples on the host there).
 
-load_audio_batch is load_audio (+ normalize_audio) for many WAV files at once: the files' data chunks go to the GPU
-as stored and are decoded, downmixed and resampled there, bit for bit (dspx_decode_ragged, dspx_resample_ragged).
+load_audio_batch is load_audio (+ normalize_audio) for many WAV and FLAC files at once: the WAV data chunks and the
+FLAC files go to the GPU as stored and are decoded, downmixed and resampled there, bit for bit (dspx_decode_ragged,
+dspx_flac_decode, dspx_resample_ragged).
 """
 from __future__ import annotations
 
@@ -554,8 +555,100 @@ def _decode(lib, data, table: np.ndarray, normalize: bool, out, dev) -> None:
                                       torch.cuda.current_stream(dev.index).cuda_stream), "dspx_decode_ragged")
 
 
+# struct dspx_flac_file, struct dspx_flac_frame
+FLAC_FILE = np.dtype([("in_offset", "<i8"), ("in_bytes", "<i8"), ("out_start", "<i8"), ("out_length", "<i8"),
+                      ("first_frame", "<i8"), ("n_frames", "<i8"), ("ws_start", "<i8"), ("ws_bytes", "<i8"),
+                      ("sample_rate", "<i4"), ("channels", "<i4"), ("bps", "<i4"), ("reserved", "<i4")])
+FLAC_FRAME = np.dtype([("in_offset", "<i8"), ("out_start", "<i8"), ("ws_offset", "<i8"), ("in_bytes", "<i4"),
+                       ("header_bytes", "<i4"), ("block_size", "<i4"), ("assignment", "<i4"), ("file", "<i4"),
+                       ("reserved", "<i4")])
+FLAC_STATUS = {1: "CRC-16 mismatch", 2: "bitstream overrun", 4: "reserved code", 8: "negative LPC shift",
+               16: "invalid subframe parameters"}
+
+
+class FlacError(ValueError):
+    """A FLAC file the GPU decoder refuses: its stream does not parse, or a frame does not decode."""
+
+
+def flac_parse(data: np.ndarray, name=None) -> tuple[np.ndarray, np.ndarray]:
+    """(file row, frame table) of one FLAC file's bytes, from one dspx_flac_layout pass over them in most cases: the
+    frame table is sized from the file's size first (a frame of compressed audio rarely takes less than 256 bytes) and
+    only a file of more frames than that, such as digital silence, is parsed a second time."""
+    lib = _lib.load()
+    ptr = (C.c_void_p * 1)(data.ctypes.data)
+    size, offset, n_frames = (C.c_int64 * 1)(len(data)), (C.c_int64 * 1)(0), C.c_int64(0)
+    files = np.zeros(1, FLAC_FILE)
+    frames = np.zeros(len(data) // 256 + 16, FLAC_FRAME)
+    for _ in range(2):
+        if lib.dspx_flac_layout(ptr, size, offset, 1, files.ctypes.data, frames.ctypes.data, len(frames),
+                                C.byref(n_frames)) < 0:
+            raise FlacError(f"{name if name is not None else 'FLAC file'}: {_lib.last_error()}")
+        if n_frames.value <= len(frames):
+            return files[0], frames[:n_frames.value]
+        frames = np.zeros(n_frames.value, FLAC_FRAME)
+    raise AssertionError("dspx_flac_layout gave two frame counts for one file")
+
+
+def _flac_layout(lib, offsets, parsed, idx) -> tuple[np.ndarray, np.ndarray, int]:
+    """The file and frame tables of the files `idx` of `parsed` (read_flac_data tuples, whose last element holds each
+    file's own tables) at byte `offsets`, and the packed output length.  The frame rows are relative to their file, so
+    joining them parses nothing again: only the file rows' offsets and the frames' `file` change."""
+    files = np.zeros(len(idx), FLAC_FILE)
+    parts = []
+    at = nf = ws = total = 0
+    for j, i in enumerate(idx):
+        row, frames = parsed[i][5] if len(parsed[i]) > 5 else flac_parse(parsed[i][0], f"file {i}")
+        files[j] = row
+        for field, v in (("in_offset", offsets[i]), ("out_start", at), ("first_frame", nf), ("ws_start", ws)):
+            files[field][j] = v
+        frames = frames.copy()
+        frames["file"] = j
+        parts.append(frames)
+        total = at + int(row["out_length"])
+        at += (int(row["out_length"]) + RAGGED_ALIGN - 1) // RAGGED_ALIGN * RAGGED_ALIGN
+        nf += len(frames)
+        ws += int(row["ws_bytes"])
+    return files, (np.concatenate(parts) if parts else np.zeros(0, FLAC_FRAME)), total
+
+
+def _flac_decode(lib, data, tabs, normalize: bool, out, dev):
+    """One dspx_flac_decode call on torch's current stream into out[base:]; returns the per-frame status tensor."""
+    import torch
+
+    files, frames, base, _ = tabs
+    files_dev = torch.from_numpy(files.view(np.uint8)).to(dev)
+    frames_dev = torch.from_numpy(frames.view(np.uint8)).to(dev)
+    status = torch.empty(len(frames), dtype=torch.int32, device=dev)
+    ws_bytes = int(lib.dspx_flac_workspace(files.ctypes.data, len(files)))
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev)
+    _lib.check(lib.dspx_flac_decode(data.data_ptr(), files_dev.data_ptr(), files.ctypes.data, len(files),
+                                    frames_dev.data_ptr(), frames.ctypes.data, len(frames), 1 if normalize else 0,
+                                    out[base:].data_ptr(), status.data_ptr(), ws.data_ptr(), ws_bytes,
+                                    torch.cuda.current_stream(dev.index).cuda_stream), "dspx_flac_decode")
+    return status
+
+
+def _flac_check(checks, status: np.ndarray, offsets, names) -> None:
+    """Raise FlacError naming the first file and frame whose status is not 0."""
+    at = 0
+    for (files, frames, _, idx), _st in checks:
+        st = status[at:at + len(frames)]
+        at += len(frames)
+        bad = np.flatnonzero(st)
+        if not len(bad):
+            continue
+        f = int(bad[0])
+        row = frames[f]
+        i = idx[int(row["file"])]
+        j = f - int(files[int(row["file"])]["first_frame"])
+        what = ", ".join(v for k, v in FLAC_STATUS.items() if int(st[f]) & k)
+        name = names[i] if names is not None else f"file {i}"
+        raise FlacError(f"{name}: FLAC frame {j} (byte {int(row['in_offset'])}): {what}")
+
+
 def pack_files(parsed: list) -> tuple[Any, np.ndarray]:
-    """(pinned uint8 tensor holding the data chunks of read_wav_data tuples, their byte offsets: multiples of 16)."""
+    """(pinned uint8 tensor holding the bytes of read_wav_data / read_flac_data tuples, their byte offsets: multiples
+    of 16)."""
     import torch
 
     sizes = np.array([len(p[0]) for p in parsed], np.int64)
@@ -568,41 +661,67 @@ def pack_files(parsed: list) -> tuple[Any, np.ndarray]:
     return staging, offsets
 
 
-def decode_device(data, offsets: np.ndarray, parsed: list, target_sr: int | None, normalize: bool) -> PackedClips:
-    """The device part of decode_packed: `data` (a uint8 torch CUDA tensor) holds the data chunks of the read_wav_data
-    tuples `parsed` at byte `offsets`; work is enqueued on torch's current stream of data's device."""
+def decode_device(data, offsets: np.ndarray, parsed: list, target_sr: int | None, normalize: bool,
+                  names: list | None = None) -> PackedClips:
+    """The device part of decode_packed: `data` (a uint8 torch CUDA tensor) holds the files of the read_wav_data /
+    read_flac_data tuples `parsed` at byte `offsets`; work is enqueued on torch's current stream of data's device.
+    When FLAC files are among them, their frames' status is read back once (a synchronisation) and a bad frame raises
+    ValueError naming the file (names[i], else its index) and the frame."""
     import torch
 
     lib = _lib.load()
     dev = data.device
     n = len(parsed)
-    direct = [i for i in range(n) if target_sr is None or parsed[i][1] == target_sr]
-    others = [i for i in range(n) if not (target_sr is None or parsed[i][1] == target_sr)]
+    flac = [parsed[i][3] == _lib.DTYPE_FLAC for i in range(n)]
+    at_rate = [target_sr is None or parsed[i][1] == target_sr for i in range(n)]
     starts, lengths = np.zeros(n, np.int64), np.array([p[4] for p in parsed], np.int64)
-    dtab, at = _decode_layout(lib, offsets, parsed, direct)
-    starts[direct] = dtab["out_start"]
-    rtab, r_total = _decode_layout(lib, offsets, parsed, others)
+
+    def packed(rate_ok):
+        """Layouts of the WAV files, then of the FLAC files, with at_rate == rate_ok, back to back from 0."""
+        wav_idx = [i for i in range(n) if at_rate[i] == rate_ok and not flac[i]]
+        flac_idx = [i for i in range(n) if at_rate[i] == rate_ok and flac[i]]
+        wtab, total = _decode_layout(lib, offsets, parsed, wav_idx)
+        at = np.zeros(n, np.int64)
+        at[wav_idx] = wtab["out_start"]
+        ftabs = None
+        if flac_idx:
+            base = (total + RAGGED_ALIGN - 1) // RAGGED_ALIGN * RAGGED_ALIGN
+            files, frames, ftotal = _flac_layout(lib, offsets, parsed, flac_idx)
+            at[flac_idx] = base + files["out_start"]
+            ftabs = (files, frames, base, flac_idx)
+            total = base + ftotal
+        return wtab, ftabs, at, total
+
+    dtab, dflac, dstart, at = packed(True)
+    direct = [i for i in range(n) if at_rate[i]]
+    others = [i for i in range(n) if not at_rate[i]]
+    starts[direct] = dstart[direct]
+    rtab, rflac, rstart, r_total = packed(False)
     groups = []
     for rate in sorted({parsed[i][1] for i in others}):
-        rows = [j for j, i in enumerate(others) if parsed[i][1] == rate]
+        idx = [i for i in others if parsed[i][1] == rate]
         up, down = reduce_ratio(target_sr, rate)
-        in_starts = np.ascontiguousarray(rtab["out_start"][rows])
-        in_lengths = np.ascontiguousarray(rtab["n_frames"][rows])
-        table = np.zeros((len(rows), 4), np.int64)
-        total = _lib.check(int(lib.dspx_resample_layout(up, down, in_starts.ctypes.data, in_lengths.ctypes.data, len(rows),
+        in_starts = np.ascontiguousarray(rstart[idx])
+        in_lengths = np.ascontiguousarray(lengths[idx])
+        table = np.zeros((len(idx), 4), np.int64)
+        total = _lib.check(int(lib.dspx_resample_layout(up, down, in_starts.ctypes.data, in_lengths.ctypes.data, len(idx),
                                                         table.ctypes.data)), "dspx_resample_layout")
         base = (at + RAGGED_ALIGN - 1) // RAGGED_ALIGN * RAGGED_ALIGN
-        idx = [others[j] for j in rows]
         starts[idx] = base + table[:, 2]
         lengths[idx] = table[:, 3]
         groups.append((up, down, table, base))
         at = base + int(total)
+    checks = []
     with torch.cuda.device(dev.index):
         out = torch.zeros(max(at, 1), dtype=torch.float32, device=dev)
         _decode(lib, data, dtab, normalize, out, dev)
+        if dflac:
+            checks.append((dflac, _flac_decode(lib, data, dflac, normalize, out, dev)))
         if groups:
             scratch = torch.empty(max(r_total, 1), dtype=torch.float32, device=dev)
             _decode(lib, data, rtab, False, scratch, dev)
+            if rflac:
+                checks.append((rflac, _flac_decode(lib, data, rflac, False, scratch, dev)))
             stream = torch.cuda.current_stream(dev.index).cuda_stream
             for up, down, table, base in groups:
                 table_dev = torch.from_numpy(table).to(dev)
@@ -612,18 +731,22 @@ def decode_device(data, offsets: np.ndarray, parsed: list, target_sr: int | None
                                                     _lib.DTYPE_F32, 1 if normalize else 0, table_dev.data_ptr(),
                                                     table.ctypes.data, len(table), out[base:].data_ptr(), ws.data_ptr(),
                                                     ws_bytes, stream), "dspx_resample_ragged")
+        if checks:
+            _flac_check(checks, torch.cat([st for _, st in checks]).cpu().numpy(), offsets, names)
     return PackedClips(out, starts, lengths)
 
 
-def decode_packed(parsed: list, target_sr: int | None, normalize: bool, device: int | None = None) -> PackedClips:
+def decode_packed(parsed: list, target_sr: int | None, normalize: bool, device: int | None = None,
+                  names: list | None = None) -> PackedClips:
     """load_audio(path, target_sr)[0] (normalize_audio of it when `normalize`) of every file, from its read_wav_data
-    tuple, into one packed buffer on the GPU.
+    or read_flac_data tuple, into one packed buffer on the GPU.
 
-    The data chunks travel as stored, at 16-byte offsets of one pinned buffer, in one host-to-device copy.  Files at
-    target_sr (or all of them when it is None) are decoded with the normalisation in one launch, straight into the
-    output buffer; the others are decoded without it into a scratch buffer (one launch), then resampled with it, one
-    dspx_resample_ragged launch per rate, each group of outputs at its own offset of the output buffer -- the
-    reference's order: decode, downmix, resample, normalise.
+    The WAV data chunks and FLAC files travel as stored, at 16-byte offsets of one pinned buffer, in one host-to-device
+    copy.  Files at target_sr (or all of them when it is None) are decoded with the normalisation, straight into the
+    output buffer (one WAV and one FLAC decode launch); the others are decoded without it into a scratch buffer (the
+    same two), then resampled with it, one dspx_resample_ragged launch per rate, each group of outputs at its own
+    offset of the output buffer -- the reference's order: decode, downmix, resample, normalise.  A FLAC frame that
+    does not decode raises ValueError naming the file (names[i] when given) and the frame.
     """
     import torch
 
@@ -632,30 +755,35 @@ def decode_packed(parsed: list, target_sr: int | None, normalize: bool, device: 
     staging, offsets = pack_files(parsed)
     with torch.cuda.device(dev.index):
         data = staging.to(dev, non_blocking=True)
-    return decode_device(data, offsets, parsed, target_sr, normalize)
+    return decode_device(data, offsets, parsed, target_sr, normalize, names)
 
 
 def load_audio_batch(paths, target_sr: int | None = None, normalize: bool = False, device: int | None = None) -> list:
     """[load_audio(p, target_sr)[0] for p in paths] (normalize_audio of each when `normalize`), decoded on the GPU.
 
     Returns float32 torch CUDA tensors, views into one packed buffer, bit-identical to the host functions.  The files
-    may mix PCM 8/16/24/32-bit and IEEE float 32/64 WAV encodings, 1 to 32 channels, lengths and rates; each is
-    decoded and downmixed on the device, then resampled there when its rate is not target_sr.  A file of another
-    kind, or without audio frames, raises ValueError naming it.
+    may mix PCM 8/16/24/32-bit and IEEE float 32/64 WAV encodings with 1 to 32 channels, FLAC files (4 to 32 bits, 1
+    to 8 channels), lengths and rates; each is decoded and downmixed on the device, then resampled there when its
+    rate is not target_sr.  A file of another kind, without audio frames, or with a FLAC frame that does not decode
+    raises ValueError naming it.
     """
-    from .audio import read_wav_data
+    from .audio import read_flac_data, read_wav_data
 
     parsed = []
+    paths = list(paths)
     for p in paths:
         d = read_wav_data(p)
         if d is None:
-            raise ValueError(f"{p}: not a WAV file of PCM 8/16/24/32-bit or IEEE float 32/64 samples with 1 to 32 channels")
+            d = read_flac_data(p)
+        if d is None:
+            raise ValueError(f"{p}: neither a FLAC file nor a WAV file of PCM 8/16/24/32-bit or IEEE float 32/64 samples "
+                             "with 1 to 32 channels")
         if d[4] < 1:
             raise ValueError(f"{p}: no audio frames")
         parsed.append(d)
     if not parsed:
         return []
-    packed = decode_packed(parsed, None if target_sr is None else int(target_sr), normalize, device)
+    packed = decode_packed(parsed, None if target_sr is None else int(target_sr), normalize, device, [str(p) for p in paths])
     return [packed.samples[s:s + n] for s, n in zip(packed.starts.tolist(), packed.lengths.tolist())]
 
 

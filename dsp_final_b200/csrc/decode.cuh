@@ -119,26 +119,27 @@ DSPX_HD float dec_sample(const unsigned char *p, int dtype)
     }
 }
 
-// np.mean(frame, axis=1) of one frame of C samples at p (C == 1: the sample itself, as load_audio does not average).
-DSPX_HD float dec_mix(const unsigned char *p, int C, int dtype)
+// np.mean over the C float32 samples sample(0) ... sample(C - 1) of one frame (C == 1: the sample itself, as load_audio
+// does not average).  Shared by the WAV and FLAC decoders (DESIGN.md 4.6, 4.7).
+template <class Sample>
+DSPX_HD float dec_mean(int C, Sample sample)
 {
-    const int b = dec_bytes(dtype);
-    if (C == 1) return dec_sample(p, dtype);
+    if (C == 1) return sample(0);
     float s;
     if (C < 8) {
         s = 0.0f;
-        for (int c = 0; c < C; c++) s = dec_add(s, dec_sample(p + c * b, dtype));
+        for (int c = 0; c < C; c++) s = dec_add(s, sample(c));
     } else {
         float r[8];
 #pragma unroll
-        for (int j = 0; j < 8; j++) r[j] = dec_sample(p + j * b, dtype);
+        for (int j = 0; j < 8; j++) r[j] = sample(j);
         int i = 8;
         for (; i + 8 <= C; i += 8) {
 #pragma unroll
-            for (int j = 0; j < 8; j++) r[j] = dec_add(r[j], dec_sample(p + (i + j) * b, dtype));
+            for (int j = 0; j < 8; j++) r[j] = dec_add(r[j], sample(i + j));
         }
         s = dec_add(dec_add(dec_add(r[0], r[1]), dec_add(r[2], r[3])), dec_add(dec_add(r[4], r[5]), dec_add(r[6], r[7])));
-        for (; i < C; i++) s = dec_add(s, dec_sample(p + i * b, dtype));
+        for (; i < C; i++) s = dec_add(s, sample(i));
         s = dec_add(0.0f, s);              // numpy adds the pairwise sum to the reduction's identity: -0 becomes +0
     }
     if (s != s) return dec_nan(s, s);
@@ -147,6 +148,13 @@ DSPX_HD float dec_mix(const unsigned char *p, int C, int dtype)
 #else
     return s / (float)C;
 #endif
+}
+
+// np.mean(frame, axis=1) of one frame of C samples at p.
+DSPX_HD float dec_mix(const unsigned char *p, int C, int dtype)
+{
+    const int b = dec_bytes(dtype);
+    return dec_mean(C, [=](int c) { return dec_sample(p + c * b, dtype); });
 }
 
 // normalize_audio's y / peak (rs_normalize), with x86's default NaN where the quotient is one (inf / inf).

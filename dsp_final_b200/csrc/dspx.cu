@@ -25,6 +25,7 @@
 #include "ingest.cuh"
 #include "resample.cuh"
 #include "decode.cuh"
+#include "flac.cuh"
 
 // the ctypes binding (dsp_final_b200/_lib.py) mirrors these layouts; tests assert the same numbers
 static_assert(sizeof(dspx_config) == 56 && offsetof(dspx_config, f_min) == 24 && offsetof(dspx_config, window) == 48,
@@ -32,6 +33,10 @@ static_assert(sizeof(dspx_config) == 56 && offsetof(dspx_config, f_min) == 24 &&
 static_assert(sizeof(dspx_plan_info) == 32, "dspx_plan_info layout changed: update _lib.DspxPlanInfo");
 static_assert(sizeof(dspx_decode_clip) == 40 && offsetof(dspx_decode_clip, out_start) == 24,
               "dspx_decode_clip layout changed: update batch.py");
+static_assert(sizeof(dspx_flac_file) == 80 && offsetof(dspx_flac_file, sample_rate) == 64,
+              "dspx_flac_file layout changed: update batch.py");
+static_assert(sizeof(dspx_flac_frame) == 48 && offsetof(dspx_flac_frame, in_bytes) == 24,
+              "dspx_flac_frame layout changed: update batch.py");
 
 namespace dspx {
 
@@ -593,6 +598,30 @@ static int decode_launch(const void *in, const dspx_decode_clip *tab, int64_t n_
             const unsigned nc = (unsigned)std::min<int64_t>(n_clips - c0, 65535);
             wav_decode_kernel<<<dim3((unsigned)max_tiles, nc), DEC_THREADS, DEC_SMEM, st>>>(
                 static_cast<const unsigned char *>(in), tab + c0, out, normalize ? peaks + c0 : nullptr, passes[p]);
+            DSPX_CUDA_CHECK(cudaGetLastError());
+        }
+    return DSPX_OK;
+}
+
+// ---- FLAC decoding (flac.cuh) ---------------------------------------------------
+
+// The workspace: a peak per file, then the frames' integers (ws_offset is relative to the latter).
+static size_t flac_peaks_bytes(int64_t n_files) { return align256((size_t)std::max<int64_t>(n_files, 1) * sizeof(unsigned)); }
+
+static int flac_launch(const void *in, const dspx_flac_file *files, const dspx_flac_frame *frames, int64_t n_frames,
+                       int64_t n_files, int normalize, float *out, int32_t *status, char *ws, cudaStream_t st)
+{
+    unsigned *peaks = reinterpret_cast<unsigned *>(ws);
+    char *samples = ws + flac_peaks_bytes(n_files);
+    if (normalize) DSPX_CUDA_CHECK(cudaMemsetAsync(peaks, 0, (size_t)n_files * sizeof(unsigned), st));
+    flac_frame_kernel<<<(unsigned)((n_frames + FL_THREADS - 1) / FL_THREADS), FL_THREADS, 0, st>>>(
+        static_cast<const unsigned char *>(in), files, frames, n_frames, samples, status);
+    DSPX_CUDA_CHECK(cudaGetLastError());
+    const int passes[2] = {normalize ? FL_PEAK : FL_STORE, FL_NORM};
+    for (int p = 0; p < (normalize ? 2 : 1); p++)
+        for (int64_t f0 = 0; f0 < n_frames; f0 += 0x7fffffff) {
+            const unsigned nf = (unsigned)std::min<int64_t>(n_frames - f0, 0x7fffffff);
+            flac_mix_kernel<<<nf, FL_MIX_THREADS, 0, st>>>(files, frames + f0, samples, status + f0, out, peaks, passes[p]);
             DSPX_CUDA_CHECK(cudaGetLastError());
         }
     return DSPX_OK;
@@ -1325,6 +1354,84 @@ int dspx_decode_ragged(const void *in_dev, const dspx_decode_clip *table_dev, co
     DSPX_REQUIRE(max_tiles < (int64_t)0x7fffffff, "clip too long for one launch");
     return decode_launch(in_dev, table_dev, n_clips, max_tiles, normalize ? 1 : 0, out_dev,
                          reinterpret_cast<unsigned *>(ws_align(workspace_dev)), static_cast<cudaStream_t>(stream));
+}
+
+// ---- FLAC decoding ----
+
+int64_t dspx_flac_layout(const void *const *files_host, const int64_t *sizes, const int64_t *in_offsets, int64_t n_files,
+                         dspx_flac_file *files_out, dspx_flac_frame *frames_out, int64_t frames_capacity,
+                         int64_t *n_frames_out)
+{
+    DSPX_REQUIRE(n_files >= 0 && frames_capacity >= 0, "negative file count or capacity");
+    DSPX_REQUIRE(n_files == 0 || (files_host && sizes && in_offsets && n_frames_out), "null argument");
+    DSPX_REQUIRE(frames_out || frames_capacity == 0, "frames_out is NULL with a non-zero capacity");
+    int64_t at = 0, end = 0, nf = 0, ws = 0;
+    FlFile f;
+    for (int64_t i = 0; i < n_files; i++) {
+        DSPX_REQUIRE(files_host[i] && sizes[i] >= 0, "file %lld: no bytes or a negative size", (long long)i);
+        DSPX_REQUIRE(in_offsets[i] >= 0 && in_offsets[i] % 16 == 0, "file %lld: in_offset negative or not a multiple of 16",
+                     (long long)i);
+        int64_t where = 0;
+        const char *bad = fl_parse_file(static_cast<const unsigned char *>(files_host[i]), sizes[i], f, &where);
+        DSPX_REQUIRE(!bad, "file %lld: byte %lld: %s", (long long)i, (long long)where, bad);
+        if (files_out)
+            files_out[i] = dspx_flac_file{in_offsets[i], sizes[i], at, f.samples, nf, (int64_t)f.frames.size(), ws,
+                                          f.ws_bytes, f.si.rate, f.si.channels, f.si.bps, 0};
+        for (size_t j = 0; j < f.frames.size() && nf + (int64_t)j < frames_capacity; j++) {
+            frames_out[nf + (int64_t)j] = f.frames[j];
+            frames_out[nf + (int64_t)j].file = (int32_t)i;
+        }
+        nf += (int64_t)f.frames.size();
+        ws += f.ws_bytes;
+        end = at + f.samples;
+        at += (f.samples + 3) & ~(int64_t)3;      // RAGGED_ALIGN: the packed output is a valid ragged batch
+    }
+    if (n_frames_out) *n_frames_out = nf;
+    return end;
+}
+
+size_t dspx_flac_workspace(const dspx_flac_file *files_host, int64_t n_files)
+{
+    size_t samples = 0;
+    for (int64_t i = 0; files_host && i < n_files; i++)
+        samples = std::max(samples, (size_t)(files_host[i].ws_start + files_host[i].ws_bytes));
+    return 256 + flac_peaks_bytes(n_files) + samples;
+}
+
+int dspx_flac_decode(const void *in_dev, const dspx_flac_file *files_dev, const dspx_flac_file *files_host, int64_t n_files,
+                     const dspx_flac_frame *frames_dev, const dspx_flac_frame *frames_host, int64_t n_frames, int normalize,
+                     float *out_dev, int32_t *status_dev, void *workspace_dev, size_t workspace_bytes, void *stream)
+{
+    DSPX_REQUIRE(n_files >= 0 && n_frames >= 0, "negative file or frame count");
+    if (n_frames == 0) return DSPX_OK;
+    DSPX_REQUIRE(in_dev && files_dev && files_host && frames_dev && frames_host && out_dev && status_dev && workspace_dev,
+                 "null argument");
+    DSPX_REQUIRE(reinterpret_cast<uintptr_t>(in_dev) % 16 == 0 && reinterpret_cast<uintptr_t>(out_dev) % 16 == 0,
+                 "in_dev and out_dev must be 16-byte aligned");
+    for (int64_t i = 0; i < n_files; i++) {
+        const dspx_flac_file &r = files_host[i];
+        DSPX_REQUIRE(r.channels >= 1 && r.channels <= DSPX_FLAC_MAX_CHANNELS && r.bps >= 4 && r.bps <= 32 &&
+                         r.in_offset >= 0 && r.in_offset % 16 == 0 && r.in_bytes >= 0 && r.out_start >= 0 &&
+                         r.out_start % 4 == 0 && r.out_length >= 0 && r.ws_start >= 0 && r.ws_start % 16 == 0 &&
+                         r.ws_bytes >= 0,
+                     "file %lld: bad table row", (long long)i);
+    }
+    const size_t need = dspx_flac_workspace(files_host, n_files);
+    DSPX_REQUIRE(workspace_bytes >= need, "workspace too small (%zu bytes, need %zu)", workspace_bytes, need);
+    for (int64_t f = 0; f < n_frames; f++) {
+        const dspx_flac_frame &fr = frames_host[f];
+        DSPX_REQUIRE(fr.file >= 0 && fr.file < n_files, "frame %lld: file outside the table", (long long)f);
+        const dspx_flac_file &r = files_host[fr.file];
+        DSPX_REQUIRE(fr.assignment >= 0 && fr.assignment <= 10 && fl_channels(fr.assignment) == r.channels &&
+                         fr.block_size >= 1 && fr.block_size <= FL_MAX_BLOCK && fr.header_bytes >= 6 &&
+                         fr.in_bytes >= fr.header_bytes + 2 && fr.in_offset >= 0 &&
+                         fr.in_offset + fr.in_bytes <= r.in_bytes && fr.out_start >= 0 &&
+                         fr.out_start + fr.block_size <= r.out_length && fr.ws_offset >= 0 && fr.ws_offset % 16 == 0 &&
+                         fr.ws_offset + fl_ws_bytes(r.bps, fr.assignment, fr.block_size) <= r.ws_bytes,
+                     "frame %lld: bad table row", (long long)f);
+    }
+    return flac_launch(in_dev, files_dev, frames_dev, n_frames, n_files, normalize ? 1 : 0, out_dev, status_dev,
+                       ws_align(workspace_dev), static_cast<cudaStream_t>(stream));
 }
 
 }  // extern "C"

@@ -17,6 +17,7 @@
 #include "feat_warp8_x2.cuh"
 #include "resample.cuh"
 #include "decode.cuh"
+#include "flac.cuh"
 #include "retrieval_select.cuh"
 #include "feat_select.cuh"
 
@@ -500,6 +501,42 @@ int emu_decode(const void *in, const dspx_decode_clip *table, int64_t n_clips, i
                 if (w.store) dec_store(t, ys, 0, 1);
             }
         }
+    return DSPX_OK;
+}
+
+// Replays flac_frame_kernel and flac_mix_kernel frame by frame: fl_frame decodes each frame into a heap buffer of
+// exactly its integers' size (block_size x channels x 4 or 8 bytes) with a coefficient scratch of the kernel's size,
+// then fl_mix_frame writes its outputs; with normalize, fl_divide runs after every frame's peak is folded, as on the
+// device.  Tables from dspx_flac_layout; in / out / status as for dspx_flac_decode.
+int emu_flac_decode(const void *in, const dspx_flac_file *files, int64_t n_files, const dspx_flac_frame *frames,
+                    int64_t n_frames, int normalize, float *out, int32_t *status)
+{
+    for (int64_t f = 0; f < n_frames; f++)
+        if (frames[f].file < 0 || frames[f].file >= n_files || frames[f].assignment < 0 || frames[f].assignment > 10 ||
+            frames[f].block_size < 1 || frames[f].block_size > FL_MAX_BLOCK)
+            return DSPX_EINVAL;
+    uint16_t table[256];
+    for (int i = 0; i < 256; i++) table[i] = fl_crc16_entry(i);
+    const unsigned char *src = static_cast<const unsigned char *>(in);
+    std::vector<std::vector<char>> samples(n_frames);
+    for (int64_t f = 0; f < n_frames; f++) {
+        const dspx_flac_frame &fr = frames[f];
+        const int bps = files[fr.file].bps;
+        samples[f].resize((size_t)fr.block_size * fl_channels(fr.assignment) * (fl_wide(bps) ? 8 : 4));
+        std::vector<int32_t> coef(FL_MAX_ORDER + 1);
+        status[f] = fl_frame(src + files[fr.file].in_offset, fr, bps, samples[f].data(), coef.data(), table);
+    }
+    std::vector<unsigned> peaks(n_files, 0u);
+    for (int64_t f = 0; f < n_frames; f++)
+        if (!status[f]) {
+            const dspx_flac_frame &fr = frames[f];
+            const dspx_flac_file &file = files[fr.file];
+            peaks[fr.file] = std::max(peaks[fr.file],
+                                      fl_mix_frame(fr, file.bps, samples[f].data(), out + file.out_start, false, 0u, 0, 1));
+        }
+    if (normalize)
+        for (int64_t f = 0; f < n_frames; f++)
+            if (!status[f]) fl_divide(frames[f], out + files[frames[f].file].out_start, peaks[frames[f].file], 0, 1);
     return DSPX_OK;
 }
 

@@ -17,7 +17,7 @@ from typing import Any, Iterable, List
 import numpy as np
 
 from . import _lib
-from .batch import PackedClips, _is_cuda_tensor, decode_packed, embed_stats, features_batch, features_packed, features_ragged
+from .batch import FlacError, PackedClips, _is_cuda_tensor, decode_packed, embed_stats, features_batch, features_packed, features_ragged
 from .dsp.mfcc import MfccConfig
 
 
@@ -40,19 +40,25 @@ def _load_clips(items: List[Any], cfg: MfccConfig, loader) -> tuple[list | Packe
     retrieval.py:35-36), bit for bit, taken in this order:
       1. every file is mono 16-bit PCM at one common rate: the raw int16 samples and that rate.  The GPU resamples
          them when that rate is not cfg.sample_rate, converts and peak-normalises inside the feature launch;
-      2. otherwise, when read_wav_data accepts every file (PCM 8/16/24/32-bit or IEEE float 32/64, 1 to 32 channels,
-         any rates): a PackedClips buffer, decoded, downmixed, resampled and normalised on the GPU (decode_packed);
-      3. otherwise: float32 arrays from load_audio + normalize_audio on the host."""
-    from .audio import load_audio, normalize_audio, read_pcm16, read_wav_data
+      2. otherwise, when read_wav_data (PCM 8/16/24/32-bit or IEEE float 32/64, 1 to 32 channels) or read_flac_data
+         (FLAC) accepts every file, at any rates: a PackedClips buffer, decoded, downmixed, resampled and normalised on
+         the GPU (decode_packed);
+      3. otherwise, or when the GPU decoder refuses a FLAC file (batch.FlacError): float32 arrays from load_audio +
+         normalize_audio on the host (without soundfile, load_audio of such a file raises FlacError naming it)."""
+    from .audio import load_audio, normalize_audio, read_flac_data, read_pcm16, read_wav_data
 
     if loader is not None:
         return [np.asarray(loader(item), dtype=np.float32).reshape(-1) for item in items], None
     pcm = [read_pcm16(item.path) for item in items]
     if all(p is not None for p in pcm) and len({rate for _, rate in pcm}) == 1:
         return [x for x, _ in pcm], pcm[0][1]
-    data = [read_wav_data(item.path) for item in items]
-    if all(d is not None and d[4] >= 1 for d in data):
-        return decode_packed(data, int(cfg.sample_rate), True), None
+    try:
+        data = [read_wav_data(item.path) for item in items]
+        data = [d if d is not None else read_flac_data(item.path) for d, item in zip(data, items)]
+        if all(d is not None and d[4] >= 1 for d in data):
+            return decode_packed(data, int(cfg.sample_rate), True, names=[str(item.path) for item in items]), None
+    except FlacError:          # a FLAC file the GPU decoder refuses: the host loader (soundfile) may still read it
+        pass
     clips = []
     for item in items:
         audio, _ = load_audio(item.path, target_sr=cfg.sample_rate)

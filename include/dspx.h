@@ -297,6 +297,75 @@ int dspx_decode_ragged(const void *in_dev, const dspx_decode_clip *table_dev, co
                        int64_t n_clips, int normalize, float *out_dev, void *workspace_dev, size_t workspace_bytes,
                        void *stream);
 
+/* ---- FLAC decode + downmix: load_audio of a FLAC file (+ normalize_audio) ----
+ * Native FLAC streams (an optional leading ID3v2 tag, "fLaC", metadata blocks, frames) go to the device as stored; one
+ * launch pair writes, per file, the float32 mono clip: each sample s of a b-bit stream is s / 2^(b-1) in float32 (the
+ * scaling read_wav applies to PCM, so a FLAC file and a WAV file of the same integers give the same bits), then the
+ * downmix of dspx_decode_ragged (DESIGN.md 4.7).  1 to 8 channels, 4 to 32 bits, block sizes 1 .. 65535, fixed and
+ * variable blocking, every subframe type. */
+#define DSPX_FLAC_MAX_CHANNELS 8
+typedef struct dspx_flac_file {
+    int64_t in_offset;    /* byte offset of the file's first byte in the input buffer: a multiple of 16 */
+    int64_t in_bytes;     /* the file's size */
+    int64_t out_start;    /* first float32 sample of the file's output: a multiple of 4 */
+    int64_t out_length;   /* samples per channel */
+    int64_t first_frame;  /* its first row of the frame table */
+    int64_t n_frames;
+    int64_t ws_start;     /* byte offset of its frames' integers in the workspace's sample region: a multiple of 16 */
+    int64_t ws_bytes;     /* their size: 4 bytes per sample and channel (8 for 32-bit streams), each frame 16-aligned */
+    int32_t sample_rate;
+    int32_t channels;
+    int32_t bps;          /* bits per sample, 4 .. 32 */
+    int32_t reserved;
+} dspx_flac_file;
+/* A frame's offsets are relative to its file's row, so one file's rows can join any batch unchanged: only the file
+ * rows' in_offset, out_start, first_frame and ws_start and the frames' `file` depend on the batch. */
+typedef struct dspx_flac_frame {
+    int64_t in_offset;    /* byte offset of the frame's sync code in its file */
+    int64_t out_start;    /* its first output sample, from the file's out_start */
+    int64_t ws_offset;    /* byte offset of its decoded integers, from the file's ws_start: a multiple of 16 */
+    int32_t in_bytes;     /* header through CRC-16 */
+    int32_t header_bytes; /* header through CRC-8 */
+    int32_t block_size;   /* 1 .. 65535 */
+    int32_t assignment;   /* 0 .. 7: that many channels plus one, coded independently; 8 left/side, 9 right/side, 10 mid/side */
+    int32_t file;         /* row of the file table */
+    int32_t reserved;
+} dspx_flac_frame;
+/* Per-frame status bits of dspx_flac_decode (0: decoded). */
+#define DSPX_FLAC_CRC 1        /* the frame's CRC-16 does not match its bytes */
+#define DSPX_FLAC_OVERRUN 2    /* a subframe reads past the frame's last byte */
+#define DSPX_FLAC_RESERVED 4   /* a reserved subframe type, residual coding method, LPC precision or padding bit */
+#define DSPX_FLAC_NEG_SHIFT 8  /* a negative LPC shift */
+#define DSPX_FLAC_INVALID 16   /* wasted bits or a predictor order the block cannot hold, a partition order that does
+                                  not divide the block */
+/* Host only, no device needed; one pass over each file.  files_host[i] holds sizes[i] bytes of file i, which sits at
+ * in_offsets[i] (a multiple of 16) of the device input buffer.  Parses STREAMINFO, skips a leading ID3v2 tag, the
+ * other metadata blocks and a trailing ID3v1 / APEv2 tag, and finds every frame: sync code, header CRC-8, header fields
+ * consistent with STREAMINFO, and the frame (fixed blocking) or first-sample (variable blocking) number equal to the
+ * running count from the first frame's -- which rejects sync-like bytes inside residual data; a frame ends where the
+ * next one starts, the last at the end of the stream.  Outputs and workspace regions are packed back to back, outputs
+ * with starts aligned to 4 samples, as dspx_decode_layout packs them.  files_out (n_files rows) may be NULL; frames_out
+ * holds frames_capacity rows and may be NULL with capacity 0.  *n_frames_out is set to the batch's frame count; when
+ * that exceeds frames_capacity, the rows past it are not written and the caller calls again with a larger table.
+ * Returns the packed output length, or DSPX_EINVAL naming the file and the byte offset of the first problem: no
+ * "fLaC", a bad metadata block, a frame header that is not valid or not the next frame (a damaged header in the middle
+ * of a stream is named at its own offset), a STREAMINFO total that is non-zero and differs from the frames' block
+ * sizes, or no frames. */
+int64_t dspx_flac_layout(const void *const *files_host, const int64_t *sizes, const int64_t *in_offsets, int64_t n_files,
+                         dspx_flac_file *files_out, dspx_flac_frame *frames_out, int64_t frames_capacity,
+                         int64_t *n_frames_out);
+/* Device scratch of one dspx_flac_decode call: a peak per file and the files' integers (their ws_start + ws_bytes):
+ * 4 bytes per sample and channel, 8 for 32-bit streams -- about 3.5 GB for 2000 five-second stereo clips at 44.1 kHz. */
+size_t dspx_flac_workspace(const dspx_flac_file *files_host, int64_t n_files);
+/* in_dev: the input buffer (16-byte aligned); the table pairs hold the same tables on the device and on the host
+ * (dspx_flac_layout's, or per-file tables joined as described above); out_dev: float32, 16-byte aligned; status_dev:
+ * one int32 per frame, DSPX_FLAC_* bits (the outputs of a frame with a non-zero status are unspecified).  normalize as
+ * for dspx_decode_ragged.  No bit reader reads outside its frame's bytes.  Two launches (three when normalising) on
+ * `stream`, no synchronisation; n_frames == 0 enqueues nothing. */
+int dspx_flac_decode(const void *in_dev, const dspx_flac_file *files_dev, const dspx_flac_file *files_host, int64_t n_files,
+                     const dspx_flac_frame *frames_dev, const dspx_flac_frame *frames_host, int64_t n_frames, int normalize,
+                     float *out_dev, int32_t *status_dev, void *workspace_dev, size_t workspace_bytes, void *stream);
+
 /* ---- fft / ifft / rfft  src/dsp/fft.py:27-77 ----
  * in_dev [batch, n_in] interleaved complex64; the first min(n_in, n) samples are used,
  * zero-padded to P = next_pow2(n).  out_dev and work_dev each hold [batch, P] complex64.
